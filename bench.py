@@ -6,6 +6,7 @@
            --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 5 --warmup 1       # CPU arm (oracle port of the reference, rank 0 only)
     python bench.py --config 3                                   # one config as the headline line (1..5)
+    python bench.py --steps 20 --dump-outputs DIR                # also write config 1's last timed step to DIR/*.npy
 
 Headline = BASELINE.json configs[0]: b_sae 512->32768 n_bits=4 gamma=4 k=32 forward at batch 4096 per GPU.
 A "step" is one forward of the hot path over one batch of synthetic activations: x [B,512] fp32 (resident in HBM) ->
@@ -67,9 +68,16 @@ def parse():
     # accepted for compatibility with round-1 command lines
     ap.add_argument("--variant", default=None, choices=[None, "batch-sharded", "dict-sharded"])
     ap.add_argument("--graph", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of config 1, write what its last step returned (latent values and indices, "
+                         "reconstruction) as DIR/<name>.npy, so that two builds can be compared output for output")
     a = ap.parse_args()
     if a.variant == "dict-sharded":
         a.config = "5"
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.config not in ("all", "1")):
+        ap.error("--dump-outputs writes the outputs of config 1 on the B200 (--impl b200, --config all or 1)")
     return a
 
 
@@ -263,14 +271,14 @@ def cpu_baseline_block(batch, k, steps, warmup):
             "best": batch / best, "median_s_per_forward": med, "best_s_per_forward": best,
             "sample": f"{batch} rows x {len(times)} timed forwards ({warmup} warm-up) of the same workload, median; "
                       f"oracle/qsae_oracle.bsae_forward_dense_port_torch == the reference's op sequence "
-                      f"(sae/binary.py:91-103), pinned to the shim-loaded reference by tests/test_oracle_golden.py; "
+                      f"(sae/binary.py:91-103), pinned to the reference's stored outputs by tests/test_oracle_golden.py; "
                       f"torch CPU, {cores} threads"}, times
 
 
 def run_reference(args, rank):
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 20)), max(1, min(args.warmup, 3))
+    steps, warmup = args.steps, max(1, min(args.warmup, 3))
     cb, times = cpu_baseline_block(args.cpu_batch, args.k, steps, warmup)
     mean_s = sum(times) / len(times)
     rate = args.cpu_batch / mean_s
@@ -425,7 +433,7 @@ def oracle_rows_check(O, np, x_rows, We, be, k, vals, idx):
 # config 1: b_sae (headline)
 # ---------------------------------------------------------------------------------------------
 def bench_bsae(args, T, rank, world, device, B, k, steps, warmup, want_e2e=True, want_roofline=True, exact_too=True,
-               graph=True):
+               graph=True, keep_last=False):
     import numpy as np
     import torch
 
@@ -481,11 +489,14 @@ def bench_bsae(args, T, rank, world, device, B, k, steps, warmup, want_e2e=True,
     T.barrier()
     e0 = T.fork(streams)
     for i in range(steps):
-        run(i)
+        last = run(i)
     e1 = T.join(streams)
     T.barrier()
     elapsed_ms = T.max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
+    if keep_last:
+        # a graph replay returns nothing: the last step's outputs are the ones its graph was captured with
+        last_step = [t.cpu().numpy() for t in (keep[(steps - 1) % len(keep)][1] if use_graph else last)]
     launches = launches_per_step * steps if use_graph else L.launch_count() - c0
     ms = elapsed_ms / steps
     out = {"value": world * B / (ms * 1e-3), "ms_per_step": ms, "elapsed_ms": elapsed_ms, "clocks": clocks, "gpu_launches": int(launches),
@@ -493,6 +504,8 @@ def bench_bsae(args, T, rank, world, device, B, k, steps, warmup, want_e2e=True,
                      (f"; {S} batches in flight: consecutive steps alternate between {S} streams, every step's kernels are inside "
                       f"the timed region (fork / join events on the timing stream)" if S > 1 else "; one stream"),
            "parity_checked": parity, "n_inputs": n_in, "batch": B, "k": k, "streams": S}
+    if keep_last:
+        out["last_step"] = last_step
     if S > 1:
         # the pipelined steps produce the same bits as a lone step, and the strictly serial number is reported beside it
         if use_graph:
@@ -1142,7 +1155,9 @@ def run_b200(args, rank, world, local_rank):
 
     if cfg in ("all", "1"):
         B, k = args.batch, args.k
-        r = bench_bsae(args, T, rank, world, device, B, k, steps, warmup)
+        r = bench_bsae(args, T, rank, world, device, B, k, steps, warmup, keep_last=bool(args.dump_outputs))
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, *r.pop("last_step"))
         flops = 2.0 * B * H * D
         out = {
             "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": world, "steps": steps, "warmup": warmup,
@@ -1225,6 +1240,28 @@ def run_b200(args, rank, world, local_rank):
         print(json.dumps(out), flush=True)
     if dist is not None:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(directory, vals, idx, recon):
+    """--dump-outputs: the last timed step's (values, indices, reconstruction) as DIR/<name>.npy, indices as float64
+    (exact). When the whole batch would exceed DUMP_BYTES, a fixed-seed sample of rows is written; rows.npy lists the
+    batch rows written, in order."""
+    import numpy as np
+
+    arrays = {"latent_values": vals.astype(np.float32), "latent_indices": idx.astype(np.float64),
+              "reconstruction": recon.astype(np.float32)}
+    B = recon.shape[0]
+    row_bytes = 8 + sum(a[0].nbytes for a in arrays.values())
+    n = min(B, (DUMP_BYTES - 4096) // row_bytes)          # 4096: the four .npy headers
+    rows = np.arange(B) if n == B else np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    d = Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "rows.npy", rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a[rows])
 
 
 def headline_from(e, metric, world, steps, warmup, scaling):

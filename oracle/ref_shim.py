@@ -8,10 +8,9 @@ individual source files are executed by path with three import shims:
   * ``nnba.adder``   -> empty module (star-imported, no name is used by any forward)
   * ``SAEs.quantized_matryoshka_SAE`` -> src/quantized_sae/sae/quantized_matryoshka.py
 
-This only works where /root/reference is mounted (the authoring container). It is used by
-``tests/golden/make_golden.py`` to generate the committed fixtures and by the CPU tests that
-cross-check the oracle restatement against the real reference. Nothing in the product
-package, the ``-m gpu`` tests, ``smoke()`` or ``bench.py`` may import this file.
+It needs a checkout of the reference project (``QSAE_REFERENCE_ROOT``), which is not part of this
+repository. Only the fixture generators ``tests/golden/make_golden*.py`` use it; the product
+package, the tests, ``build()``, ``smoke()`` and ``bench.py`` never import this file.
 """
 from __future__ import annotations
 

@@ -22,8 +22,8 @@ BUILD = PKG / "_build"
 LIB = PKG / "libqsae_b200.so"
 SOURCES = ["qsae_api.cu", "encode_topk_sm100.cu", "select_topk.cu", "pack.cu", "decode.cu", "encode_dense.cu", "rescue.cu", "matryoshka.cu",
            "dense_decode_sm100.cu", "analysis.cu", "peer.cu", "train.cu"]
-HEADERS = [CSRC / "kernels.h", CSRC / "ptx_sm100.cuh", CSRC / "topk_common.cuh", CSRC / "tmap_cache.cuh",
-           PKG.parent / "include" / "qsae_b200.h"]
+# every header a source can include: an edit to any of them rebuilds every object
+HEADERS = [*sorted(CSRC.glob("*.h")), *sorted(CSRC.glob("*.cuh")), PKG.parent / "include" / "qsae_b200.h"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -1,7 +1,7 @@
 """Pin the CPU oracle (oracle/qsae_oracle.py) against outputs of the unmodified reference.
 
 The fixtures under tests/golden/ were produced by tests/golden/make_golden.py, which runs the
-reference's own nn.Modules. These tests need no GPU and no /root/reference.
+reference's own nn.Modules. These tests need no GPU and no copy of the reference.
 """
 import numpy as np
 import pytest
@@ -86,8 +86,9 @@ def test_bsae_matches_reference(golden_dir, name):
 def test_timed_cpu_arm_matches_reference_fixture(golden_dir, name):
     """bench.py's CPU arm (`--impl reference`, `cpu_baseline`) times O.bsae_forward_dense_port_torch, the reference's own
     op sequence (sae/binary.py:91-103 + :24-47) on torch CPU tensors. Pin it to the outputs of the unmodified reference
-    stored in the fixtures (runs everywhere, the GPU box included): sparse latent = k non-zeros at the reference's
-    indices with its values, reconstruction and polarize loss equal up to fp32 summation order."""
+    stored in the fixtures: the dense latent is bit-equal to the reference's (its k non-zeros at the reference's indices
+    with the reference's values), reconstruction and polarize loss are equal up to fp32 summation order (the bits of
+    a CPU matmul depend on the host's thread count and instruction set, so stored outputs can only pin them this far)."""
     import torch
 
     cfg = cases.BSAE_CASES[name]
@@ -97,38 +98,11 @@ def test_timed_cpu_arm_matches_reference_fixture(golden_dir, name):
     t = {n: torch.from_numpy(v) for n, v in inp.items()}
     lat, recon, pol = O.bsae_forward_dense_port_torch(t["x"], t["We"], t["be"], t["logits"], t["bd"], n_bits=cfg["n_bits"],
                                                       gamma=cfg["gamma"], k=k)
-    lat = lat.numpy()
-    assert ((lat != 0).sum(1) <= k).all()
-    got_vals = np.take_along_axis(lat, g["latent_idx"].astype(np.int64), axis=1)
-    np.testing.assert_allclose(got_vals, g["latent_vals"], rtol=1e-6, atol=1e-7)
-    assert np.count_nonzero(lat) == np.count_nonzero(g["latent_vals"])
+    ref_lat = np.zeros((cfg["B"], cfg["H"]), dtype=np.float32)
+    np.put_along_axis(ref_lat, g["latent_idx"].astype(np.int64), g["latent_vals"], axis=1)
+    assert np.array_equal(lat.numpy(), ref_lat)
     _close(recon.numpy(), g["recon"])
     assert float(pol) == pytest.approx(float(g["polarize"]), rel=1e-5, abs=1e-9)
-
-
-def test_timed_cpu_arm_is_bit_equal_to_the_shim_loaded_reference():
-    """Where /root/reference is mounted (the authoring container): the port and the reference module, same tensors,
-    same torch -> bit-equal latent, reconstruction and polarize loss."""
-    import torch
-
-    from oracle import ref_shim
-
-    if not ref_shim.available():
-        pytest.skip("/root/reference is not mounted here (GPU box)")
-    ref = ref_shim.load()
-    cfg = dict(D=64, H=2048, n_bits=4, gamma=4.0, B=48, polar=False, bf16=False, seed=123)
-    inp = cases.bsae_inputs(cfg)
-    m = ref.BinarySAE(cfg["D"], cfg["H"], cfg["gamma"], cfg["n_bits"])
-    m.load_state_dict({"encoder.0.weight": torch.from_numpy(inp["We"]), "encoder.0.bias": torch.from_numpy(inp["be"]),
-                       "decoder.weight": torch.from_numpy(inp["logits"]), "decoder.bias": torch.from_numpy(inp["bd"])})
-    m.eval()
-    with torch.no_grad():
-        rl, rr, rp = m(torch.from_numpy(inp["x"]))
-    k = int(cfg["H"] * m.k)
-    t = {n: torch.from_numpy(v) for n, v in inp.items()}
-    lat, recon, pol = O.bsae_forward_dense_port_torch(t["x"], t["We"], t["be"], t["logits"], t["bd"], n_bits=cfg["n_bits"],
-                                                      gamma=cfg["gamma"], k=k)
-    assert torch.equal(lat, rl) and torch.equal(recon, rr) and float(pol) == float(rp)
 
 
 def test_bsae_state_dict_layout(golden_dir):

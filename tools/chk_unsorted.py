@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from quantizedsae_b200 import _lib as L
 B, H, D, k = (int(sys.argv[2]) if len(sys.argv) > 2 else 512), 131072, 512, int(sys.argv[1]) if len(sys.argv) > 1 else 2097
 dev = torch.device("cuda:0")
