@@ -368,6 +368,120 @@ __device__ __forceinline__ void epilogue_loop(const EncodeLaunch& p, int n_my_ti
   }
 }
 
+// MODE 4 on its own: the epilogue of the specialised sweep (SEL == 4 below). It keeps exactly the survivor lists of
+// epilogue_loop<4> (same threshold, same column order, same counts and bounds) and has no debug paths. Compiled
+// without the other modes' per-class registers, it has room for a pipelined TMEM drain: chunk c + 1's tcgen05.ld is
+// in flight while chunk c is compared and its survivors stored (tcgen05.wait::ld waits for every outstanding load of
+// the thread, so the wait for chunk c + 1 comes after chunk c's work). The chunk loop is unrolled so that the
+// two load buffers never have to be copied while a load is landing in one of them.
+__device__ __forceinline__ void epilogue_prior(const EncodeLaunch& p, int n_my_tiles, int tile_begin, int sub_base, int m0,
+                                               int tt0, int zero_from, int e, int lane, uint32_t tmem_base,
+                                               const float* bias_smem, uint64_t* tmem_full, uint64_t* tmem_empty,
+                                               uint64_t* bias_full, uint64_t* pair_empty) {
+  const unsigned full = 0xffffffffu;
+  const int quad = e & 3;       // TMEM lanes 32*quad .. +31 (hardware: warp_id % 4)
+  const int half = e >> 2;      // columns [half*128, half*128+128) of the tile
+  const int row = m0 + quad * 32 + lane;
+  const bool row_ok = row < p.B;
+  const int nsub = p.nsub;
+  const int cap = p.cap;
+  const int k = p.k_sel;
+  const size_t slot = static_cast<size_t>(row_ok ? row : 0) * nsub + sub_base + half;
+  uint2* buf = reinterpret_cast<uint2*>(p.cand) + slot * cap;
+  int cnt = 0;
+  const uint32_t half_taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + half * 128;
+
+  // as in epilogue_loop<4>: a value survives iff v >= thr, thr = max(lowest finite float, prior of the row)
+  float thr = INFINITY;
+  float valid_bound = -INFINITY;
+  if (row_ok) {
+    thr = fmaxf(-3.402823466e+38f, p.prior != nullptr ? __ldg(p.prior + static_cast<size_t>(row) * p.prior_stride) : p.prior_const);
+    valid_bound = thr;
+  }
+
+  for (int t = 0; t < n_my_tiles; ++t) {
+    const int acc = (tt0 + t) & 1;
+    const uint32_t ph = ((tt0 + t) >> 1) & 1;
+    mbar_wait(&tmem_full[acc], ph);
+    mbar_wait(&bias_full[acc], ph);
+    tc_fence_after();
+    const int n_tile = (tile_begin + t) * BN + half * 128;
+    const float4* bias4 = reinterpret_cast<const float4*>(bias_smem + acc * BN + half * 128);
+    const uint32_t taddr = half_taddr + acc * BN;
+    uint32_t r[2][32];
+    tmem_ld_32x32b_x32(taddr, r[0]);
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      uint32_t (&rc)[32] = r[c & 1];
+      tmem_ld_wait(rc);                                              // chunk c has landed; nothing else is in flight
+      if (c < 3) tmem_ld_32x32b_x32(taddr + (c + 1) * 32, r[(c + 1) & 1]);
+      const int col0 = n_tile + c * 32;
+      float v[32];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const float4 b = bias4[c * 8 + j];
+        v[4 * j + 0] = __uint_as_float(rc[4 * j + 0]) + b.x;
+        v[4 * j + 1] = __uint_as_float(rc[4 * j + 1]) + b.y;
+        v[4 * j + 2] = __uint_as_float(rc[4 * j + 2]) + b.z;
+        v[4 * j + 3] = __uint_as_float(rc[4 * j + 3]) + b.w;
+      }
+      if (p.act == 1) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j], 0.f);
+      }
+      if (col0 + 32 > p.H) {  // last, partial tile only
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+          if (col0 + j >= p.H) v[j] = -INFINITY;
+      }
+      uint32_t hits = 0u;
+#pragma unroll
+      for (int j = 0; j < 32; ++j) hits |= (v[j] >= thr) ? (1u << j) : 0u;
+      while (__any_sync(full, hits != 0u)) {
+        if (hits != 0u) {
+          const int j = __ffs(hits) - 1;
+          hits &= hits - 1u;
+          buf[cnt] = make_uint2(__float_as_uint(pick32(v, j)), static_cast<uint32_t>(col0 + j));
+          ++cnt;
+        }
+      }
+      if (__any_sync(full, cnt > cap - 32)) {
+        if (k <= 0) {
+          // threshold-only use (q_sae): a full buffer cannot be cut, so stop collecting and report the overflow
+          if (cnt > cap - 32) {
+            thr = INFINITY;
+            if (p.overflow != nullptr) atomicExch(p.overflow, 1);
+          }
+        } else {
+          // the call may save and restore registers: let the next chunk land first. It takes its in / out
+          // arguments by address, so they are copies: cnt, thr and valid_bound stay in registers on the common path.
+          if (c < 3) tmem_ld_wait(r[(c + 1) & 1]);
+          int cnt_r = cnt;
+          float thr_r = thr, bound_r = valid_bound;
+          relieve_warp_buffers(buf, cnt_r, thr_r, bound_r, k, cap, lane);
+          cnt = cnt_r; thr = thr_r; valid_bound = bound_r;
+        }
+      }
+    }
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) {
+      mbar_arrive(&tmem_empty[acc]);
+      if (pair_empty != nullptr) mbar_arrive_cluster(&pair_empty[acc], 0);   // the leader's MMA thread waits for both CTAs
+    }
+  }
+  if (row_ok) {
+    p.cand_cnt[slot] = cnt;
+    p.cand_thr[slot] = valid_bound;
+    if (zero_from >= 0 && half == 0) {
+      for (int s2 = zero_from; s2 < nsub; ++s2) {
+        p.cand_cnt[static_cast<size_t>(row) * nsub + s2] = 0;
+        p.cand_thr[static_cast<size_t>(row) * nsub + s2] = -INFINITY;
+      }
+    }
+  }
+}
+
 // ---- range schedule --------------------------------------------------------------------------------------
 // Small batches do not fill the machine with (split, row block) CTAs: B = 4096 gives 32 row blocks x 4 splits = 128
 // CTAs on 148 SMs. With p.range_g > 0 the grid is range_g CTAs (one per SM) and the U = row_blocks x n_tiles tile
@@ -661,14 +775,17 @@ __device__ __forceinline__ void epilogue_dense(const EncodeLaunch& p, int n_my_t
   if (p.act == 2) flush_level_count();
 }
 
-// one piece of the epilogue role: dense epilogue, or the selection mode of this launch
-template <bool DENSE, bool PAIR>
+// one piece of the epilogue role: dense epilogue, the prior-threshold epilogue of the specialised sweep (SEL == 4), or
+// the selection mode of this launch
+template <bool DENSE, bool PAIR, int SEL>
 __device__ __forceinline__ void run_epilogue_piece(const EncodeLaunch& p, int n, int tile0, int sub_base, int m0, int tt0,
                                                    int zero_from, int e, int lane, uint32_t tmem_base, const float* bias_smem,
                                                    uint16_t* share, uint8_t* staging, uint64_t* tmem_full, uint64_t* tmem_empty,
                                                    uint64_t* bias_full, uint64_t* pe) {
   if constexpr (DENSE) {
     epilogue_dense<PAIR>(p, n, tile0, m0, tt0, e, lane, tmem_base, bias_smem, staging, tmem_full, tmem_empty, bias_full, pe);
+  } else if constexpr (SEL == 4) {
+    epilogue_prior(p, n, tile0, sub_base, m0, tt0, zero_from, e, lane, tmem_base, bias_smem, tmem_full, tmem_empty, bias_full, pe);
   } else {
     switch (p.mode) {
       case 1:
@@ -703,7 +820,9 @@ __device__ __forceinline__ void run_epilogue_piece(const EncodeLaunch& p, int n,
 //   their own 128 accumulator rows from their own TMEM. Halves the W bytes per SM (L2 -> SM traffic
 //   and shared-memory reads) and frees 16 KiB per stage: 4-stage ring for the selection epilogues,
 //   3 stages next to the store staging area for the dense epilogue.
-template <int K_CHUNKS, bool DENSE, int CL>
+// SEL = -1: the selection mode is p.mode, chosen at run time; SEL = 4: prior threshold only (epilogue_prior). Producer,
+//   MMA and bias roles are the same for both.
+template <int K_CHUNKS, bool DENSE, int CL, int SEL>
 __global__ void __launch_bounds__(cta_threads(DENSE), 1)
 encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
                    const __grid_constant__ CUtensorMap tmap_b0,
@@ -932,7 +1051,7 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
       // epilogue's register allocation where it was before pieces existed: the B = 65536 sweep lost 7 % otherwise)
       const int tile_begin = split * p.tiles_per_split;
       const int n = max(0, min(p.n_tiles, tile_begin + p.tiles_per_split) - tile_begin);
-      if (n > 0) run_epilogue_piece<DENSE, PAIR>(p, n, tile_begin, split * 2, m0_grid, 0, -1, e, lane, tmem_base, bias_smem, share, smem + L.staging_off,
+      if (n > 0) run_epilogue_piece<DENSE, PAIR, SEL>(p, n, tile_begin, split * 2, m0_grid, 0, -1, e, lane, tmem_base, bias_smem, share, smem + L.staging_off,
                                                  tmem_full, tmem_empty, bias_full, pe);
     } else {
       const int n_pieces = *piece_n;
@@ -940,7 +1059,7 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
 #pragma unroll 1
       for (int pi = 0; pi < n_pieces; ++pi) {
         const Piece pc = piece_tab[pi];
-        run_epilogue_piece<DENSE, PAIR>(p, pc.n, pc.tile0, pc.sub_base, pc.rb * BM, tt0, pc.zero_from, e, lane, tmem_base, bias_smem, share,
+        run_epilogue_piece<DENSE, PAIR, SEL>(p, pc.n, pc.tile0, pc.sub_base, pc.rb * BM, tt0, pc.zero_from, e, lane, tmem_base, bias_smem, share,
                                         smem + L.staging_off, tmem_full, tmem_empty, bias_full, pe);
         tt0 += pc.n;
       }
@@ -1465,12 +1584,12 @@ bool make_tmap_bf16(CUtensorMap* map, const void* base, int rows, int cols, int 
 
 struct BMaps { CUtensorMap m[3]; };   // the (up to three) bf16 parts of W, boxed for the chosen cluster variant
 
-template <int K_CHUNKS, bool DENSE, int CL>
+template <int K_CHUNKS, bool DENSE, int CL, int SEL>
 cudaError_t launch_k(const CUtensorMap& tx, const BMaps& b, const EncodeLaunch& p, cudaStream_t stream) {
   const SmemLayout L = smem_layout(K_CHUNKS, DENSE, CL >= 2);
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(encode_topk_kernel<K_CHUNKS, DENSE, CL>,
+    cudaError_t e = cudaFuncSetAttribute(encode_topk_kernel<K_CHUNKS, DENSE, CL, SEL>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, L.total);
     if (e != cudaSuccess) return e;
     attr_set = true;
@@ -1493,33 +1612,46 @@ cudaError_t launch_k(const CUtensorMap& tx, const BMaps& b, const EncodeLaunch& 
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, encode_topk_kernel<K_CHUNKS, DENSE, CL>, tx, b.m[0], b.m[1], b.m[2], p);
+    return cudaLaunchKernelEx(&cfg, encode_topk_kernel<K_CHUNKS, DENSE, CL, SEL>, tx, b.m[0], b.m[1], b.m[2], p);
   } else {
-    encode_topk_kernel<K_CHUNKS, DENSE, CL><<<grid, cta_threads(DENSE), L.total, stream>>>(tx, b.m[0], b.m[1], b.m[2], p);
+    encode_topk_kernel<K_CHUNKS, DENSE, CL, SEL><<<grid, cta_threads(DENSE), L.total, stream>>>(tx, b.m[0], b.m[1], b.m[2], p);
     return cudaGetLastError();
   }
 }
 
+template <bool DENSE, int SEL>
+cudaError_t launch_kc(const CUtensorMap& tx, const BMaps& b, const EncodeLaunch& p, cudaStream_t stream) {
+  switch ((p.D + BK - 1) / BK) {
+    case 1: return launch_k<1, DENSE, 0, SEL>(tx, b, p, stream);
+    case 2: return launch_k<2, DENSE, 0, SEL>(tx, b, p, stream);
+    case 3: return launch_k<3, DENSE, 0, SEL>(tx, b, p, stream);
+    case 4: return launch_k<4, DENSE, 0, SEL>(tx, b, p, stream);
+    case 5: return launch_k<5, DENSE, 0, SEL>(tx, b, p, stream);
+    case 6: return launch_k<6, DENSE, 0, SEL>(tx, b, p, stream);
+    case 7: return launch_k<7, DENSE, 0, SEL>(tx, b, p, stream);
+    default:   // the headline width: the cluster variants exist here (launch_any has checked D <= 512)
+      if (p.cluster == 3) return launch_k<8, DENSE, 3, SEL>(tx, b, p, stream);
+      if (p.cluster == 2) return launch_k<8, DENSE, 2, SEL>(tx, b, p, stream);
+      if (p.cluster == 1) return launch_k<8, DENSE, 1, SEL>(tx, b, p, stream);
+      return launch_k<8, DENSE, 0, SEL>(tx, b, p, stream);
+  }
+}
+
+// Prior-threshold sweeps (mode 4) run on the kernel compiled for that mode alone unless QSAE_ENCODE_SPECIALISED=0;
+// the diagnostics (debug_mode, debug_z) exist in the generic kernel only.
 template <bool DENSE>
 const char* launch_any(const CUtensorMap& tx, const BMaps& b, const EncodeLaunch& p, cudaStream_t stream) {
   const int kc = (p.D + BK - 1) / BK;
+  if (kc < 1 || kc > 8) return "D must be <= 512";
   if (p.cluster == 3 && kc != 8) return "the pair range schedule exists for D > 448 only";
   cudaError_t e;
-  switch (kc) {
-    case 1: e = launch_k<1, DENSE, 0>(tx, b, p, stream); break;
-    case 2: e = launch_k<2, DENSE, 0>(tx, b, p, stream); break;
-    case 3: e = launch_k<3, DENSE, 0>(tx, b, p, stream); break;
-    case 4: e = launch_k<4, DENSE, 0>(tx, b, p, stream); break;
-    case 5: e = launch_k<5, DENSE, 0>(tx, b, p, stream); break;
-    case 6: e = launch_k<6, DENSE, 0>(tx, b, p, stream); break;
-    case 7: e = launch_k<7, DENSE, 0>(tx, b, p, stream); break;
-    case 8:   // the headline width: the cluster variants exist here
-      if (p.cluster == 3) e = launch_k<8, DENSE, 3>(tx, b, p, stream);
-      else if (p.cluster == 2) e = launch_k<8, DENSE, 2>(tx, b, p, stream);
-      else if (p.cluster == 1) e = launch_k<8, DENSE, 1>(tx, b, p, stream);
-      else e = launch_k<8, DENSE, 0>(tx, b, p, stream);
-      break;
-    default: return "D must be <= 512";
+  if constexpr (!DENSE) {
+    if (p.mode == 4 && p.debug_mode == 0 && p.debug_z == nullptr && tuning().encode_specialised != 0)
+      e = launch_kc<false, 4>(tx, b, p, stream);
+    else
+      e = launch_kc<false, -1>(tx, b, p, stream);
+  } else {
+    e = launch_kc<true, -1>(tx, b, p, stream);
   }
   return e == cudaSuccess ? nullptr : cudaGetErrorString(e);
 }

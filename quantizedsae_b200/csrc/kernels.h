@@ -28,6 +28,7 @@ struct Tuning {
   int encode_cluster;     // QSAE_ENCODE_CLUSTER: 0 / 1 / 2 forces the cluster variant (-1 = automatic)
   int encode_range;       // QSAE_ENCODE_RANGE: 0 keeps the (split, row block) grid at small batches
   int encode_range_pair;  // QSAE_ENCODE_RANGE_PAIR: 1 = cta_group::2 pairs on the range schedule (sparse sweeps)
+  int encode_specialised; // QSAE_ENCODE_SPECIALISED: 0 = prior-threshold sweeps on the generic kernel (all modes compiled in)
   int mat_bps;            // QSAE_MAT_BPS: 6 / 7 / 8 forces the resident blocks per SM of the q_sae level decoder (0 = automatic, -1 = always 6)
   int prepass_range;      // QSAE_PREPASS_RANGE: 1 = sample pre-pass of large batches on the pair range schedule (experiment; no gain measured)
   int merge_tier;         // QSAE_MERGE_TIER: 8 / 12 / 16 forces the keys per lane of the warp merge (0 = from the expected survivor count)

@@ -194,6 +194,18 @@ __device__ __forceinline__ void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&r)
 __device__ __forceinline__ void tmem_ld_wait() {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
+// the same wait, with the destination registers of the outstanding load as operands: when other work sits between
+// a tcgen05.ld and its wait, this keeps the compiler from reading (or copying) r before the load has landed
+__device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[32]) {
+  asm volatile("tcgen05.wait::ld.sync.aligned;"
+               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
+                 "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]),
+                 "+r"(r[15]), "+r"(r[16]), "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]),
+                 "+r"(r[22]), "+r"(r[23]), "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]),
+                 "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
+               :
+               : "memory");
+}
 
 // ---------------------------------------------------------------- tcgen05, CTA pairs (cta_group::2)
 // Two CTAs of a cluster (ranks 2i, 2i+1, same TPC) execute one MMA of M = 256: each holds its own

@@ -33,6 +33,7 @@ void reload_tuning() {
   t.encode_cluster = env_int("QSAE_ENCODE_CLUSTER", -1);
   t.encode_range = env_int("QSAE_ENCODE_RANGE", 1);
   t.encode_range_pair = env_int("QSAE_ENCODE_RANGE_PAIR", 1);
+  t.encode_specialised = env_int("QSAE_ENCODE_SPECIALISED", 1);
   t.prior_prep = env_int("QSAE_PRIOR_PREP", 1);
   t.mat_bps = env_int("QSAE_MAT_BPS", 0);
   t.prepass_range = env_int("QSAE_PREPASS_RANGE", 0);
