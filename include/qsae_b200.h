@@ -367,6 +367,37 @@ int qsae_tsae_forward(const float* x_f32, const uint16_t* w_hi /* [H, D]: bf16(W
                       float* h_out /* [B, H] */, float* recon /* [B, D] */, void* workspace,
                       size_t workspace_bytes, void* stream);
 
+/* t_t_bf16 [H, D] = T^T as bf16 (exact: the entries are ternary), the B operand of the backward's g T. */
+int qsae_pack_ternary_t(const float* w /* [D, H] */, int D, int H, float threshold, uint16_t* t_t_bf16, void* stream);
+
+/* Weight-gradient GEMM on the tensor cores: c[M, N] = sum_k A(k, m) B(k, n), a contraction over K batch rows.
+ * b_parts: host array of n_parts device pointers, row-major bf16 [K, N]. a_parts: row-major bf16 [K, M]
+ * (a_kmajor = 0), or [M, K] (a_kmajor = 1, then K % 8 == 0). Both MN-major operands are read as they are, no
+ * transposes. n_parts = 1: one bf16 product; n_parts = 3: the operands are three-part splits
+ * (qsae_split_bf16x3) and the six products above 2^-24 go into one fp32 accumulator (fp32-accurate products).
+ * N % 8 == 0 and M % 8 == 0 (a_kmajor = 0) or K % 8 == 0 (a_kmajor = 1); any K >= 1 (TMA zero-fills the tail).
+ * c [M, N] fp32 is overwritten. */
+int qsae_wgrad(const uint16_t* const* a_parts, const uint16_t* const* b_parts, int n_parts, int M, int N, int K,
+               int a_kmajor, float* c, void* stream);
+
+/* Backward of TernarySparseAutoencoder.forward (what torch autograd computes on the reference, training.py):
+ *   gz = (g T + g_h) * 1[h > 0]            g = d loss / d recon [B, D], g_h = d loss / d h [B, H] or NULL
+ *   grad_w_enc = gz^T x [H, D]    grad_b_enc = sum_b gz [H]    grad_w_dec = mask * (g^T h) [D, H] (mask NULL: 1)
+ *   grad_x = gz W_enc [B, D] (NULL: not computed; w_hi / w_mid / w_lo are then unused)
+ * gz comes from the dense encoder kernel with a ReLU-backward epilogue (g T never reaches memory), which also sums it
+ * per column into grad_b_enc; the three weight products are qsae_wgrad GEMMs. exact = 1: g, gz, h, x (and W_enc: w_mid / w_lo from qsae_split_bf16x3) as three
+ * bf16 parts, fp32-accurate products; exact = 0: one bf16 product each. grad_b_enc is a column sum with atomics
+ * (not bit-deterministic); everything else is. Outputs are overwritten. h, x, g, g_h, gradients 16-byte aligned.
+ * Same shape limits as qsae_tsae_forward; B may be 0 (zero gradients). */
+int qsae_tsae_backward_workspace_bytes(int B, int H, int D, int exact, size_t* bytes);
+int qsae_tsae_backward(const float* x /* [B, D] */, const float* h /* [B, H] forward output */,
+                       const float* g_recon /* [B, D] */, const float* g_h /* [B, H] or NULL */,
+                       const uint16_t* t_t_bf16 /* [H, D] from qsae_pack_ternary_t */, const float* mask /* [D, H] or NULL */,
+                       const uint16_t* w_hi, const uint16_t* w_mid, const uint16_t* w_lo /* [H, D], grad_x only */,
+                       int B, int H, int D, int exact, float* grad_w_enc /* [H, D] */, float* grad_b_enc /* [H] */,
+                       float* grad_w_dec /* [D, H] */, float* grad_x /* [B, D] or NULL */, void* workspace,
+                       size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Dictionary-sharded b_sae (2^20-latent dictionaries over G GPUs; SURVEY.md 8e). Shard g owns the
  * latents [g * shard_latents, (g + 1) * shard_latents) of nn.Linear / binary_decoder

@@ -103,6 +103,10 @@ SYMBOLS = {
     "qsae_rigl_init_mask": (_i, [_vp, _vp, _i, _i, C.c_ulonglong, _vp, _sz, _vp]),
     "qsae_rigl_update_mask": (_i, [_vp, _vp, _vp, _vp, _i, _i, C.c_ulonglong, C.c_ulonglong, _vp, _sz, _vp]),
     "qsae_mul_inplace": (_i, [_vp, _vp, _sz, _vp]),
+    "qsae_pack_ternary_t": (_i, [_vp, _i, _i, _f, _vp, _vp]),
+    "qsae_wgrad": (_i, [C.POINTER(_vp), C.POINTER(_vp), _i, _i, _i, _i, _i, _vp, _vp]),
+    "qsae_tsae_backward_workspace_bytes": (_i, [_i, _i, _i, _i, C.POINTER(_sz)]),
+    "qsae_tsae_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
 }
 
 
@@ -692,6 +696,77 @@ def tsae_forward(x: torch.Tensor, w_parts, b_enc: torch.Tensor, t_bf16: torch.Te
                                    t_bf16.data_ptr(), B, H, D, 1 if exact else 0, h.data_ptr(), recon.data_ptr(),
                                    ws.data_ptr(), ws.numel(), _stream()))
     return h, recon
+
+
+def pack_ternary_t(w: torch.Tensor, threshold: float = 0.5) -> torch.Tensor:
+    """decoder.weight [D, H] -> T^T bf16 [H, D], T = sign(w) * (|w| >= thr) (B operand of the t_sae backward)."""
+    _need_cuda(w)
+    assert w.dtype == torch.float32
+    D, H = w.shape
+    t_t = torch.empty((H, D), dtype=torch.bfloat16, device=w.device)
+    check(load().qsae_pack_ternary_t(w.data_ptr(), D, H, float(threshold), t_t.data_ptr(), _stream()))
+    return t_t
+
+
+def _bf16_parts(parts, what: str):
+    parts = tuple(parts)
+    if len(parts) not in (1, 3):
+        raise ValueError(f"{what}: 1 or 3 bf16 parts expected, got {len(parts)}")
+    _need_cuda(*parts)
+    if any(p.dtype != torch.bfloat16 or p.dim() != 2 or p.shape != parts[0].shape for p in parts):
+        raise ValueError(f"{what}: parts must be bf16 matrices of one shape")
+    return parts
+
+
+def wgrad(a_parts, b_parts, a_kmajor: bool = False) -> torch.Tensor:
+    """c [M, N] fp32 = sum_k A(k, m) B(k, n) on the tensor cores (qsae_wgrad). b_parts: bf16 [K, N];
+    a_parts: bf16 [K, M], or [M, K] with a_kmajor. One part each (one bf16 product) or three (split_bf16x3 parts:
+    the six products above 2^-24 in one fp32 accumulator)."""
+    a_parts = _bf16_parts(a_parts, "wgrad A")
+    b_parts = _bf16_parts(b_parts, "wgrad B")
+    if len(a_parts) != len(b_parts):
+        raise ValueError("wgrad: A and B need the same number of parts")
+    K, N = b_parts[0].shape
+    M, Ka = (a_parts[0].shape if a_kmajor else a_parts[0].shape[::-1])
+    if Ka != K:
+        raise ValueError(f"wgrad: contraction lengths differ ({Ka} vs {K})")
+    c = torch.empty((M, N), dtype=torch.float32, device=b_parts[0].device)
+    n = len(a_parts)
+    ap = (_vp * n)(*[p.data_ptr() for p in a_parts])
+    bp = (_vp * n)(*[p.data_ptr() for p in b_parts])
+    check(load().qsae_wgrad(ap, bp, n, M, N, K, 1 if a_kmajor else 0, c.data_ptr(), _stream()))
+    return c
+
+
+def tsae_backward(x: torch.Tensor, h: torch.Tensor, g_recon: torch.Tensor, g_h: torch.Tensor | None, t_t: torch.Tensor,
+                  mask: torch.Tensor | None, w_parts, exact: bool, want_grad_x: bool):
+    """Backward of t_sae's forward (qsae_tsae_backward). w_parts: (bf16(W_enc),) or split_bf16x3(W_enc), used for
+    grad_x only. -> (grad W_enc [H, D], grad b_enc [H], grad W_dec [D, H], grad x [B, D] | None)"""
+    _need_cuda(x, h, g_recon, g_h, t_t, mask)
+    _f32c(x, h, g_recon, g_h, mask)
+    B, D = x.shape
+    H = h.shape[1]
+    assert h.shape == (B, H) and g_recon.shape == (B, D) and t_t.shape == (H, D) and t_t.dtype == torch.bfloat16
+    assert g_h is None or g_h.shape == (B, H)
+    assert mask is None or mask.shape == (D, H)
+    w = tuple(w_parts) if want_grad_x else (None, None, None)
+    if want_grad_x:
+        _need_cuda(*w)
+        if len(w) != (3 if exact else 1):
+            raise ValueError("tsae_backward: grad_x needs the encoder weight as 3 bf16 parts (exact) or 1 (fast)")
+        w = w + (None,) * (3 - len(w))
+    dev = x.device
+    gwe = torch.empty((H, D), dtype=torch.float32, device=dev)
+    gbe = torch.empty((H,), dtype=torch.float32, device=dev)
+    gwd = torch.empty((D, H), dtype=torch.float32, device=dev)
+    gx = torch.empty((B, D), dtype=torch.float32, device=dev) if want_grad_x else None
+    n = _sz(0)
+    check(load().qsae_tsae_backward_workspace_bytes(B, H, D, 1 if exact else 0, C.byref(n)))
+    ws = _workspace(dev, int(n.value))
+    check(load().qsae_tsae_backward(x.data_ptr(), h.data_ptr(), g_recon.data_ptr(), _ptr(g_h), t_t.data_ptr(), _ptr(mask),
+                                    _ptr(w[0]), _ptr(w[1]), _ptr(w[2]), B, H, D, 1 if exact else 0, gwe.data_ptr(),
+                                    gbe.data_ptr(), gwd.data_ptr(), _ptr(gx), ws.data_ptr(), ws.numel(), _stream()))
+    return gwe, gbe, gwd, gx
 
 
 def pack_candidates(vals: torch.Tensor, idx: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:

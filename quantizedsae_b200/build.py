@@ -21,7 +21,7 @@ CSRC = PKG / "csrc"
 BUILD = PKG / "_build"
 LIB = PKG / "libqsae_b200.so"
 SOURCES = ["qsae_api.cu", "encode_topk_sm100.cu", "select_topk.cu", "pack.cu", "decode.cu", "encode_dense.cu", "rescue.cu", "matryoshka.cu",
-           "dense_decode_sm100.cu", "analysis.cu", "peer.cu", "train.cu"]
+           "dense_decode_sm100.cu", "analysis.cu", "peer.cu", "train.cu", "wgrad_sm100.cu"]
 # every header a source can include: an edit to any of them rebuilds every object
 HEADERS = [*sorted(CSRC.glob("*.h")), *sorted(CSRC.glob("*.cuh")), PKG.parent / "include" / "qsae_b200.h"]
 

@@ -632,11 +632,12 @@ __device__ __forceinline__ void epilogue_dense(const EncodeLaunch& p, int n_my_t
         }
         if (row0 + lane < p.B) n_act += n;
       }
-      if (p.accum_mode != 0) {
+      if (p.accum_mode != 0 || p.act == 3) {
         // Split-operand passes (exact fp32 encoder): r holds this pass's raw partial products (the
         // launcher passes no bias for these passes; the final pass adds p.accum_bias here).
         //   1: out = acc            2: out = out + acc            3: out = act(out + acc + bias), + bf16 hi / lo
         // The transformation runs in the row-contiguous read-back layout, where `out` is read coalesced.
+        // act == 3 (ReLU backward, streamed-operand kernel only, no bias): see the WIDE branch below.
         auto finish = [&](int rr, int cc, const uint4 u) {
           if (row0 + rr >= p.B || cc >= p.H) return;
           const size_t off = static_cast<size_t>(row0 + rr) * H + cc;
@@ -667,6 +668,59 @@ __device__ __forceinline__ void epilogue_dense(const EncodeLaunch& p, int n_my_t
           for (int q = 0; q < 8; ++q)
             st_shared_v4(st + lane * 128 + ((q ^ (lane & 7)) << 4), r[4 * q], r[4 * q + 1], r[4 * q + 2], r[4 * q + 3]);
           __syncwarp();
+          if (p.act == 3) {
+            // ReLU backward at the forward's output: out = (acc + gate_add) * (gate > 0); torch masks on the returned h
+            // and selects, so a non-finite acc where h <= 0 gives 0. gate / gate_add do not depend on the accumulator:
+            // four rows of both are loaded before any of them is used (a load per row in turn left the kernel
+            // latency-bound). The warp's 32 rows are summed per column (p.gate_colsum += sum_b out: the bias
+            // gradient, one atomic per column and warp).
+            const int cc = col0 + f_col;
+            float4 cs = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+            for (int j0 = 0; j0 < 8; j0 += 4) {
+              float4 hv[4], av[4];
+#pragma unroll
+              for (int i = 0; i < 4; ++i) {
+                const int rr = 4 * (j0 + i) + f_row;
+                const bool ok = row0 + rr < p.B && cc < p.H;
+                const size_t off = static_cast<size_t>(row0 + rr) * H + cc;
+                hv[i] = ok ? __ldg(reinterpret_cast<const float4*>(p.gate + off)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                av[i] = ok && p.gate_add != nullptr ? __ldg(reinterpret_cast<const float4*>(p.gate_add + off))
+                                                    : make_float4(0.f, 0.f, 0.f, 0.f);
+              }
+#pragma unroll
+              for (int i = 0; i < 4; ++i) {
+                const int rr = 4 * (j0 + i) + f_row;
+                if (row0 + rr >= p.B || cc >= p.H) continue;
+                const size_t off = static_cast<size_t>(row0 + rr) * H + cc;
+                const uint4 u = ld_shared_v4(st + rr * 128 + (((lane & 7) ^ (rr & 7)) << 4));
+                float4 v = make_float4(__uint_as_float(u.x) + av[i].x, __uint_as_float(u.y) + av[i].y,
+                                       __uint_as_float(u.z) + av[i].z, __uint_as_float(u.w) + av[i].w);
+                v.x = hv[i].x > 0.f ? v.x : 0.f; v.y = hv[i].y > 0.f ? v.y : 0.f;
+                v.z = hv[i].z > 0.f ? v.z : 0.f; v.w = hv[i].w > 0.f ? v.w : 0.f;
+                cs.x += v.x; cs.y += v.y; cs.z += v.z; cs.w += v.w;
+                if (flags & 1) *reinterpret_cast<float4*>(p.out_f32 + off) = v;
+                if (flags & 2)
+                  *reinterpret_cast<uint2*>(p.out_hi + off) = make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w));
+              }
+            }
+            if (p.gate_colsum != nullptr) {   // lanes l, l + 8, l + 16, l + 24 hold the same four columns
+#pragma unroll
+              for (int sh = 8; sh <= 16; sh <<= 1) {
+                cs.x += __shfl_xor_sync(0xffffffffu, cs.x, sh);
+                cs.y += __shfl_xor_sync(0xffffffffu, cs.y, sh);
+                cs.z += __shfl_xor_sync(0xffffffffu, cs.z, sh);
+                cs.w += __shfl_xor_sync(0xffffffffu, cs.w, sh);
+              }
+              if (lane < 8 && cc < p.H) {
+                atomicAdd(p.gate_colsum + cc, cs.x);
+                atomicAdd(p.gate_colsum + cc + 1, cs.y);
+                atomicAdd(p.gate_colsum + cc + 2, cs.z);
+                atomicAdd(p.gate_colsum + cc + 3, cs.w);
+              }
+            }
+            continue;
+          }
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             const int rr = 4 * j + f_row;
@@ -1110,7 +1164,7 @@ __global__ void __launch_bounds__(cta_threads(true), 1)
 encode_dense_split_kernel(const __grid_constant__ CUtensorMap tmap_xh, const __grid_constant__ CUtensorMap tmap_xm,
                           const __grid_constant__ CUtensorMap tmap_xl, const __grid_constant__ CUtensorMap tmap_wh,
                           const __grid_constant__ CUtensorMap tmap_wm, const __grid_constant__ CUtensorMap tmap_wl,
-                          EncodeLaunch p, int k_chunks, int n_prod) {
+                          EncodeLaunch p, int k_chunks, int n_prod, uint32_t prods) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const SmemLayout L = split_smem_layout();
   uint8_t* ring = smem;
@@ -1138,10 +1192,10 @@ encode_dense_split_kernel(const __grid_constant__ CUtensorMap tmap_xh, const __g
   const int n_my = static_cast<int>(range_start(blockIdx.x / 2 + 1, U, G) - u0);
   const int rbp0 = static_cast<int>(u0 / n_tiles);
   const int tile0 = static_cast<int>(u0 - static_cast<long long>(rbp0) * n_tiles);
-  // n_prod = 6: the split-operand product; n_prod = 1: only xh wh (the fast mode's single bf16 product on this
-  // kernel's schedule: all 148 SMs at any batch, nothing resident)
+  // products: (x part, W part) of product i = ((prods >> 4i + 2) & 3, (prods >> 4i) & 3), see the launcher.
+  // n_prod = 6: the split-operand product; n_prod = 3: three x parts against one W part; n_prod = 1: only xh wh (the
+  // fast mode's single bf16 product on this kernel's schedule: all 148 SMs at any batch, nothing resident)
   const int k_iters = n_prod * k_chunks;
-  const int prod0 = 6 - n_prod;
 
   if (threadIdx.x == 0) {
     if ((smem_u32(smem) & 1023u) != 0u) {
@@ -1180,10 +1234,11 @@ encode_dense_split_kernel(const __grid_constant__ CUtensorMap tmap_xh, const __g
         const int n0 = tile * BN + static_cast<int>(cta_rank) * (BN / 2);
 #pragma unroll 1
         for (int it = 0; it < k_iters; ++it) {
-          const int pi = it / k_chunks, kc = it - pi * k_chunks, prod = prod0 + pi;
-          // product order (smallest first): xl wh, xm wm, xh wl, xm wh, xh wm, xh wh
-          const CUtensorMap* tx = (prod == 0) ? &tmap_xl : ((prod == 1 || prod == 3) ? &tmap_xm : &tmap_xh);
-          const CUtensorMap* tw = (prod == 2) ? &tmap_wl : ((prod == 1 || prod == 4) ? &tmap_wm : &tmap_wh);
+          const int pi = it / k_chunks, kc = it - pi * k_chunks;
+          const uint32_t pr = prods >> (4 * pi);
+          const uint32_t xi = (pr >> 2) & 3u, wi = pr & 3u;
+          const CUtensorMap* tx = (xi == 2) ? &tmap_xl : (xi == 1 ? &tmap_xm : &tmap_xh);
+          const CUtensorMap* tw = (wi == 2) ? &tmap_wl : (wi == 1 ? &tmap_wm : &tmap_wh);
           mbar_wait(&empty[stage], phase ^ 1u);
           const uint32_t full_leader = mapa_u32(smem_u32(&full[stage]), 0);
           if (leader) mbar_arrive_expect_tx(&full[stage], 2 * kSplitStageBytes);   // 32 KiB from each CTA
@@ -1758,6 +1813,7 @@ const char* encode_dense_tc_launch(const uint16_t* x_bf16, const uint16_t* const
   if (p.accum_mode != 0 && !out_f32) return "dense encoder: accumulating passes need the fp32 output";
   if (p.act == 2 && (p.accum_mode != 0 || !p.step_scale || !p.step_level_start || !p.step_level_count || (p.H % 128) != 0))
     return "dense encoder: the step-operand epilogue needs scale / levels / counts, H % 128 == 0 and a plain pass";
+  if (p.act == 3) return "dense encoder: the ReLU-backward epilogue runs on the streamed-operand kernel only";
   CUtensorMap tx;
   if (!make_tmap_bf16(&tx, x_bf16, p.B, p.D, BM)) return "cuTensorMapEncodeTiled(x) failed";
   p.out_f32 = out_f32; p.out_hi = out_hi; p.out_lo = out_lo;
@@ -1772,9 +1828,15 @@ const char* encode_dense_tc_launch(const uint16_t* x_bf16, const uint16_t* const
 }
 
 const char* encode_dense_split_launch(const uint16_t* const* x_parts, const uint16_t* const* w_parts, int n_parts, EncodeLaunch p,
-                                      float* out_f32, uint16_t* out_hi, uint16_t* out_lo, int num_sms, cudaStream_t stream) {
+                                      float* out_f32, uint16_t* out_hi, uint16_t* out_lo, int num_sms, cudaStream_t stream,
+                                      int n_w_parts) {
+  if (n_w_parts == 0) n_w_parts = n_parts;
   if (n_parts != 1 && n_parts != 3) return "dense tensor-core encoder (streamed operands): 1 or 3 parts per operand";
+  if (n_w_parts != n_parts && !(n_parts == 3 && n_w_parts == 1))
+    return "dense tensor-core encoder (streamed operands): 1 x 1, 3 x 3 or 3 x 1 parts";
   if ((p.H % 8) != 0) return "dense tensor-core encoder needs H % 8 == 0";
+  if (p.act == 3 && (!p.gate || out_lo || p.bias != nullptr))
+    return "dense encoder: the ReLU-backward epilogue needs the gate, writes fp32 and / or bf16 hi, and takes no bias";
   if ((reinterpret_cast<uintptr_t>(out_f32) | reinterpret_cast<uintptr_t>(out_hi) | reinterpret_cast<uintptr_t>(out_lo)) & 15)
     return "dense tensor-core encoder: outputs must be 16-byte aligned";
   if (p.act == 2 && (!p.step_scale || !p.step_level_start || !p.step_level_count || (p.H % 128) != 0))
@@ -1789,9 +1851,21 @@ const char* encode_dense_split_launch(const uint16_t* const* x_parts, const uint
   if (tuning().dense_flags_mask >= 0) p.dense_flags &= tuning().dense_flags_mask;  // timing experiments only
   CUtensorMap tx[3], tw[3];
   for (int i = 0; i < 3; ++i) {
-    const int j = i < n_parts ? i : 0;
-    if (!make_tmap_bf16(&tx[i], x_parts[j], p.B, p.D, BM)) return "cuTensorMapEncodeTiled(x part) failed";
-    if (!make_tmap_bf16(&tw[i], w_parts[j], p.H, p.D, BN / 2)) return "cuTensorMapEncodeTiled(W part) failed";
+    if (!make_tmap_bf16(&tx[i], x_parts[i < n_parts ? i : 0], p.B, p.D, BM)) return "cuTensorMapEncodeTiled(x part) failed";
+    if (!make_tmap_bf16(&tw[i], w_parts[i < n_w_parts ? i : 0], p.H, p.D, BN / 2)) return "cuTensorMapEncodeTiled(W part) failed";
+  }
+  // product list (x part, W part), smallest first: 3 x 3: xl wh, xm wm, xh wl, xm wh, xh wm, xh wh;
+  // 3 x 1: xl wh, xm wh, xh wh; 1 x 1: xh wh
+  static const uint32_t kSix[6][2] = {{2, 0}, {1, 1}, {0, 2}, {1, 0}, {0, 1}, {0, 0}};
+  static const uint32_t kThree[3][2] = {{2, 0}, {1, 0}, {0, 0}};
+  int n_prod = 1;
+  uint32_t prods = 0u;
+  if (n_parts == 3) {
+    n_prod = n_w_parts == 3 ? 6 : 3;
+    for (int i = 0; i < n_prod; ++i) {
+      const uint32_t* pr = n_prod == 6 ? kSix[i] : kThree[i];
+      prods |= ((pr[0] << 2) | pr[1]) << (4 * i);
+    }
   }
   const SmemLayout L = split_smem_layout();
   static bool attr_set = false;
@@ -1818,7 +1892,7 @@ const char* encode_dense_split_launch(const uint16_t* const* x_parts, const uint
   cfg.numAttrs = 1;
   const int k_chunks = (p.D + BK - 1) / BK;
   cudaError_t e = cudaLaunchKernelEx(&cfg, encode_dense_split_kernel, tx[0], tx[1], tx[2], tw[0], tw[1], tw[2], p, k_chunks,
-                                     n_parts == 3 ? 6 : 1);
+                                     n_prod, prods);
   return e == cudaSuccess ? nullptr : cudaGetErrorString(e);
 }
 

@@ -59,7 +59,8 @@ struct EncodeLaunch {
   int range_pair;       // range schedule over cta_group::2 pairs (range_g pairs, 2 range_g CTAs)
   int tiles_per_split;  // in units of kEncBN latents
   int n_tiles;          // ceil(H / kEncBN)
-  int act;              // 0 none, 1 relu; dense epilogue only: 2 = step operand, out = (z >= step_thr) ? step_scale[col] : 0
+  int act;              // 0 none, 1 relu; dense epilogue only: 2 = step operand, out = (z >= step_thr) ? step_scale[col] : 0,
+                        // 3 = ReLU backward, out = (acc + gate_add) * (gate > 0) (streamed-operand kernel, no bias)
   int mode;             // epilogue bound: 0 bisection only, 1/2/3 class maxima, 4 prior (see .cu)
   int cap;              // entries per survivor buffer
   const float* bias;    // [H]
@@ -85,6 +86,10 @@ struct EncodeLaunch {
   const int* step_level_start;        // [step_n_levels + 1] device, multiples of 128
   int step_n_levels;
   unsigned long long* step_level_count;   // [step_n_levels] += active (row, latent) pairs per level
+  // act == 3 (t_sae backward: gz = (g T + g_h) * 1[h > 0] straight from the accumulator of g T)
+  const float* gate;      // [B, H] the forward's ReLU output h
+  const float* gate_add;  // [B, H] d loss / d h, or null
+  float* gate_colsum;     // [H] += column sums of the output (the bias gradient), or null
   int debug_mode;       // 0 normal; timing experiments: 1 no survivors, 2 no TMEM drain
   float* debug_z;       // optional dense [B, H] dump of the accumulator (+bias, act); diagnostics only
 };
@@ -126,8 +131,10 @@ const char* encode_dense_tc_launch(const uint16_t* x_bf16, const uint16_t* const
 // stream through the ring, every product lands in the same TMEM accumulator, the output is written once
 // (p.bias / p.act applied; p.n_tiles as for encode_dense_tc_launch; a range schedule over num_sms / 2 CTA pairs)
 // n_parts = 1: only the bf16 product x_parts[0] w_parts[0] (fast mode) on the same schedule
+// n_w_parts = 1 with n_parts = 3: the three x parts against ONE W part (exact when W is bf16-representable, e.g. ternary)
 const char* encode_dense_split_launch(const uint16_t* const* x_parts, const uint16_t* const* w_parts, int n_parts, EncodeLaunch p,
-                                      float* out_f32, uint16_t* out_hi, uint16_t* out_lo, int num_sms, cudaStream_t stream);
+                                      float* out_f32, uint16_t* out_hi, uint16_t* out_lo, int num_sms, cudaStream_t stream,
+                                      int n_w_parts = 0);
 // src -> three bf16 parts with hi + mid + lo == src exactly (24 mantissa bits); mid / lo may be null
 const char* split_bf16x3_launch(const float* src, uint16_t* hi, uint16_t* mid, uint16_t* lo, size_t n, cudaStream_t stream);
 
@@ -139,6 +146,13 @@ size_t dense_decode_workspace_bytes(int B, int K, int N, int num_sms);
 const char* dense_decode_launch(const uint16_t* a_hi, const uint16_t* a_lo, int lda, const uint16_t* b_t, int ldb, int B,
                                 int K, int N, const float* bias, const float* prev, float* out, void* workspace,
                                 int num_sms, cudaStream_t stream);
+
+// wgrad_sm100.cu: c[M, N] = sum_k A(k, m) B(k, n) over K rows (the batch), bf16 parts, fp32 accumulation.
+// b_parts: row-major [K, N]; a_parts: row-major [K, M], or [M, K] when a_kmajor. n_parts = 1 (one product) or 3 (the six
+// products of three-part splits above 2^-24, one accumulator). N and the row pitch of A multiples of 8; c [M, N] fp32,
+// overwritten.
+const char* wgrad_launch(const uint16_t* const* a_parts, const uint16_t* const* b_parts, int n_parts, int M, int N, int K,
+                         bool a_kmajor, float* c, int num_sms, cudaStream_t stream);
 
 // select_topk.cu
 struct SelectLaunch {
@@ -244,8 +258,9 @@ const char* residual_update_launch(const float* r, const float* recon, size_t n,
 // src -> hi = bf16(src), lo = bf16(src - hi) (lo may be null)
 const char* split_bf16_launch(const float* src, uint16_t* hi, uint16_t* lo, size_t n, cudaStream_t stream);
 // t_sae decoder.weight [D, H] -> sign(w) * (|w| >= threshold): bf16 [D, H] and/or int8 rows [H, D]
+// t_t_bf16: the same T transposed, bf16 [H, D] (K-major B operand of the t_sae backward's g T); may be null
 const char* pack_ternary_launch(const float* w, int D, int H, float threshold, uint16_t* t_bf16, int8_t* t_rows,
-                                cudaStream_t stream);
+                                cudaStream_t stream, uint16_t* t_t_bf16 = nullptr);
 
 // decode.cu
 // idx_offset: the dictionary holds latents [idx_offset, idx_offset + H); other entries are skipped

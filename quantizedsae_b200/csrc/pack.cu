@@ -176,9 +176,10 @@ __global__ void split_bf16x3_kernel(const float* __restrict__ src, uint16_t* __r
 
 // STEWeights hard weights (sae/ternary.py:46-49): sign(w) * (|w| >= threshold) in {-1, 0, +1}.
 // 32 x 32 tiles of w [D, H]: bf16 in place ([D, H], K-major B operand of the decoder GEMM) and
-// transposed int8 rows ([H, D], gather layout of the sparse decoder).
+// transposed int8 rows ([H, D], gather layout of the sparse decoder) and / or transposed bf16 ([H, D], K-major B
+// operand of the t_sae backward's g T).
 __global__ void pack_ternary_kernel(const float* __restrict__ w, int D, int H, float threshold,
-                                    uint16_t* __restrict__ t_bf16, int8_t* __restrict__ t_rows) {
+                                    uint16_t* __restrict__ t_bf16, int8_t* __restrict__ t_rows, uint16_t* __restrict__ t_t_bf16) {
   __shared__ int8_t tile[32][33];
   const int h0 = blockIdx.x * 32, d0 = blockIdx.y * 32;
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
@@ -192,11 +193,15 @@ __global__ void pack_ternary_kernel(const float* __restrict__ w, int D, int H, f
     }
     tile[i][threadIdx.x] = t;
   }
-  if (t_rows == nullptr) return;
+  if (t_rows == nullptr && t_t_bf16 == nullptr) return;
   __syncthreads();
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
     const int h = h0 + i, d = d0 + threadIdx.x;
-    if (h < H && d < D) t_rows[static_cast<size_t>(h) * D + d] = tile[threadIdx.x][i];
+    if (h < H && d < D) {
+      const int8_t t = tile[threadIdx.x][i];
+      if (t_rows != nullptr) t_rows[static_cast<size_t>(h) * D + d] = t;
+      if (t_t_bf16 != nullptr) t_t_bf16[static_cast<size_t>(h) * D + d] = t == 0 ? 0x0000u : (t > 0 ? 0x3F80u : 0xBF80u);
+    }
   }
 }
 
@@ -307,9 +312,9 @@ const char* split_bf16_launch(const float* src, uint16_t* hi, uint16_t* lo, size
 }
 
 const char* pack_ternary_launch(const float* w, int D, int H, float threshold, uint16_t* t_bf16, int8_t* t_rows,
-                                cudaStream_t stream) {
+                                cudaStream_t stream, uint16_t* t_t_bf16) {
   dim3 grid((H + 31) / 32, (D + 31) / 32), block(32, 8);
-  pack_ternary_kernel<<<grid, block, 0, stream>>>(w, D, H, threshold, t_bf16, t_rows);
+  pack_ternary_kernel<<<grid, block, 0, stream>>>(w, D, H, threshold, t_bf16, t_rows, t_t_bf16);
   return cuda_err(cudaGetLastError());
 }
 

@@ -270,10 +270,28 @@ __device__ __forceinline__ uint64_t umma_desc_kmajor_sw128(uint32_t smem_addr) {
   d |= static_cast<uint64_t>(2) << 61;
   return d;
 }
+// MN-major, 128-byte swizzled operand tile: each K index is one row of 64 MN-consecutive bf16 (128 B), 8-row atoms
+// of 1024 B (the layout a {64 x rows} TMA box of a row-major [K, MN] tensor lands in with SWIZZLE_128B).
+//   [16,30) LBO >> 4: byte distance between consecutive 64-element MN columns of atoms |
+//   [32,46) SBO >> 4: byte distance between consecutive groups of 8 K rows (1024 for a contiguous column)
+// A K step of 16 rows advances the start address by 2 SBO.
+__device__ __forceinline__ uint64_t umma_desc_mnmajor_sw128(uint32_t smem_addr, uint32_t lbo_bytes) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr & 0x3FFFF) >> 4);
+  d |= static_cast<uint64_t>((lbo_bytes >> 4) & 0x3FFF) << 16;
+  d |= static_cast<uint64_t>(1024 >> 4) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(2) << 61;
+  return d;
+}
 // kind::f16 instruction descriptor: D=f32, A=B=bf16, both K-major, dense
 __host__ __device__ constexpr uint32_t umma_idesc_bf16_f32(int M, int N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(N >> 3) << 17) |
          (static_cast<uint32_t>(M >> 4) << 24);
+}
+// the same with the transpose bits: bit 15 = A is MN-major, bit 16 = B is MN-major
+__host__ __device__ constexpr uint32_t umma_idesc_bf16_f32_major(int M, int N, bool a_mn, bool b_mn) {
+  return umma_idesc_bf16_f32(M, N) | (a_mn ? (1u << 15) : 0u) | (b_mn ? (1u << 16) : 0u);
 }
 
 // ---------------------------------------------------------------- cluster

@@ -1263,6 +1263,151 @@ int qsae_tsae_forward(const float* x_f32, const uint16_t* w_hi, const uint16_t* 
                                                            ws + tp.dec_off, num_sms(), st));
 }
 
+// ---- t_sae backward (training.py: _TernarySAEFn)
+int qsae_pack_ternary_t(const float* w, int D, int H, float threshold, uint16_t* t_t_bf16, void* stream) {
+  if (!w || !t_t_bf16) return fail(QSAE_ERR_INVALID_ARGUMENT, "pack_ternary_t: null pointer");
+  if (D <= 0 || H <= 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "pack_ternary_t: bad shape");
+  return launch_status("pack_ternary_t", pack_ternary_launch(w, D, H, threshold, nullptr, nullptr, S(stream), t_t_bf16));
+}
+
+int qsae_wgrad(const uint16_t* const* a_parts, const uint16_t* const* b_parts, int n_parts, int M, int N, int K, int a_kmajor,
+               float* c, void* stream) {
+  if (!a_parts || !b_parts || !c) return fail(QSAE_ERR_INVALID_ARGUMENT, "wgrad: null pointer");
+  if (n_parts != 1 && n_parts != 3) return fail(QSAE_ERR_INVALID_ARGUMENT, "wgrad: n_parts must be 1 or 3, got %d", n_parts);
+  if (M <= 0 || N <= 0 || K <= 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "wgrad: bad shape M=%d N=%d K=%d", M, N, K);
+  if ((N % 8) != 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "wgrad: N must be a multiple of 8, got %d", N);
+  if (a_kmajor ? (K % 8) != 0 : (M % 8) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "wgrad: %s must be a multiple of 8 (row pitch of A), got %d", a_kmajor ? "K" : "M",
+                a_kmajor ? K : M);
+  uintptr_t bits = reinterpret_cast<uintptr_t>(c);
+  for (int i = 0; i < n_parts; ++i) {
+    if (!a_parts[i] || !b_parts[i]) return fail(QSAE_ERR_INVALID_ARGUMENT, "wgrad: null operand part");
+    bits |= reinterpret_cast<uintptr_t>(a_parts[i]) | reinterpret_cast<uintptr_t>(b_parts[i]);
+  }
+  if (bits & 15) return fail(QSAE_ERR_INVALID_ARGUMENT, "wgrad: operands and output must be 16-byte aligned");
+  return launch_status("wgrad", wgrad_launch(a_parts, b_parts, n_parts, M, N, K, a_kmajor != 0, c, num_sms(), S(stream)));
+}
+
+namespace {
+// workspace of the backward: bf16 parts of g, x [B, D]; the bf16 parts of gz, h [B, H] and (exact mode) fp32 gz
+struct TsaeBwdPlan { size_t bd, bh, g_off, x_off, gz_off, gzp_off, hp_off, total; };
+int plan_tsae_backward(int B, int H, int D, int exact, TsaeBwdPlan* bp) {
+  TsaePlan tp;
+  int rc = plan_tsae(B > 0 ? B : 1, H, D, exact, &tp);   // the forward's shape limits
+  if (rc != QSAE_OK) return rc;
+  const int np = exact ? 3 : 1;
+  bp->bd = align_up(static_cast<size_t>(B) * D * 2, 1024);
+  bp->bh = align_up(static_cast<size_t>(B) * H * 2, 1024);
+  bp->g_off = 0;
+  bp->x_off = bp->g_off + np * bp->bd;
+  bp->gz_off = bp->x_off + np * bp->bd;
+  bp->gzp_off = bp->gz_off + (exact ? align_up(static_cast<size_t>(B) * H * 4, 1024) : 0);   // fp32 gz: exact only
+  bp->hp_off = bp->gzp_off + np * bp->bh;
+  bp->total = bp->hp_off + np * bp->bh;
+  return QSAE_OK;
+}
+}  // namespace
+
+int qsae_tsae_backward_workspace_bytes(int B, int H, int D, int exact, size_t* bytes) {
+  if (!bytes) return fail(QSAE_ERR_INVALID_ARGUMENT, "workspace query: null pointer");
+  if (B < 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "tsae_backward: negative batch");
+  TsaeBwdPlan bp;
+  int rc = plan_tsae_backward(B, H, D, exact, &bp);
+  if (rc != QSAE_OK) return rc;
+  *bytes = bp.total;
+  return QSAE_OK;
+}
+
+int qsae_tsae_backward(const float* x, const float* h, const float* g_recon, const float* g_h, const uint16_t* t_t_bf16,
+                       const float* mask, const uint16_t* w_hi, const uint16_t* w_mid, const uint16_t* w_lo, int B, int H, int D,
+                       int exact, float* grad_w_enc, float* grad_b_enc, float* grad_w_dec, float* grad_x, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  if (B < 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "tsae_backward: negative batch");
+  TsaeBwdPlan bp;
+  int rc = plan_tsae_backward(B, H, D, exact, &bp);
+  if (rc != QSAE_OK) return rc;
+  if (!grad_w_enc || !grad_b_enc || !grad_w_dec) return fail(QSAE_ERR_INVALID_ARGUMENT, "tsae_backward: null gradient pointer");
+  cudaStream_t st = S(stream);
+  const size_t nbd = static_cast<size_t>(B) * D, nbh = static_cast<size_t>(B) * H, nhd = static_cast<size_t>(H) * D;
+  if (B == 0) {   // nothing to contract: zero gradients
+    cudaError_t e = cudaMemsetAsync(grad_w_enc, 0, nhd * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_b_enc, 0, static_cast<size_t>(H) * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_w_dec, 0, nhd * 4, st);
+    return e == cudaSuccess ? QSAE_OK : fail(QSAE_ERR_CUDA, "tsae_backward: %s", cudaGetErrorString(e));
+  }
+  if (!x || !h || !g_recon || !t_t_bf16 || !workspace) return fail(QSAE_ERR_INVALID_ARGUMENT, "tsae_backward: null pointer");
+  if (grad_x && (!w_hi || (exact && (!w_mid || !w_lo))))
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "tsae_backward: grad_x needs the parts of W_enc (three in exact mode)");
+  if (workspace_bytes < bp.total)
+    return fail(QSAE_ERR_WORKSPACE_TOO_SMALL, "tsae_backward: workspace %zu < %zu bytes", workspace_bytes, bp.total);
+  const uintptr_t align16 = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(h) | reinterpret_cast<uintptr_t>(g_recon) |
+                            reinterpret_cast<uintptr_t>(g_h) | reinterpret_cast<uintptr_t>(t_t_bf16) |
+                            reinterpret_cast<uintptr_t>(grad_w_enc) | reinterpret_cast<uintptr_t>(grad_w_dec) |
+                            reinterpret_cast<uintptr_t>(grad_x) | reinterpret_cast<uintptr_t>(w_hi) |
+                            reinterpret_cast<uintptr_t>(w_mid) | reinterpret_cast<uintptr_t>(w_lo);
+  if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0 || (align16 & 15) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "tsae_backward: workspace must be 1024-byte and tensors 16-byte aligned");
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  const int np = exact ? 3 : 1;
+  uint16_t *gp[3], *xp[3], *gzp[3], *hp[3];
+  for (int i = 0; i < 3; ++i) {
+    const int j = i < np ? i : 0;
+    gp[i] = reinterpret_cast<uint16_t*>(ws + bp.g_off + j * bp.bd);
+    xp[i] = reinterpret_cast<uint16_t*>(ws + bp.x_off + j * bp.bd);
+    gzp[i] = reinterpret_cast<uint16_t*>(ws + bp.gzp_off + j * bp.bh);
+    hp[i] = reinterpret_cast<uint16_t*>(ws + bp.hp_off + j * bp.bh);
+  }
+  float* gz = reinterpret_cast<float*>(ws + bp.gz_off);
+  auto parts = [&](const char* what, const float* src, uint16_t* const* dst, size_t n) {
+    return launch_status(what, exact ? split_bf16x3_launch(src, dst[0], dst[1], dst[2], n, st) : cast_bf16_launch(src, dst[0], n, st));
+  };
+  // gz = (g T + g_h) * 1[h > 0]: the dense encoder over g (M = B, K = D) against T^T [H, D] with the ReLU-backward
+  // epilogue, which also sums gz per column into grad_b_enc. Fast mode writes only bf16(gz), the operand of the
+  // weight GEMMs; exact mode writes fp32 gz, the source of its three-part split.
+  rc = parts("split g", g_recon, gp, nbd);
+  if (rc != QSAE_OK) return rc;
+  // grad b_enc = sum_b gz: column sums from the same epilogue (atomics)
+  cudaError_t e = cudaMemsetAsync(grad_b_enc, 0, static_cast<size_t>(H) * 4, st);
+  if (e != cudaSuccess) return fail(QSAE_ERR_CUDA, "tsae_backward: %s", cudaGetErrorString(e));
+  EncodeLaunch el;
+  memset(&el, 0, sizeof(el));
+  el.B = B; el.H = H; el.D = D; el.act = 3; el.bias = nullptr; el.gate = h; el.gate_add = g_h; el.gate_colsum = grad_b_enc;
+  el.n_tiles = (H + kEncBN - 1) / kEncBN;
+  el.n_splits = 1;
+  el.tiles_per_split = el.n_tiles;
+  const uint16_t* wt[1] = {t_t_bf16};
+  const uint16_t* gpc[3] = {gp[0], gp[1], gp[2]};
+  rc = launch_status("encode kernel (dense, ReLU backward)",
+                     encode_dense_split_launch(gpc, wt, np, el, exact ? gz : nullptr, exact ? nullptr : gzp[0], nullptr,
+                                               num_sms(), st, 1));
+  if (rc != QSAE_OK) return rc;
+  if (exact) {
+    rc = launch_status("split gz", split_bf16x3_launch(gz, gzp[0], gzp[1], gzp[2], nbh, st));
+    if (rc != QSAE_OK) return rc;
+  }
+  rc = parts("split h", h, hp, nbh);
+  if (rc != QSAE_OK) return rc;
+  rc = parts("split x", x, xp, nbd);
+  if (rc != QSAE_OK) return rc;
+  const uint16_t* gzc[3] = {gzp[0], gzp[1], gzp[2]};
+  const uint16_t* xc[3] = {xp[0], xp[1], xp[2]};
+  const uint16_t* hc[3] = {hp[0], hp[1], hp[2]};
+  // grad W_enc [H, D] = gz^T x;  grad W_dec [D, H] = g^T h (already in decoder.weight's layout), then * mask
+  rc = launch_status("wgrad (encoder)", wgrad_launch(gzc, xc, np, H, D, B, false, grad_w_enc, num_sms(), st));
+  if (rc != QSAE_OK) return rc;
+  rc = launch_status("wgrad (decoder)", wgrad_launch(gpc, hc, np, D, H, B, false, grad_w_dec, num_sms(), st));
+  if (rc != QSAE_OK) return rc;
+  if (mask) {
+    rc = launch_status("mul_inplace", mul_inplace_launch(grad_w_dec, mask, nhd, st));
+    if (rc != QSAE_OK) return rc;
+  }
+  if (grad_x) {   // grad x [B, D] = gz W_enc: gz is the K-major A (K = H), W_enc [H, D] the MN-major B
+    const uint16_t* wc[3] = {w_hi, exact ? w_mid : w_hi, exact ? w_lo : w_hi};
+    rc = launch_status("wgrad (input)", wgrad_launch(gzc, wc, np, B, D, H, true, grad_x, num_sms(), st));
+  }
+  return rc;
+}
+
 // ---- q_sae dense fallback: any activity level (an untrained model is ~50 % active), level sums as GEMMs
 int qsae_unpack_matryoshka_t(const uint32_t* packed, int H, int D, uint16_t* t_bf16, void* stream) {
   if (!packed || !t_bf16 || H <= 0 || D <= 0 || (D % 16) != 0)

@@ -1,0 +1,282 @@
+// Weight-gradient GEMM for sm_100a:  C[M, N] = sum_k A(k, m) B(k, n),  bf16 operands, fp32 accumulation in TMEM.
+//
+// The backward of a dense layer contracts over the batch (t_sae, training.py): grad encoder.0.weight = gz^T x [H, D]
+// and grad decoder.weight = g^T h [D, H]. Both operands are the row-major batch tensors as they are, A = [K, M] and
+// B = [K, N]: MN-major UMMA operands, so no [B, H] tensor is ever transposed. A TMA box of 64 columns x 64 batch rows
+// with the 128-byte swizzle lands as one MN-major column of atoms (64 rows of 128 B); a stage holds two such columns
+// of A (128 rows of the output) and four of B (256 columns). The batch is K and may have any length: TMA zero-fills
+// the tail rows, and columns past M or N.
+//
+// A may instead be K-major, [M, K] row-major (x.grad = gz W_enc contracts over H, and gz is [B, H]).
+//
+// Products: a list of (A part, B part) pairs contracted into the SAME accumulator. Fast mode is one bf16 product;
+// exact mode splits both fp32 operands into three bf16 parts and keeps the six partial products above 2^-24,
+// smallest first (the order of encode_dense_split_kernel).
+//
+// Persistent CTAs over 128 x 256 output tiles (the dimension with fewer tiles runs fastest, so the CTAs working at
+// the same time share the slice of the large operand in L2), a 4-stage ring of 48 KiB stages, and two TMEM
+// accumulators: the epilogue drains tile t while the MMAs of tile t + 1 run.
+#include <cuda.h>
+#include <cuda_runtime.h>
+#include <stdint.h>
+#include <stdio.h>
+#include <stdlib.h>
+
+#include "kernels.h"
+#include "ptx_sm100.cuh"
+#include "tmap_cache.cuh"
+
+namespace qsae {
+
+namespace {
+
+constexpr int BM = 128, BN = 256, BK = 64, UMMA_K = 16;
+constexpr int kABytes = BM * BK * 2;        // 16 KiB: two MN columns of 64 rows x 128 B (or 128 K-major rows)
+constexpr int kBBytes = BN * BK * 2;        // 32 KiB: four MN columns
+constexpr int kColBytes = BK * 128;         // one MN column of atoms: 64 K rows x 128 B
+constexpr int kStageBytes = kABytes + kBBytes;
+constexpr int kStages = 4;
+constexpr int kThreads = 256;               // warps: 0 TMA, 1 MMA, 2 TMEM alloc, 3 idle, 4-7 epilogue
+constexpr int kTmemCols = 2 * BN;           // two accumulators
+constexpr int kBarOff = kStages * kStageBytes;
+constexpr int kSmem = kBarOff + 8 * (2 * kStages + 4) + 16;
+static_assert(kSmem <= 227 * 1024, "wgrad_kernel: shared memory budget");
+
+struct WgradParams {
+  int M, N;
+  int m_tiles, n_tiles;
+  int k_chunks;          // ceil(K / 64)
+  int n_prod;
+  uint32_t prods;        // product i: A part (prods >> 4i + 2) & 3, B part (prods >> 4i) & 3
+  int a_kmajor;
+  int m_fast;            // tile u -> (u % m_tiles, u / m_tiles), else (u / n_tiles, u % n_tiles)
+  float* c;              // [M, N] row-major
+};
+
+template <bool A_KMAJOR>
+__global__ void __launch_bounds__(kThreads, 1)
+wgrad_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ CUtensorMap ta1,
+             const __grid_constant__ CUtensorMap ta2, const __grid_constant__ CUtensorMap tb0,
+             const __grid_constant__ CUtensorMap tb1, const __grid_constant__ CUtensorMap tb2, WgradParams p) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kBarOff);
+  uint64_t* full = bars;
+  uint64_t* empty = bars + kStages;
+  uint64_t* tmem_full = bars + 2 * kStages;
+  uint64_t* tmem_empty = tmem_full + 2;
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 4);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int n_units = p.m_tiles * p.n_tiles;
+  const int k_iters = p.n_prod * p.k_chunks;
+  auto tile_of = [&](int u, int* m0, int* n0) {
+    const int mt = p.m_fast ? u % p.m_tiles : u / p.n_tiles;
+    const int nt = p.m_fast ? u / p.m_tiles : u % p.n_tiles;
+    *m0 = mt * BM;
+    *n0 = nt * BN;
+  };
+
+  if (threadIdx.x == 0) {
+    if ((smem_u32(smem) & 1023u) != 0u) {
+      printf("qsae: dynamic shared memory is not 1024-byte aligned\n");
+      __trap();
+    }
+    for (int s = 0; s < kStages; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], 1);
+    }
+    for (int a = 0; a < 2; ++a) {
+      mbar_init(&tmem_full[a], 1);
+      mbar_init(&tmem_empty[a], 4);
+    }
+    fence_mbar_init();
+    fence_proxy_async_smem();
+  }
+  if (warp == 2) tmem_alloc<kTmemCols>(tmem_ptr);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_ptr;
+
+  if (warp == 0) {
+    if (lane == 0) {
+      tma_prefetch_desc(&ta0);
+      tma_prefetch_desc(&tb0);
+      int stage = 0;
+      uint32_t phase = 0;
+      for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
+        int m0, n0;
+        tile_of(u, &m0, &n0);
+#pragma unroll 1
+        for (int it = 0; it < k_iters; ++it) {
+          const int pi = it / p.k_chunks, kc = it - pi * p.k_chunks;
+          const uint32_t pr = p.prods >> (4 * pi);
+          const int ai = (pr >> 2) & 3, bi = pr & 3;
+          const CUtensorMap* ta = ai == 0 ? &ta0 : (ai == 1 ? &ta1 : &ta2);
+          const CUtensorMap* tb = bi == 0 ? &tb0 : (bi == 1 ? &tb1 : &tb2);
+          mbar_wait(&empty[stage], phase ^ 1u);
+          uint8_t* st = smem + stage * kStageBytes;
+          mbar_arrive_expect_tx(&full[stage], kStageBytes);
+          const int k0 = kc * BK;
+          if constexpr (A_KMAJOR) {
+            tma_load_2d(st, ta, &full[stage], k0, m0, kPolicyEvictNormal);
+          } else {
+#pragma unroll
+            for (int c = 0; c < BM / 64; ++c) tma_load_2d(st + c * kColBytes, ta, &full[stage], m0 + 64 * c, k0, kPolicyEvictNormal);
+          }
+#pragma unroll
+          for (int c = 0; c < BN / 64; ++c)
+            tma_load_2d(st + kABytes + c * kColBytes, tb, &full[stage], n0 + 64 * c, k0, kPolicyEvictNormal);
+          if (++stage == kStages) { stage = 0; phase ^= 1u; }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      constexpr uint32_t idesc = umma_idesc_bf16_f32_major(BM, BN, !A_KMAJOR, true);
+      int stage = 0;
+      uint32_t phase = 0;
+      int t = 0;
+      for (int u = blockIdx.x; u < n_units; u += gridDim.x, ++t) {
+        const int acc = t & 1;
+        mbar_wait(&tmem_empty[acc], ((t >> 1) & 1) ^ 1u);
+        tc_fence_after();
+        const uint32_t d_tmem = tmem_base + acc * BN;
+#pragma unroll 1
+        for (int it = 0; it < k_iters; ++it) {
+          mbar_wait(&full[stage], phase);
+          tc_fence_after();
+          const uint32_t st = smem_u32(smem + stage * kStageBytes);
+          const uint64_t a_desc = A_KMAJOR ? umma_desc_kmajor_sw128(st) : umma_desc_mnmajor_sw128(st, kColBytes);
+          const uint64_t b_desc = umma_desc_mnmajor_sw128(st + kABytes, kColBytes);
+#pragma unroll
+          for (int ks = 0; ks < BK / UMMA_K; ++ks) {
+            // K-major: 16 elements = 32 B along the row; MN-major: 16 K rows = two 1024-byte atoms
+            const uint64_t a_step = A_KMAJOR ? 2u * ks : static_cast<uint64_t>(ks) * (2048 >> 4);
+            umma_f16_ss(d_tmem, a_desc + a_step, b_desc + static_cast<uint64_t>(ks) * (2048 >> 4), idesc,
+                        (it | ks) != 0 ? 1u : 0u);
+          }
+          umma_commit(&empty[stage]);
+          if (it == k_iters - 1) umma_commit(&tmem_full[acc]);
+          if (++stage == kStages) { stage = 0; phase ^= 1u; }
+        }
+      }
+    }
+  } else if (warp >= 4) {
+    const int quad = warp - 4;   // TMEM lanes 32 quad .. +31 (warp_id % 4)
+    const uint32_t lane_taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
+    int t = 0;
+    for (int u = blockIdx.x; u < n_units; u += gridDim.x, ++t) {
+      int m0, n0;
+      tile_of(u, &m0, &n0);
+      const int acc = t & 1;
+      mbar_wait(&tmem_full[acc], (t >> 1) & 1);
+      tc_fence_after();
+      const int row = m0 + quad * 32 + lane;
+      float* dst = p.c + static_cast<size_t>(row) * p.N;
+#pragma unroll 1
+      for (int c0 = 0; c0 < BN; c0 += 32) {
+        if (n0 + c0 >= p.N) break;   // warp-uniform
+        uint32_t r[32];
+        tmem_ld_32x32b_x32(lane_taddr + acc * BN + c0, r);
+        tmem_ld_wait();
+        if (row < p.M) {
+#pragma unroll
+          for (int j = 0; j < 32; j += 4)
+            if (n0 + c0 + j < p.N)   // N % 8 == 0
+              *reinterpret_cast<uint4*>(dst + n0 + c0 + j) = make_uint4(r[j], r[j + 1], r[j + 2], r[j + 3]);
+        }
+      }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&tmem_empty[acc]);
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  if (warp == 2) tmem_dealloc<kTmemCols>(tmem_base);
+}
+
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+// row-major bf16 [rows, cols] with a {64 x box_rows} box, 128-byte swizzle
+bool make_tmap(CUtensorMap* map, const void* base, int rows, int cols, int box_rows) {
+  static EncodeTiledFn enc = nullptr;
+  if (!enc) {
+    void* ptr = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) != cudaSuccess ||
+        q != cudaDriverEntryPointSuccess)
+      return false;
+    enc = reinterpret_cast<EncodeTiledFn>(ptr);
+  }
+  const TmapKey key{base, static_cast<unsigned long long>(rows), static_cast<unsigned long long>(cols),
+                    static_cast<unsigned long long>(cols) * 2, static_cast<unsigned int>(BK), static_cast<unsigned int>(box_rows),
+                    static_cast<int>(CU_TENSOR_MAP_DATA_TYPE_BFLOAT16), static_cast<int>(CU_TENSOR_MAP_SWIZZLE_128B),
+                    tmap_current_device()};
+  EncodeTiledFn fn = enc;
+  return tmap_cache().get(key, map, [&](CUtensorMap* m) {
+    cuuint64_t dims[2] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(rows)};
+    cuuint64_t strides[1] = {static_cast<cuuint64_t>(cols) * 2};
+    cuuint32_t box[2] = {BK, static_cast<cuuint32_t>(box_rows)};
+    cuuint32_t estr[2] = {1, 1};
+    return fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  });
+}
+
+template <bool A_KMAJOR>
+cudaError_t launch(const CUtensorMap* ta, const CUtensorMap* tb, const WgradParams& p, int grid, cudaStream_t stream) {
+  static bool attr = false;
+  if (!attr) {
+    cudaError_t e = cudaFuncSetAttribute(wgrad_kernel<A_KMAJOR>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+    if (e != cudaSuccess) return e;
+    attr = true;
+  }
+  wgrad_kernel<A_KMAJOR><<<grid, kThreads, kSmem, stream>>>(ta[0], ta[1], ta[2], tb[0], tb[1], tb[2], p);
+  return cudaGetLastError();
+}
+
+}  // namespace
+
+const char* wgrad_launch(const uint16_t* const* a_parts, const uint16_t* const* b_parts, int n_parts, int M, int N, int K,
+                         bool a_kmajor, float* c, int num_sms, cudaStream_t stream) {
+  if (n_parts != 1 && n_parts != 3) return "wgrad: 1 or 3 parts per operand";
+  if (M <= 0 || N <= 0 || K <= 0 || (N % 8) != 0) return "wgrad: M, N, K must be positive and N a multiple of 8";
+  if (a_kmajor ? (K % 8) != 0 : (M % 8) != 0) return "wgrad: the row pitch of A (M, or K when A is K-major) must be a multiple of 8";
+  CUtensorMap ta[3], tb[3];
+  for (int i = 0; i < 3; ++i) {
+    const int j = i < n_parts ? i : 0;
+    const bool ok_a = a_kmajor ? make_tmap(&ta[i], a_parts[j], M, K, BM) : make_tmap(&ta[i], a_parts[j], K, M, BK);
+    if (!ok_a) return "cuTensorMapEncodeTiled(wgrad A) failed";
+    if (!make_tmap(&tb[i], b_parts[j], K, N, BK)) return "cuTensorMapEncodeTiled(wgrad B) failed";
+  }
+  WgradParams p;
+  p.M = M; p.N = N;
+  p.m_tiles = (M + BM - 1) / BM;
+  p.n_tiles = (N + BN - 1) / BN;
+  p.k_chunks = (K + BK - 1) / BK;
+  if (n_parts == 1) {
+    p.n_prod = 1;
+    p.prods = 0u;
+  } else {
+    // (A part, B part), smallest first: lo hi, mid mid, hi lo, mid hi, hi mid, hi hi
+    const uint32_t pairs[6][2] = {{2, 0}, {1, 1}, {0, 2}, {1, 0}, {0, 1}, {0, 0}};
+    p.n_prod = 6;
+    p.prods = 0u;
+    for (int i = 0; i < 6; ++i) p.prods |= ((pairs[i][0] << 2) | pairs[i][1]) << (4 * i);
+  }
+  p.a_kmajor = a_kmajor ? 1 : 0;
+  p.m_fast = p.m_tiles <= p.n_tiles ? 1 : 0;
+  p.c = c;
+  const int units = p.m_tiles * p.n_tiles;
+  const int grid = units < num_sms ? units : num_sms;
+  const cudaError_t e = a_kmajor ? launch<true>(ta, tb, p, grid, stream) : launch<false>(ta, tb, p, grid, stream);
+  return cuda_err(e);
+}
+
+}  // namespace qsae

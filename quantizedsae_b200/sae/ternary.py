@@ -70,6 +70,13 @@ class STEWeights(nn.Module):
         from .. import training
         training.rigl_mask_grad(self)
 
+    def _ternary_t(self):
+        """T^T as bf16 [H, D] for the current weights (B operand of the backward's g T, training.py)."""
+        if not self.weight.is_cuda:
+            raise RuntimeError("STEWeights runs only on CUDA (no CPU fallback)")
+        return self._prep.get("ternary_t", param_key(self.weight) + (self.threshold,),
+                              lambda: _lib.pack_ternary_t(self.weight.detach().contiguous(), self.threshold))
+
     def hard_weights(self) -> torch.Tensor:
         """sign(W) * (|W| >= threshold) as float32 [D, H] (sae/ternary.py:46-49)."""
         return self._ternary()[0].float()
@@ -97,6 +104,10 @@ class TernarySparseAutoencoder(nn.Module):
         self.input_dim = input_dim
         self.hidden_dim = hidden_dim
         self.exact = True
+        # True: forward builds one autograd node (training.py, _TernarySAEFn) whenever grad mode is on, so the
+        # trainer's loss.backward() fills encoder.0.weight / .bias, decoder.weight (and x) .grad and
+        # decoder.output_grad
+        self.autograd = False
         self._prep = PreparedCache()
 
 
@@ -141,13 +152,19 @@ class TernarySparseAutoencoder(nn.Module):
         latents = self.encode_topk(x)
         return latents, self.decoder.decode_sparse(latents)
 
-    def forward(self, x):
-        x = require_cuda_input(x, self)
+    def _enc_parts(self):
+        """The encoder weight as the forward contracts it: split_bf16x3 parts (exact) or (bf16(W),)."""
+        return self._w_parts() if self.exact else (self._w_bf16(),)
+
+    def _forward_dense(self, x):
         lin = self.encoder[0]
-        t_bf16 = self.decoder._ternary()[0]
-        if self.exact:
-            h, recon = _lib.tsae_forward(x, self._w_parts(), lin.bias.detach(), t_bf16, True)
-        else:
-            h, recon = _lib.tsae_forward(x, (self._w_bf16(),), lin.bias.detach(), t_bf16, False)
+        return _lib.tsae_forward(x, self._enc_parts(), lin.bias.detach(), self.decoder._ternary()[0], self.exact)
+
+    def forward(self, x):
+        if self.autograd and torch.is_grad_enabled():
+            from .. import training
+            return training.tsae_forward(self, x)
+        x = require_cuda_input(x, self)
+        h, recon = self._forward_dense(x)
         self.decoder.input_activations = h        # the reference's forward hook (sae/ternary.py:21-22)
         return h, recon

@@ -16,8 +16,21 @@ q_sae   `QuantizedMatryoshkaDecoder.ste_backward(grad_levels)`: what loss.backwa
         False), from the active lists of `QuantizedMatryoshkaSAE.forward_active`; `apply_secant_grad()` (:145-190).
         `qsae_trainer_decoder_grads` strings them together under the trainer's loss (training/trainer.py:88-113).
         The encoder side of q_sae's backward is dense (the STE passes a gradient to every latent, :99) and is not
-        built: it is two plain dense GEMMs with no quantisation-specific structure.
-t_sae   `STEWeights.init_mask / update_mask / mask_grad` (sae/ternary.py:27-90): exact RigL drop / grow by radix
+        built: its STE and sparsity-term semantics are not pinned here.
+t_sae   `tsae_forward(model, x)` (what `TernarySparseAutoencoder.forward` runs when `model.autograd = True` and grad
+        mode is on): the same (h, recon) as the plain forward, behind ONE autograd node, so the reference trainer's
+        loop (training/trainer.py:152-173) runs as written: loss.backward() fills .grad of encoder.0.weight /
+        encoder.0.bias / decoder.weight (and of x when it requires grad) and sets decoder.output_grad (the
+        reference's backward hook, sae/ternary.py:24-25). With g = d loss / d recon and g_h = d loss / d h:
+            gz = (g T + g_h) * 1[h > 0]: the dense encoder kernel over g against T^T with a ReLU-backward epilogue
+                 (g T never reaches memory);
+            grad W_enc = gz^T x, grad W_dec = mask * (g^T h) (the STE's weight * mask, sae/ternary.py:41-52),
+            grad x = gz W_enc: tensor-core GEMMs over the batch (csrc/wgrad_sm100.cu) on the row-major batch
+                 tensors as they are (MN-major operands, no transposes);
+            grad b_enc = column sums of gz (atomics: not bit-deterministic, the other gradients are).
+        model.exact (default) contracts three-part bf16 splits of every fp32 operand (fp32-accurate products);
+        exact = False one bf16 product per GEMM.
+        `STEWeights.init_mask / update_mask / mask_grad` (sae/ternary.py:27-90): exact RigL drop / grow by radix
         select on the device.
 No CPU fallback: CUDA tensors only.
 """
@@ -139,6 +152,51 @@ def qsae_trainer_decoder_grads(model, x, active_cap: int = 256):
     return {"recon_losses": losses, "latent_groups": out["latent_groups"], "reconstruction_levels": levels}
 
 
+# ---- t_sae: autograd node ------------------------------------------------------------------------------
+
+class _TernarySAEFn(torch.autograd.Function):
+    """(x, W_enc, b_enc, W_dec) -> (h, recon), one node: g T feeds the ReLU mask inside one epilogue."""
+
+    @staticmethod
+    def forward(ctx, x, w_enc, b_enc, w_dec, model):
+        ctx.set_materialize_grads(False)
+        h, recon = model._forward_dense(x.detach())
+        dec = model.decoder
+        # what the forward contracted, kept for the backward (the reference differentiates through these values)
+        ctx.t_t = dec._ternary_t()
+        ctx.mask = dec.mask.detach().contiguous().float()
+        ctx.w_parts = model._enc_parts()
+        ctx.exact = bool(model.exact)
+        ctx.dec = dec
+        ctx.save_for_backward(x, h)
+        return h, recon
+
+    @staticmethod
+    def backward(ctx, g_h, g_recon):
+        x, h = ctx.saved_tensors
+        B, D = x.shape
+        if g_recon is not None:
+            g = g_recon.detach().contiguous().float()
+            ctx.dec.output_grad = g                   # the reference's backward hook (sae/ternary.py:24-25)
+        else:
+            g = torch.zeros((B, D), dtype=torch.float32, device=x.device)
+        gh = None if g_h is None else g_h.detach().contiguous().float()
+        gwe, gbe, gwd, gx = _lib.tsae_backward(x.detach().contiguous(), h.detach(), g, gh, ctx.t_t, ctx.mask, ctx.w_parts,
+                                               ctx.exact, want_grad_x=ctx.needs_input_grad[0])
+        return gx, gwe, gbe, gwd, None
+
+
+def tsae_forward(model, x):
+    """TernarySparseAutoencoder.forward with an autograd node behind (h, recon) (see module docstring)."""
+    from .sae.base import require_cuda_input
+
+    x = require_cuda_input(x, model)
+    lin = model.encoder[0]
+    h, recon = _TernarySAEFn.apply(x, lin.weight, lin.bias, model.decoder.weight, model)
+    model.decoder.input_activations = h.detach()  # the reference's forward hook (sae/ternary.py:21-22)
+    return h, recon
+
+
 # ---- t_sae: RigL mask maintenance ---------------------------------------------------------------------
 
 def rigl_init_mask(ste, sparsity: float) -> None:
@@ -167,7 +225,8 @@ def rigl_update_mask(ste, f_decay: float, sparsity_rate: float = 0.7) -> None:
     if n_grow > 0 and ste.input_activations is not None:
         if ste.output_grad is None:
             raise RuntimeError("update_mask: output_grad is not set (the reference captures it in a backward hook, "
-                               "sae/ternary.py:24-25); assign decoder.output_grad = d loss / d reconstruction")
+                               "sae/ternary.py:24-25); set model.autograd = True and call loss.backward(), or assign "
+                               "decoder.output_grad = d loss / d reconstruction")
         a = ste.input_activations.detach().contiguous().float()
         d = ste.output_grad.detach().contiguous().float()
         a_mean = _lib.column_sum(a, 1.0 / a.shape[0])
