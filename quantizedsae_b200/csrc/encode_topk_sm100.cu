@@ -1735,7 +1735,10 @@ int encode_pick_splits(int B, int H, int num_sms) {
                        (static_cast<double>(n_tiles) / (static_cast<double>(tps) * s));
     if (eff > best * 1.03) { best = eff; best_s = s; }
   }
-  return best_s;
+  // no split without tiles (9 tiles over 8 splits of 2 leave 3 empty): the cluster variants launch no epilogue for an
+  // empty split, so its survivor-list counts would never be written. The same tile ranges over fewer splits.
+  const int tps = (n_tiles + best_s - 1) / best_s;
+  return (n_tiles + tps - 1) / tps;
 }
 
 int encode_pick_range(int B, int H, int num_sms, int* nsub, int* pair, bool any_batch) {

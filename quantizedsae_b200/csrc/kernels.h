@@ -299,6 +299,9 @@ const char* matryoshka_dense_operand_launch(const float* z, int B, int H, const 
                                             const int* level_start, int n_levels, uint16_t* a_hi, uint16_t* a_lo,
                                             unsigned long long* level_count, void* scratch, cudaStream_t stream);
 size_t matryoshka_dense_operand_scratch_bytes();
+const char* matryoshka_dense_tail_launch(const uint16_t* a_hi, const uint16_t* a_lo, const uint16_t* t_bf16,
+                                        const int* level_start, int n_levels, int B, int H, int D, const float* bias,
+                                        float* result, cudaStream_t stream);
 const char* max_row_norm_launch(const float* w, int H, int D, float* out, cudaStream_t stream);
 const char* row_threshold_launch(const float* x, int B, int D, const float* wmax, float thr_value, float* thr,
                                  cudaStream_t stream);

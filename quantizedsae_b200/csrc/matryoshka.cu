@@ -114,9 +114,9 @@ __global__ void unpack_matryoshka_t_kernel(const uint32_t* __restrict__ packed, 
 }
 
 // a[b, h] = (z[b, h] >= thr) ? scale[h] : 0, as bf16 hi + lo (hi + lo = scale to 2^-17); per-level activity counts.
-// HBM-streaming (4 B read, 4 B written per element): 8 consecutive latents per thread through 16-byte accesses; a
-// group of 8 lies inside one level (level boundaries are multiples of 8), its count is added once per warp when
-// the warp's groups share the level (the usual case), else per lane.
+// HBM-streaming (4 B read, 4 B written per element): 8 consecutive latents per thread through 16-byte accesses. A
+// group's count is added once per warp when the warp's groups lie inside one level (the usual case), else per lane;
+// a group that straddles a level boundary (boundaries need not be multiples of 8) is counted element by element.
 __global__ void __launch_bounds__(256)
 matryoshka_dense_operand_kernel(const float* __restrict__ z, int B, int H, const float* __restrict__ scale, float thr,
                                 const int* __restrict__ level_start, int n_levels, uint16_t* __restrict__ a_hi,
@@ -137,9 +137,11 @@ matryoshka_dense_operand_kernel(const float* __restrict__ z, int B, int H, const
     const size_t g = g0 + lane;
     const bool live = g < groups;
     int lvl = -1;
-    unsigned n_act = 0u;
+    int h = 0;
+    unsigned n_act = 0u, act_bits = 0u;
+    bool straddle = false;
     if (live) {
-      const int h = static_cast<int>(g % h8) << 3;
+      h = static_cast<int>(g % h8) << 3;
       const float4 z0 = __ldcs(reinterpret_cast<const float4*>(z + g * 8));
       const float4 z1 = __ldcs(reinterpret_cast<const float4*>(z + g * 8) + 1);
       const float4 s0 = __ldg(reinterpret_cast<const float4*>(scale + h));
@@ -151,6 +153,7 @@ matryoshka_dense_operand_kernel(const float* __restrict__ z, int B, int H, const
       for (int i = 0; i < 4; ++i) {
         const bool a0 = zv[2 * i] >= thr, a1 = zv[2 * i + 1] >= thr;
         n_act += (a0 ? 1u : 0u) + (a1 ? 1u : 0u);
+        act_bits |= (a0 ? 1u : 0u) << (2 * i) | (a1 ? 1u : 0u) << (2 * i + 1);
         const float v0 = a0 ? sv[2 * i] : 0.f, v1 = a1 ? sv[2 * i + 1] : 0.f;
         const __nv_bfloat162 hh = __floats2bfloat162_rn(v0, v1);
         const __nv_bfloat162 ll = __floats2bfloat162_rn(v0 - __bfloat162float(hh.x), v1 - __bfloat162float(hh.y));
@@ -161,17 +164,63 @@ matryoshka_dense_operand_kernel(const float* __restrict__ z, int B, int H, const
       *reinterpret_cast<uint4*>(a_lo + g * 8) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
       lvl = 0;
       while (lvl + 1 < n_levels && h >= s_start[lvl + 1]) ++lvl;
+      straddle = lvl + 1 < n_levels && h + 8 > s_start[lvl + 1];
     }
     const int lvl0 = __shfl_sync(full, lvl, 0);
-    if (__all_sync(full, lvl == lvl0)) {
+    if (__all_sync(full, lvl == lvl0 && !straddle)) {
       const unsigned tot = __reduce_add_sync(full, n_act);
       if (lane == 0 && tot != 0u) atomicAdd(&s_cnt[lvl0], tot);
-    } else if (n_act != 0u) {
-      atomicAdd(&s_cnt[lvl], n_act);
+    } else if (!straddle) {
+      if (n_act != 0u) atomicAdd(&s_cnt[lvl], n_act);
+    } else {
+      for (int i = 0; i < 8; ++i) {
+        while (lvl + 1 < n_levels && h + i >= s_start[lvl + 1]) ++lvl;
+        if ((act_bits >> i) & 1u) atomicAdd(&s_cnt[lvl], 1u);
+      }
     }
   }
   __syncthreads();
   if (threadIdx.x < 32) count_partial[static_cast<size_t>(blockIdx.x) * 32 + threadIdx.x] = s_cnt[threadIdx.x];
+}
+
+// The dense level GEMMs run over the cuts c_l = floor8(level_start[l + 1]), because a TMA base address must be 16-byte
+// aligned: their chain leaves R[l] = bias + sum over h < c_l in result[l] for every level whose range [c_{l-1}, c_l)
+// is not empty. This kernel completes every level:
+//   result[l] = R[m] + sum over h in [c_l, level_start[l + 1]) of (a_hi + a_lo)[b, h] T[h, :],
+// m = the last level <= l that had a GEMM (none: R = bias). The at most 7 leftover columns of level l lie in level
+// l + 1's GEMM range, so they go to result[l] only. Block per row, thread per output feature, levels in order.
+__global__ void __launch_bounds__(128)
+matryoshka_dense_tail_kernel(const uint16_t* __restrict__ a_hi, const uint16_t* __restrict__ a_lo,
+                             const uint16_t* __restrict__ t_bf16 /* [D, H] */, const int* __restrict__ level_start,
+                             int n_levels, int B, int H, int D, const float* __restrict__ bias,
+                             float* __restrict__ result /* [n_levels, B, D] */) {
+  for (int b = blockIdx.x; b < B; b += gridDim.x) {
+    for (int d = threadIdx.x; d < D; d += blockDim.x) {
+      float chain = bias != nullptr ? __ldg(bias + d) : 0.f;
+      int c_prev = 0;
+      for (int l = 0; l < n_levels; ++l) {
+        const int end = __ldg(level_start + l + 1), c = end & ~7;
+        float* out = result + (static_cast<size_t>(l) * B + b) * D + d;
+        if (c > c_prev) chain = *out;
+        float tail = 0.f;
+        if (end > c) {
+          const uint4 hv = __ldg(reinterpret_cast<const uint4*>(a_hi + static_cast<size_t>(b) * H + c));
+          const uint4 lv = __ldg(reinterpret_cast<const uint4*>(a_lo + static_cast<size_t>(b) * H + c));
+          const uint4 tv = __ldg(reinterpret_cast<const uint4*>(t_bf16 + static_cast<size_t>(d) * H + c));
+          const uint32_t hw[4] = {hv.x, hv.y, hv.z, hv.w}, lw[4] = {lv.x, lv.y, lv.z, lv.w}, tw[4] = {tv.x, tv.y, tv.z, tv.w};
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            const int sh = (j & 1) ? 0 : 16;   // bf16 j of a word: low half for even j
+            const float a = __uint_as_float((hw[j >> 1] << sh) & 0xFFFF0000u) + __uint_as_float((lw[j >> 1] << sh) & 0xFFFF0000u);
+            const float t = __uint_as_float((tw[j >> 1] << sh) & 0xFFFF0000u);
+            if (c + j < end) tail = fmaf(a, t, tail);
+          }
+        }
+        *out = chain + tail;
+        c_prev = c;
+      }
+    }
+  }
 }
 
 constexpr int kMatWarps = 4;
@@ -390,6 +439,15 @@ const char* matryoshka_dense_operand_launch(const float* z, int B, int H, const 
   if (e != cudaSuccess) return cudaGetErrorString(e);
   count_launches(1);
   sum_level_counts_kernel<<<n_levels, 256, 0, stream>>>(partial, static_cast<int>(g), 32, n_levels, level_count);
+  return cuda_err(cudaGetLastError());
+}
+
+const char* matryoshka_dense_tail_launch(const uint16_t* a_hi, const uint16_t* a_lo, const uint16_t* t_bf16,
+                                        const int* level_start, int n_levels, int B, int H, int D, const float* bias,
+                                        float* result, cudaStream_t stream) {
+  if ((H % 8) != 0) return "matryoshka_dense_tail: H must be a multiple of 8";
+  const int g = B < 148 * 16 ? B : 148 * 16;
+  matryoshka_dense_tail_kernel<<<g, 128, 0, stream>>>(a_hi, a_lo, t_bf16, level_start, n_levels, B, H, D, bias, result);
   return cuda_err(cudaGetLastError());
 }
 

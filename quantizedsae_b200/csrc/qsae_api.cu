@@ -1421,7 +1421,9 @@ int plan_matryoshka_dense(int B, int H, int D, MatDensePlan* mp) {
   if (B <= 0 || H <= 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "B and H must be positive");
   if (D < 16 || D > 512 || (D % 16) != 0)
     return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka: D must be a multiple of 16 in [16, 512], got %d", D);
-  if ((H % 8) != 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka dense path: hidden_dim must be a multiple of 8, got %d", H);
+  if ((H % 8) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka dense path: hidden_dim must be a multiple of 8, got %d (the A "
+                "operand and T^T rows are not padded to 16 bytes; other hidden_dim values have the sparse path only)", H);
   const size_t bh = static_cast<size_t>(B) * H;
   mp->x_off = 0;
   mp->z_off = 3 * align_up(static_cast<size_t>(B) * D * 2, 1024);   // room for the three bf16 parts of x
@@ -1454,9 +1456,9 @@ int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, cons
     return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_forward_dense: null pointer");
   if (!w_hi) return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_forward_dense: no encoder weights");
   if (n_levels < 1 || n_levels > 32) return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_forward_dense: 1 <= n_levels <= 32");
-  for (int i = 0; i <= n_levels; ++i) {
-    if ((level_start_host[i] % 8) != 0 || (i > 0 && level_start_host[i] <= level_start_host[i - 1]))
-      return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka dense path: level boundaries must be increasing multiples of 8");
+  for (int i = 1; i <= n_levels; ++i) {
+    if (level_start_host[i] <= level_start_host[i - 1])
+      return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka dense path: level boundaries must be increasing");
   }
   if (level_start_host[0] != 0 || level_start_host[n_levels] != H)
     return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka dense path: levels must cover [0, H)");
@@ -1494,17 +1496,29 @@ int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, cons
                                                        level_count, ws + mp.cnt_off, st));
     if (rc != QSAE_OK) return rc;
   }
-  // 3. one GEMM per level over its K range, outputs accumulated level by level (:121-129)
+  // 3. one GEMM per level over its K range, outputs accumulated level by level (:121-129). A TMA base address must be
+  //    16-byte aligned, so the ranges end at the cuts floor8(level_start[i + 1]); a level whose range is empty after
+  //    the cut has no GEMM. When a boundary is off the 8-grid, a last kernel adds each level's leftover columns
+  //    [cut, level_start[i + 1]) to that level alone and fills the levels without a GEMM (matryoshka.cu)
   const size_t bd = static_cast<size_t>(B) * D;
+  int k0 = 0, prev = -1;
+  bool tail = false;
   for (int i = 0; i < n_levels; ++i) {
-    const int k0 = level_start_host[i], kn = level_start_host[i + 1] - k0;
+    const int cut = level_start_host[i + 1] & ~7;
+    tail = tail || cut != level_start_host[i + 1];
+    if (cut == k0) continue;
     rc = launch_status("dense_decode (level)",
-                       dense_decode_launch(a_hi + k0, a_lo + k0, H, t_bf16 + k0, H, B, kn, D, i == 0 ? dec_bias : nullptr,
-                                           i == 0 ? nullptr : result + (i - 1) * bd, result + i * bd, ws + mp.dec_off,
+                       dense_decode_launch(a_hi + k0, a_lo + k0, H, t_bf16 + k0, H, B, cut - k0, D, prev < 0 ? dec_bias : nullptr,
+                                           prev < 0 ? nullptr : result + prev * bd, result + i * bd, ws + mp.dec_off,
                                            num_sms(), st));
     if (rc != QSAE_OK) return rc;
+    k0 = cut;
+    prev = i;
   }
-  return QSAE_OK;
+  if (tail)
+    rc = launch_status("matryoshka_dense_tail", matryoshka_dense_tail_launch(a_hi, a_lo, t_bf16, level_start_dev, n_levels, B,
+                                                                             H, D, dec_bias, result, st));
+  return rc;
 }
 
 int qsae_residual_update(const float* residual, const float* recon, size_t n, float* out, void* stream) {

@@ -975,7 +975,8 @@ def test_pack_ternary_bit_exact(cuda_device):
     assert ref[0, :8].tolist() == [1, -1, 0, 0, 0, 0, 1, -1]
 
 
-@pytest.mark.parametrize("B,K,N", [(128, 1024, 512), (200, 4096, 64), (77, 1000, 256), (1, 72, 8), (300, 2048, 384)])
+@pytest.mark.parametrize("B,K,N", [(128, 1024, 512), (200, 4096, 64), (77, 1000, 256), (1, 72, 8), (300, 2048, 384),
+                                   (33, 8, 64), (130, 32, 512), (1, 40, 16)])
 def test_decode_dense_vs_fp64(cuda_device, B, K, N):
     rng = np.random.default_rng(B + K + N)
     a = np.maximum(rng.standard_normal((B, K)), 0).astype(np.float32)
@@ -1143,7 +1144,7 @@ def test_qsae_untrained_model_falls_back_to_dense(cuda_device):
 
 
 @pytest.mark.parametrize("exact", [False, True])
-@pytest.mark.parametrize("B,H", [(160, 32768), (700, 4096), (40, 1024), (90, 832)])
+@pytest.mark.parametrize("B,H", [(160, 32768), (700, 4096), (40, 1024), (90, 832), (120, 2056)])
 def test_qsae_dense_operand_from_the_encoder_epilogue(cuda_device, tuning, B, H, exact):
     """The dense path's A operand (active * scale as bf16 hi / lo) and the per-level activity counts written by the
     encoder epilogue itself (act = 2) against the first form: fp32 pre-activations to HBM + the streaming operand kernel.
