@@ -132,7 +132,7 @@ def check_decisions(act, forced, band, what):
 
 def level_sums_f64(act, rows, starts, bias):
     """Cumulative float64 level sums of act [B, H] over the dictionary rows [H, D] -> ([L, B, D], terms [L, B])."""
-    A = sp.csr_matrix(act.astype(np.float64))
+    A = sp.csr_matrix(act, dtype=np.float64)   # from the non-zeros: no dense float64 copy of a [B, H] mask
     B, D = act.shape[0], rows.shape[1]
     L = len(starts) - 1
     out, n = np.empty((L, B, D)), np.empty((L, B))
