@@ -126,8 +126,8 @@ int qsae_default_sample_rows(int H);
 /* Kernels this library has launched in this process (all threads, monotonic): what bench.py reports as gpu_launches. */
 unsigned long long qsae_launch_count(void);
 
-/* Tuning / diagnostic switches (QSAE_ENCODE_SPLITS, QSAE_ENCODE_PRIOR, QSAE_ENCODE_CLUSTER, QSAE_ENCODE_RANGE,
- * QSAE_PRIOR_PREP, QSAE_SAMPLE_DIV, QSAE_DENSE_SPLIT_FUSED, QSAE_DENSE_STEP_FUSED, QSAE_DECODE_PAIR, QSAE_DEBUG_*) are
+/* Tuning / diagnostic switches (QSAE_ENCODE_CLUSTER, QSAE_ENCODE_RANGE, QSAE_PRIOR_PREP, QSAE_SAMPLE_DIV,
+ * QSAE_DENSE_STEP_FUSED, QSAE_DECODE_PAIR, QSAE_DEBUG_*; INTEGRATION.md lists them all) are
  * read from the environment once, on first use, never on a
  * launch path. A process that changes them afterwards (tests, tuning runs) calls this to re-read them. */
 int qsae_reload_tuning(void);
@@ -355,9 +355,8 @@ int qsae_decode_dense(const uint16_t* a_hi /* [B, K] */, const uint16_t* a_lo /*
  *            from the GEMM epilogue; recon from one pass over bf16(h) (relative error <= 2^-9 per term).
  * exact = 1: any fp32 operands. x and W are split exactly into three bf16 parts each and the six partial
  *            products above 2^-24 are accumulated on the tensor cores in ONE launch (both operands streamed,
- *            all six products into the same TMEM accumulator, smallest first; QSAE_DENSE_SPLIT_FUSED=0: the
- *            three accumulating launches of the first version); recon from two accumulating passes over the
- *            hi/lo split of h (2^-17 per term).
+ *            all six products into the same TMEM accumulator, smallest first); recon from two accumulating
+ *            passes over the hi/lo split of h (2^-17 per term).
  * H % 8 == 0, D % 8 == 0, 8 <= D <= 512. */
 int qsae_tsae_workspace_bytes(int B, int H, int D, int exact, size_t* bytes);
 int qsae_tsae_forward(const float* x_f32, const uint16_t* w_hi /* [H, D]: bf16(W) */,

@@ -66,8 +66,8 @@ __host__ __device__ constexpr int epi_warps(bool dense) { return 8; }
 __host__ __device__ constexpr int cta_threads(bool dense) { return 128 + epi_warps(dense) * 32; }
 constexpr int kTmemCols = 512;                  // 2 accumulators x 256 columns
 
-constexpr int kMaxPieces = 8;   // pieces of one CTA's range: 2 when a range is shorter than a row block (full sweeps), up to
-                                // ceil(range / tiles per row block) + 1 for short sweeps (the sample pre-pass); checked by encode_pick_range
+constexpr int kMaxPieces = 8;   // pieces of one CTA's range: ceil(range / tiles per row block) + 1 at most, i.e. 2 when there are
+                                // fewer row blocks than CTAs (every range-scheduled sweep on 148 SMs); checked by encode_pick_range
 struct SmemLayout {
   uint32_t a_off, b_off, staging_off, bias_off, share_off, bar_off, tmem_ptr_off, piece_off, total;
 };
@@ -610,7 +610,7 @@ __device__ __forceinline__ void epilogue_dense(const EncodeLaunch& p, int n_my_t
         r[4 * j + 2] = __float_as_uint(__uint_as_float(r[4 * j + 2]) + b.z);
         r[4 * j + 3] = __float_as_uint(__uint_as_float(r[4 * j + 3]) + b.w);
       }
-      if (p.act == 1 && p.accum_mode == 0) {
+      if (p.act == 1) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(fmaxf(__uint_as_float(r[j]), 0.f));
       }
@@ -632,117 +632,66 @@ __device__ __forceinline__ void epilogue_dense(const EncodeLaunch& p, int n_my_t
         }
         if (row0 + lane < p.B) n_act += n;
       }
-      if (p.accum_mode != 0 || p.act == 3) {
-        // Split-operand passes (exact fp32 encoder): r holds this pass's raw partial products (the
-        // launcher passes no bias for these passes; the final pass adds p.accum_bias here).
-        //   1: out = acc            2: out = out + acc            3: out = act(out + acc + bias), + bf16 hi / lo
-        // The transformation runs in the row-contiguous read-back layout, where `out` is read coalesced.
-        // act == 3 (ReLU backward, streamed-operand kernel only, no bias): see the WIDE branch below.
-        auto finish = [&](int rr, int cc, const uint4 u) {
-          if (row0 + rr >= p.B || cc >= p.H) return;
-          const size_t off = static_cast<size_t>(row0 + rr) * H + cc;
-          float4 v = make_float4(__uint_as_float(u.x), __uint_as_float(u.y), __uint_as_float(u.z), __uint_as_float(u.w));
-          if (p.accum_mode >= 2) {
-            const float4 o = *reinterpret_cast<const float4*>(p.out_f32 + off);
-            v.x += o.x; v.y += o.y; v.z += o.z; v.w += o.w;
-          }
-          if (p.accum_mode == 3) {
-            const float4 b = *reinterpret_cast<const float4*>(p.accum_bias + cc);
-            v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-            if (p.act == 1) { v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f); }
-            if (flags & 6) {
-              const uint32_t h0 = pack_bf16x2(v.x, v.y), h1 = pack_bf16x2(v.z, v.w);
-              if (flags & 2) *reinterpret_cast<uint2*>(p.out_hi + off) = make_uint2(h0, h1);
-              if (flags & 4) {
-                const uint32_t l0 = pack_bf16x2(v.x - __uint_as_float(h0 << 16), v.y - __uint_as_float(h0 & 0xFFFF0000u));
-                const uint32_t l1 = pack_bf16x2(v.z - __uint_as_float(h1 << 16), v.w - __uint_as_float(h1 & 0xFFFF0000u));
-                *reinterpret_cast<uint2*>(p.out_lo + off) = make_uint2(l0, l1);
-              }
-            }
-          }
-          *reinterpret_cast<float4*>(p.out_f32 + off) = v;
-        };
-        if constexpr (WIDE) {
+      if constexpr (WIDE) {
+        if (p.act == 3) {
+          // ReLU backward at the forward's output (streamed-operand kernel only, no bias): out = (acc + gate_add) *
+          // (gate > 0); torch masks on the returned h and selects, so a non-finite acc where h <= 0 gives 0. gate /
+          // gate_add do not depend on the accumulator: four rows of both are loaded before any of them is used (a load
+          // per row in turn left the kernel latency-bound). The warp's 32 rows are summed per column (p.gate_colsum +=
+          // sum_b out: the bias gradient, one atomic per column and warp). The transformation runs in the
+          // row-contiguous read-back layout, where gate and gate_add are read coalesced.
           __syncwarp();
 #pragma unroll
           for (int q = 0; q < 8; ++q)
             st_shared_v4(st + lane * 128 + ((q ^ (lane & 7)) << 4), r[4 * q], r[4 * q + 1], r[4 * q + 2], r[4 * q + 3]);
           __syncwarp();
-          if (p.act == 3) {
-            // ReLU backward at the forward's output: out = (acc + gate_add) * (gate > 0); torch masks on the returned h
-            // and selects, so a non-finite acc where h <= 0 gives 0. gate / gate_add do not depend on the accumulator:
-            // four rows of both are loaded before any of them is used (a load per row in turn left the kernel
-            // latency-bound). The warp's 32 rows are summed per column (p.gate_colsum += sum_b out: the bias
-            // gradient, one atomic per column and warp).
-            const int cc = col0 + f_col;
-            float4 cs = make_float4(0.f, 0.f, 0.f, 0.f);
+          const int cc = col0 + f_col;
+          float4 cs = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
-            for (int j0 = 0; j0 < 8; j0 += 4) {
-              float4 hv[4], av[4];
+          for (int j0 = 0; j0 < 8; j0 += 4) {
+            float4 hv[4], av[4];
 #pragma unroll
-              for (int i = 0; i < 4; ++i) {
-                const int rr = 4 * (j0 + i) + f_row;
-                const bool ok = row0 + rr < p.B && cc < p.H;
-                const size_t off = static_cast<size_t>(row0 + rr) * H + cc;
-                hv[i] = ok ? __ldg(reinterpret_cast<const float4*>(p.gate + off)) : make_float4(0.f, 0.f, 0.f, 0.f);
-                av[i] = ok && p.gate_add != nullptr ? __ldg(reinterpret_cast<const float4*>(p.gate_add + off))
-                                                    : make_float4(0.f, 0.f, 0.f, 0.f);
-              }
-#pragma unroll
-              for (int i = 0; i < 4; ++i) {
-                const int rr = 4 * (j0 + i) + f_row;
-                if (row0 + rr >= p.B || cc >= p.H) continue;
-                const size_t off = static_cast<size_t>(row0 + rr) * H + cc;
-                const uint4 u = ld_shared_v4(st + rr * 128 + (((lane & 7) ^ (rr & 7)) << 4));
-                float4 v = make_float4(__uint_as_float(u.x) + av[i].x, __uint_as_float(u.y) + av[i].y,
-                                       __uint_as_float(u.z) + av[i].z, __uint_as_float(u.w) + av[i].w);
-                v.x = hv[i].x > 0.f ? v.x : 0.f; v.y = hv[i].y > 0.f ? v.y : 0.f;
-                v.z = hv[i].z > 0.f ? v.z : 0.f; v.w = hv[i].w > 0.f ? v.w : 0.f;
-                cs.x += v.x; cs.y += v.y; cs.z += v.z; cs.w += v.w;
-                if (flags & 1) *reinterpret_cast<float4*>(p.out_f32 + off) = v;
-                if (flags & 2)
-                  *reinterpret_cast<uint2*>(p.out_hi + off) = make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w));
-              }
+            for (int i = 0; i < 4; ++i) {
+              const int rr = 4 * (j0 + i) + f_row;
+              const bool ok = row0 + rr < p.B && cc < p.H;
+              const size_t off = static_cast<size_t>(row0 + rr) * H + cc;
+              hv[i] = ok ? __ldg(reinterpret_cast<const float4*>(p.gate + off)) : make_float4(0.f, 0.f, 0.f, 0.f);
+              av[i] = ok && p.gate_add != nullptr ? __ldg(reinterpret_cast<const float4*>(p.gate_add + off))
+                                                  : make_float4(0.f, 0.f, 0.f, 0.f);
             }
-            if (p.gate_colsum != nullptr) {   // lanes l, l + 8, l + 16, l + 24 hold the same four columns
 #pragma unroll
-              for (int sh = 8; sh <= 16; sh <<= 1) {
-                cs.x += __shfl_xor_sync(0xffffffffu, cs.x, sh);
-                cs.y += __shfl_xor_sync(0xffffffffu, cs.y, sh);
-                cs.z += __shfl_xor_sync(0xffffffffu, cs.z, sh);
-                cs.w += __shfl_xor_sync(0xffffffffu, cs.w, sh);
-              }
-              if (lane < 8 && cc < p.H) {
-                atomicAdd(p.gate_colsum + cc, cs.x);
-                atomicAdd(p.gate_colsum + cc + 1, cs.y);
-                atomicAdd(p.gate_colsum + cc + 2, cs.z);
-                atomicAdd(p.gate_colsum + cc + 3, cs.w);
-              }
-            }
-            continue;
-          }
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const int rr = 4 * j + f_row;
-            finish(rr, col0 + f_col, ld_shared_v4(st + rr * 128 + (((lane & 7) ^ (rr & 7)) << 4)));
-          }
-        } else {
-#pragma unroll
-          for (int hf = 0; hf < 2; ++hf) {
-            __syncwarp();
-#pragma unroll
-            for (int q = 0; q < 4; ++q)
-              st_shared_v4(st + lane * 64 + ((q ^ ((lane >> 1) & 3)) << 4), r[16 * hf + 4 * q], r[16 * hf + 4 * q + 1],
-                           r[16 * hf + 4 * q + 2], r[16 * hf + 4 * q + 3]);
-            __syncwarp();
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const int rr = 8 * j + h_row;
-              finish(rr, col0 + 16 * hf + (lane & 3) * 4, ld_shared_v4(st + rr * 64 + (((lane & 3) ^ ((rr >> 1) & 3)) << 4)));
+            for (int i = 0; i < 4; ++i) {
+              const int rr = 4 * (j0 + i) + f_row;
+              if (row0 + rr >= p.B || cc >= p.H) continue;
+              const size_t off = static_cast<size_t>(row0 + rr) * H + cc;
+              const uint4 u = ld_shared_v4(st + rr * 128 + (((lane & 7) ^ (rr & 7)) << 4));
+              float4 v = make_float4(__uint_as_float(u.x) + av[i].x, __uint_as_float(u.y) + av[i].y,
+                                     __uint_as_float(u.z) + av[i].z, __uint_as_float(u.w) + av[i].w);
+              v.x = hv[i].x > 0.f ? v.x : 0.f; v.y = hv[i].y > 0.f ? v.y : 0.f;
+              v.z = hv[i].z > 0.f ? v.z : 0.f; v.w = hv[i].w > 0.f ? v.w : 0.f;
+              cs.x += v.x; cs.y += v.y; cs.z += v.z; cs.w += v.w;
+              if (flags & 1) *reinterpret_cast<float4*>(p.out_f32 + off) = v;
+              if (flags & 2)
+                *reinterpret_cast<uint2*>(p.out_hi + off) = make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w));
             }
           }
+          if (p.gate_colsum != nullptr) {   // lanes l, l + 8, l + 16, l + 24 hold the same four columns
+#pragma unroll
+            for (int sh = 8; sh <= 16; sh <<= 1) {
+              cs.x += __shfl_xor_sync(0xffffffffu, cs.x, sh);
+              cs.y += __shfl_xor_sync(0xffffffffu, cs.y, sh);
+              cs.z += __shfl_xor_sync(0xffffffffu, cs.z, sh);
+              cs.w += __shfl_xor_sync(0xffffffffu, cs.w, sh);
+            }
+            if (lane < 8 && cc < p.H) {
+              atomicAdd(p.gate_colsum + cc, cs.x);
+              atomicAdd(p.gate_colsum + cc + 1, cs.y);
+              atomicAdd(p.gate_colsum + cc + 2, cs.z);
+              atomicAdd(p.gate_colsum + cc + 3, cs.w);
+            }
+          }
+          continue;
         }
-        continue;
       }
       if (flags & 1) {
         if constexpr (WIDE) {
@@ -878,10 +827,7 @@ __device__ __forceinline__ void run_epilogue_piece(const EncodeLaunch& p, int n,
 //   MMA and bias roles are the same for both.
 template <int K_CHUNKS, bool DENSE, int CL, int SEL>
 __global__ void __launch_bounds__(cta_threads(DENSE), 1)
-encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
-                   const __grid_constant__ CUtensorMap tmap_b0,
-                   const __grid_constant__ CUtensorMap tmap_b1,
-                   const __grid_constant__ CUtensorMap tmap_b2, EncodeLaunch p) {
+encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_w, EncodeLaunch p) {
   constexpr bool MCAST = CL == 1;
   constexpr bool PAIR = CL >= 2;            // CL = 3: cta_group::2 pairs ON the range schedule (sparse sweeps, small batches)
   constexpr int kStages = ring_stages(DENSE, PAIR);
@@ -912,7 +858,6 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
   const int m0_grid = ranged ? 0 : ((CL != 0) ? blockIdx.x : blockIdx.y) * BM;
   const uint32_t cta_rank = (CL != 0) ? cluster_ctarank() : 0u;
   const bool leader = cta_rank == 0u;
-  const int k_iters = (p.k_parts > 1 ? p.k_parts : 1) * K_CHUNKS;
   // the CTA's pieces, computed once by thread 0 (64-bit divisions) and read from shared memory by every role
   int* piece_n = reinterpret_cast<int*>(smem + L.piece_off);
   Piece* piece_tab = reinterpret_cast<Piece*>(smem + L.piece_off + 16);
@@ -981,7 +926,7 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
     // ------------------------------------------------------------- TMA producer
     if (lane == 0) {
       tma_prefetch_desc(&tmap_x);
-      tma_prefetch_desc(&tmap_b0);
+      tma_prefetch_desc(&tmap_w);
       const int n_pieces = *piece_n;
       int stage = 0;
       uint32_t phase = 0;
@@ -1005,24 +950,21 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
         }
         for (int t = 0; t < pc.n; ++t) {
           const int n0 = (pc.tile0 + t) * BN;
-          // p.k_parts B operands (bf16 parts of W) are contracted against the same resident x tile
 #pragma unroll 1
-          for (int it2 = 0; it2 < k_iters; ++it2) {
-            const int part = it2 / K_CHUNKS, kc = it2 - part * K_CHUNKS;
-            const CUtensorMap* tb = part == 0 ? &tmap_b0 : (part == 1 ? &tmap_b1 : &tmap_b2);
+          for (int kc = 0; kc < K_CHUNKS; ++kc) {
             mbar_wait(&empty[stage], phase ^ 1u);
             if constexpr (PAIR) {
               if (leader) mbar_arrive_expect_tx(&full[stage], kBBytesPerStage);   // 16 KiB from each CTA
-              tma_load_2d_pair(b_smem + stage * kStageBytes, tb, mapa_u32(smem_u32(&full[stage]), 0), kc * BK,
+              tma_load_2d_pair(b_smem + stage * kStageBytes, &tmap_w, mapa_u32(smem_u32(&full[stage]), 0), kc * BK,
                                n0 + static_cast<int>(cta_rank) * (BN / 2), kPolicyEvictLast);
             } else if constexpr (MCAST) {
               mbar_arrive_expect_tx(&full[stage], kBBytesPerStage);
               // my half of the stage lands in both CTAs; the other half arrives from the peer
-              tma_load_2d_mcast(b_smem + stage * kBBytesPerStage + cta_rank * (kBBytesPerStage / 2), tb,
+              tma_load_2d_mcast(b_smem + stage * kBBytesPerStage + cta_rank * (kBBytesPerStage / 2), &tmap_w,
                                 &full[stage], kc * BK, n0 + static_cast<int>(cta_rank) * (BN / 2), 0x3, kPolicyEvictLast);
             } else {
               mbar_arrive_expect_tx(&full[stage], kBBytesPerStage);
-              tma_load_2d(b_smem + stage * kBBytesPerStage, tb, &full[stage], kc * BK, n0, kPolicyEvictLast);
+              tma_load_2d(b_smem + stage * kBBytesPerStage, &tmap_w, &full[stage], kc * BK, n0, kPolicyEvictLast);
             }
             if (++stage == kStages) { stage = 0; phase ^= 1u; }
           }
@@ -1049,8 +991,7 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
           tc_fence_after();
           const uint32_t d_tmem = tmem_base + acc * BN;
 #pragma unroll 1
-          for (int it2 = 0; it2 < k_iters; ++it2) {
-            const int kc = it2 % K_CHUNKS;      // every part of W meets the same x chunks
+          for (int kc = 0; kc < K_CHUNKS; ++kc) {
             mbar_wait(&full[stage], phase);
             tc_fence_after();
             const uint64_t a_desc = a_desc0 + static_cast<uint64_t>((kc * kABytesPerChunk) >> 4);
@@ -1059,16 +1000,16 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
             for (int ks = 0; ks < BK / UMMA_K; ++ks) {
               // advance 16 elements = 32 bytes along K inside the swizzle atom: +2 in the
               // (address >> 4) field of the descriptor
-              if constexpr (PAIR) umma_f16_ss_pair(d_tmem, a_desc + ks * 2, b_desc + ks * 2, idesc, (it2 | ks) != 0 ? 1u : 0u);
-              else umma_f16_ss(d_tmem, a_desc + ks * 2, b_desc + ks * 2, idesc, (it2 | ks) != 0 ? 1u : 0u);
+              if constexpr (PAIR) umma_f16_ss_pair(d_tmem, a_desc + ks * 2, b_desc + ks * 2, idesc, (kc | ks) != 0 ? 1u : 0u);
+              else umma_f16_ss(d_tmem, a_desc + ks * 2, b_desc + ks * 2, idesc, (kc | ks) != 0 ? 1u : 0u);
             }
             if constexpr (PAIR) {
               umma_commit_pair(&empty[stage], 0x3);
-              if (it2 == k_iters - 1) umma_commit_pair(&tmem_full[acc], 0x3);
+              if (kc == K_CHUNKS - 1) umma_commit_pair(&tmem_full[acc], 0x3);
             } else {
               if constexpr (MCAST) umma_commit_mcast(&empty[stage], 0x3);
               else umma_commit(&empty[stage]);
-              if (it2 == k_iters - 1) umma_commit(&tmem_full[acc]);
+              if (kc == K_CHUNKS - 1) umma_commit(&tmem_full[acc]);
             }
             if (++stage == kStages) { stage = 0; phase ^= 1u; }
           }
@@ -1135,10 +1076,10 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_x,
 // launch. x = xh + xm + xl and W = wh + wm + wl (bf16 parts, both sums exact); the six partial products above 2^-24
 // are contracted into the SAME TMEM accumulator, smallest first:
 //     xl wh, xm wm, xh wl, xm wh, xh wm, xh wh        (K = 6 D in effect)
-// so the dense fp32 output is written once (the three-pass form read-modify-wrote it twice: 2.1 ms of a 2.3 ms
-// forward at B = 4096). No x tile is resident: every ring stage carries one 128 x 64 chunk of an x part next to
-// the CTA's half (128 latents) of the matching W chunk, the cta_group::2 pair executes M = 256 MMAs (CL = 2 of the
-// kernel above), and the epilogue is the same dense epilogue (accum_mode 0: bias + activation, fp32 / hi / lo).
+// so the dense fp32 output is written once (three launches that read-modify-wrote it took 2054 us against 595 us at
+// B = 4096, profiles/r2s3_measurements.md 1). No x tile is resident: every ring stage carries one 128 x 64 chunk of an
+// x part next to the CTA's half (128 latents) of the matching W chunk, the cta_group::2 pair executes M = 256 MMAs
+// (CL = 2 of the kernel above), and the epilogue is the same dense epilogue (bias + activation, fp32 / hi / lo).
 // The MMAs of a tile take six times as long as its drain, so the stores hide behind the tensor pipe here.
 // Six 32 KiB stages next to the 32 KiB store staging area: 231.6 KB, all the shared memory a CTA can have (five stages:
 // 620 us at B = 4096, H = 32768; six: 595 us -- this kernel is bound by the tensor pipe, and ring depth shows).
@@ -1194,7 +1135,7 @@ encode_dense_split_kernel(const __grid_constant__ CUtensorMap tmap_xh, const __g
   const int tile0 = static_cast<int>(u0 - static_cast<long long>(rbp0) * n_tiles);
   // products: (x part, W part) of product i = ((prods >> 4i + 2) & 3, (prods >> 4i) & 3), see the launcher.
   // n_prod = 6: the split-operand product; n_prod = 3: three x parts against one W part; n_prod = 1: only xh wh (the
-  // fast mode's single bf16 product on this kernel's schedule: all 148 SMs at any batch, nothing resident)
+  // single bf16 product of the fast-mode t_sae backward)
   const int k_iters = n_prod * k_chunks;
 
   if (threadIdx.x == 0) {
@@ -1637,10 +1578,8 @@ bool make_tmap_bf16(CUtensorMap* map, const void* base, int rows, int cols, int 
                       CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
-struct BMaps { CUtensorMap m[3]; };   // the (up to three) bf16 parts of W, boxed for the chosen cluster variant
-
 template <int K_CHUNKS, bool DENSE, int CL, int SEL>
-cudaError_t launch_k(const CUtensorMap& tx, const BMaps& b, const EncodeLaunch& p, cudaStream_t stream) {
+cudaError_t launch_k(const CUtensorMap& tx, const CUtensorMap& tw, const EncodeLaunch& p, cudaStream_t stream) {
   const SmemLayout L = smem_layout(K_CHUNKS, DENSE, CL >= 2);
   static bool attr_set = false;
   if (!attr_set) {
@@ -1667,46 +1606,48 @@ cudaError_t launch_k(const CUtensorMap& tx, const BMaps& b, const EncodeLaunch& 
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, encode_topk_kernel<K_CHUNKS, DENSE, CL, SEL>, tx, b.m[0], b.m[1], b.m[2], p);
+    return cudaLaunchKernelEx(&cfg, encode_topk_kernel<K_CHUNKS, DENSE, CL, SEL>, tx, tw, p);
   } else {
-    encode_topk_kernel<K_CHUNKS, DENSE, CL, SEL><<<grid, cta_threads(DENSE), L.total, stream>>>(tx, b.m[0], b.m[1], b.m[2], p);
+    encode_topk_kernel<K_CHUNKS, DENSE, CL, SEL><<<grid, cta_threads(DENSE), L.total, stream>>>(tx, tw, p);
     return cudaGetLastError();
   }
 }
 
 template <bool DENSE, int SEL>
-cudaError_t launch_kc(const CUtensorMap& tx, const BMaps& b, const EncodeLaunch& p, cudaStream_t stream) {
+cudaError_t launch_kc(const CUtensorMap& tx, const CUtensorMap& tw, const EncodeLaunch& p, cudaStream_t stream) {
   switch ((p.D + BK - 1) / BK) {
-    case 1: return launch_k<1, DENSE, 0, SEL>(tx, b, p, stream);
-    case 2: return launch_k<2, DENSE, 0, SEL>(tx, b, p, stream);
-    case 3: return launch_k<3, DENSE, 0, SEL>(tx, b, p, stream);
-    case 4: return launch_k<4, DENSE, 0, SEL>(tx, b, p, stream);
-    case 5: return launch_k<5, DENSE, 0, SEL>(tx, b, p, stream);
-    case 6: return launch_k<6, DENSE, 0, SEL>(tx, b, p, stream);
-    case 7: return launch_k<7, DENSE, 0, SEL>(tx, b, p, stream);
+    case 1: return launch_k<1, DENSE, 0, SEL>(tx, tw, p, stream);
+    case 2: return launch_k<2, DENSE, 0, SEL>(tx, tw, p, stream);
+    case 3: return launch_k<3, DENSE, 0, SEL>(tx, tw, p, stream);
+    case 4: return launch_k<4, DENSE, 0, SEL>(tx, tw, p, stream);
+    case 5: return launch_k<5, DENSE, 0, SEL>(tx, tw, p, stream);
+    case 6: return launch_k<6, DENSE, 0, SEL>(tx, tw, p, stream);
+    case 7: return launch_k<7, DENSE, 0, SEL>(tx, tw, p, stream);
     default:   // the headline width: the cluster variants exist here (launch_any has checked D <= 512)
-      if (p.cluster == 3) return launch_k<8, DENSE, 3, SEL>(tx, b, p, stream);
-      if (p.cluster == 2) return launch_k<8, DENSE, 2, SEL>(tx, b, p, stream);
-      if (p.cluster == 1) return launch_k<8, DENSE, 1, SEL>(tx, b, p, stream);
-      return launch_k<8, DENSE, 0, SEL>(tx, b, p, stream);
+      if constexpr (!DENSE) {   // the dense epilogue has the single-CTA and the cta_group::2 variants only
+        if (p.cluster == 3) return launch_k<8, DENSE, 3, SEL>(tx, tw, p, stream);
+        if (p.cluster == 1) return launch_k<8, DENSE, 1, SEL>(tx, tw, p, stream);
+      }
+      if (p.cluster == 2) return launch_k<8, DENSE, 2, SEL>(tx, tw, p, stream);
+      return launch_k<8, DENSE, 0, SEL>(tx, tw, p, stream);
   }
 }
 
 // Prior-threshold sweeps (mode 4) run on the kernel compiled for that mode alone unless QSAE_ENCODE_SPECIALISED=0;
 // the diagnostics (debug_mode, debug_z) exist in the generic kernel only.
 template <bool DENSE>
-const char* launch_any(const CUtensorMap& tx, const BMaps& b, const EncodeLaunch& p, cudaStream_t stream) {
+const char* launch_any(const CUtensorMap& tx, const CUtensorMap& tw, const EncodeLaunch& p, cudaStream_t stream) {
   const int kc = (p.D + BK - 1) / BK;
   if (kc < 1 || kc > 8) return "D must be <= 512";
   if (p.cluster == 3 && kc != 8) return "the pair range schedule exists for D > 448 only";
   cudaError_t e;
   if constexpr (!DENSE) {
     if (p.mode == 4 && p.debug_mode == 0 && p.debug_z == nullptr && tuning().encode_specialised != 0)
-      e = launch_kc<false, 4>(tx, b, p, stream);
+      e = launch_kc<false, 4>(tx, tw, p, stream);
     else
-      e = launch_kc<false, -1>(tx, b, p, stream);
+      e = launch_kc<false, -1>(tx, tw, p, stream);
   } else {
-    e = launch_kc<true, -1>(tx, b, p, stream);
+    e = launch_kc<true, -1>(tx, tw, p, stream);
   }
   return e == cudaSuccess ? nullptr : cudaGetErrorString(e);
 }
@@ -1741,10 +1682,10 @@ int encode_pick_splits(int B, int H, int num_sms) {
   return (n_tiles + tps - 1) / tps;
 }
 
-int encode_pick_range(int B, int H, int num_sms, int* nsub, int* pair, bool any_batch) {
+int encode_pick_range(int B, int H, int num_sms, int* nsub, int* pair) {
   *nsub = 0;
   if (pair) *pair = 0;
-  if (tuning().encode_range == 0 || (B >= 16384 && !any_batch)) return 0;   // large batches: the multicast pairs take over
+  if (tuning().encode_range == 0 || B >= 16384) return 0;   // large batches: the multicast pairs take over
   const long long m_tiles = (B + BM - 1) / BM;
   const long long n_tiles = (H + BN - 1) / BN;
   const long long U = m_tiles * n_tiles;
@@ -1754,7 +1695,7 @@ int encode_pick_range(int B, int H, int num_sms, int* nsub, int* pair, bool any_
   const long long tps = (n_tiles + s - 1) / s;
   const double eff = (static_cast<double>(units) / (waves * num_sms)) *
                      (static_cast<double>(n_tiles) / (static_cast<double>(tps) * s));
-  if ((eff >= 0.95 && !any_batch) || U < 2ll * num_sms) return 0;
+  if (eff >= 0.95 || U < 2ll * num_sms) return 0;
   // cta_group::2 pairs on the range schedule: the units are (pair of row blocks, tile), one pair per two SMs. Halves the
   // W bytes every SM pulls from L2 (the single-CTA sweep runs at the L2 slice limit: 3.5 us per tile against 3.1 us
   // for the pair). Needs whole pairs of full row blocks.
@@ -1784,13 +1725,9 @@ void encode_pick_mode(int k_sel, int* mode, int* cap) {
   else *mode = 0;
 }
 
-// tensor maps of the W parts with the box the cluster variant loads (256 latents, or 128 per CTA of a pair)
-const char* make_b_maps(BMaps* bm, const uint16_t* const* parts, int n_parts, const EncodeLaunch& p) {
-  const int box = p.cluster ? BN / 2 : BN;
-  for (int i = 0; i < 3; ++i) {
-    const uint16_t* w = parts[i < n_parts ? i : 0];
-    if (!make_tmap_bf16(&bm->m[i], w, p.H, p.D, box)) return "cuTensorMapEncodeTiled(W) failed";
-  }
+// tensor map of W with the box the cluster variant loads (256 latents, or 128 per CTA of a pair)
+const char* make_w_map(CUtensorMap* tw, const uint16_t* w_bf16, const EncodeLaunch& p) {
+  if (!make_tmap_bf16(tw, w_bf16, p.H, p.D, p.cluster ? BN / 2 : BN)) return "cuTensorMapEncodeTiled(W) failed";
   return nullptr;
 }
 
@@ -1799,35 +1736,32 @@ const char* encode_topk_launch(const uint16_t* x_bf16, const uint16_t* w_bf16, E
   CUtensorMap tx;
   if (!make_tmap_bf16(&tx, x_bf16, p.B, p.D, BM)) return "cuTensorMapEncodeTiled(x) failed";
   p.dense_flags = 0;
-  p.k_parts = 1;
-  p.accum_mode = 0;
   p.cluster = p.range_g > 0 ? (p.range_pair ? 3 : 0) : pick_cluster(p, p.B >= 16384 ? 1 : 0);
-  BMaps bm;
-  if (const char* err = make_b_maps(&bm, &w_bf16, 1, p)) return err;
-  return launch_any<false>(tx, bm, p, stream);
+  CUtensorMap tw;
+  if (const char* err = make_w_map(&tw, w_bf16, p)) return err;
+  return launch_any<false>(tx, tw, p, stream);
 }
 
-const char* encode_dense_tc_launch(const uint16_t* x_bf16, const uint16_t* const* w_parts, int n_parts, EncodeLaunch p,
-                                   float* out_f32, uint16_t* out_hi, uint16_t* out_lo, cudaStream_t stream) {
+const char* encode_dense_tc_launch(const uint16_t* x_bf16, const uint16_t* w_bf16, EncodeLaunch p, float* out_f32,
+                                   uint16_t* out_hi, uint16_t* out_lo, cudaStream_t stream) {
   if ((p.H % 8) != 0) return "dense tensor-core encoder needs H % 8 == 0";
-  if (n_parts < 1 || n_parts > 3) return "dense tensor-core encoder: 1 to 3 parts of W";
   if ((reinterpret_cast<uintptr_t>(out_f32) | reinterpret_cast<uintptr_t>(out_hi) | reinterpret_cast<uintptr_t>(out_lo)) & 15)
     return "dense tensor-core encoder: outputs must be 16-byte aligned";
-  if (p.accum_mode != 0 && !out_f32) return "dense encoder: accumulating passes need the fp32 output";
-  if (p.act == 2 && (p.accum_mode != 0 || !p.step_scale || !p.step_level_start || !p.step_level_count || (p.H % 128) != 0))
-    return "dense encoder: the step-operand epilogue needs scale / levels / counts, H % 128 == 0 and a plain pass";
+  if (p.act == 2 && (!p.step_scale || !p.step_level_start || !p.step_level_count || (p.H % 128) != 0))
+    return "dense encoder: the step-operand epilogue needs scale / levels / counts and H % 128 == 0";
   if (p.act == 3) return "dense encoder: the ReLU-backward epilogue runs on the streamed-operand kernel only";
   CUtensorMap tx;
   if (!make_tmap_bf16(&tx, x_bf16, p.B, p.D, BM)) return "cuTensorMapEncodeTiled(x) failed";
   p.out_f32 = out_f32; p.out_hi = out_hi; p.out_lo = out_lo;
-  p.k_parts = n_parts;
   p.dense_flags = (out_f32 ? 1 : 0) | (out_hi ? 2 : 0) | (out_lo ? 4 : 0);
   if (p.dense_flags == 0) return "dense encoder: no output requested";
   if (tuning().dense_flags_mask >= 0) p.dense_flags &= tuning().dense_flags_mask;  // timing experiments only
-  p.cluster = p.range_g > 0 ? (p.range_pair ? 3 : 0) : pick_cluster(p, kDefaultClusterDense);
-  BMaps bm;
-  if (const char* err = make_b_maps(&bm, w_parts, n_parts, p)) return err;
-  return launch_any<true>(tx, bm, p, stream);
+  p.range_g = 0;
+  p.cluster = pick_cluster(p, kDefaultClusterDense);
+  if (p.cluster == 1) p.cluster = kDefaultClusterDense;   // no multicast variant: it gained nothing here (DESIGN.md 5.1)
+  CUtensorMap tw;
+  if (const char* err = make_w_map(&tw, w_bf16, p)) return err;
+  return launch_any<true>(tx, tw, p, stream);
 }
 
 const char* encode_dense_split_launch(const uint16_t* const* x_parts, const uint16_t* const* w_parts, int n_parts, EncodeLaunch p,
@@ -1845,8 +1779,6 @@ const char* encode_dense_split_launch(const uint16_t* const* x_parts, const uint
   if (p.act == 2 && (!p.step_scale || !p.step_level_start || !p.step_level_count || (p.H % 128) != 0))
     return "dense encoder: the step-operand epilogue needs scale / levels / counts and H % 128 == 0";
   p.out_f32 = out_f32; p.out_hi = out_hi; p.out_lo = out_lo;
-  p.k_parts = n_parts;
-  p.accum_mode = 0;
   p.range_g = 0;
   p.cluster = 2;
   p.dense_flags = (out_f32 ? 1 : 0) | (out_hi ? 2 : 0) | (out_lo ? 4 : 0);

@@ -22,23 +22,16 @@ constexpr int kPriorCounters = 4 + kRescueSlots;   // ints zeroed per call: [0] 
 // Tuning / diagnostic switches, read ONCE from the environment (never on a launch path); qsae_reload_tuning()
 // re-reads them (tests and tuning experiments that change the environment of a live process).
 struct Tuning {
-  int encode_splits;      // QSAE_ENCODE_SPLITS: latent-axis splits of the sweep (0 = automatic)
-  int encode_prior;       // QSAE_ENCODE_PRIOR: 0 switches the sampled prior off
   int encode_debug_mode;  // QSAE_ENCODE_DEBUG_MODE: timing experiments (EncodeLaunch::debug_mode)
-  int encode_cluster;     // QSAE_ENCODE_CLUSTER: 0 / 1 / 2 forces the cluster variant (-1 = automatic)
+  int encode_cluster;     // QSAE_ENCODE_CLUSTER: 0 / 1 / 2 forces the cluster variant (-1 = automatic; dense: 0 / 2)
   int encode_range;       // QSAE_ENCODE_RANGE: 0 keeps the (split, row block) grid at small batches
   int encode_range_pair;  // QSAE_ENCODE_RANGE_PAIR: 1 = cta_group::2 pairs on the range schedule (sparse sweeps)
   int encode_specialised; // QSAE_ENCODE_SPECIALISED: 0 = prior-threshold sweeps on the generic kernel (all modes compiled in)
-  int mat_bps;            // QSAE_MAT_BPS: 6 / 7 / 8 forces the resident blocks per SM of the q_sae level decoder (0 = automatic, -1 = always 6)
-  int prepass_range;      // QSAE_PREPASS_RANGE: 1 = sample pre-pass of large batches on the pair range schedule (experiment; no gain measured)
   int merge_tier;         // QSAE_MERGE_TIER: 8 / 12 / 16 forces the keys per lane of the warp merge (0 = from the expected survivor count)
   int sample_div;         // QSAE_SAMPLE_DIV: the sampled prior works on H / sample_div of the latents
   int prior_prep;         // QSAE_PRIOR_PREP: 0 keeps the separate cast / pre-pass / prior kernels
-  int dense_range;        // QSAE_DENSE_RANGE: dense epilogue (t_sae) on the range schedule: 1 = single CTAs, 2 = cta_group::2 pairs (experiments; both slower)
   int dense_flags_mask;   // QSAE_DENSE_FLAGS_MASK: masks dense epilogue outputs (-1 = off; timing experiments)
   int dense_step_fused;   // QSAE_DENSE_STEP_FUSED: 0 = q_sae dense path writes fp32 pre-activations and runs the separate operand kernel
-  int dense_fast_streamed;  // QSAE_DENSE_FAST_STREAMED: 1 = fast-mode dense encoder on the streamed-operand kernel (range schedule over CTA pairs)
-  int dense_split_fused;  // QSAE_DENSE_SPLIT_FUSED: 0 = exact dense encoder as three accumulating passes instead of the one-launch kernel
   int decode_pair;        // QSAE_DECODE_PAIR: 0 / 1 forces the decoder GEMM variant (-1 = automatic)
   int peer_timeout_ms;    // QSAE_PEER_TIMEOUT_MS: bound of a peer-memory flag wait (default 20000)
   int debug_large;        // QSAE_DEBUG_LARGE: survivor statistics of the large-k path on stderr (synchronises)
@@ -74,9 +67,6 @@ struct EncodeLaunch {
   float* cand_thr;      // [B][n_splits*2] inclusive lower bound of the row's k_sel-th largest value
   int cluster;          // 0 single CTA, 1 TMA-multicast pair, 2 cta_group::2 pair (set by the launcher)
   int dense_flags;      // dense epilogue outputs: 1 fp32, 2 bf16 hi, 4 bf16 lo (set by the launcher)
-  int k_parts;          // 1..3 bf16 parts of W contracted against the same x tile (set by the launcher)
-  int accum_mode;       // dense epilogue, split-operand passes: 0 off, 1 out = acc, 2 out += acc, 3 out = act(out + acc + bias)
-  const float* accum_bias;  // [H], added by the final accumulating pass
   float* out_f32;       // dense epilogue: [B, H] row-major outputs (set by the launcher)
   uint16_t* out_hi;
   uint16_t* out_lo;
@@ -97,9 +87,7 @@ struct EncodeLaunch {
 // encode_topk_sm100.cu
 int encode_pick_splits(int B, int H, int num_sms);
 // range schedule for this shape: CTAs to launch (0 = keep the (split, row block) grid) and lists per row
-// any_batch: also for B >= 16384 (short sweeps such as the sample pre-pass, where a (split, row block) CTA has only a
-// few tiles to amortise its x tile over)
-int encode_pick_range(int B, int H, int num_sms, int* nsub, int* pair = nullptr, bool any_batch = false);
+int encode_pick_range(int B, int H, int num_sms, int* nsub, int* pair = nullptr);
 void encode_pick_mode(int k_sel, int* mode, int* cap);
 const char* encode_topk_launch(const uint16_t* x_bf16, const uint16_t* w_bf16, EncodeLaunch p,
                                cudaStream_t stream);
@@ -122,15 +110,14 @@ struct PrepLaunch {
 int prior_prep_pick_ns(int B, int D, int n_sample, int m, int num_sms);
 const char* prior_prep_launch(const uint16_t* w_sample, const PrepLaunch& p, cudaStream_t stream);
 
-// dense epilogue variant (t_sae): h = act(x W^T + b) as fp32 and/or bf16 hi (+ lo) [B, H], TMA stores
-// w_parts: 1..3 bf16 matrices [H, D] whose sum is W (hi, mid, lo of a split fp32 matrix): all are contracted
-// against x into the same accumulator. p.accum_mode selects plain / accumulating output (see EncodeLaunch).
-const char* encode_dense_tc_launch(const uint16_t* x_bf16, const uint16_t* const* w_parts, int n_parts, EncodeLaunch p,
-                                   float* out_f32, uint16_t* out_hi, uint16_t* out_lo, cudaStream_t stream);
-// the same fp32-accurate product (x and W as three bf16 parts each, six partial products) in ONE launch: both operands
+// dense epilogue variant (t_sae fast mode, q_sae dense path): h = act(x W^T + b) from one bf16 product, written as fp32
+// and/or bf16 hi (+ lo) [B, H]; x tile resident, W streamed (single CTAs or cta_group::2 pairs, p.range_g ignored)
+const char* encode_dense_tc_launch(const uint16_t* x_bf16, const uint16_t* w_bf16, EncodeLaunch p, float* out_f32,
+                                   uint16_t* out_hi, uint16_t* out_lo, cudaStream_t stream);
+// the fp32-accurate product (x and W as three bf16 parts each, six partial products) in ONE launch: both operands
 // stream through the ring, every product lands in the same TMEM accumulator, the output is written once
 // (p.bias / p.act applied; p.n_tiles as for encode_dense_tc_launch; a range schedule over num_sms / 2 CTA pairs)
-// n_parts = 1: only the bf16 product x_parts[0] w_parts[0] (fast mode) on the same schedule
+// n_parts = 1: only the bf16 product x_parts[0] w_parts[0] (fast-mode t_sae backward) on the same schedule
 // n_w_parts = 1 with n_parts = 3: the three x parts against ONE W part (exact when W is bf16-representable, e.g. ternary)
 const char* encode_dense_split_launch(const uint16_t* const* x_parts, const uint16_t* const* w_parts, int n_parts, EncodeLaunch p,
                                       float* out_f32, uint16_t* out_hi, uint16_t* out_lo, int num_sms, cudaStream_t stream,

@@ -481,12 +481,9 @@ const char* decode_matryoshka_launch(const void* cand, const int* cand_cnt, int 
   // wave of 7 or 8 blocks per SM but not of 6 (B = 4096 on 148 SMs: 27.7 rows per SM against 24 warps) would run two
   // half-empty waves of a latency-bound kernel, so it takes the smallest occupancy that holds every row at once.
   int bps = 6;
-  if (tuning().mat_bps >= 6 && tuning().mat_bps <= 8) bps = tuning().mat_bps;
-  else if (tuning().mat_bps == 0) {
-    const long long rows_per_wave6 = static_cast<long long>(num_sms) * 6 * kMatWarps;
-    if (B > rows_per_wave6 && B <= static_cast<long long>(num_sms) * 7 * kMatWarps) bps = 7;
-    else if (B > rows_per_wave6 && B <= static_cast<long long>(num_sms) * 8 * kMatWarps) bps = 8;
-  }
+  const long long rows_per_wave6 = static_cast<long long>(num_sms) * 6 * kMatWarps;
+  if (B > rows_per_wave6 && B <= static_cast<long long>(num_sms) * 7 * kMatWarps) bps = 7;
+  else if (B > rows_per_wave6 && B <= static_cast<long long>(num_sms) * 8 * kMatWarps) bps = 8;
   int blocks = (B + kMatWarps - 1) / kMatWarps;
   if (blocks > num_sms * bps) blocks = num_sms * bps;   // = resident blocks
   (void)scratch;   // round 1: per-warp partial counts for a second kernel; the counts now leave through atomics

@@ -27,23 +27,16 @@ int env_int(const char* name, int dflt) {
 }  // namespace
 void reload_tuning() {
   Tuning t;
-  t.encode_splits = env_int("QSAE_ENCODE_SPLITS", 0);
-  t.encode_prior = env_int("QSAE_ENCODE_PRIOR", 1);
   t.encode_debug_mode = env_int("QSAE_ENCODE_DEBUG_MODE", 0);
   t.encode_cluster = env_int("QSAE_ENCODE_CLUSTER", -1);
   t.encode_range = env_int("QSAE_ENCODE_RANGE", 1);
   t.encode_range_pair = env_int("QSAE_ENCODE_RANGE_PAIR", 1);
   t.encode_specialised = env_int("QSAE_ENCODE_SPECIALISED", 1);
   t.prior_prep = env_int("QSAE_PRIOR_PREP", 1);
-  t.mat_bps = env_int("QSAE_MAT_BPS", 0);
-  t.prepass_range = env_int("QSAE_PREPASS_RANGE", 0);
   t.merge_tier = env_int("QSAE_MERGE_TIER", 0);
   t.sample_div = env_int("QSAE_SAMPLE_DIV", 16);
   if (t.sample_div < 8) t.sample_div = 8;   // the plan samples only when H >= 8 n_sample
-  t.dense_range = env_int("QSAE_DENSE_RANGE", 0);
   t.dense_flags_mask = env_int("QSAE_DENSE_FLAGS_MASK", -1);
-  t.dense_split_fused = env_int("QSAE_DENSE_SPLIT_FUSED", 1);
-  t.dense_fast_streamed = env_int("QSAE_DENSE_FAST_STREAMED", 0);
   t.dense_step_fused = env_int("QSAE_DENSE_STEP_FUSED", 1);
   t.decode_pair = env_int("QSAE_DECODE_PAIR", -1);
   t.peer_timeout_ms = env_int("QSAE_PEER_TIMEOUT_MS", 20000);
@@ -111,19 +104,15 @@ struct StagePlan {
 
 enum StageKind { kStageClassBound = 0, kStagePriorMain = 1, kStageSamplePre = 2 };
 
-// D: width of the contraction when the caller allows the range schedule (the pair variant exists for D = 512 only)
-void plan_stage(int B, int H, int k_sel, StageKind kind, bool allow_split_override, size_t base, StagePlan* sp,
-                bool allow_range = false, int D = 0) {
+// allow_range (prior-threshold sweeps): the range schedule at small batches; D: width of the contraction (the pair
+// variant exists for D = 512 only)
+void plan_stage(int B, int H, int k_sel, StageKind kind, size_t base, StagePlan* sp, bool allow_range = false, int D = 0) {
   sp->H = H;
   sp->k_sel = k_sel;
   sp->range_g = 0;
   sp->range_pair = 0;
   sp->n_tiles = (H + kEncBN - 1) / kEncBN;
   sp->n_splits = encode_pick_splits(B, H, num_sms());
-  if (allow_split_override) {
-    const int s = tuning().encode_splits;   // tuning experiments only
-    if (s >= 1 && s <= kMaxSplits && s <= sp->n_tiles) sp->n_splits = s;
-  }
   if (kind == kStageSamplePre && (B + kEncBM - 1) / kEncBM >= num_sms()) sp->n_splits = 1;  // enough row blocks
   if (kind == kStageSamplePre && sp->n_splits > 4) sp->n_splits = 4;   // the prior kernel sorts at most 8 x kTopM values per row
   sp->tiles_per_split = (sp->n_tiles + sp->n_splits - 1) / sp->n_splits;
@@ -131,20 +120,8 @@ void plan_stage(int B, int H, int k_sel, StageKind kind, bool allow_split_overri
   if (kind == kStageSamplePre) {
     sp->mode = 5;   // register-resident class top-2, no survivor buffers: cand region = the kept values
     sp->cap = 0;
-    // Large batches: a (1 split, row block) CTA sweeps only the sample's few tiles (8 at H = 32768) per x tile and 512
-    // CTAs make 3.46 waves on 148 SMs. Experiment (QSAE_PREPASS_RANGE=1, off by default): CTA pairs on the range
-    // schedule sweep ~28 contiguous units each on every SM; a row block is then shared by at most two pairs (4 lists of
-    // kTopM values per row). Measured at B = 65536: pre-pass 139 -> 124 us (each of a range's 3-4 x-tile reloads drains
-    // the MMA pipeline) but the prior kernel reads twice the values (+15 us): no gain.
-    if (allow_range && tuning().prepass_range != 0 && sp->n_splits == 1 && (B + kEncBM - 1) / kEncBM >= num_sms() && D > 448) {
-      int range_nsub = 0, range_pair = 0;
-      const int g = encode_pick_range(B, H, num_sms(), &range_nsub, &range_pair, true);
-      if (g > 0 && range_pair && range_nsub <= 8) {
-        sp->range_g = g;
-        sp->range_pair = 1;
-        sp->nsub = range_nsub;
-      }
-    }
+    // Large batches stay on the (1 split, row block) grid: the range schedule shortened the pre-pass but doubled the
+    // values the prior kernel reads, no gain (profiles/r2s3_measurements.md 3f)
     sp->cand_off = align_up(base, 256);
     sp->cnt_off = sp->thr_off = sp->cand_off;
     sp->end = align_up(sp->cand_off + static_cast<size_t>(B) * sp->nsub * kTopM * 4, 256);
@@ -157,8 +134,7 @@ void plan_stage(int B, int H, int k_sel, StageKind kind, bool allow_split_overri
     // covers ~1 / nsub of a row's latents (a few dozen survivors), so 256 entries are plenty (a full list is cut
     // exactly in the kernel, as always)
     int range_nsub = 0, range_pair = 0;
-    const int g = (allow_range && tuning().encode_splits == 0)
-                      ? encode_pick_range(B, H, num_sms(), &range_nsub, D > 448 ? &range_pair : nullptr) : 0;
+    const int g = allow_range ? encode_pick_range(B, H, num_sms(), &range_nsub, D > 448 ? &range_pair : nullptr) : 0;
     if (g > 0) {
       sp->range_g = g;
       sp->range_pair = range_pair;
@@ -219,14 +195,14 @@ int plan_encode(int B, int H, int D, int k, int exact, int n_sample, EncodePlan*
     // the warp merge holds 512 survivors per row in registers; the prior pays while mean + sigma of the survivor
     // count (m / r, sqrt(m) / r) stays inside (k_sel <= 128 at r = 1 / 16), above that the class-bound modes take over
     const bool fits = (m + sqrt(static_cast<double>(m))) * (static_cast<double>(H) / n_sample) <= 512.0;
-    if (tuning().encode_prior != 0 && m <= kPriorMaxRank && m <= n_sample && fits) {
+    if (m <= kPriorMaxRank && m <= n_sample && fits) {
       pl->use_prior = true;
       pl->m = m;
     }
   }
   pl->x_off = 0;
   size_t off = align_up(static_cast<size_t>(B) * D * 2, 1024);
-  plan_stage(B, H, k_sel, pl->use_prior ? kStagePriorMain : kStageClassBound, true, off, &pl->main, true, D);
+  plan_stage(B, H, k_sel, pl->use_prior ? kStagePriorMain : kStageClassBound, off, &pl->main, true, D);
   off = pl->main.end;
   pl->counters_off = off; off += 256;
   pl->rescue_rows_off = off; off = align_up(off + static_cast<size_t>(B) * 4, 256);
@@ -234,7 +210,7 @@ int plan_encode(int B, int H, int D, int k, int exact, int n_sample, EncodePlan*
     pl->prior_off = off; off = align_up(off + static_cast<size_t>(B) * 4, 256);
     pl->ovf_rows_off = off; off = align_up(off + static_cast<size_t>(B) * 4, 256);
     pl->rescue_z_off = off; off = align_up(off + static_cast<size_t>(kRescueSlots) * H * 4, 256);
-    plan_stage(B, n_sample, pl->m, kStageSamplePre, false, off, &pl->pre, true, D);
+    plan_stage(B, n_sample, pl->m, kStageSamplePre, off, &pl->pre);
     off = pl->pre.end;
   }
   pl->total = off;
@@ -293,7 +269,7 @@ int plan_encode_large(int B, int H, int D, int k, int exact, int n_sample, Large
     const double r = static_cast<double>(n_sample) / H;
     const int m = choose_prior_rank(k_sel, r);
     if (m <= kMaxK && m <= n_sample) {
-      plan_stage(B, H, 0, kStagePriorMain, true, off, &lp->main);
+      plan_stage(B, H, 0, kStagePriorMain, off, &lp->main);
       // survivors of a row = rank of the m-th largest sample value in the full row: mean m / r, standard
       // deviation ~ sqrt(m) / r (negative binomial); a list holds 1 / nsub of them (+ Poisson spread).
       // Lists sized for mean + 7 sigma of both: a filled list costs an exact recomputation of the row.
@@ -319,7 +295,7 @@ int plan_encode_large(int B, int H, int D, int k, int exact, int n_sample, Large
     lp->pre_vals_off = off; off = align_up(off + static_cast<size_t>(B) * lp->m * 4, 256);
     lp->pre_idx_off = off; off = align_up(off + static_cast<size_t>(B) * lp->m * 4, 256);
     lp->scratch_off = off; off = align_up(off + rescue_large_scratch_bytes(H, num_sms()), 256);
-    plan_stage(B, n_sample, lp->m, kStageClassBound, false, off, &lp->pre);
+    plan_stage(B, n_sample, lp->m, kStageClassBound, off, &lp->pre);
     off = lp->pre.end;
   } else {
     // dense pre-activations in row chunks of at most ~1 GB
@@ -329,7 +305,7 @@ int plan_encode_large(int B, int H, int D, int k, int exact, int n_sample, Large
     if (rows > B) rows = B;
     lp->chunk_rows = static_cast<int>(rows);
     lp->z_off = off; off = align_up(off + static_cast<size_t>(rows) * H * 4, 256);
-    plan_stage(static_cast<int>(rows), H, 1, kStageClassBound, false, off, &lp->dense);
+    plan_stage(static_cast<int>(rows), H, 1, kStageClassBound, off, &lp->dense);
     off = lp->dense.end;
   }
   lp->total = off;
@@ -816,7 +792,7 @@ int plan_matryoshka(int B, int H, int D, MatPlan* mp) {
     return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka: D must be a multiple of 16 in [16, 512], got %d", D);
   mp->x_off = 0;
   mp->prior_off = align_up(static_cast<size_t>(B) * D * 2, 1024);
-  plan_stage(B, H, 0, kStagePriorMain, false, mp->prior_off + align_up(static_cast<size_t>(B) * 4, 256), &mp->st, true, D);
+  plan_stage(B, H, 0, kStagePriorMain, mp->prior_off + align_up(static_cast<size_t>(B) * 4, 256), &mp->st, true, D);
   // every active latent is kept: largest buffers. Range schedule: more, shorter lists per row (the same capacity per row)
   mp->st.cap = mp->st.range_g > 0 ? kCandCapMax / 2 : kCandCapMax;
   mp->st.cnt_off = mp->st.cand_off + static_cast<size_t>(B) * mp->st.nsub * mp->st.cap * 8;
@@ -1121,15 +1097,10 @@ int qsae_decode_dense(const uint16_t* a_hi, const uint16_t* a_lo, const uint16_t
 
 namespace {
 // Dense pre-activations (+ activation) on the tensor cores.
-//   w_mid == w_lo == nullptr: one pass over bf16(x) and w_hi (fast mode).
+//   w_mid == w_lo == nullptr: one pass over bf16(x) and w_hi (fast mode; encode_dense_tc_launch).
 //   otherwise: fp32-accurate product through 8 + 8 + 8-bit operand splits, x = xh + xm + xl and
-//   W = wh + wm + wl (both exact), keeping the six partial products above 2^-24 -- by default in ONE launch
-//   (encode_dense_split_kernel: both operands streamed, one accumulator, outputs written once); with
-//   QSAE_DENSE_SPLIT_FUSED=0 as the three accumulating passes of the first version:
-//     pass 1: xh * (wh + wm + wl) -> out      pass 2: out += xm * (wh + wm)
-//     pass 3: out = act(out + xl * wh + bias), bf16 hi (+ lo) of the result written alongside.
-//   Each pass is one launch of the dense encoder kernel (the x tile is resident in shared memory, the W
-//   parts stream through the ring into the same TMEM accumulator).
+//   W = wh + wm + wl (both exact), keeping the six partial products above 2^-24 in ONE launch
+//   (encode_dense_split_kernel: both operands streamed, one accumulator, outputs written once).
 // x_parts: workspace for the bf16 part(s) of x, 3 * align_up(B * D * 2, 1024) bytes in split mode.
 // step: act == 2 only (EncodeLaunch::step_*): the q_sae dense path's A operand written by the epilogue.
 struct StepOperand { float thr; const float* scale; const int* level_start; int n_levels; unsigned long long* level_count; };
@@ -1147,29 +1118,14 @@ int dense_encode_tc(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_
   el.n_tiles = (H + kEncBN - 1) / kEncBN;
   el.n_splits = encode_pick_splits(B, H, num_sms());
   el.tiles_per_split = (el.n_tiles + el.n_splits - 1) / el.n_splits;
-  if (tuning().dense_range == 1) {   // one CTA per SM over contiguous tile ranges (single-CTA variant) instead of CTA pairs
-    int unused = 0;
-    el.range_g = encode_pick_range(B, H, num_sms(), &unused);
-  } else if (tuning().dense_range == 2 && D > 448) {   // cta_group::2 pairs ON the range schedule (all SMs at small batches)
-    int unused = 0, pair = 0;
-    const int g = encode_pick_range(B, H, num_sms(), &unused, &pair);
-    if (g > 0 && pair) { el.range_g = g; el.range_pair = 1; }
-  }
   const size_t xn = static_cast<size_t>(B) * D;
   const size_t xstride = align_up(xn * 2, 1024);
   uint16_t* xh = reinterpret_cast<uint16_t*>(x_parts);
   if (!w_mid || !w_lo) {
     int rc = launch_status("cast x", cast_bf16_launch(x_f32, xh, xn, st));
     if (rc != QSAE_OK) return rc;
-    const uint16_t* parts[1] = {w_hi};
     if (g_enc_ev_start) cudaEventRecord(g_enc_ev_start, st);
-    if (tuning().dense_fast_streamed != 0 && tuning().dense_range != 1) {
-      const uint16_t* xp[1] = {xh};
-      rc = launch_status("encode kernel (dense, streamed operands)",
-                         encode_dense_split_launch(xp, parts, 1, el, out_f32, out_hi, out_lo, num_sms(), st));
-    } else {
-      rc = launch_status("encode kernel (dense)", encode_dense_tc_launch(xh, parts, 1, el, out_f32, out_hi, out_lo, st));
-    }
+    rc = launch_status("encode kernel (dense)", encode_dense_tc_launch(xh, w_hi, el, out_f32, out_hi, out_lo, st));
     if (g_enc_ev_stop) cudaEventRecord(g_enc_ev_stop, st);
     return rc;
   }
@@ -1177,31 +1133,10 @@ int dense_encode_tc(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_
   uint16_t* xl = reinterpret_cast<uint16_t*>(x_parts + 2 * xstride);
   int rc = launch_status("split x", split_bf16x3_launch(x_f32, xh, xm, xl, xn, st));
   if (rc != QSAE_OK) return rc;
-  if (act == 2 && !(tuning().dense_split_fused != 0 && tuning().dense_range != 1))
-    return fail(QSAE_ERR_INVALID_ARGUMENT, "dense encoder: the step operand needs the one-launch split kernel");
-  if (tuning().dense_split_fused != 0 && tuning().dense_range != 1) {
-    // one launch: all six partial products into one TMEM accumulator, outputs written once
-    const uint16_t* xp[3] = {xh, xm, xl};
-    const uint16_t* wp[3] = {w_hi, w_mid, w_lo};
-    if (g_enc_ev_start) cudaEventRecord(g_enc_ev_start, st);
-    rc = launch_status("encode kernel (dense, split operands)", encode_dense_split_launch(xp, wp, 3, el, out_f32, out_hi, out_lo, num_sms(), st));
-    if (g_enc_ev_stop) cudaEventRecord(g_enc_ev_stop, st);
-    return rc;
-  }
-  el.bias = nullptr;            // the kernel's bias loader treats a null bias as zeros; the final pass adds b_enc
-  el.accum_bias = b_enc;
-  const uint16_t* p1[3] = {w_hi, w_mid, w_lo};
-  const uint16_t* p2[2] = {w_hi, w_mid};
-  const uint16_t* p3[1] = {w_hi};
+  const uint16_t* xp[3] = {xh, xm, xl};
+  const uint16_t* wp[3] = {w_hi, w_mid, w_lo};
   if (g_enc_ev_start) cudaEventRecord(g_enc_ev_start, st);
-  el.accum_mode = 1;
-  rc = launch_status("encode kernel (dense, xh)", encode_dense_tc_launch(xh, p1, 3, el, out_f32, nullptr, nullptr, st));
-  if (rc != QSAE_OK) return rc;
-  el.accum_mode = 2;
-  rc = launch_status("encode kernel (dense, xm)", encode_dense_tc_launch(xm, p2, 2, el, out_f32, nullptr, nullptr, st));
-  if (rc != QSAE_OK) return rc;
-  el.accum_mode = 3;
-  rc = launch_status("encode kernel (dense, xl)", encode_dense_tc_launch(xl, p3, 1, el, out_f32, out_hi, out_lo, st));
+  rc = launch_status("encode kernel (dense, split operands)", encode_dense_split_launch(xp, wp, 3, el, out_f32, out_hi, out_lo, num_sms(), st));
   if (g_enc_ev_stop) cudaEventRecord(g_enc_ev_stop, st);
   return rc;
 }
@@ -1481,8 +1416,7 @@ int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, cons
   // 2. A = active * scale, split into bf16 hi / lo; activity counts per level -- written by the encoder's
   //    epilogue itself when the level boundaries are multiples of 128 (the fp32 pre-activations never reach
   //    HBM: 1.07 GB of traffic and two launches less at B = 4096, H = 32768), else by a streaming kernel
-  bool fuse_step = tuning().dense_step_fused != 0 && tuning().dense_range != 1 &&
-                   ((w_mid == nullptr || w_lo == nullptr) || tuning().dense_split_fused != 0);
+  bool fuse_step = tuning().dense_step_fused != 0;
   for (int i = 0; i <= n_levels; ++i) fuse_step = fuse_step && (level_start_host[i] % 128) == 0;
   if (fuse_step) {
     const StepOperand so = {kActiveThreshold, scale, level_start_dev, n_levels, level_count};
