@@ -279,6 +279,15 @@ int qsae_activation_counts(const int32_t* idx, const float* vals, int B, int cap
 int qsae_coactivation(const int32_t* idx, const float* vals, int B, int cap, int H, int32_t* cooc /* [H, H] */,
                       void* stream);
 int qsae_sq_error_accumulate(const float* a, const float* b, size_t n, double* out /* device scalar */, void* stream);
+/* The same statistics from a dense activity mask, for rows whose active sets are too long for the lists (a q_sae at
+ * high activity; qsae_matryoshka_forward_dense_active writes the mask): cooc[i * H + j] += sum_k M[k, i] M[k, j] for
+ * mask [K, H] bf16 0.0 / 1.0, row-major, and counts[h] += sum_k M[k, h] (counts may be NULL). A tcgen05 product over
+ * the tiles of the upper triangle; each element is added to cooc[m, n] and cooc[n, m] by one thread, so there are no
+ * atomics, the result is bit-deterministic and cooc is complete and symmetric after every call (list and mask batches
+ * may add into the same matrix in any order). H % 8 == 0, K <= 2^24 (fp32 accumulation of 0/1 products is exact there);
+ * mask and cooc 16-byte aligned. */
+int qsae_coactivation_dense(const uint16_t* mask /* [K, H] */, int K, int H, int32_t* cooc /* [H, H] */,
+                            long long* counts /* [H] or NULL */, void* stream);
 
 /* Dense [B, H] latents (what the reference hands to its decoders: sae/binary.py:24, sae/quantized_matryoshka.py:47)
  * -> sparse per-row lists, ascending latent order. mode 0: entries != 0; mode 1: entries > thr (q_sae activity, :99).
@@ -304,6 +313,18 @@ int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, cons
                                   int D, float* result /* [n_levels, B, D] */,
                                   unsigned long long* level_count /* [n_levels] */, void* workspace,
                                   size_t workspace_bytes, void* stream);
+/* The same forward, also writing its activity mask: active_mask[b * mask_pitch + mask_col + h] = 1.0 (bf16) where
+ * latent h of row b is active (sigmoid(z) > 0.5, the decision that forms A; a latent with a zero decoder scale is still
+ * active), else 0.0. mask_pitch and mask_col are multiples of 8 with mask_col + H <= mask_pitch, so the stages of an
+ * rq_sae can write side by side into one [B, sum of stage widths] mask. Input for qsae_coactivation_dense. */
+int qsae_matryoshka_forward_dense_active(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_mid,
+                                         const uint16_t* w_lo, const float* b_enc, const uint16_t* t_bf16,
+                                         const float* scale, const int* level_start_dev, const int* level_start_host,
+                                         int n_levels, const float* dec_bias, int B, int H, int D,
+                                         float* result /* [n_levels, B, D] */,
+                                         unsigned long long* level_count /* [n_levels] */,
+                                         uint16_t* active_mask /* [B, mask_pitch] */, int mask_pitch, int mask_col,
+                                         void* workspace, size_t workspace_bytes, void* stream);
 
 /* rq_sae (ResidualQuantizedSAE.forward, sae/residual_quantized.py:53-69): a cascade of one-bit q_saes, each
  * run with qsae_matryoshka_forward (n_levels = 1) on the residual of the previous stage;

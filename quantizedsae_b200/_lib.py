@@ -55,6 +55,7 @@ SYMBOLS = {
                                             _vp, _i, _vp, _vp, _vp, _sz, _vp]),
     "qsae_activation_counts": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "qsae_coactivation": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
+    "qsae_coactivation_dense": (_i, [_vp, _i, _i, _vp, _vp, _vp]),
     "qsae_sq_error_accumulate": (_i, [_vp, _vp, _sz, _vp, _vp]),
     "qsae_compact_dense": (_i, [_vp, _i, _i, _i, _f, _i, _vp, _vp, _vp, _vp, _vp]),
     "qsae_max_row_norm": (_i, [_vp, _i, _i, _vp, _vp]),
@@ -63,6 +64,8 @@ SYMBOLS = {
     "qsae_matryoshka_dense_workspace_bytes": (_i, [_i, _i, _i, C.POINTER(_sz)]),
     "qsae_matryoshka_forward_dense": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(_i), _i, _vp, _i, _i, _i, _vp,
                                            _vp, _vp, _sz, _vp]),
+    "qsae_matryoshka_forward_dense_active": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(_i), _i, _vp, _i, _i, _i,
+                                                  _vp, _vp, _vp, _i, _i, _vp, _sz, _vp]),
     "qsae_decode_matryoshka_lists_workspace_bytes": (_i, [C.POINTER(_sz)]),
     "qsae_decode_matryoshka_lists": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "qsae_pack_ternary": (_i, [_vp, _i, _i, _f, _vp, _vp, _vp]),
@@ -482,6 +485,16 @@ def coactivation(idx: torch.Tensor, vals: torch.Tensor | None, cooc: torch.Tenso
     check(load().qsae_coactivation(idx.data_ptr(), _ptr(vals), B, cap, cooc.shape[0], cooc.data_ptr(), _stream()))
 
 
+def coactivation_dense(mask: torch.Tensor, cooc: torch.Tensor, counts: torch.Tensor | None = None) -> None:
+    """cooc [H, H] int32 += mask^T mask and counts [H] int64 += mask.sum(0), for a bf16 0/1 activity mask [K, H]
+    (tensor cores; K <= 2^24, H % 8 == 0)."""
+    _need_cuda(mask, cooc, counts)
+    assert mask.dtype == torch.bfloat16 and mask.dim() == 2 and cooc.dtype == torch.int32
+    K, H = mask.shape
+    assert cooc.shape == (H, H) and (counts is None or (counts.dtype == torch.int64 and counts.numel() == H))
+    check(load().qsae_coactivation_dense(mask.data_ptr(), K, H, cooc.data_ptr(), _ptr(counts), _stream()))
+
+
 def sq_error_accumulate(a: torch.Tensor, b: torch.Tensor, out: torch.Tensor) -> None:
     """out (device float64 scalar) += sum (a - b)^2."""
     _need_cuda(a, b, out)
@@ -822,9 +835,11 @@ def unpack_matryoshka_t(packed: torch.Tensor, D: int) -> torch.Tensor:
     return t
 
 
-def matryoshka_forward_dense(x, w_parts, b_enc, t_bf16, scale, level_start_dev, level_start_host, dec_bias):
+def matryoshka_forward_dense(x, w_parts, b_enc, t_bf16, scale, level_start_dev, level_start_host, dec_bias,
+                             mask=None, mask_col=0):
     """Dense q_sae forward -> (result [n_levels, B, D] f32, level_count [n_levels] int64).
-    w_parts: (bf16(W),) or split_bf16x3(W) for fp32-accurate activity decisions."""
+    w_parts: (bf16(W),) or split_bf16x3(W) for fp32-accurate activity decisions. mask: bf16 [B, P] that also receives
+    the activity (1.0 = active) in columns [mask_col, mask_col + H) (qsae_matryoshka_forward_dense_active)."""
     w_hi = w_parts[0]
     w_mid, w_lo = (w_parts[1], w_parts[2]) if len(w_parts) == 3 else (None, None)
     _need_cuda(x, w_hi, w_mid, w_lo, b_enc, t_bf16, scale, level_start_dev, dec_bias)
@@ -839,6 +854,14 @@ def matryoshka_forward_dense(x, w_parts, b_enc, t_bf16, scale, level_start_dev, 
     check(load().qsae_matryoshka_dense_workspace_bytes(B, H, D, C.byref(n)))
     ws = _workspace(x.device, int(n.value))
     starts = (_i * (n_levels + 1))(*[int(v) for v in level_start_host])
+    if mask is not None:
+        _need_cuda(mask)
+        assert mask.dtype == torch.bfloat16 and mask.dim() == 2 and mask.shape[0] == B
+        check(load().qsae_matryoshka_forward_dense_active(
+            x.data_ptr(), w_hi.data_ptr(), _ptr(w_mid), _ptr(w_lo), b_enc.data_ptr(), t_bf16.data_ptr(), scale.data_ptr(),
+            level_start_dev.data_ptr(), starts, n_levels, _ptr(dec_bias), B, H, D, result.data_ptr(), counts.data_ptr(),
+            mask.data_ptr(), mask.shape[1], int(mask_col), ws.data_ptr(), ws.numel(), _stream()))
+        return result, counts
     check(load().qsae_matryoshka_forward_dense(x.data_ptr(), w_hi.data_ptr(), _ptr(w_mid), _ptr(w_lo), b_enc.data_ptr(),
                                                t_bf16.data_ptr(),
                                                scale.data_ptr(), level_start_dev.data_ptr(), starts, n_levels,

@@ -615,6 +615,7 @@ __device__ __forceinline__ void epilogue_dense(const EncodeLaunch& p, int n_my_t
         for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(fmaxf(__uint_as_float(r[j]), 0.f));
       }
       if (!warp_live || col0 >= p.H) continue;  // warp-uniform
+      uint32_t act_bits = 0u;   // act == 2: bit j = column col0 + j of this lane's row is active
       if (p.act == 2) {
         // q_sae dense path: r = active ? scale[col] : 0 (the A operand of the level GEMMs; hi / lo leave below)
         const float4* sc4 = reinterpret_cast<const float4*>(p.step_scale + col0);
@@ -625,6 +626,7 @@ __device__ __forceinline__ void epilogue_dense(const EncodeLaunch& p, int n_my_t
           const bool a0 = __uint_as_float(r[4 * j + 0]) >= p.step_thr, a1 = __uint_as_float(r[4 * j + 1]) >= p.step_thr;
           const bool a2 = __uint_as_float(r[4 * j + 2]) >= p.step_thr, a3 = __uint_as_float(r[4 * j + 3]) >= p.step_thr;
           n += (a0 ? 1u : 0u) + (a1 ? 1u : 0u) + (a2 ? 1u : 0u) + (a3 ? 1u : 0u);
+          act_bits |= ((a0 ? 1u : 0u) | (a1 ? 2u : 0u) | (a2 ? 4u : 0u) | (a3 ? 8u : 0u)) << (4 * j);
           r[4 * j + 0] = a0 ? __float_as_uint(s.x) : 0u;
           r[4 * j + 1] = a1 ? __float_as_uint(s.y) : 0u;
           r[4 * j + 2] = a2 ? __float_as_uint(s.z) : 0u;
@@ -765,6 +767,25 @@ __device__ __forceinline__ void epilogue_dense(const EncodeLaunch& p, int n_my_t
             if (row0 + rr < p.B && col0 + h_col < p.H)
               *reinterpret_cast<uint4*>(p.out_lo + static_cast<size_t>(row0 + rr) * H + col0 + h_col) = v;
           }
+        }
+      }
+      if (p.act == 2 && p.step_mask != nullptr) {
+        // activity mask of the same decisions: bf16 1.0 (0x3F80) / 0, through the staging layout of the bf16 outputs
+        uint32_t mk[16];
+#pragma unroll
+        for (int j = 0; j < 16; ++j)
+          mk[j] = (((act_bits >> (2 * j)) & 1u) ? 0x3F80u : 0u) | (((act_bits >> (2 * j + 1)) & 1u) ? 0x3F800000u : 0u);
+        __syncwarp();
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+          st_shared_v4(st + lane * 64 + ((q ^ ((lane >> 1) & 3)) << 4), mk[4 * q], mk[4 * q + 1], mk[4 * q + 2], mk[4 * q + 3]);
+        __syncwarp();
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const int rr = 8 * j + h_row;
+          const uint4 v = ld_shared_v4(st + rr * 64 + (((lane & 3) ^ ((rr >> 1) & 3)) << 4));
+          if (row0 + rr < p.B && col0 + h_col < p.H)
+            *reinterpret_cast<uint4*>(p.step_mask + static_cast<size_t>(row0 + rr) * p.step_mask_pitch + col0 + h_col) = v;
         }
       }
     }

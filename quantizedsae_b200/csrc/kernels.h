@@ -76,6 +76,8 @@ struct EncodeLaunch {
   const int* step_level_start;        // [step_n_levels + 1] device, multiples of 128
   int step_n_levels;
   unsigned long long* step_level_count;   // [step_n_levels] += active (row, latent) pairs per level
+  uint16_t* step_mask;                // or null: bf16 activity mask, 1.0 where z >= step_thr; row r at step_mask + r * pitch
+  int step_mask_pitch;                // elements, a multiple of 8
   // act == 3 (t_sae backward: gz = (g T + g_h) * 1[h > 0] straight from the accumulator of g T)
   const float* gate;      // [B, H] the forward's ReLU output h
   const float* gate_add;  // [B, H] d loss / d h, or null
@@ -138,6 +140,11 @@ const char* dense_decode_launch(const uint16_t* a_hi, const uint16_t* a_lo, int 
 // b_parts: row-major [K, N]; a_parts: row-major [K, M], or [M, K] when a_kmajor. n_parts = 1 (one product) or 3 (the six
 // products of three-part splits above 2^-24, one accumulator). N and the row pitch of A multiples of 8; c [M, N] fp32,
 // overwritten.
+// cooc[H, H] int32 += M^T M of a bf16 0/1 mask M [K, H] (K <= 2^24, H % 8 == 0), upper-triangle tiles only, each
+// product element added to cooc[m, n] and, for n > m, to cooc[n, m] (one writer per element, no atomics);
+// counts[h] += the diagonal (or null)
+const char* coactivation_dense_launch(const uint16_t* mask, int K, int H, int32_t* cooc, long long* counts, int num_sms,
+                                      cudaStream_t stream);
 const char* wgrad_launch(const uint16_t* const* a_parts, const uint16_t* const* b_parts, int n_parts, int M, int N, int K,
                          bool a_kmajor, float* c, int num_sms, cudaStream_t stream);
 
@@ -281,10 +288,12 @@ const char* decode_matryoshka_launch(const void* cand, const int* cand_cnt, int 
 size_t decode_matryoshka_scratch_bytes(int num_sms);
 // packed 2-bit codes [H, D/16] -> T^T as bf16 [D, H] with entries {-2, 0, +2} (B operand of the dense level GEMMs)
 const char* unpack_matryoshka_t_launch(const uint32_t* packed, int H, int D, uint16_t* t_bf16, cudaStream_t stream);
-// z [B, H] -> a = (z >= thr) * scale[h] split into bf16 hi / lo [B, H]; level_count[l] += active entries of level l
+// z [B, H] -> a = (z >= thr) * scale[h] split into bf16 hi / lo [B, H]; level_count[l] += active entries of level l;
+// mask (or null): bf16 1.0 / 0.0 = (z >= thr), row b at mask + b * mask_pitch (a multiple of 8 elements)
 const char* matryoshka_dense_operand_launch(const float* z, int B, int H, const float* scale, float thr,
                                             const int* level_start, int n_levels, uint16_t* a_hi, uint16_t* a_lo,
-                                            unsigned long long* level_count, void* scratch, cudaStream_t stream);
+                                            unsigned long long* level_count, void* scratch, cudaStream_t stream,
+                                            uint16_t* mask = nullptr, int mask_pitch = 0);
 size_t matryoshka_dense_operand_scratch_bytes();
 const char* matryoshka_dense_tail_launch(const uint16_t* a_hi, const uint16_t* a_lo, const uint16_t* t_bf16,
                                         const int* level_start, int n_levels, int B, int H, int D, const float* bias,

@@ -113,14 +113,16 @@ __global__ void unpack_matryoshka_t_kernel(const uint32_t* __restrict__ packed, 
   }
 }
 
-// a[b, h] = (z[b, h] >= thr) ? scale[h] : 0, as bf16 hi + lo (hi + lo = scale to 2^-17); per-level activity counts.
+// a[b, h] = (z[b, h] >= thr) ? scale[h] : 0, as bf16 hi + lo (hi + lo = scale to 2^-17); per-level activity counts;
+// with a mask, also mask[b * mask_pitch + h] = bf16 (z[b, h] >= thr) (the activity itself: a zero scale is still active).
 // HBM-streaming (4 B read, 4 B written per element): 8 consecutive latents per thread through 16-byte accesses. A
 // group's count is added once per warp when the warp's groups lie inside one level (the usual case), else per lane;
 // a group that straddles a level boundary (boundaries need not be multiples of 8) is counted element by element.
 __global__ void __launch_bounds__(256)
 matryoshka_dense_operand_kernel(const float* __restrict__ z, int B, int H, const float* __restrict__ scale, float thr,
                                 const int* __restrict__ level_start, int n_levels, uint16_t* __restrict__ a_hi,
-                                uint16_t* __restrict__ a_lo, unsigned* __restrict__ count_partial /* [gridDim.x, 32] */) {
+                                uint16_t* __restrict__ a_lo, unsigned* __restrict__ count_partial /* [gridDim.x, 32] */,
+                                uint16_t* __restrict__ mask, int mask_pitch) {
   __shared__ unsigned s_cnt[32];
   __shared__ int s_start[33];
   if (threadIdx.x < 32) s_cnt[threadIdx.x] = 0u;
@@ -162,6 +164,13 @@ matryoshka_dense_operand_kernel(const float* __restrict__ z, int B, int H, const
       }
       *reinterpret_cast<uint4*>(a_hi + g * 8) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
       *reinterpret_cast<uint4*>(a_lo + g * 8) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+      if (mask != nullptr) {
+        uint32_t mk[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+          mk[i] = (((act_bits >> (2 * i)) & 1u) ? 0x3F80u : 0u) | (((act_bits >> (2 * i + 1)) & 1u) ? 0x3F800000u : 0u);
+        *reinterpret_cast<uint4*>(mask + (g / h8) * static_cast<size_t>(mask_pitch) + h) = make_uint4(mk[0], mk[1], mk[2], mk[3]);
+      }
       lvl = 0;
       while (lvl + 1 < n_levels && h >= s_start[lvl + 1]) ++lvl;
       straddle = lvl + 1 < n_levels && h + 8 > s_start[lvl + 1];
@@ -427,14 +436,17 @@ size_t matryoshka_dense_operand_scratch_bytes() { return static_cast<size_t>(148
 
 const char* matryoshka_dense_operand_launch(const float* z, int B, int H, const float* scale, float thr,
                                             const int* level_start, int n_levels, uint16_t* a_hi, uint16_t* a_lo,
-                                            unsigned long long* level_count, void* scratch, cudaStream_t stream) {
+                                            unsigned long long* level_count, void* scratch, cudaStream_t stream,
+                                            uint16_t* mask, int mask_pitch) {
   if ((H % 8) != 0) return "matryoshka_dense_operand: H must be a multiple of 8";
+  if (mask != nullptr && ((mask_pitch % 8) != 0 || (reinterpret_cast<uintptr_t>(mask) & 15) != 0))
+    return "matryoshka_dense_operand: the mask needs 16-byte aligned rows";
   if (n_levels > 32) return "matryoshka_dense_operand: at most 32 levels";
   size_t g = (static_cast<size_t>(B) * (H / 8) + 255) / 256;
   if (g > 148 * 16) g = 148 * 16;
   unsigned* partial = static_cast<unsigned*>(scratch);
   matryoshka_dense_operand_kernel<<<static_cast<int>(g), 256, 0, stream>>>(z, B, H, scale, thr, level_start, n_levels,
-                                                                           a_hi, a_lo, partial);
+                                                                           a_hi, a_lo, partial, mask, mask_pitch);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cudaGetErrorString(e);
   count_launches(1);

@@ -924,6 +924,19 @@ int qsae_coactivation(const int32_t* idx, const float* vals, int B, int cap, int
   return launch_status("coactivation", coactivation_launch(idx, vals, B, cap, H, cooc, S(stream)));
 }
 
+int qsae_coactivation_dense(const uint16_t* mask, int K, int H, int32_t* cooc, long long* counts, void* stream) {
+  if (K < 0 || H <= 0 || (H % 8) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "coactivation_dense: K >= 0 and H a positive multiple of 8 (K=%d H=%d)", K, H);
+  if (K > (1 << 24))
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "coactivation_dense: at most 2^24 rows per call (the fp32 counts are exact to "
+                "2^24), got %d", K);
+  if (K == 0) return QSAE_OK;
+  if (!mask || !cooc) return fail(QSAE_ERR_INVALID_ARGUMENT, "coactivation_dense: null pointer");
+  if (((reinterpret_cast<uintptr_t>(mask) | reinterpret_cast<uintptr_t>(cooc)) & 15) || (reinterpret_cast<uintptr_t>(counts) & 7))
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "coactivation_dense: mask and cooc must be 16-byte aligned, counts 8-byte");
+  return launch_status("coactivation_dense", coactivation_dense_launch(mask, K, H, cooc, counts, num_sms(), S(stream)));
+}
+
 int qsae_sq_error_accumulate(const float* a, const float* b, size_t n, double* out, void* stream) {
   if (n == 0) return QSAE_OK;
   if (!a || !b || !out) return fail(QSAE_ERR_INVALID_ARGUMENT, "sq_error: null pointer");
@@ -1103,7 +1116,10 @@ namespace {
 //   (encode_dense_split_kernel: both operands streamed, one accumulator, outputs written once).
 // x_parts: workspace for the bf16 part(s) of x, 3 * align_up(B * D * 2, 1024) bytes in split mode.
 // step: act == 2 only (EncodeLaunch::step_*): the q_sae dense path's A operand written by the epilogue.
-struct StepOperand { float thr; const float* scale; const int* level_start; int n_levels; unsigned long long* level_count; };
+struct StepOperand {
+  float thr; const float* scale; const int* level_start; int n_levels; unsigned long long* level_count;
+  uint16_t* mask; int mask_pitch;   // or null: activity mask (EncodeLaunch::step_mask)
+};
 int dense_encode_tc(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_mid, const uint16_t* w_lo,
                     const float* b_enc, int B, int H, int D, int act, uint8_t* x_parts, float* out_f32, uint16_t* out_hi,
                     uint16_t* out_lo, cudaStream_t st, const StepOperand* step = nullptr) {
@@ -1114,6 +1130,7 @@ int dense_encode_tc(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_
     if (!step) return fail(QSAE_ERR_INVALID_ARGUMENT, "dense encoder: step operand without its description");
     el.step_thr = step->thr; el.step_scale = step->scale; el.step_level_start = step->level_start;
     el.step_n_levels = step->n_levels; el.step_level_count = step->level_count;
+    el.step_mask = step->mask; el.step_mask_pitch = step->mask_pitch;
   }
   el.n_tiles = (H + kEncBN - 1) / kEncBN;
   el.n_splits = encode_pick_splits(B, H, num_sms());
@@ -1380,12 +1397,13 @@ int qsae_matryoshka_dense_workspace_bytes(int B, int H, int D, size_t* bytes) {
   return QSAE_OK;
 }
 
-int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_mid, const uint16_t* w_lo,
-                                  const float* b_enc,
-                                  const uint16_t* t_bf16, const float* scale, const int* level_start_dev,
+namespace {
+// mask (or null): the activity mask of the forward's own decisions, bf16 [B, >= H] rows of mask_pitch elements
+int matryoshka_forward_dense_impl(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_mid, const uint16_t* w_lo,
+                                  const float* b_enc, const uint16_t* t_bf16, const float* scale, const int* level_start_dev,
                                   const int* level_start_host, int n_levels, const float* dec_bias, int B, int H, int D,
-                                  float* result, unsigned long long* level_count, void* workspace,
-                                  size_t workspace_bytes, void* stream) {
+                                  float* result, unsigned long long* level_count, uint16_t* mask, int mask_pitch,
+                                  void* workspace, size_t workspace_bytes, void* stream) {
   if (B == 0) return QSAE_OK;
   if (!x_f32 || !b_enc || !t_bf16 || !scale || !level_start_dev || !level_start_host || !result || !level_count || !workspace)
     return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_forward_dense: null pointer");
@@ -1419,7 +1437,7 @@ int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, cons
   bool fuse_step = tuning().dense_step_fused != 0;
   for (int i = 0; i <= n_levels; ++i) fuse_step = fuse_step && (level_start_host[i] % 128) == 0;
   if (fuse_step) {
-    const StepOperand so = {kActiveThreshold, scale, level_start_dev, n_levels, level_count};
+    const StepOperand so = {kActiveThreshold, scale, level_start_dev, n_levels, level_count, mask, mask_pitch};
     rc = dense_encode_tc(x_f32, w_hi, w_mid, w_lo, b_enc, B, H, D, 2, ws + mp.x_off, nullptr, a_hi, a_lo, st, &so);
     if (rc != QSAE_OK) return rc;
   } else {
@@ -1427,7 +1445,7 @@ int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, cons
     if (rc != QSAE_OK) return rc;
     rc = launch_status("matryoshka_dense_operand",
                        matryoshka_dense_operand_launch(z, B, H, scale, kActiveThreshold, level_start_dev, n_levels, a_hi, a_lo,
-                                                       level_count, ws + mp.cnt_off, st));
+                                                       level_count, ws + mp.cnt_off, st, mask, mask_pitch));
     if (rc != QSAE_OK) return rc;
   }
   // 3. one GEMM per level over its K range, outputs accumulated level by level (:121-129). A TMA base address must be
@@ -1453,6 +1471,34 @@ int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, cons
     rc = launch_status("matryoshka_dense_tail", matryoshka_dense_tail_launch(a_hi, a_lo, t_bf16, level_start_dev, n_levels, B,
                                                                              H, D, dec_bias, result, st));
   return rc;
+}
+}  // namespace
+
+int qsae_matryoshka_forward_dense(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_mid, const uint16_t* w_lo,
+                                  const float* b_enc,
+                                  const uint16_t* t_bf16, const float* scale, const int* level_start_dev,
+                                  const int* level_start_host, int n_levels, const float* dec_bias, int B, int H, int D,
+                                  float* result, unsigned long long* level_count, void* workspace,
+                                  size_t workspace_bytes, void* stream) {
+  return matryoshka_forward_dense_impl(x_f32, w_hi, w_mid, w_lo, b_enc, t_bf16, scale, level_start_dev, level_start_host,
+                                       n_levels, dec_bias, B, H, D, result, level_count, nullptr, 0, workspace,
+                                       workspace_bytes, stream);
+}
+
+int qsae_matryoshka_forward_dense_active(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_mid, const uint16_t* w_lo,
+                                         const float* b_enc, const uint16_t* t_bf16, const float* scale,
+                                         const int* level_start_dev, const int* level_start_host, int n_levels,
+                                         const float* dec_bias, int B, int H, int D, float* result,
+                                         unsigned long long* level_count, uint16_t* active_mask, int mask_pitch,
+                                         int mask_col, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!active_mask) return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_forward_dense_active: null mask");
+  if (mask_col < 0 || mask_col + H > mask_pitch || (mask_pitch % 8) != 0 || (mask_col % 8) != 0 ||
+      (reinterpret_cast<uintptr_t>(active_mask) & 15) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_forward_dense_active: the mask needs 16-byte aligned rows and columns "
+                "(pitch %d, column %d, H %d: multiples of 8, column + H <= pitch)", mask_pitch, mask_col, H);
+  return matryoshka_forward_dense_impl(x_f32, w_hi, w_mid, w_lo, b_enc, t_bf16, scale, level_start_dev, level_start_host,
+                                       n_levels, dec_bias, B, H, D, result, level_count, active_mask + mask_col, mask_pitch,
+                                       workspace, workspace_bytes, stream);
 }
 
 int qsae_residual_update(const float* residual, const float* recon, size_t n, float* out, void* stream) {

@@ -198,6 +198,214 @@ wgrad_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ CU
   if (warp == 2) tmem_dealloc<kTmemCols>(tmem_base);
 }
 
+// ---- Co-activation counts of a dense activity mask: cooc[H, H] int32 += M^T M, M [K, H] bf16 0/1 (the analysis
+// consumers' dense route, analysis.py). The producer and MMA warps are those of wgrad_kernel with A = B = M (both
+// MN-major, one product); the schedule and the epilogue differ:
+//   - only the 128 x 256 tiles that reach the upper triangle (some n >= m) are computed, column by column of tiles
+//     (m fastest: the CTAs working at the same time share the 256-column slice of M in L2);
+//   - the epilogue reads the exact integer counts (products of 0/1 summed in fp32: exact up to 2^24 rows) and, for
+//     every element with n >= m, adds it to cooc[m, n] and, when n > m, to cooc[n, m] -- one writer per element and
+//     launch, so no atomics, the result is bit-deterministic and complete after every launch. Lanes hold consecutive
+//     rows m, so the mirrored read-modify-writes are coalesced 128-byte rows. The diagonal also goes to counts[m].
+//   - eight epilogue warps (two per TMEM lane quarter, 128 columns each) keep enough loads in flight for the
+//     read-modify-write to hide behind the MMAs of the next tile at K = 4096.
+constexpr int kCoThreads = 384;             // warps: 0 TMA, 1 MMA, 2 TMEM alloc, 3 idle, 4-11 epilogue
+constexpr int kCoEpiWarps = 8;
+
+struct CoactParams {
+  int H;
+  int m_tiles;
+  int k_chunks;
+  int n_units;           // tiles that reach the upper triangle
+  int32_t* c;            // [H, H]
+  long long* counts;     // [H] or null
+};
+
+// unit u -> tile (m0, n0): columns of tiles in order, tile column nt holding row tiles 0 .. min(2 nt + 2, m_tiles) - 1
+__device__ __forceinline__ void coact_tile_of(int u, int m_tiles, int* m0, int* n0) {
+  int nt = 0;
+  for (;;) {
+    const int c = min(2 * nt + 2, m_tiles);
+    if (u < c) break;
+    u -= c;
+    ++nt;
+  }
+  *m0 = u * BM;
+  *n0 = nt * BN;
+}
+
+__global__ void __launch_bounds__(kCoThreads, 1)
+coactivation_dense_kernel(const __grid_constant__ CUtensorMap tm, CoactParams p) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kBarOff);
+  uint64_t* full = bars;
+  uint64_t* empty = bars + kStages;
+  uint64_t* tmem_full = bars + 2 * kStages;
+  uint64_t* tmem_empty = tmem_full + 2;
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 4);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) {
+    if ((smem_u32(smem) & 1023u) != 0u) {
+      printf("qsae: dynamic shared memory is not 1024-byte aligned\n");
+      __trap();
+    }
+    for (int s = 0; s < kStages; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], 1);
+    }
+    for (int a = 0; a < 2; ++a) {
+      mbar_init(&tmem_full[a], 1);
+      mbar_init(&tmem_empty[a], kCoEpiWarps);
+    }
+    fence_mbar_init();
+    fence_proxy_async_smem();
+  }
+  if (warp == 2) tmem_alloc<kTmemCols>(tmem_ptr);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_ptr;
+
+  if (warp == 0) {
+    if (lane == 0) {
+      tma_prefetch_desc(&tm);
+      int stage = 0;
+      uint32_t phase = 0;
+      for (int u = blockIdx.x; u < p.n_units; u += gridDim.x) {
+        int m0, n0;
+        coact_tile_of(u, p.m_tiles, &m0, &n0);
+#pragma unroll 1
+        for (int kc = 0; kc < p.k_chunks; ++kc) {
+          mbar_wait(&empty[stage], phase ^ 1u);
+          uint8_t* st = smem + stage * kStageBytes;
+          mbar_arrive_expect_tx(&full[stage], kStageBytes);
+          const int k0 = kc * BK;
+#pragma unroll
+          for (int c = 0; c < BM / 64; ++c) tma_load_2d(st + c * kColBytes, &tm, &full[stage], m0 + 64 * c, k0, kPolicyEvictNormal);
+#pragma unroll
+          for (int c = 0; c < BN / 64; ++c)
+            tma_load_2d(st + kABytes + c * kColBytes, &tm, &full[stage], n0 + 64 * c, k0, kPolicyEvictNormal);
+          if (++stage == kStages) { stage = 0; phase ^= 1u; }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      constexpr uint32_t idesc = umma_idesc_bf16_f32_major(BM, BN, true, true);
+      int stage = 0;
+      uint32_t phase = 0;
+      int t = 0;
+      for (int u = blockIdx.x; u < p.n_units; u += gridDim.x, ++t) {
+        const int acc = t & 1;
+        mbar_wait(&tmem_empty[acc], ((t >> 1) & 1) ^ 1u);
+        tc_fence_after();
+        const uint32_t d_tmem = tmem_base + acc * BN;
+#pragma unroll 1
+        for (int kc = 0; kc < p.k_chunks; ++kc) {
+          mbar_wait(&full[stage], phase);
+          tc_fence_after();
+          const uint32_t st = smem_u32(smem + stage * kStageBytes);
+          const uint64_t a_desc = umma_desc_mnmajor_sw128(st, kColBytes);
+          const uint64_t b_desc = umma_desc_mnmajor_sw128(st + kABytes, kColBytes);
+#pragma unroll
+          for (int ks = 0; ks < BK / UMMA_K; ++ks) {
+            const uint64_t step = static_cast<uint64_t>(ks) * (2048 >> 4);   // 16 K rows = two 1024-byte atoms
+            umma_f16_ss(d_tmem, a_desc + step, b_desc + step, idesc, (kc | ks) != 0 ? 1u : 0u);
+          }
+          umma_commit(&empty[stage]);
+          if (kc == p.k_chunks - 1) umma_commit(&tmem_full[acc]);
+          if (++stage == kStages) { stage = 0; phase ^= 1u; }
+        }
+      }
+    }
+  } else if (warp >= 4) {
+    const int e = warp - 4;
+    const int quad = e & 3;                    // TMEM lanes 32 quad .. +31 (warp_id % 4)
+    const int cbase = (e >> 2) * (BN / 2);     // this warp's 128 columns of the tile
+    const uint32_t lane_taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
+    const size_t H = static_cast<size_t>(p.H);
+    int t = 0;
+    for (int u = blockIdx.x; u < p.n_units; u += gridDim.x, ++t) {
+      int m0, n0;
+      coact_tile_of(u, p.m_tiles, &m0, &n0);
+      const int acc = t & 1;
+      mbar_wait(&tmem_full[acc], (t >> 1) & 1);
+      tc_fence_after();
+      const int wrow0 = m0 + quad * 32;
+      const int m = wrow0 + lane;
+      const bool row_ok = m < p.H;
+#pragma unroll 1
+      for (int c0 = cbase; c0 < cbase + BN / 2; c0 += 32) {
+        const int nc = n0 + c0;
+        if (nc >= p.H) break;                       // warp-uniform
+        if (nc + 31 < wrow0 || wrow0 >= p.H) continue;   // wholly below the diagonal for every row of the warp
+        uint32_t r[32];
+        tmem_ld_32x32b_x32(lane_taddr + acc * BN + c0, r);
+        tmem_ld_wait();
+        int* v = reinterpret_cast<int*>(r);       // exact integer counts, in place
+#pragma unroll
+        for (int j = 0; j < 32; ++j) v[j] = __float2int_rn(__uint_as_float(r[j]));
+        // cooc[m, n] for n >= m: the lane's own row, 16-byte groups (H % 8 == 0: a group is inside [0, H) or past it)
+        int32_t* drow = p.c + static_cast<size_t>(m) * H + nc;
+        int4 old[8];
+#pragma unroll
+        for (int q = 0; q < 8; ++q)
+          old[q] = (row_ok && nc + 4 * q + 3 >= m && nc + 4 * q < p.H) ? *reinterpret_cast<const int4*>(drow + 4 * q)
+                                                                        : make_int4(0, 0, 0, 0);
+        // cooc[n, m] for n > m: column j of the tile is a row of cooc, the warp's 32 rows m are 32 consecutive ints;
+        // 16 columns at a time, their loads issued together with the row's
+        int mir[16];
+#pragma unroll
+        for (int j = 0; j < 16; ++j) {
+          const int n = nc + j;
+          mir[j] = (row_ok && n > m && n < p.H) ? p.c[static_cast<size_t>(n) * H + m] : 0;
+        }
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+          const int n = nc + 4 * q;
+          if (!row_ok || n + 3 < m || n >= p.H) continue;
+          if (n >= m) {
+            *reinterpret_cast<int4*>(drow + 4 * q) =
+                make_int4(old[q].x + v[4 * q], old[q].y + v[4 * q + 1], old[q].z + v[4 * q + 2], old[q].w + v[4 * q + 3]);
+          } else {                                  // the group holding the diagonal: elements n + i >= m only
+            if (n + 1 >= m) drow[4 * q + 1] = old[q].y + v[4 * q + 1];
+            if (n + 2 >= m) drow[4 * q + 2] = old[q].z + v[4 * q + 2];
+            drow[4 * q + 3] = old[q].w + v[4 * q + 3];
+          }
+        }
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          if (h == 1) {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+              const int n = nc + 16 + j;
+              mir[j] = (row_ok && n > m && n < p.H) ? p.c[static_cast<size_t>(n) * H + m] : 0;
+            }
+          }
+#pragma unroll
+          for (int j = 0; j < 16; ++j) {
+            const int n = nc + 16 * h + j;
+            if (row_ok && n > m && n < p.H) p.c[static_cast<size_t>(n) * H + m] = mir[j] + v[16 * h + j];
+          }
+        }
+        if (p.counts != nullptr && row_ok && m >= nc && m < nc + 32) {
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (nc + j == m) p.counts[m] += v[j];
+        }
+      }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&tmem_empty[acc]);
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  if (warp == 2) tmem_dealloc<kTmemCols>(tmem_base);
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -277,6 +485,31 @@ const char* wgrad_launch(const uint16_t* const* a_parts, const uint16_t* const* 
   const int grid = units < num_sms ? units : num_sms;
   const cudaError_t e = a_kmajor ? launch<true>(ta, tb, p, grid, stream) : launch<false>(ta, tb, p, grid, stream);
   return cuda_err(e);
+}
+
+const char* coactivation_dense_launch(const uint16_t* mask, int K, int H, int32_t* cooc, long long* counts, int num_sms,
+                                      cudaStream_t stream) {
+  if (K <= 0 || H <= 0 || (H % 8) != 0) return "coactivation_dense: K and H must be positive and H a multiple of 8";
+  if (K > (1 << 24)) return "coactivation_dense: at most 2^24 rows per launch (fp32 counts are exact up to 2^24)";
+  CUtensorMap tm;
+  if (!make_tmap(&tm, mask, K, H, BK)) return "cuTensorMapEncodeTiled(coactivation mask) failed";
+  CoactParams p;
+  p.H = H;
+  p.m_tiles = (H + BM - 1) / BM;
+  p.k_chunks = (K + BK - 1) / BK;
+  p.n_units = 0;
+  for (int nt = 0; nt < (H + BN - 1) / BN; ++nt) p.n_units += 2 * nt + 2 < p.m_tiles ? 2 * nt + 2 : p.m_tiles;
+  p.c = cooc;
+  p.counts = counts;
+  static bool attr = false;
+  if (!attr) {
+    cudaError_t e = cudaFuncSetAttribute(coactivation_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+    if (e != cudaSuccess) return cuda_err(e);
+    attr = true;
+  }
+  const int grid = p.n_units < num_sms ? p.n_units : num_sms;
+  coactivation_dense_kernel<<<grid, kCoThreads, kSmem, stream>>>(tm, p);
+  return cuda_err(cudaGetLastError());
 }
 
 }  // namespace qsae

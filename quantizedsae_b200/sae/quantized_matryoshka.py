@@ -193,7 +193,8 @@ class QuantizedMatryoshkaSAE(SparseAutoencoder):
         lin = self.encoder[0]
         return torch.sigmoid(_lib.encode_dense(x, lin.weight.detach().contiguous(), lin.bias.detach()))
 
-    def _forward_dense(self, x):
+    def _dense_levels(self, x, mask=None, mask_col=0):
+        """The dense path -> (result [n_bits, B, D], level counts); mask: also its activity (forward_dense_active)."""
         lin = self.encoder[0]
         dec = self.decoder
         _, scale = dec._packed()
@@ -201,18 +202,42 @@ class QuantizedMatryoshkaSAE(SparseAutoencoder):
         w_parts = self._w_parts() if self.exact else (self._w_bf16(),)
         result, counts = _lib.matryoshka_forward_dense(
             x, w_parts, lin.bias.detach(), dec._t_bf16(), scale, ls, dec._level_starts_host(),
-            dec.bias.detach() if self.allow_bias else None)
+            dec.bias.detach() if self.allow_bias else None, mask=mask, mask_col=mask_col)
         self.last_path = "dense"
-        return dec._finish(result, counts, None, x.shape[0])
+        return result, counts
 
-    def forward_active(self, x, active_cap: int = 256):
-        """forward(x) plus each row's active latents in sparse form, for the analysis consumers
-        (scripts/analysis/dynamic_analysis.py:30-73 builds a dense [B, H] mask from a second encoder pass).
-        -> dict(latent_groups, reconstruction_levels, level_counts int64 [n_bits],
-                active_idx [B, cap] int32 (-1 = empty, unordered), active_cnt [B] int32).
-        Sparse path only: a model whose rows overflow the survivor lists (~50 % active, untrained) has no
-        sparse active form and raises."""
+    def _forward_dense(self, x):
+        result, counts = self._dense_levels(x)
+        return self.decoder._finish(result, counts, None, x.shape[0])
+
+    def forward_dense_active(self, x, mask=None, mask_col: int = 0):
+        """The dense path's forward with its activity as a mask, for the analysis consumers at any activity
+        (scripts/analysis/dynamic_analysis.py:30-73 builds the same [B, H] mask from `encoder(x) > 0.5`).
+        -> dict(latent_groups, reconstruction_levels, level_counts int64 [n_bits], active_mask [B, H] bf16 1.0 / 0.0).
+        The mask comes from the decisions that form the level GEMMs' operand, so it matches the forward bit for bit; it
+        records activity, so a latent whose decoder row is all zero is still active. mask / mask_col: write into columns [mask_col, mask_col + H) of
+        a caller's bf16 [B, P] mask instead (multiples of 8; rq_sae puts its stages side by side)."""
         x = require_cuda_input(x, self)
+        if self.hidden_dim % 8 != 0:
+            raise ValueError(f"q_sae: hidden_dim {self.hidden_dim} is not a multiple of 8, so there is no dense path "
+                             "(its operands need 16-byte aligned rows) and no activity mask; use forward_active")
+        if mask is None:
+            mask = torch.empty((x.shape[0], self.hidden_dim), dtype=torch.bfloat16, device=x.device)
+            mask_col = 0
+        result, counts = self._dense_levels(x, mask, mask_col)
+        groups, levels = self.decoder._finish(result, counts, None, x.shape[0])
+        return {"latent_groups": groups, "reconstruction_levels": levels, "level_counts": counts,
+                "active_mask": mask[:, mask_col:mask_col + self.hidden_dim]}
+
+    def _known_dense(self) -> bool:
+        """True when this weight version's regime is already known to be dense (model(x) takes the dense path)."""
+        if self.dense_mode == "always":
+            return True
+        return (self.dense_mode == "auto" and self._regime is not None and self._regime[0] == self._weights_key()
+                and self._regime[1] == "dense")
+
+    def _forward_lists(self, x, active_cap: int = 256):
+        """forward_active's body: the dict, or None when the rows overflow the sparse survivor lists."""
         lin = self.encoder[0]
         packed, scale = self.decoder._packed()
         ls, _ = self.decoder._levels()
@@ -224,8 +249,7 @@ class QuantizedMatryoshkaSAE(SparseAutoencoder):
                 w_f32=lin.weight.detach().contiguous() if self.exact else None,
                 w_norm_max=self._w_norm_max() if self.exact else None, active_cap=cap)
             if int(overflow.item()) != 0:
-                raise RuntimeError("q_sae: rows with more active latents than the sparse path holds have no sparse "
-                                   "active-list form (dense activity); use model.encode(x) > 0.5")
+                return None
             need = int(a_cnt.max().item()) if a_cnt.numel() else 0
             if need <= cap:
                 break
@@ -234,6 +258,20 @@ class QuantizedMatryoshkaSAE(SparseAutoencoder):
         groups, levels = self.decoder._finish(result, counts, overflow, x.shape[0])
         return {"latent_groups": groups, "reconstruction_levels": levels, "level_counts": counts,
                 "active_idx": a_idx, "active_cnt": a_cnt}
+
+    def forward_active(self, x, active_cap: int = 256):
+        """forward(x) plus each row's active latents in sparse form, for the analysis consumers
+        (scripts/analysis/dynamic_analysis.py:30-73 builds a dense [B, H] mask from a second encoder pass).
+        -> dict(latent_groups, reconstruction_levels, level_counts int64 [n_bits],
+                active_idx [B, cap] int32 (-1 = empty, unordered), active_cnt [B] int32).
+        Sparse path only: a model whose rows overflow the survivor lists (~50 % active, untrained) has no
+        sparse active form and raises; forward_dense_active gives the same forward's activity as a dense mask."""
+        x = require_cuda_input(x, self)
+        r = self._forward_lists(x, active_cap)
+        if r is None:
+            raise RuntimeError("q_sae: rows with more active latents than the sparse path holds have no sparse "
+                               "active-list form (dense activity); use forward_dense_active(x) or model.encode(x) > 0.5")
+        return r
 
     def _forward_sparse(self, x, want_residual: bool = False):
         """The sparse path without the host-side overflow check: -> (result [n_bits, B, D], counts, overflow [1]
