@@ -194,7 +194,6 @@ __device__ __forceinline__ void epilogue_loop(const EncodeLaunch& p, int n_my_ti
   const int row_in_tile = quad * 32 + lane;
   const int row = m0 + row_in_tile;
   const bool row_ok = row < p.B;
-  const bool live = row_ok && p.debug_mode == 0;
   const int nsub = p.nsub;
   const int sub = sub_base + half;
   const int cap = p.cap;
@@ -206,12 +205,12 @@ __device__ __forceinline__ void epilogue_loop(const EncodeLaunch& p, int n_my_ti
 
   // a value survives iff v >= thr (inclusive; starts at the lowest finite float so that the
   // -inf used to mask out-of-range columns never survives)
-  float thr = live ? -3.402823466e+38f : INFINITY;
+  float thr = row_ok ? -3.402823466e+38f : INFINITY;
   float valid_bound = -INFINITY;  // inclusive lower bound of the k-th largest, reported to the merge
   float tm[MODE == 5 ? kTopM : 1];
 #pragma unroll
   for (int i = 0; i < (MODE == 5 ? kTopM : 1); ++i) tm[i] = -INFINITY;
-  if (MODE == 4 && live) {
+  if (MODE == 4 && row_ok) {
     // prior threshold: the m-th largest pre-activation of a sample of this row's latents
     // (itself one of the row's values). Tight, but only probably <= the k-th largest: the merge
     // kernel verifies it by counting survivors and sends the rare failing row to the rescue path.
@@ -222,7 +221,7 @@ __device__ __forceinline__ void epilogue_loop(const EncodeLaunch& p, int n_my_ti
   constexpr bool kTop2 = (MODE == 2 || MODE == 3);
   float top1[kClasses ? 32 : 1];
   float top2[kTop2 ? 32 : 1];
-  const float init = live ? -INFINITY : INFINITY;
+  const float init = row_ok ? -INFINITY : INFINITY;
 #pragma unroll
   for (int j = 0; j < (kClasses ? 32 : 1); ++j) top1[j] = init;
 #pragma unroll
@@ -238,7 +237,6 @@ __device__ __forceinline__ void epilogue_loop(const EncodeLaunch& p, int n_my_ti
     const float4* bias4 = reinterpret_cast<const float4*>(bias_smem + acc * BN + half * 128);
 #pragma unroll 1
     for (int c = 0; c < 4; ++c) {
-      if (p.debug_mode == 2) break;  // timing experiment: pipeline without the TMEM drain
       uint32_t r[32];
       tmem_ld_32x32b_x32(lane_taddr + acc * BN + half * 128 + c * 32, r);
       tmem_ld_wait();
@@ -291,7 +289,7 @@ __device__ __forceinline__ void epilogue_loop(const EncodeLaunch& p, int n_my_ti
           share[half * BM + row_in_tile] = bf16_floor_bits(bound);
           bound = fminf(bound, bf16_bits_to_float(share[(half ^ 1) * BM + row_in_tile]));
         }
-        if (live) { thr = fmaxf(thr, bound); valid_bound = fmaxf(valid_bound, bound); }
+        if (row_ok) { thr = fmaxf(thr, bound); valid_bound = fmaxf(valid_bound, bound); }
       }
       // survivors: per-lane hit mask, then rounds in which every lane with a pending hit stores
       // one entry. Scattered stores cost one LSU transaction per lane, so the number of store
@@ -358,7 +356,7 @@ __device__ __forceinline__ void epilogue_loop(const EncodeLaunch& p, int n_my_ti
     }
   } else if (row_ok) {
     p.cand_cnt[slot] = cnt;
-    p.cand_thr[slot] = live ? valid_bound : -INFINITY;
+    p.cand_thr[slot] = valid_bound;
     if (zero_from >= 0 && half == 0) {
       for (int s2 = zero_from; s2 < nsub; ++s2) {
         p.cand_cnt[static_cast<size_t>(row) * nsub + s2] = 0;
@@ -1655,7 +1653,7 @@ cudaError_t launch_kc(const CUtensorMap& tx, const CUtensorMap& tw, const Encode
 }
 
 // Prior-threshold sweeps (mode 4) run on the kernel compiled for that mode alone unless QSAE_ENCODE_SPECIALISED=0;
-// the diagnostics (debug_mode, debug_z) exist in the generic kernel only.
+// the dense dump (debug_z) exists in the generic kernel only.
 template <bool DENSE>
 const char* launch_any(const CUtensorMap& tx, const CUtensorMap& tw, const EncodeLaunch& p, cudaStream_t stream) {
   const int kc = (p.D + BK - 1) / BK;
@@ -1663,7 +1661,7 @@ const char* launch_any(const CUtensorMap& tx, const CUtensorMap& tw, const Encod
   if (p.cluster == 3 && kc != 8) return "the pair range schedule exists for D > 448 only";
   cudaError_t e;
   if constexpr (!DENSE) {
-    if (p.mode == 4 && p.debug_mode == 0 && p.debug_z == nullptr && tuning().encode_specialised != 0)
+    if (p.mode == 4 && p.debug_z == nullptr && tuning().encode_specialised != 0)
       e = launch_kc<false, 4>(tx, tw, p, stream);
     else
       e = launch_kc<false, -1>(tx, tw, p, stream);
@@ -1776,7 +1774,6 @@ const char* encode_dense_tc_launch(const uint16_t* x_bf16, const uint16_t* w_bf1
   p.out_f32 = out_f32; p.out_hi = out_hi; p.out_lo = out_lo;
   p.dense_flags = (out_f32 ? 1 : 0) | (out_hi ? 2 : 0) | (out_lo ? 4 : 0);
   if (p.dense_flags == 0) return "dense encoder: no output requested";
-  if (tuning().dense_flags_mask >= 0) p.dense_flags &= tuning().dense_flags_mask;  // timing experiments only
   p.range_g = 0;
   p.cluster = pick_cluster(p, kDefaultClusterDense);
   if (p.cluster == 1) p.cluster = kDefaultClusterDense;   // no multicast variant: it gained nothing here (DESIGN.md 5.1)
@@ -1804,7 +1801,6 @@ const char* encode_dense_split_launch(const uint16_t* const* x_parts, const uint
   p.cluster = 2;
   p.dense_flags = (out_f32 ? 1 : 0) | (out_hi ? 2 : 0) | (out_lo ? 4 : 0);
   if (p.dense_flags == 0) return "dense encoder: no output requested";
-  if (tuning().dense_flags_mask >= 0) p.dense_flags &= tuning().dense_flags_mask;  // timing experiments only
   CUtensorMap tx[3], tw[3];
   for (int i = 0; i < 3; ++i) {
     if (!make_tmap_bf16(&tx[i], x_parts[i < n_parts ? i : 0], p.B, p.D, BM)) return "cuTensorMapEncodeTiled(x part) failed";

@@ -22,7 +22,6 @@ constexpr int kPriorCounters = 4 + kRescueSlots;   // ints zeroed per call: [0] 
 // Tuning / diagnostic switches, read ONCE from the environment (never on a launch path); qsae_reload_tuning()
 // re-reads them (tests and tuning experiments that change the environment of a live process).
 struct Tuning {
-  int encode_debug_mode;  // QSAE_ENCODE_DEBUG_MODE: timing experiments (EncodeLaunch::debug_mode)
   int encode_cluster;     // QSAE_ENCODE_CLUSTER: 0 / 1 / 2 forces the cluster variant (-1 = automatic; dense: 0 / 2)
   int encode_range;       // QSAE_ENCODE_RANGE: 0 keeps the (split, row block) grid at small batches
   int encode_range_pair;  // QSAE_ENCODE_RANGE_PAIR: 1 = cta_group::2 pairs on the range schedule (sparse sweeps)
@@ -30,7 +29,6 @@ struct Tuning {
   int merge_tier;         // QSAE_MERGE_TIER: 8 / 12 / 16 forces the keys per lane of the warp merge (0 = from the expected survivor count)
   int sample_div;         // QSAE_SAMPLE_DIV: the sampled prior works on H / sample_div of the latents
   int prior_prep;         // QSAE_PRIOR_PREP: 0 keeps the separate cast / pre-pass / prior kernels
-  int dense_flags_mask;   // QSAE_DENSE_FLAGS_MASK: masks dense epilogue outputs (-1 = off; timing experiments)
   int dense_step_fused;   // QSAE_DENSE_STEP_FUSED: 0 = q_sae dense path writes fp32 pre-activations and runs the separate operand kernel
   int decode_pair;        // QSAE_DECODE_PAIR: 0 / 1 forces the decoder GEMM variant (-1 = automatic)
   int peer_timeout_ms;    // QSAE_PEER_TIMEOUT_MS: bound of a peer-memory flag wait (default 20000)
@@ -82,7 +80,6 @@ struct EncodeLaunch {
   const float* gate;      // [B, H] the forward's ReLU output h
   const float* gate_add;  // [B, H] d loss / d h, or null
   float* gate_colsum;     // [H] += column sums of the output (the bias gradient), or null
-  int debug_mode;       // 0 normal; timing experiments: 1 no survivors, 2 no TMEM drain
   float* debug_z;       // optional dense [B, H] dump of the accumulator (+bias, act); diagnostics only
 };
 

@@ -27,7 +27,6 @@ int env_int(const char* name, int dflt) {
 }  // namespace
 void reload_tuning() {
   Tuning t;
-  t.encode_debug_mode = env_int("QSAE_ENCODE_DEBUG_MODE", 0);
   t.encode_cluster = env_int("QSAE_ENCODE_CLUSTER", -1);
   t.encode_range = env_int("QSAE_ENCODE_RANGE", 1);
   t.encode_range_pair = env_int("QSAE_ENCODE_RANGE_PAIR", 1);
@@ -36,7 +35,6 @@ void reload_tuning() {
   t.merge_tier = env_int("QSAE_MERGE_TIER", 0);
   t.sample_div = env_int("QSAE_SAMPLE_DIV", 16);
   if (t.sample_div < 8) t.sample_div = 8;   // the plan samples only when H >= 8 n_sample
-  t.dense_flags_mask = env_int("QSAE_DENSE_FLAGS_MASK", -1);
   t.dense_step_fused = env_int("QSAE_DENSE_STEP_FUSED", 1);
   t.decode_pair = env_int("QSAE_DECODE_PAIR", -1);
   t.peer_timeout_ms = env_int("QSAE_PEER_TIMEOUT_MS", 20000);
@@ -83,6 +81,12 @@ int launch_status(const char* what, const char* err) {
 }
 inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+// carves `bytes` from a workspace at `off` and returns their offset; the next region starts at the aligned end
+size_t take(size_t& off, size_t bytes, size_t align = 256) {
+  const size_t start = off;
+  off = align_up(off + bytes, align);
+  return start;
+}
 
 int num_sms() {
   static int cached[64] = {0};
@@ -103,6 +107,16 @@ struct StagePlan {
 };
 
 enum StageKind { kStageClassBound = 0, kStagePriorMain = 1, kStageSamplePre = 2 };
+
+// The survivor lists of a sweep from `base` on: [B][nsub][cap] entries {float bits, int32 column}, then the counts
+// [B][nsub], then the thresholds [B][nsub].
+void place_lists(int B, size_t base, StagePlan* sp) {
+  const size_t lists = static_cast<size_t>(B) * sp->nsub;
+  sp->cand_off = align_up(base, 256);
+  sp->cnt_off = sp->cand_off + lists * sp->cap * 8;
+  sp->thr_off = sp->cnt_off + lists * 4;
+  sp->end = align_up(sp->thr_off + lists * 4, 256);
+}
 
 // allow_range (prior-threshold sweeps): the range schedule at small batches; D: width of the contraction (the pair
 // variant exists for D = 512 only)
@@ -145,10 +159,7 @@ void plan_stage(int B, int H, int k_sel, StageKind kind, size_t base, StagePlan*
     encode_pick_mode(k_sel, &sp->mode, &sp->cap);
     if (sp->tiles_per_split * (kEncBN / 2) <= 448) sp->cap = 512;  // a sub-stream this short cannot fill more
   }
-  sp->cand_off = align_up(base, 256);
-  sp->cnt_off = sp->cand_off + static_cast<size_t>(B) * sp->nsub * sp->cap * 8;
-  sp->thr_off = sp->cnt_off + static_cast<size_t>(B) * sp->nsub * 4;
-  sp->end = align_up(sp->thr_off + static_cast<size_t>(B) * sp->nsub * 4, 256);
+  place_lists(B, base, sp);
 }
 
 // Prior threshold = m-th largest pre-activation over a sample of n_sample of the H latents.
@@ -174,10 +185,17 @@ struct EncodePlan {
   size_t x_off, prior_off, counters_off, rescue_rows_off, ovf_rows_off, rescue_z_off, total;
 };
 
-int plan_encode(int B, int H, int D, int k, int exact, int n_sample, EncodePlan* pl) {
+// shapes the tensor-core encoder takes (b_sae, t_sae): B, H > 0; D a multiple of 8 in [8, 512]
+int check_encode_shape(int B, int H, int D) {
   if (B <= 0 || H <= 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "B and H must be positive (B=%d H=%d)", B, H);
   if (D < 8 || D > 512 || (D % 8) != 0)
     return fail(QSAE_ERR_INVALID_ARGUMENT, "D must be a multiple of 8 in [8, 512], got %d", D);
+  return QSAE_OK;
+}
+
+int plan_encode(int B, int H, int D, int k, int exact, int n_sample, EncodePlan* pl) {
+  const int rc = check_encode_shape(B, H, D);
+  if (rc != QSAE_OK) return rc;
   if (k < 1) return fail(QSAE_ERR_INVALID_ARGUMENT, "k must be >= 1, got %d", k);
   if (k > H) return fail(QSAE_ERR_K_OUT_OF_RANGE, "selected index k out of range (k=%d > H=%d)", k, H);
   if (k > kMaxK) return fail(QSAE_ERR_INVALID_ARGUMENT, "k=%d exceeds QSAE_MAX_K=%d on the warp-level path", k, kMaxK);
@@ -200,16 +218,16 @@ int plan_encode(int B, int H, int D, int k, int exact, int n_sample, EncodePlan*
       pl->m = m;
     }
   }
-  pl->x_off = 0;
-  size_t off = align_up(static_cast<size_t>(B) * D * 2, 1024);
+  size_t off = 0;
+  pl->x_off = take(off, static_cast<size_t>(B) * D * 2, 1024);
   plan_stage(B, H, k_sel, pl->use_prior ? kStagePriorMain : kStageClassBound, off, &pl->main, true, D);
   off = pl->main.end;
-  pl->counters_off = off; off += 256;
-  pl->rescue_rows_off = off; off = align_up(off + static_cast<size_t>(B) * 4, 256);
+  pl->counters_off = take(off, 256);
+  pl->rescue_rows_off = take(off, static_cast<size_t>(B) * 4);
   if (pl->use_prior) {
-    pl->prior_off = off; off = align_up(off + static_cast<size_t>(B) * 4, 256);
-    pl->ovf_rows_off = off; off = align_up(off + static_cast<size_t>(B) * 4, 256);
-    pl->rescue_z_off = off; off = align_up(off + static_cast<size_t>(kRescueSlots) * H * 4, 256);
+    pl->prior_off = take(off, static_cast<size_t>(B) * 4);
+    pl->ovf_rows_off = take(off, static_cast<size_t>(B) * 4);
+    pl->rescue_z_off = take(off, static_cast<size_t>(kRescueSlots) * H * 4);
     plan_stage(B, n_sample, pl->m, kStageSamplePre, off, &pl->pre);
     off = pl->pre.end;
   }
@@ -217,18 +235,40 @@ int plan_encode(int B, int H, int D, int k, int exact, int n_sample, EncodePlan*
   return QSAE_OK;
 }
 
-void fill_encode_launch(EncodeLaunch* el, const StagePlan& sp, int B, int D, int act, const float* bias,
-                        uint8_t* ws) {
-  memset(el, 0, sizeof(*el));
-  el->B = B; el->H = sp.H; el->D = D; el->k_sel = sp.k_sel;
-  el->n_splits = sp.n_splits; el->tiles_per_split = sp.tiles_per_split; el->n_tiles = sp.n_tiles;
-  el->nsub = sp.nsub; el->range_g = sp.range_g; el->range_pair = sp.range_pair;
-  el->act = act; el->mode = sp.mode; el->cap = sp.cap; el->bias = bias;
-  el->cand = ws + sp.cand_off;
-  el->cand_cnt = reinterpret_cast<int*>(ws + sp.cnt_off);
-  el->cand_thr = reinterpret_cast<float*>(ws + sp.thr_off);
+EncodeLaunch stage_launch(const StagePlan& sp, int B, int D, int act, const float* bias, uint8_t* ws) {
+  EncodeLaunch el{};
+  el.B = B; el.H = sp.H; el.D = D; el.k_sel = sp.k_sel;
+  el.n_splits = sp.n_splits; el.tiles_per_split = sp.tiles_per_split; el.n_tiles = sp.n_tiles;
+  el.nsub = sp.nsub; el.range_g = sp.range_g; el.range_pair = sp.range_pair;
+  el.act = act; el.mode = sp.mode; el.cap = sp.cap; el.bias = bias;
+  el.cand = ws + sp.cand_off;
+  el.cand_cnt = reinterpret_cast<int*>(ws + sp.cnt_off);
+  el.cand_thr = reinterpret_cast<float*>(ws + sp.thr_off);
+  return el;
 }
 
+// Merge of the survivor lists the sweep `el` has just written: k_sel kept per row, the first k_out emitted.
+// x_f32, w_f32, bias: the fp32 operands of the exact re-scoring and rescue (or null).
+SelectLaunch merge_launch(const EncodeLaunch& el, int k_sel, int k_out, int exact, const float* x_f32, const float* w_f32,
+                          const float* bias, float* out_vals, int32_t* out_idx, int32_t* out_flags) {
+  SelectLaunch sl{};
+  sl.B = el.B; sl.H = el.H; sl.D = el.D; sl.k_sel = k_sel; sl.k_out = k_out; sl.nsub = el.nsub; sl.cap = el.cap;
+  sl.act = el.act; sl.exact = exact;
+  sl.cand = el.cand; sl.cand_cnt = el.cand_cnt; sl.cand_thr = el.cand_thr;
+  sl.x_f32 = x_f32; sl.w_f32 = w_f32; sl.bias = bias;
+  sl.out_vals = out_vals; sl.out_idx = out_idx; sl.out_flags = out_flags;
+  return sl;
+}
+
+// Exact recomputation of the rows the merge `sl` put on its rescue list, into the same outputs
+RescueLaunch rescue_launch(const SelectLaunch& sl, const uint16_t* x_bf16, const uint16_t* w_bf16) {
+  RescueLaunch rl{};
+  rl.B = sl.B; rl.H = sl.H; rl.D = sl.D; rl.k_sel = sl.k_sel; rl.k_out = sl.k_out; rl.act = sl.act; rl.exact = sl.exact;
+  rl.x_bf16 = x_bf16; rl.w_bf16 = w_bf16; rl.x_f32 = sl.x_f32; rl.w_f32 = sl.w_f32; rl.bias = sl.bias;
+  rl.rescue_count = sl.rescue_count; rl.rescue_rows = sl.rescue_rows;
+  rl.out_vals = sl.out_vals; rl.out_idx = sl.out_idx; rl.out_flags = sl.out_flags;
+  return rl;
+}
 
 int next_pow2_host(int v) {
   int p = 1;
@@ -249,9 +289,8 @@ struct LargePlan {
 };
 
 int plan_encode_large(int B, int H, int D, int k, int exact, int n_sample, LargePlan* lp) {
-  if (B <= 0 || H <= 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "B and H must be positive (B=%d H=%d)", B, H);
-  if (D < 8 || D > 512 || (D % 8) != 0)
-    return fail(QSAE_ERR_INVALID_ARGUMENT, "D must be a multiple of 8 in [8, 512], got %d", D);
+  const int rc = check_encode_shape(B, H, D);
+  if (rc != QSAE_OK) return rc;
   if (k > H) return fail(QSAE_ERR_K_OUT_OF_RANGE, "selected index k out of range (k=%d > H=%d)", k, H);
   if (k > kMaxKLarge) return fail(QSAE_ERR_INVALID_ARGUMENT, "k=%d exceeds QSAE_MAX_K_LARGE=%d", k, kMaxKLarge);
   // re-scoring margin: the density of pre-activations around the k-th largest grows with k, so the number of
@@ -263,8 +302,8 @@ int plan_encode_large(int B, int H, int D, int k, int exact, int n_sample, Large
   lp->m = 0;
   lp->chunk_rows = 0;
   const int ksort = next_pow2_host(k_sel);
-  lp->x_off = 0;
-  size_t off = align_up(static_cast<size_t>(B) * D * 2, 1024);
+  size_t off = 0;
+  lp->x_off = take(off, static_cast<size_t>(B) * D * 2, 1024);
   if (n_sample >= 256 && H >= 8 * static_cast<long long>(n_sample)) {
     const double r = static_cast<double>(n_sample) / H;
     const int m = choose_prior_rank(k_sel, r);
@@ -282,19 +321,17 @@ int plan_encode_large(int B, int H, int D, int k, int exact, int n_sample, Large
         lp->use_prior = true;
         lp->m = m;
         lp->main.cap = cap;
-        lp->main.cnt_off = lp->main.cand_off + static_cast<size_t>(B) * lp->main.nsub * cap * 8;
-        lp->main.thr_off = lp->main.cnt_off + static_cast<size_t>(B) * lp->main.nsub * 4;
-        lp->main.end = align_up(lp->main.thr_off + static_cast<size_t>(B) * lp->main.nsub * 4, 256);
+        place_lists(B, off, &lp->main);
       }
     }
   }
   if (lp->use_prior) {
     off = lp->main.end;
-    lp->counters_off = off; off += 256;
-    lp->rescue_rows_off = off; off = align_up(off + static_cast<size_t>(B) * 4, 256);
-    lp->pre_vals_off = off; off = align_up(off + static_cast<size_t>(B) * lp->m * 4, 256);
-    lp->pre_idx_off = off; off = align_up(off + static_cast<size_t>(B) * lp->m * 4, 256);
-    lp->scratch_off = off; off = align_up(off + rescue_large_scratch_bytes(H, num_sms()), 256);
+    lp->counters_off = take(off, 256);
+    lp->rescue_rows_off = take(off, static_cast<size_t>(B) * 4);
+    lp->pre_vals_off = take(off, static_cast<size_t>(B) * lp->m * 4);
+    lp->pre_idx_off = take(off, static_cast<size_t>(B) * lp->m * 4);
+    lp->scratch_off = take(off, rescue_large_scratch_bytes(H, num_sms()));
     plan_stage(B, n_sample, lp->m, kStageClassBound, off, &lp->pre);
     off = lp->pre.end;
   } else {
@@ -304,7 +341,7 @@ int plan_encode_large(int B, int H, int D, int k, int exact, int n_sample, Large
     if (rows < kEncBM) rows = kEncBM;
     if (rows > B) rows = B;
     lp->chunk_rows = static_cast<int>(rows);
-    lp->z_off = off; off = align_up(off + static_cast<size_t>(rows) * H * 4, 256);
+    lp->z_off = take(off, static_cast<size_t>(rows) * H * 4);
     plan_stage(static_cast<int>(rows), H, 1, kStageClassBound, off, &lp->dense);
     off = lp->dense.end;
   }
@@ -337,8 +374,7 @@ int encode_topk_large(const float* x_f32, const uint16_t* w_bf16, const float* w
         rc = launch_status("encode_dense", encode_dense_launch(x_f32 + static_cast<size_t>(r0) * D, nullptr, rows, w_f32,
                                                                b_enc, H, D, act, z, st));
       } else {
-        EncodeLaunch el;
-        fill_encode_launch(&el, lp.dense, rows, D, act, b_enc, ws);   // the chunk's split plan, possibly fewer rows
+        EncodeLaunch el = stage_launch(lp.dense, rows, D, act, b_enc, ws);   // the chunk's split plan, possibly fewer rows
         el.debug_z = z;
         rc = launch_status("encode_topk kernel (dense dump)",
                            encode_topk_launch(x_bf16 + static_cast<size_t>(r0) * D, w_bf16, el, st));
@@ -366,22 +402,15 @@ int encode_topk_large(const float* x_f32, const uint16_t* w_bf16, const float* w
   if (rc != QSAE_OK) return rc;
   // 1. ordered top-m over the sampled rows (tensor-core values: the same arithmetic as the full sweep)
   {
-    EncodeLaunch pe;
-    fill_encode_launch(&pe, lp.pre, B, D, act, b_sample, ws);
+    const EncodeLaunch pe = stage_launch(lp.pre, B, D, act, b_sample, ws);
     rc = launch_status("encode_topk kernel (sample top-m)", encode_topk_launch(x_bf16, w_sample, pe, st));
     if (rc != QSAE_OK) return rc;
-    SelectLaunch sl;
-    memset(&sl, 0, sizeof(sl));
-    sl.B = B; sl.H = n_sample; sl.D = D; sl.k_sel = lp.m; sl.k_out = lp.m; sl.nsub = lp.pre.nsub; sl.cap = lp.pre.cap;
-    sl.act = act;
-    sl.cand = pe.cand; sl.cand_cnt = pe.cand_cnt; sl.cand_thr = pe.cand_thr;
-    sl.out_vals = pre_vals; sl.out_idx = pre_idx;
+    const SelectLaunch sl = merge_launch(pe, lp.m, lp.m, 0, nullptr, nullptr, nullptr, pre_vals, pre_idx, nullptr);
     rc = launch_status("select_topk kernel (sample top-m)", select_topk_launch(sl, st));
     if (rc != QSAE_OK) return rc;
   }
   // 2. full sweep, everything >= the row's m-th largest sample value
-  EncodeLaunch el;
-  fill_encode_launch(&el, lp.main, B, D, act, b_enc, ws);
+  EncodeLaunch el = stage_launch(lp.main, B, D, act, b_enc, ws);
   el.k_sel = 0;
   el.prior = pre_vals + (lp.m - 1); el.prior_stride = lp.m;
   el.overflow = counters + 1;
@@ -390,13 +419,7 @@ int encode_topk_large(const float* x_f32, const uint16_t* w_bf16, const float* w
   if (g_enc_ev_stop) cudaEventRecord(g_enc_ev_stop, st);
   if (rc != QSAE_OK) return rc;
   // 3. block-per-row merge (radix select), count check
-  SelectLaunch sl;
-  memset(&sl, 0, sizeof(sl));
-  sl.B = B; sl.H = H; sl.D = D; sl.k_sel = lp.k_sel; sl.k_out = k; sl.nsub = lp.main.nsub; sl.cap = lp.main.cap;
-  sl.act = act; sl.exact = exact;
-  sl.cand = el.cand; sl.cand_cnt = el.cand_cnt; sl.cand_thr = el.cand_thr;
-  sl.x_f32 = x_f32; sl.w_f32 = w_f32; sl.bias = b_enc;
-  sl.out_vals = out_vals; sl.out_idx = out_idx; sl.out_flags = out_flags;
+  SelectLaunch sl = merge_launch(el, lp.k_sel, k, exact, x_f32, w_f32, b_enc, out_vals, out_idx, out_flags);
   sl.rescue_count = counters; sl.rescue_rows = rescue_rows; sl.check_count = 1;
   sl.unsorted = g_unordered_topk;
   rc = launch_status("select_topk kernel", select_topk_launch(sl, st));
@@ -419,13 +442,8 @@ int encode_topk_large(const float* x_f32, const uint16_t* w_bf16, const float* w
     free(h_cnt);
   }
   // 4. failed rows: exact recomputation
-  RescueLaunch rl;
-  memset(&rl, 0, sizeof(rl));
-  rl.B = B; rl.H = H; rl.D = D; rl.k_sel = lp.k_sel; rl.k_out = k; rl.act = act; rl.exact = exact;
-  rl.x_bf16 = x_bf16; rl.w_bf16 = w_bf16; rl.x_f32 = x_f32; rl.w_f32 = w_f32; rl.bias = b_enc;
-  rl.rescue_count = counters; rl.rescue_rows = rescue_rows;
-  rl.out_vals = out_vals; rl.out_idx = out_idx; rl.out_flags = out_flags;
-  return launch_status("rescue kernel (large k)", rescue_large_launch(rl, ws + lp.scratch_off, num_sms(), st));
+  return launch_status("rescue kernel (large k)",
+                       rescue_large_launch(rescue_launch(sl, x_bf16, w_bf16), ws + lp.scratch_off, num_sms(), st));
 }
 
 }  // namespace
@@ -572,13 +590,12 @@ int encode_topk_impl(const float* x_f32, const uint16_t* w_bf16, const float* w_
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   uint16_t* x_bf16 = reinterpret_cast<uint16_t*>(ws + pl.x_off);
   cudaStream_t st = S(stream);
-  const int debug_mode = tuning().encode_debug_mode;
 
   int* counters = reinterpret_cast<int*>(ws + pl.counters_off);   // [0] rescue rows, [1] merge overflow rows
   int32_t* rescue_rows = reinterpret_cast<int32_t*>(ws + pl.rescue_rows_off);
   stage_mark(0, st);
   // small batches on the prior path: cast, sample pre-pass, prior and the counter reset are ONE launch
-  const int prep_ns = (pl.use_prior && debug_mode == 0) ? prior_prep_pick_ns(B, D, n_sample, pl.m, num_sms()) : 0;
+  const int prep_ns = pl.use_prior ? prior_prep_pick_ns(B, D, n_sample, pl.m, num_sms()) : 0;
   if (prep_ns == 0) {
     rc = launch_status("cast x", cast_bf16_launch(x_f32, x_bf16, static_cast<size_t>(B) * D, st));
     if (rc != QSAE_OK) return rc;
@@ -588,32 +605,18 @@ int encode_topk_impl(const float* x_f32, const uint16_t* w_bf16, const float* w_
 
   if (!pl.use_prior) {
     // ---- class-bound path: one sweep, block-per-row merge
-    EncodeLaunch el;
-    fill_encode_launch(&el, pl.main, B, D, act, b_enc, ws);
-    el.debug_mode = debug_mode;
+    const EncodeLaunch el = stage_launch(pl.main, B, D, act, b_enc, ws);
     if (g_enc_ev_start) cudaEventRecord(g_enc_ev_start, st);
     rc = launch_status("encode_topk kernel", encode_topk_launch(x_bf16, w_bf16, el, st));
     if (g_enc_ev_stop) cudaEventRecord(g_enc_ev_stop, st);
     if (rc != QSAE_OK) return rc;
-    SelectLaunch sl;
-    memset(&sl, 0, sizeof(sl));
-    sl.B = B; sl.H = H; sl.D = D; sl.k_sel = pl.k_sel; sl.k_out = k; sl.nsub = pl.main.nsub; sl.cap = pl.main.cap;
-    sl.act = act; sl.exact = exact;
-    sl.cand = el.cand; sl.cand_cnt = el.cand_cnt; sl.cand_thr = el.cand_thr;
-    sl.x_f32 = x_f32; sl.w_f32 = w_f32; sl.bias = b_enc;
-    sl.out_vals = out_vals; sl.out_idx = out_idx; sl.out_flags = out_flags;
+    SelectLaunch sl = merge_launch(el, pl.k_sel, k, exact, x_f32, w_f32, b_enc, out_vals, out_idx, out_flags);
     if (exact) { sl.rescue_count = counters; sl.rescue_rows = rescue_rows; }   // uncertified rows only (the bound itself is exact)
     rc = launch_status("select_topk kernel", select_topk_launch(sl, st));
     if (rc != QSAE_OK || !exact) return rc;
     // exact mode: a row whose fp32 re-scoring could not certify the selection is recomputed exactly, as on the
     // prior path (round 1 left such rows flagged with their bf16-chosen candidates)
-    RescueLaunch rl;
-    memset(&rl, 0, sizeof(rl));
-    rl.B = B; rl.H = H; rl.D = D; rl.k_sel = pl.k_sel; rl.k_out = k; rl.act = act; rl.exact = exact;
-    rl.x_bf16 = x_bf16; rl.w_bf16 = w_bf16; rl.x_f32 = x_f32; rl.w_f32 = w_f32; rl.bias = b_enc;
-    rl.rescue_count = counters; rl.rescue_rows = rescue_rows;
-    rl.out_vals = out_vals; rl.out_idx = out_idx; rl.out_flags = out_flags;
-    return launch_status("rescue kernel", rescue_rows_launch(rl, num_sms(), st));
+    return launch_status("rescue kernel", rescue_rows_launch(rescue_launch(sl, x_bf16, w_bf16), num_sms(), st));
   }
 
   // ---- prior-threshold path
@@ -621,16 +624,14 @@ int encode_topk_impl(const float* x_f32, const uint16_t* w_bf16, const float* w_
   int32_t* ovf_rows = reinterpret_cast<int32_t*>(ws + pl.ovf_rows_off);
   if (prep_ns > 0) {
     // 1. cast + sample pre-pass + prior in one cluster launch (prior_prep_kernel)
-    PrepLaunch pp;
-    memset(&pp, 0, sizeof(pp));
+    PrepLaunch pp{};
     pp.B = B; pp.D = D; pp.n_sample = n_sample; pp.act = act; pp.m = pl.m; pp.ns = prep_ns;
     pp.x_f32 = x_f32; pp.x_bf16 = x_bf16; pp.bias = b_sample; pp.prior = prior; pp.zero_counters = counters;
     rc = launch_status("prior_prep kernel", prior_prep_launch(w_sample, pp, st));
     if (rc != QSAE_OK) return rc;
   } else {
     // 1. pre-pass: the fused kernel over the sampled dictionary rows, top list kept in registers
-    EncodeLaunch pe;
-    fill_encode_launch(&pe, pl.pre, B, D, act, b_sample, ws);
+    EncodeLaunch pe = stage_launch(pl.pre, B, D, act, b_sample, ws);
     pe.top_out = reinterpret_cast<float*>(ws + pl.pre.cand_off);
     rc = launch_status("encode_topk kernel (sample pre-pass)", encode_topk_launch(x_bf16, w_sample, pe, st));
     if (rc != QSAE_OK) return rc;
@@ -639,9 +640,7 @@ int encode_topk_impl(const float* x_f32, const uint16_t* w_bf16, const float* w_
   }
   stage_mark(1, st);
   // 2. full sweep against the prior
-  EncodeLaunch el;
-  fill_encode_launch(&el, pl.main, B, D, act, b_enc, ws);
-  el.debug_mode = debug_mode;
+  EncodeLaunch el = stage_launch(pl.main, B, D, act, b_enc, ws);
   el.prior = prior; el.prior_stride = 1;
   if (g_enc_ev_start) cudaEventRecord(g_enc_ev_start, st);
   rc = launch_status("encode_topk kernel", encode_topk_launch(x_bf16, w_bf16, el, st));
@@ -649,13 +648,7 @@ int encode_topk_impl(const float* x_f32, const uint16_t* w_bf16, const float* w_
   if (rc != QSAE_OK) return rc;
   stage_mark(2, st);
   // 3. merge (warp per row; rows with too many survivors go through the block kernel)
-  SelectLaunch sl;
-  memset(&sl, 0, sizeof(sl));
-  sl.B = B; sl.H = H; sl.D = D; sl.k_sel = pl.k_sel; sl.k_out = k; sl.nsub = pl.main.nsub; sl.cap = pl.main.cap;
-  sl.act = act; sl.exact = exact;
-  sl.cand = el.cand; sl.cand_cnt = el.cand_cnt; sl.cand_thr = el.cand_thr;
-  sl.x_f32 = x_f32; sl.w_f32 = w_f32; sl.bias = b_enc;
-  sl.out_vals = out_vals; sl.out_idx = out_idx; sl.out_flags = out_flags;
+  SelectLaunch sl = merge_launch(el, pl.k_sel, k, exact, x_f32, w_f32, b_enc, out_vals, out_idx, out_flags);
   sl.rescue_count = counters; sl.rescue_rows = rescue_rows; sl.check_count = 1;
   // warp per row: up to 512 survivors in registers (the expected count is ~32 m); rows with more take a two-pass
   // prefilter inside the same warp (round 1 had a second launch with 32 keys per lane for them: 25 us at B = 4096
@@ -683,12 +676,7 @@ int encode_topk_impl(const float* x_f32, const uint16_t* w_bf16, const float* w_
   stage_mark(3, st);
   // tail, one launch: rows the warp merge could not hold (floods of equal values) through the block-per-row select,
   // rows whose prior failed the count check through the exact recomputation; both decoded there when fused
-  RescueLaunch rl;
-  memset(&rl, 0, sizeof(rl));
-  rl.B = B; rl.H = H; rl.D = D; rl.k_sel = pl.k_sel; rl.k_out = k; rl.act = act; rl.exact = exact;
-  rl.x_bf16 = x_bf16; rl.w_bf16 = w_bf16; rl.x_f32 = x_f32; rl.w_f32 = w_f32; rl.bias = b_enc;
-  rl.rescue_count = counters; rl.rescue_rows = rescue_rows;
-  rl.out_vals = out_vals; rl.out_idx = out_idx; rl.out_flags = out_flags;
+  RescueLaunch rl = rescue_launch(sl, x_bf16, w_bf16);
   rl.z_scratch = reinterpret_cast<float*>(ws + pl.rescue_z_off); rl.slot_done = counters + 4;
   rc = launch_status("select_tail kernel", select_tail_launch(sl, rl, counters + 1, ovf_rows, num_sms(), st));
   stage_mark(4, st);
@@ -717,8 +705,7 @@ int qsae_prior_prep(const float* x_f32, const uint16_t* w_sample, const float* b
   const int ns = prior_prep_pick_ns(B, D, n_sample, m, num_sms());
   if (ns_out) *ns_out = ns;
   if (ns == 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "prior_prep: no single-launch variant for B=%d D=%d n_sample=%d m=%d", B, D, n_sample, m);
-  PrepLaunch pp;
-  memset(&pp, 0, sizeof(pp));
+  PrepLaunch pp{};
   pp.B = B; pp.D = D; pp.n_sample = n_sample; pp.act = act; pp.m = m; pp.ns = ns;
   pp.x_f32 = x_f32; pp.x_bf16 = x_bf16; pp.bias = b_sample; pp.prior = prior;
   return launch_status("prior_prep kernel", prior_prep_launch(w_sample, pp, S(stream)));
@@ -764,8 +751,7 @@ int qsae_encode_dense_tc(const float* x_f32, const uint16_t* w_bf16, const float
   uint16_t* x_bf16 = reinterpret_cast<uint16_t*>(ws + pl.x_off);
   rc = launch_status("cast x", cast_bf16_launch(x_f32, x_bf16, static_cast<size_t>(B) * D, S(stream)));
   if (rc != QSAE_OK) return rc;
-  EncodeLaunch el;
-  fill_encode_launch(&el, pl.main, B, D, act, b_enc, ws);
+  EncodeLaunch el = stage_launch(pl.main, B, D, act, b_enc, ws);
   el.debug_z = z;
   return launch_status("encode_topk kernel (dense dump)", encode_topk_launch(x_bf16, w_bf16, el, S(stream)));
 }
@@ -790,16 +776,16 @@ int plan_matryoshka(int B, int H, int D, MatPlan* mp) {
   if (B <= 0 || H <= 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "B and H must be positive");
   if (D < 16 || D > 512 || (D % 16) != 0)
     return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka: D must be a multiple of 16 in [16, 512], got %d", D);
-  mp->x_off = 0;
-  mp->prior_off = align_up(static_cast<size_t>(B) * D * 2, 1024);
-  plan_stage(B, H, 0, kStagePriorMain, mp->prior_off + align_up(static_cast<size_t>(B) * 4, 256), &mp->st, true, D);
+  size_t off = 0;
+  mp->x_off = take(off, static_cast<size_t>(B) * D * 2, 1024);
+  mp->prior_off = take(off, static_cast<size_t>(B) * 4);
+  plan_stage(B, H, 0, kStagePriorMain, off, &mp->st, true, D);
   // every active latent is kept: largest buffers. Range schedule: more, shorter lists per row (the same capacity per row)
   mp->st.cap = mp->st.range_g > 0 ? kCandCapMax / 2 : kCandCapMax;
-  mp->st.cnt_off = mp->st.cand_off + static_cast<size_t>(B) * mp->st.nsub * mp->st.cap * 8;
-  mp->st.thr_off = mp->st.cnt_off + static_cast<size_t>(B) * mp->st.nsub * 4;
-  mp->st.end = align_up(mp->st.thr_off + static_cast<size_t>(B) * mp->st.nsub * 4, 256);
-  mp->scratch_off = mp->st.end;
-  mp->total = align_up(mp->scratch_off + decode_matryoshka_scratch_bytes(num_sms()), 256);
+  place_lists(B, off, &mp->st);
+  off = mp->st.end;
+  mp->scratch_off = take(off, decode_matryoshka_scratch_bytes(num_sms()));
+  mp->total = off;
   return QSAE_OK;
 }
 }  // namespace
@@ -887,8 +873,7 @@ int qsae_matryoshka_forward_active(const float* x_f32, const uint16_t* w_bf16, c
   }
   rc = launch_status("cast x", cast_bf16_launch(x_f32, x_bf16, static_cast<size_t>(B) * D, st));
   if (rc != QSAE_OK) return rc;
-  EncodeLaunch el;
-  fill_encode_launch(&el, mp.st, B, D, QSAE_ACT_NONE, b_enc, ws);
+  EncodeLaunch el = stage_launch(mp.st, B, D, QSAE_ACT_NONE, b_enc, ws);
   el.prior = exact ? thr : nullptr; el.prior_stride = 1; el.prior_const = kActiveThreshold;   // per-row band, or one constant threshold (by value)
   el.overflow = overflow;
   rc = launch_status("encode kernel (threshold)", encode_topk_launch(x_bf16, w_bf16, el, st));
@@ -1123,8 +1108,7 @@ struct StepOperand {
 int dense_encode_tc(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_mid, const uint16_t* w_lo,
                     const float* b_enc, int B, int H, int D, int act, uint8_t* x_parts, float* out_f32, uint16_t* out_hi,
                     uint16_t* out_lo, cudaStream_t st, const StepOperand* step = nullptr) {
-  EncodeLaunch el;
-  memset(&el, 0, sizeof(el));
+  EncodeLaunch el{};
   el.B = B; el.H = H; el.D = D; el.act = act; el.bias = b_enc;
   if (act == 2) {
     if (!step) return fail(QSAE_ERR_INVALID_ARGUMENT, "dense encoder: step operand without its description");
@@ -1162,9 +1146,8 @@ int dense_encode_tc(const float* x_f32, const uint16_t* w_hi, const uint16_t* w_
 namespace {
 struct TsaePlan { size_t x_off, hi_off, lo_off, dec_off, total; };
 int plan_tsae(int B, int H, int D, int exact, TsaePlan* tp) {
-  if (B <= 0 || H <= 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "B and H must be positive (B=%d H=%d)", B, H);
-  if (D < 8 || D > 512 || (D % 8) != 0)
-    return fail(QSAE_ERR_INVALID_ARGUMENT, "D must be a multiple of 8 in [8, 512], got %d", D);
+  const int rc = check_encode_shape(B, H, D);
+  if (rc != QSAE_OK) return rc;
   if ((H % 8) != 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "t_sae: hidden_dim must be a multiple of 8, got %d", H);
   tp->x_off = 0;
   tp->hi_off = (exact ? 3 : 1) * align_up(static_cast<size_t>(B) * D * 2, 1024);
@@ -1321,8 +1304,7 @@ int qsae_tsae_backward(const float* x, const float* h, const float* g_recon, con
   // grad b_enc = sum_b gz: column sums from the same epilogue (atomics)
   cudaError_t e = cudaMemsetAsync(grad_b_enc, 0, static_cast<size_t>(H) * 4, st);
   if (e != cudaSuccess) return fail(QSAE_ERR_CUDA, "tsae_backward: %s", cudaGetErrorString(e));
-  EncodeLaunch el;
-  memset(&el, 0, sizeof(el));
+  EncodeLaunch el{};
   el.B = B; el.H = H; el.D = D; el.act = 3; el.bias = nullptr; el.gate = h; el.gate_add = g_h; el.gate_colsum = grad_b_enc;
   el.n_tiles = (H + kEncBN - 1) / kEncBN;
   el.n_splits = 1;
@@ -1540,8 +1522,7 @@ int qsae_topk_dense(const float* z, int R, int H, int k, float* out_vals, int32_
   int* cnt = reinterpret_cast<int*>(ws + static_cast<size_t>(R) * kDenseCap * 8);
   int rc = launch_status("dense_candidates", dense_candidates_launch(z, R, H, k, cand, cnt, S(stream)));
   if (rc != QSAE_OK) return rc;
-  SelectLaunch sl;
-  memset(&sl, 0, sizeof(sl));
+  SelectLaunch sl{};
   sl.B = R; sl.H = H; sl.D = 0; sl.k_sel = k; sl.k_out = k; sl.nsub = 1; sl.cap = kDenseCap;
   sl.cand = cand; sl.cand_cnt = cnt; sl.out_vals = out_vals; sl.out_idx = out_idx;
   return launch_status("select_topk kernel", select_topk_launch(sl, S(stream)));
@@ -1615,8 +1596,7 @@ int merge_candidates_impl(const void* cand_all, const void* const* list_bases, i
   int32_t* ovf_rows = reinterpret_cast<int32_t*>(static_cast<uint8_t*>(workspace) + 256);
   cudaError_t ce = cudaMemsetAsync(counters, 0, 2 * sizeof(int), st);
   if (ce != cudaSuccess) return fail(QSAE_ERR_CUDA, "merge_candidates: %s", cudaGetErrorString(ce));
-  SelectLaunch sl;
-  memset(&sl, 0, sizeof(sl));
+  SelectLaunch sl{};
   sl.B = B; sl.H = n_shards * shard_latents; sl.k_sel = k_out; sl.k_out = k_out; sl.nsub = n_shards; sl.cap = k_in;
   sl.cand = cand_all;                 // [n_shards][B][k_in] entries, every list full
   sl.list_bases = list_bases;         // or one [B][k_in] list array per shard, in that shard's (peer) memory

@@ -25,4 +25,4 @@ for _ in range(iters):
 e.record()
 torch.cuda.synchronize()
 t = s.elapsed_time(e) / iters
-print(f"mode={os.environ.get('QSAE_ENCODE_DEBUG_MODE','0')} B={B} k={k}: {t*1e3:.1f} us  {2.0*B*H*D/t/1e9:.1f} TFLOP/s  {B/t/1e3:.2f} Mtok/s", flush=True)
+print(f"B={B} k={k}: {t*1e3:.1f} us  {2.0*B*H*D/t/1e9:.1f} TFLOP/s  {B/t/1e3:.2f} Mtok/s", flush=True)

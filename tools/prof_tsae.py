@@ -33,8 +33,7 @@ e1.record()
 torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / iters
 L.check(L.load().qsae_set_encode_kernel_events(None, None))
-import os
-print(f"dense encoder kernel (mask={os.environ.get('QSAE_DENSE_FLAGS_MASK', '-')}): {k0.elapsed_time(k1) * 1e3:.1f} us")
+print(f"dense encoder kernel: {k0.elapsed_time(k1) * 1e3:.1f} us")
 print(f"t_sae fwd B={B} exact={exact}: {ms:.3f} ms/step, {B / ms * 1e3 / 1e6:.2f} Mtok/s, "
       f"{4.0 * B * H * D / ms / 1e9:.0f} TFLOP/s (two GEMMs)")
 hi, lo = L.split_bf16(h)
