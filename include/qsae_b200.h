@@ -559,6 +559,24 @@ int qsae_matryoshka_backward_finish(const float* w, const float* w_mirror, const
                                     int n_levels, int H, int D, float c, int joint_bits, float* grad_w, float* grad_w_mirror,
                                     void* stream);
 
+/* The same STE term at any activity, from the bf16 0/1 activity mask [B, H] of qsae_matryoshka_forward_dense (an
+ * untrained q_sae has ~50 % of its latents active, far more than the active lists hold):
+ *   grad_w[h,d] += alpha[h] M[h,d] s'(w[h,d]), same for the mirror,  M[h,:] = sum_b mask[b,h] grad_levels[level(h)][b,:]
+ *   z2[h] = sum_b mask[b,h]  (WRITTEN, exact int32; the input of the secant step, qsae_matryoshka_backward_finish)
+ * M is a tensor-core product mask^T g per level whose epilogue applies the STE factor (M never reaches memory); every
+ * element of the .grad buffers has one writer, so the result is bit-deterministic. exact != 0: the gradients enter as
+ * three bf16 parts (fp32-accurate; the mask is exact in bf16), exact = 0: one bf16 part. Workspace: the bf16 parts of
+ * the level gradients (qsae_matryoshka_backward_dense_workspace_bytes), 1024-byte aligned. No host synchronisation.
+ * Limits: H % 8 == 0, D % 16 == 0 and D <= 512, 1..8 levels; mask, gradients, weights and .grad 16-byte aligned.
+ * B == 0 zeroes z2 and leaves the gradients untouched. */
+int qsae_matryoshka_backward_dense_workspace_bytes(int B, int D, int n_levels, int exact, size_t* bytes);
+int qsae_matryoshka_backward_dense(const uint16_t* mask /* bf16 [B, H] */, int B, int H, int D,
+                                   const float* const* grad_levels /* host array of n_levels device pointers [B,D] */,
+                                   const int* level_start /* host, n_levels + 1 */, int n_levels, const float* w,
+                                   const float* w_mirror, const float* alpha /* [H] scale_vector */, int exact,
+                                   float* grad_w, float* grad_w_mirror, int32_t* z2 /* [H] */, void* workspace,
+                                   size_t workspace_bytes, void* stream);
+
 /* RigL mask maintenance of STEWeights (sae/ternary.py:27-90); weight, mask [D,H] float32 (mask holds 0 / 1), both
  * updated in place; exact order statistics by a three-pass radix select on the device, no host synchronisation.
  * Ties at a cut that torch.topk leaves unspecified are resolved by the lowest flat index.

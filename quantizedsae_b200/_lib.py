@@ -102,6 +102,9 @@ SYMBOLS = {
     "qsae_bsae_logit_grad": (_i, [_vp, _vp, _i, _i, _i, _vp, _f, _i, _vp, _vp]),
     "qsae_matryoshka_backward_scatter": (_i, [_vp, _i, _i, _i, _i, C.POINTER(_vp), C.POINTER(_i), _i, _vp, _vp, _vp]),
     "qsae_matryoshka_backward_finish": (_i, [_vp, _vp, _vp, _vp, _vp, C.POINTER(_i), _i, _i, _i, _f, _i, _vp, _vp, _vp]),
+    "qsae_matryoshka_backward_dense_workspace_bytes": (_i, [_i, _i, _i, _i, C.POINTER(_sz)]),
+    "qsae_matryoshka_backward_dense": (_i, [_vp, _i, _i, _i, C.POINTER(_vp), C.POINTER(_i), _i, _vp, _vp, _vp, _i, _vp, _vp, _vp,
+                                            _vp, _sz, _vp]),
     "qsae_rigl_workspace_bytes": (_i, [C.POINTER(_sz)]),
     "qsae_rigl_init_mask": (_i, [_vp, _vp, _i, _i, C.c_ulonglong, _vp, _sz, _vp]),
     "qsae_rigl_update_mask": (_i, [_vp, _vp, _vp, _vp, _i, _i, C.c_ulonglong, C.c_ulonglong, _vp, _sz, _vp]),
@@ -589,6 +592,29 @@ def matryoshka_backward_finish(w, w_mirror, M, z2, alpha, level_start_host, c: f
     n, ls = _level_array(level_start_host)
     check(load().qsae_matryoshka_backward_finish(w.data_ptr(), w_mirror.data_ptr(), _ptr(M), _ptr(z2), alpha.data_ptr(), ls, n, H, D,
                                                  float(c), int(joint_bits), grad_w.data_ptr(), grad_w_mirror.data_ptr(), _stream()))
+
+
+def matryoshka_backward_dense(mask: torch.Tensor, grad_levels, level_start_host, w, w_mirror, alpha, exact: bool, grad_w,
+                              grad_w_mirror) -> torch.Tensor:
+    """grad_w += alpha M s'(w), same for the mirror, M[h,:] = mask[:,h]^T grad_levels[level(h)], from a bf16 0/1 mask
+    [B, H] (tensor cores; exact: three bf16 parts of each gradient). -> z2 [H] int32 = mask.sum(0)."""
+    _need_cuda(mask, w, w_mirror, alpha, grad_w, grad_w_mirror, *grad_levels)
+    _f32c(w, w_mirror, alpha, grad_w, grad_w_mirror, *grad_levels)
+    assert mask.dtype == torch.bfloat16 and mask.dim() == 2
+    B, H = mask.shape
+    D = w.shape[1]
+    n, ls = _level_array(level_start_host)
+    assert len(grad_levels) == n and all(tuple(g.shape) == (B, D) for g in grad_levels)
+    assert tuple(w.shape) == (H, D) and grad_w.shape == w.shape and w_mirror.shape == w.shape and grad_w_mirror.shape == w.shape
+    nb = _sz(0)
+    check(load().qsae_matryoshka_backward_dense_workspace_bytes(B, D, n, int(bool(exact)), C.byref(nb)))
+    ws = _workspace(mask.device, int(nb.value))
+    z2 = torch.empty((H,), dtype=torch.int32, device=mask.device)
+    ptrs = (_vp * n)(*[g.data_ptr() for g in grad_levels])
+    check(load().qsae_matryoshka_backward_dense(mask.data_ptr(), B, H, D, ptrs, ls, n, w.data_ptr(), w_mirror.data_ptr(),
+                                                alpha.data_ptr(), int(bool(exact)), grad_w.data_ptr(), grad_w_mirror.data_ptr(),
+                                                z2.data_ptr(), ws.data_ptr(), int(nb.value), _stream()))
+    return z2
 
 
 def _rigl_ws(device) -> torch.Tensor:

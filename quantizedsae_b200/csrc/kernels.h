@@ -144,6 +144,13 @@ const char* coactivation_dense_launch(const uint16_t* mask, int K, int H, int32_
                                       cudaStream_t stream);
 const char* wgrad_launch(const uint16_t* const* a_parts, const uint16_t* const* b_parts, int n_parts, int M, int N, int K,
                          bool a_kmajor, float* c, int num_sms, cudaStream_t stream);
+// q_sae STE backward from a dense activity mask: grad_w[h, :] += alpha[h] (mask[:, h]^T g_level(h)) s'(w[h, :]), the same
+// for the mirror. mask bf16 0/1 [B, H] (H % 8 == 0); g_parts: n_parts (1 or 3) bf16 parts, each the n_levels level
+// gradients stacked [n_levels B, D] (D % 16 == 0); level_start host [n_levels + 1]. One writer per element, no atomics.
+const char* matryoshka_ste_dense_launch(const uint16_t* mask, int B, int H, int D, const uint16_t* const* g_parts, int n_parts,
+                                        const int* level_start, int n_levels, const float* w, const float* w_mirror,
+                                        const float* alpha, float* grad_w, float* grad_w_mirror, int num_sms,
+                                        cudaStream_t stream);
 
 // select_topk.cu
 struct SelectLaunch {
@@ -321,6 +328,8 @@ const char* matryoshka_scatter_launch(const int32_t* idx, int B, int cap, int H,
 const char* matryoshka_grad_finish_launch(const float* W, const float* Wm, const float* M, const int32_t* z2,
                                           const float* alpha, const int* level_start, int n_levels, int H, int D, float c,
                                           int joint_bits, float* gW, float* gWm, cudaStream_t stream);
+// z2[h] += number of rows b with mask[b, h] != 0 (bf16 mask [B, H], H % 8 == 0, 16-byte aligned rows; integer atomics)
+const char* mask_column_count_launch(const uint16_t* mask, int B, int H, int32_t* z2, cudaStream_t stream);
 size_t rigl_workspace_bytes(int sms);
 const char* rigl_init_mask_launch(float* weight, float* mask, int D, int H, unsigned long long n_inactive, void* ws, int sms,
                                   cudaStream_t stream);

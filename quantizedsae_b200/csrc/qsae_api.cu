@@ -1009,6 +1009,76 @@ int qsae_matryoshka_backward_finish(const float* w, const float* w_mirror, const
                                                      grad_w, grad_w_mirror, S(stream)));
 }
 
+namespace {
+// workspace of the dense STE backward: n_parts bf16 parts, each the n_levels level gradients stacked [n_levels B, D]
+int plan_matryoshka_backward_dense(int B, int D, int n_levels, int exact, size_t* part_bytes, size_t* total) {
+  if (B < 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_backward_dense: negative batch");
+  if (D < 16 || D > 512 || (D % 16) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_backward_dense: D must be a multiple of 16 in [16, 512], got %d", D);
+  if (n_levels < 1 || n_levels > 8) return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_backward_dense: 1..8 levels, got %d", n_levels);
+  *part_bytes = align_up(static_cast<size_t>(n_levels) * B * D * 2, 1024);
+  *total = (exact ? 3 : 1) * *part_bytes;
+  return QSAE_OK;
+}
+}  // namespace
+
+int qsae_matryoshka_backward_dense_workspace_bytes(int B, int D, int n_levels, int exact, size_t* bytes) {
+  if (!bytes) return fail(QSAE_ERR_INVALID_ARGUMENT, "workspace query: null pointer");
+  size_t part = 0;
+  return plan_matryoshka_backward_dense(B, D, n_levels, exact, &part, bytes);
+}
+
+int qsae_matryoshka_backward_dense(const uint16_t* mask, int B, int H, int D, const float* const* grad_levels,
+                                   const int* level_start, int n_levels, const float* w, const float* w_mirror,
+                                   const float* alpha, int exact, float* grad_w, float* grad_w_mirror, int32_t* z2,
+                                   void* workspace, size_t workspace_bytes, void* stream) {
+  size_t part = 0, total = 0;
+  int rc = plan_matryoshka_backward_dense(B, D, n_levels, exact, &part, &total);
+  if (rc != QSAE_OK) return rc;
+  if (H <= 0 || (H % 8) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_backward_dense: H must be a positive multiple of 8, got %d", H);
+  rc = check_levels("matryoshka_backward_dense", level_start, n_levels, H);
+  if (rc != QSAE_OK) return rc;
+  if (!w || !w_mirror || !alpha || !grad_w || !grad_w_mirror || !z2)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_backward_dense: null pointer");
+  cudaStream_t st = S(stream);
+  cudaError_t e = cudaMemsetAsync(z2, 0, static_cast<size_t>(H) * 4, st);
+  if (e != cudaSuccess) return fail(QSAE_ERR_CUDA, "matryoshka_backward_dense: %s", cudaGetErrorString(e));
+  if (B == 0) return QSAE_OK;
+  if (!mask || !grad_levels || !workspace) return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_backward_dense: null pointer");
+  if (workspace_bytes < total)
+    return fail(QSAE_ERR_WORKSPACE_TOO_SMALL, "matryoshka_backward_dense: workspace %zu < %zu bytes", workspace_bytes, total);
+  uintptr_t align16 = reinterpret_cast<uintptr_t>(mask) | reinterpret_cast<uintptr_t>(w) | reinterpret_cast<uintptr_t>(w_mirror) |
+                      reinterpret_cast<uintptr_t>(grad_w) | reinterpret_cast<uintptr_t>(grad_w_mirror);
+  for (int i = 0; i < n_levels; ++i) {
+    if (!grad_levels[i]) return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_backward_dense: grad_levels[%d] is null", i);
+    align16 |= reinterpret_cast<uintptr_t>(grad_levels[i]);
+  }
+  if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0 || (align16 & 15) != 0 || (reinterpret_cast<uintptr_t>(alpha) & 3) != 0 ||
+      (reinterpret_cast<uintptr_t>(z2) & 3) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "matryoshka_backward_dense: workspace must be 1024-byte aligned, the mask, gradients, "
+                "weights and .grad buffers 16-byte aligned");
+  // the bf16 parts of every level gradient, stacked per part: part i, level l at ws + i part + l B D
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  const int np = exact ? 3 : 1;
+  const size_t nbd = static_cast<size_t>(B) * D;
+  uint16_t* gp[3];
+  for (int i = 0; i < 3; ++i) gp[i] = reinterpret_cast<uint16_t*>(ws + (i < np ? i : 0) * part);
+  for (int l = 0; l < n_levels; ++l) {
+    const size_t off = static_cast<size_t>(l) * nbd;
+    rc = launch_status("matryoshka_backward_dense (gradient parts)",
+                       exact ? split_bf16x3_launch(grad_levels[l], gp[0] + off, gp[1] + off, gp[2] + off, nbd, st)
+                             : cast_bf16_launch(grad_levels[l], gp[0] + off, nbd, st));
+    if (rc != QSAE_OK) return rc;
+  }
+  rc = launch_status("matryoshka_backward_dense (z2)", mask_column_count_launch(mask, B, H, z2, st));
+  if (rc != QSAE_OK) return rc;
+  const uint16_t* gpc[3] = {gp[0], gp[1], gp[2]};
+  return launch_status("matryoshka_backward_dense (product)",
+                       matryoshka_ste_dense_launch(mask, B, H, D, gpc, np, level_start, n_levels, w, w_mirror, alpha, grad_w,
+                                                   grad_w_mirror, num_sms(), st));
+}
+
 int qsae_rigl_workspace_bytes(size_t* bytes) {
   if (!bytes) return fail(QSAE_ERR_INVALID_ARGUMENT, "workspace query: null pointer");
   *bytes = align_up(rigl_workspace_bytes(num_sms()), 256);

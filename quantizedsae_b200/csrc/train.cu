@@ -6,6 +6,8 @@
 //   * bsae_logit_grad: chain rule through the sigmoid bits + the polarize_loss gradient (sae/binary.py:26-43);
 //   * matryoshka_scatter / matryoshka_grad_finish: STE backward of the q_sae level decoder wrt weight and
 //     weight_mirror (sae/quantized_matryoshka.py:94-121) and apply_secant_grad (:145-190);
+//   * mask_column_count: z2 of the same backward from a dense activity mask (the product itself runs on the tensor
+//     cores, wgrad_sm100.cu);
 //   * radix select + apply kernels: STEWeights.init_mask / update_mask (RigL drop / grow, sae/ternary.py:27-87) and
 //     mask_grad (:89-90).
 // All HBM-bound elementwise / scatter work: no tensor cores. Compiled without fast-math: the logistic is the literal
@@ -261,6 +263,32 @@ matryoshka_grad_finish_kernel(const float* __restrict__ W, const float* __restri
     gW[e] += (up - (p >= 0.5f ? sec : -sec)) * (p * (1.f - p));
     gWm[e] += (up - (pm >= 0.5f ? sec : -sec)) * (pm * (1.f - pm));
   }
+}
+
+// z2[h] += #{b : mask[b,h] != 0} for a bf16 0/1 activity mask [B, H] (the dense route's z2, :137): 8 columns per
+// thread (16-byte loads, a warp reads 512 consecutive bytes of a row), a slice of the rows per grid row, one integer
+// atomic per column and slice -- exact, and the same bits in any order.
+__global__ void __launch_bounds__(256)
+mask_column_count_kernel(const uint16_t* __restrict__ mask, int B, int H, int rows_per, int32_t* __restrict__ z2) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (8 * g >= H) return;
+  const int r0 = blockIdx.y * rows_per;
+  const int r1 = min(B, r0 + rows_per);
+  int c[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  const uint16_t* col = mask + 8 * static_cast<size_t>(g);
+#pragma unroll 4
+  for (int r = r0; r < r1; ++r) {
+    const uint4 v = __ldcs(reinterpret_cast<const uint4*>(col + static_cast<size_t>(r) * H));
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      c[2 * q] += (w[q] & 0x7fffu) != 0u;
+      c[2 * q + 1] += (w[q] & 0x7fff0000u) != 0u;
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < 8; ++j)
+    if (c[j] != 0) atomicAdd(z2 + 8 * g + j, c[j]);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -731,6 +759,18 @@ const char* matryoshka_grad_finish_launch(const float* W, const float* Wm, const
   const size_t n = static_cast<size_t>(H) * D;
   if (n == 0) return nullptr;
   matryoshka_grad_finish_kernel<<<grid_for(n, 256, 148 * 16), 256, 0, stream>>>(W, Wm, M, z2, alpha, lv, H, D, c, joint_bits, gW, gWm);
+  return cuda_err(cudaGetLastError());
+}
+
+const char* mask_column_count_launch(const uint16_t* mask, int B, int H, int32_t* z2, cudaStream_t stream) {
+  if (B <= 0 || H <= 0) return nullptr;
+  const int gx = (H / 8 + 255) / 256;
+  int gy = (148 * 8 + gx - 1) / gx;              // ~8 blocks per SM
+  if (gy > B) gy = B;
+  if (gy > 65535) gy = 65535;
+  const int rows_per = (B + gy - 1) / gy;
+  gy = (B + rows_per - 1) / rows_per;
+  mask_column_count_kernel<<<dim3(gx, gy), 256, 0, stream>>>(mask, B, H, rows_per, z2);
   return cuda_err(cudaGetLastError());
 }
 

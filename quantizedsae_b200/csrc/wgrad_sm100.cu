@@ -406,6 +406,239 @@ coactivation_dense_kernel(const __grid_constant__ CUtensorMap tm, CoactParams p)
   if (warp == 2) tmem_dealloc<kTmemCols>(tmem_base);
 }
 
+// ---- STE backward of the q_sae level decoder from a dense activity mask (training.py, dense route):
+//   M[h, :] = sum_b a[b, h] g_level(h)[b, :]      (a: bf16 0/1 mask [B, H], g_l: d loss / d result[l] [B, D])
+//   grad_w[h, d] += alpha[h] M[h, d] s(w[h, d]) (1 - s(w[h, d])), the same for the mirror
+// (the STE term of matryoshka_grad_finish_kernel, train.cu, with M never written to memory). The producer and MMA
+// warps are those of wgrad_kernel (A = the mask, MN-major; B = the gradient parts, MN-major); schedule and epilogue
+// differ:
+//   - B is one stacked bf16 tensor [n_levels B, D] per part: level l's K rows start at l B. The TMA zero-fills mask
+//     rows past B, so whatever the B tile holds there (the next level's first rows) adds nothing;
+//   - a work unit is (128-row tile, level, 256-column tile), one for each level the row tile intersects (level
+//     boundaries may fall anywhere); a unit's epilogue writes only its level's rows, so each element has one writer:
+//     no atomics, and the result is bit-deterministic. Segments (row tile, level) run in row order; the dimension
+//     with fewer tiles runs fastest;
+//   - products: mask x each bf16 part of g into one accumulator (1 or 3; the mask is exact in bf16);
+//   - eight epilogue warps (two per TMEM lane quarter, 128 columns each) read w, w_mirror and both .grad rows
+//     while the next unit's MMAs run.
+struct SteDenseParams {
+  int H, D, B;
+  int m_tiles, n_tiles, n_segs, k_chunks;
+  int n_prod;
+  uint32_t prods;        // as WgradParams (A part always 0: the mask)
+  int n_fast;            // unit u -> (segment u / n_tiles, n tile u % n_tiles), else (u % n_segs, u / n_segs)
+  int n_levels;
+  int start[9];          // level l owns rows [start[l], start[l + 1])
+  const float* w;
+  const float* wm;
+  const float* alpha;
+  float* gw;
+  float* gwm;
+};
+
+// segments (row tile, non-empty level intersecting it) before row tile mt
+__host__ __device__ inline int ste_seg_first(const int* start, int n_levels, int mt) {
+  int s = 0;
+  for (int l = 0; l < n_levels; ++l) {
+    if (start[l] >= start[l + 1]) continue;
+    const int lo = start[l] / BM, hi = (start[l + 1] - 1) / BM + 1;   // row tiles [lo, hi) of level l
+    const int e = hi < mt ? hi : mt;
+    if (e > lo) s += e - lo;
+  }
+  return s;
+}
+
+// segment index -> (row tile, level); a tile holds at most n_levels segments, so the search is short
+__device__ __forceinline__ void ste_seg_of(const SteDenseParams& p, int s, int* mt, int* level) {
+  int t = s < p.m_tiles - 1 ? s : p.m_tiles - 1;
+  int f = ste_seg_first(p.start, p.n_levels, t);
+  while (f > s) f = ste_seg_first(p.start, p.n_levels, --t);
+  int j = s - f;
+  const int r0 = t * BM, r1 = r0 + BM;
+  int lv = 0;
+  for (int l = 0; l < p.n_levels; ++l) {
+    if (p.start[l] < p.start[l + 1] && p.start[l] < r1 && p.start[l + 1] > r0) {
+      if (j == 0) { lv = l; break; }
+      --j;
+    }
+  }
+  *mt = t;
+  *level = lv;
+}
+
+__device__ __forceinline__ void ste_unit(const SteDenseParams& p, int u, int* m0, int* n0, int* level) {
+  const int s = p.n_fast ? u / p.n_tiles : u % p.n_segs;
+  const int nt = p.n_fast ? u % p.n_tiles : u / p.n_segs;
+  int mt;
+  ste_seg_of(p, s, &mt, level);
+  *m0 = mt * BM;
+  *n0 = nt * BN;
+}
+
+// the literal fp32 logistic of train.cu (this file is compiled without fast-math as well)
+__device__ __forceinline__ float ste_logistic(float w) { return 1.0f / (1.0f + expf(-w)); }
+
+__global__ void __launch_bounds__(kCoThreads, 1)
+matryoshka_ste_dense_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ CUtensorMap tg0,
+                            const __grid_constant__ CUtensorMap tg1, const __grid_constant__ CUtensorMap tg2,
+                            const __grid_constant__ SteDenseParams p) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kBarOff);
+  uint64_t* full = bars;
+  uint64_t* empty = bars + kStages;
+  uint64_t* tmem_full = bars + 2 * kStages;
+  uint64_t* tmem_empty = tmem_full + 2;
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 4);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int n_units = p.n_segs * p.n_tiles;
+  const int k_iters = p.n_prod * p.k_chunks;
+  if (threadIdx.x == 0) {
+    if ((smem_u32(smem) & 1023u) != 0u) {
+      printf("qsae: dynamic shared memory is not 1024-byte aligned\n");
+      __trap();
+    }
+    for (int s = 0; s < kStages; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], 1);
+    }
+    for (int a = 0; a < 2; ++a) {
+      mbar_init(&tmem_full[a], 1);
+      mbar_init(&tmem_empty[a], kCoEpiWarps);
+    }
+    fence_mbar_init();
+    fence_proxy_async_smem();
+  }
+  if (warp == 2) tmem_alloc<kTmemCols>(tmem_ptr);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_ptr;
+
+  if (warp == 0) {
+    if (lane == 0) {
+      tma_prefetch_desc(&tm);
+      tma_prefetch_desc(&tg0);
+      int stage = 0;
+      uint32_t phase = 0;
+      for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
+        int m0, n0, level;
+        ste_unit(p, u, &m0, &n0, &level);
+        const int kbase = level * p.B;
+#pragma unroll 1
+        for (int it = 0; it < k_iters; ++it) {
+          const int pi = it / p.k_chunks, kc = it - pi * p.k_chunks;
+          const int bi = (p.prods >> (4 * pi)) & 3;
+          const CUtensorMap* tg = bi == 0 ? &tg0 : (bi == 1 ? &tg1 : &tg2);
+          mbar_wait(&empty[stage], phase ^ 1u);
+          uint8_t* st = smem + stage * kStageBytes;
+          mbar_arrive_expect_tx(&full[stage], kStageBytes);
+          const int k0 = kc * BK;
+#pragma unroll
+          for (int c = 0; c < BM / 64; ++c) tma_load_2d(st + c * kColBytes, &tm, &full[stage], m0 + 64 * c, k0, kPolicyEvictNormal);
+#pragma unroll
+          for (int c = 0; c < BN / 64; ++c)
+            tma_load_2d(st + kABytes + c * kColBytes, tg, &full[stage], n0 + 64 * c, kbase + k0, kPolicyEvictNormal);
+          if (++stage == kStages) { stage = 0; phase ^= 1u; }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      constexpr uint32_t idesc = umma_idesc_bf16_f32_major(BM, BN, true, true);
+      int stage = 0;
+      uint32_t phase = 0;
+      int t = 0;
+      for (int u = blockIdx.x; u < n_units; u += gridDim.x, ++t) {
+        const int acc = t & 1;
+        mbar_wait(&tmem_empty[acc], ((t >> 1) & 1) ^ 1u);
+        tc_fence_after();
+        const uint32_t d_tmem = tmem_base + acc * BN;
+#pragma unroll 1
+        for (int it = 0; it < k_iters; ++it) {
+          mbar_wait(&full[stage], phase);
+          tc_fence_after();
+          const uint32_t st = smem_u32(smem + stage * kStageBytes);
+          const uint64_t a_desc = umma_desc_mnmajor_sw128(st, kColBytes);
+          const uint64_t b_desc = umma_desc_mnmajor_sw128(st + kABytes, kColBytes);
+#pragma unroll
+          for (int ks = 0; ks < BK / UMMA_K; ++ks) {
+            const uint64_t step = static_cast<uint64_t>(ks) * (2048 >> 4);   // 16 K rows = two 1024-byte atoms
+            umma_f16_ss(d_tmem, a_desc + step, b_desc + step, idesc, (it | ks) != 0 ? 1u : 0u);
+          }
+          umma_commit(&empty[stage]);
+          if (it == k_iters - 1) umma_commit(&tmem_full[acc]);
+          if (++stage == kStages) { stage = 0; phase ^= 1u; }
+        }
+      }
+    }
+  } else if (warp >= 4) {
+    const int e = warp - 4;
+    const int quad = e & 3;                    // TMEM lanes 32 quad .. +31 (warp_id % 4)
+    const int cbase = (e >> 2) * (BN / 2);     // this warp's 128 columns of the tile
+    const uint32_t lane_taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
+    int t = 0;
+    for (int u = blockIdx.x; u < n_units; u += gridDim.x, ++t) {
+      int m0, n0, level;
+      ste_unit(p, u, &m0, &n0, &level);
+      const int acc = t & 1;
+      mbar_wait(&tmem_full[acc], (t >> 1) & 1);
+      tc_fence_after();
+      const int row = m0 + quad * 32 + lane;
+      const bool row_ok = row >= p.start[level] && row < p.start[level + 1];
+      if (__ballot_sync(0xffffffffu, row_ok) != 0u) {
+        const float a = row_ok ? p.alpha[row] : 0.f;
+        const size_t roff = static_cast<size_t>(row) * p.D;
+#pragma unroll 1
+        for (int c0 = cbase; c0 < cbase + BN / 2; c0 += 32) {
+          const int nc = n0 + c0;
+          if (nc >= p.D) break;                 // warp-uniform; D % 16 == 0
+          uint32_t r[32];
+          tmem_ld_32x32b_x32(lane_taddr + acc * BN + c0, r);
+          tmem_ld_wait();
+          if (!row_ok) continue;
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            const int cc = nc + 16 * h;
+            if (cc >= p.D) break;
+            float4 w4[4], wm4[4], g4[4], gm4[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+              w4[q] = *reinterpret_cast<const float4*>(p.w + roff + cc + 4 * q);
+              wm4[q] = *reinterpret_cast<const float4*>(p.wm + roff + cc + 4 * q);
+              g4[q] = *reinterpret_cast<const float4*>(p.gw + roff + cc + 4 * q);
+              gm4[q] = *reinterpret_cast<const float4*>(p.gwm + roff + cc + 4 * q);
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+              const float* wv = reinterpret_cast<const float*>(&w4[q]);
+              const float* wmv = reinterpret_cast<const float*>(&wm4[q]);
+              float* gv = reinterpret_cast<float*>(&g4[q]);
+              float* gmv = reinterpret_cast<float*>(&gm4[q]);
+#pragma unroll
+              for (int i = 0; i < 4; ++i) {
+                const float up = a * __uint_as_float(r[16 * h + 4 * q + i]);
+                const float s = ste_logistic(wv[i]), sm = ste_logistic(wmv[i]);
+                gv[i] += up * (s * (1.f - s));
+                gmv[i] += up * (sm * (1.f - sm));
+              }
+              *reinterpret_cast<float4*>(p.gw + roff + cc + 4 * q) = g4[q];
+              *reinterpret_cast<float4*>(p.gwm + roff + cc + 4 * q) = gm4[q];
+            }
+          }
+        }
+      }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&tmem_empty[acc]);
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  if (warp == 2) tmem_dealloc<kTmemCols>(tmem_base);
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -509,6 +742,48 @@ const char* coactivation_dense_launch(const uint16_t* mask, int K, int H, int32_
   }
   const int grid = p.n_units < num_sms ? p.n_units : num_sms;
   coactivation_dense_kernel<<<grid, kCoThreads, kSmem, stream>>>(tm, p);
+  return cuda_err(cudaGetLastError());
+}
+
+const char* matryoshka_ste_dense_launch(const uint16_t* mask, int B, int H, int D, const uint16_t* const* g_parts, int n_parts,
+                                        const int* level_start, int n_levels, const float* w, const float* w_mirror,
+                                        const float* alpha, float* grad_w, float* grad_w_mirror, int num_sms,
+                                        cudaStream_t stream) {
+  if (n_parts != 1 && n_parts != 3) return "matryoshka_ste_dense: 1 or 3 parts of the gradients";
+  if (n_levels < 1 || n_levels > 8) return "matryoshka_ste_dense: 1..8 levels";
+  if (B <= 0 || H <= 0 || (H % 8) != 0 || D <= 0 || (D % 16) != 0)
+    return "matryoshka_ste_dense: B, H, D must be positive, H a multiple of 8 and D of 16";
+  CUtensorMap tm, tg[3];
+  if (!make_tmap(&tm, mask, B, H, BK)) return "cuTensorMapEncodeTiled(ste mask) failed";
+  for (int i = 0; i < 3; ++i)
+    if (!make_tmap(&tg[i], g_parts[i < n_parts ? i : 0], n_levels * B, D, BK)) return "cuTensorMapEncodeTiled(ste gradients) failed";
+  SteDenseParams p;
+  p.H = H; p.D = D; p.B = B;
+  p.m_tiles = (H + BM - 1) / BM;
+  p.n_tiles = (D + BN - 1) / BN;
+  p.k_chunks = (B + BK - 1) / BK;
+  p.n_levels = n_levels;
+  for (int i = 0; i < 9; ++i) p.start[i] = level_start[i <= n_levels ? i : n_levels];
+  p.n_segs = ste_seg_first(p.start, n_levels, p.m_tiles);
+  if (n_parts == 1) {
+    p.n_prod = 1;
+    p.prods = 0u;
+  } else {
+    // mask x (lo, mid, hi): smallest first
+    p.n_prod = 3;
+    p.prods = 2u | (1u << 4) | (0u << 8);
+  }
+  p.n_fast = p.n_tiles <= p.n_segs ? 1 : 0;
+  p.w = w; p.wm = w_mirror; p.alpha = alpha; p.gw = grad_w; p.gwm = grad_w_mirror;
+  static bool attr = false;
+  if (!attr) {
+    cudaError_t e = cudaFuncSetAttribute(matryoshka_ste_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+    if (e != cudaSuccess) return cuda_err(e);
+    attr = true;
+  }
+  const int units = p.n_segs * p.n_tiles;
+  const int grid = units < num_sms ? units : num_sms;
+  matryoshka_ste_dense_kernel<<<grid, kCoThreads, kSmem, stream>>>(tm, tg[0], tg[1], tg[2], p);
   return cuda_err(cudaGetLastError());
 }
 

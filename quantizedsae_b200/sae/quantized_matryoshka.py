@@ -126,8 +126,9 @@ class QuantizedMatryoshkaDecoder(nn.Module):
     # ---- training-side (SURVEY 8f-4; quantizedsae_b200/training.py) --------------------------
     def ste_backward(self, active_idx, grad_levels, batch_size=None):
         """Accumulate the STE gradients of weight / weight_mirror / bias for upstream gradients
-        grad_levels[i] = d loss / d result[i] (what loss.backward() leaves there in the reference, :94-124);
-        active_idx [B, cap] from QuantizedMatryoshkaSAE.forward_active. Returns z2 (:137)."""
+        grad_levels[i] = d loss / d result[i] (what loss.backward() leaves there in the reference, :94-124) at any
+        activity: active_idx is the int32 active lists [B, cap] of QuantizedMatryoshkaSAE.forward_active, or the bf16
+        activity mask [B, H] of forward_dense_active (a tensor-core product, fp32-accurate). Returns z2 (:137)."""
         from .. import training
         return training.qsae_ste_backward(self, active_idx, grad_levels, batch_size)
 
@@ -172,6 +173,7 @@ class QuantizedMatryoshkaSAE(SparseAutoencoder):
         self.last_overflow = None            # device flag of the last sparse forward (1: lists overflowed, outputs NaN)
         self._regime = None                  # (weight key, "sparse" | "dense"): decided by the first forward of a weight version
         self._pending = None                 # (pinned host flag, event) of the last unchecked sparse forward
+        self._train_l0_over_h = 0.0          # mean active latents per row / H of the last training step (training.py)
         self._prep = PreparedCache()
 
     def _w_bf16(self):

@@ -11,10 +11,14 @@ b_sae   `bsae_forward(model, x)` (what `BinarySAE.forward` runs when `model.auto
         decoder.bias. Backward of sae/binary.py:24-47 and :91-99: sparse outer products (16-byte vector reductions),
         row dots against the soft dictionary, one streaming pass over the bit logits that applies the sigmoid chain
         rule and adds the polarize gradient. The returned latent carries no gradient (the trainer only logs it).
-q_sae   `QuantizedMatryoshkaDecoder.ste_backward(grad_levels)`: what loss.backward() leaves in decoder.weight.grad,
-        weight_mirror.grad and bias.grad (STE through the sign, sae/quantized_matryoshka.py:94-124, joint_gradient =
-        False), from the active lists of `QuantizedMatryoshkaSAE.forward_active`; `apply_secant_grad()` (:145-190).
-        `qsae_trainer_decoder_grads` strings them together under the trainer's loss (training/trainer.py:88-113).
+q_sae   `QuantizedMatryoshkaDecoder.ste_backward(active, grad_levels)`: what loss.backward() leaves in
+        decoder.weight.grad, weight_mirror.grad and bias.grad (STE through the sign, sae/quantized_matryoshka.py:94-124,
+        joint_gradient = False), at any activity: from the active lists of `QuantizedMatryoshkaSAE.forward_active`
+        (int32, a scatter of the level gradients) or from the bf16 activity mask of `forward_dense_active` (a
+        tensor-core product mask^T g per level with the STE factor in its epilogue); `apply_secant_grad()`
+        (:145-190). `qsae_trainer_decoder_grads` strings them together under the trainer's loss
+        (training/trainer.py:88-113) and picks the route from the activity, so it runs from initialisation (~50 %
+        of the latents active) to the end of the sparsity schedule.
         The encoder side of q_sae's backward is dense (the STE passes a gradient to every latent, :99) and is not
         built: its STE and sparsity-term semantics are not pinned here.
 t_sae   `tsae_forward(model, x)` (what `TernarySparseAutoencoder.forward` runs when `model.autograd = True` and grad
@@ -103,22 +107,31 @@ def bsae_forward(model, x):
 
 # ---- q_sae --------------------------------------------------------------------------------------------
 
-def qsae_ste_backward(decoder, active_idx: torch.Tensor, grad_levels, batch_size: int | None = None) -> torch.Tensor:
+def qsae_ste_backward(decoder, active_idx, grad_levels, batch_size: int | None = None, *, exact: bool = True) -> torch.Tensor:
     """Accumulate into decoder.weight.grad / weight_mirror.grad / bias.grad what autograd leaves there for upstream
-    gradients grad_levels[i] = d loss / d result[i] (sae/quantized_matryoshka.py:94-124). Returns z2 [H] int32 (the
-    per-latent activity counts, :137) and stashes it for apply_secant_grad."""
+    gradients grad_levels[i] = d loss / d result[i] (sae/quantized_matryoshka.py:94-124). `active_idx`: the int32
+    active lists [B, cap] of forward_active, or the bf16 activity mask [B, H] of forward_dense_active (any activity;
+    exact: the mask product takes three bf16 parts of each gradient, fp32-accurate, else one). Returns z2 [H] int32
+    (the per-latent activity counts, :137) and stashes it for apply_secant_grad."""
     H, D = decoder.in_features, decoder.out_features
     dev = decoder.weight.device
     gl = [g.detach().contiguous().float() for g in grad_levels]
     if len(gl) != decoder.n_bits:
         raise ValueError(f"expected {decoder.n_bits} level gradients, got {len(gl)}")
-    M = torch.zeros((H, D), dtype=torch.float32, device=dev)
-    z2 = torch.zeros((H,), dtype=torch.int32, device=dev)
     starts = decoder._level_starts_host()
-    _lib.matryoshka_backward_scatter(active_idx, gl, starts, M, z2)
     _, alpha = decoder._packed()
-    _lib.matryoshka_backward_finish(decoder.weight.detach(), decoder.weight_mirror.detach(), M, None, alpha, starts, 0.0, 0,
-                                    _acc_grad(decoder.weight), _acc_grad(decoder.weight_mirror))
+    if active_idx.dtype == torch.bfloat16:
+        z2 = _lib.matryoshka_backward_dense(active_idx.contiguous(), gl, starts, decoder.weight.detach(),
+                                            decoder.weight_mirror.detach(), alpha, exact, _acc_grad(decoder.weight),
+                                            _acc_grad(decoder.weight_mirror))
+    elif active_idx.dtype == torch.int32:
+        M = torch.zeros((H, D), dtype=torch.float32, device=dev)
+        z2 = torch.zeros((H,), dtype=torch.int32, device=dev)
+        _lib.matryoshka_backward_scatter(active_idx, gl, starts, M, z2)
+        _lib.matryoshka_backward_finish(decoder.weight.detach(), decoder.weight_mirror.detach(), M, None, alpha, starts, 0.0, 0,
+                                        _acc_grad(decoder.weight), _acc_grad(decoder.weight_mirror))
+    else:
+        raise TypeError(f"ste_backward: int32 active lists or a bf16 activity mask expected, got {active_idx.dtype}")
     if decoder.allow_bias:
         _lib.column_sum(gl[0], 1.0, _acc_grad(decoder.bias))
     decoder._ctx = {"z2": z2, "batch_size": int(batch_size if batch_size is not None else active_idx.shape[0])}
@@ -138,15 +151,48 @@ def qsae_apply_secant_grad(decoder) -> None:
                                     _acc_grad(decoder.weight), _acc_grad(decoder.weight_mirror))
 
 
+# Sparse / dense crossover of the decoder-side step: the sparse step (forward_active + scatter) grows with the mean
+# list length L0 (the scatter issues L0 D reductions per row), the dense step (forward_dense_active + mask product)
+# costs the same at any activity. Measured with tools/prof_qsae_train_dense.py on a B200 (1000 W limit;
+# profiles/r6_qsae_train_dense.md), 512 -> 32768, n_bits 4, B = 4096, exact: sparse 0.93 ms at L0 = 33, 1.90 ms at
+# 128, 2.59 ms at 256; dense 1.62-1.66 ms throughout. Linear between the first two, they cross at L0 ~ 100, L0 / H ~ 1/320.
+# The step cannot know its own L0 before its forward, so the decision uses the previous step's (activity moves
+# slowly under training); a step that overflows the lists goes dense at once.
+_DENSE_TRAIN_L0_OVER_H = 1.0 / 320
+
+
+def _qsae_train_active(model, x, active_cap: int) -> dict:
+    """The forward of a training step with its activity: forward_active's lists, or forward_dense_active's bf16 mask
+    when the model's regime is already dense, the previous step's mean list length passed the crossover, or the rows
+    overflow the lists (the regime is then recorded as dense, as model(x) does). Records this step's L0 / H."""
+    H = model.hidden_dim
+    dense_ok = model.dense_mode != "never" and H % 8 == 0
+    r = None
+    if not model._known_dense() and not (dense_ok and model._train_l0_over_h > _DENSE_TRAIN_L0_OVER_H):
+        r = model._forward_lists(x, active_cap)
+        if r is None:
+            if model.dense_mode == "never":
+                raise RuntimeError("q_sae: a row has more active latents than the sparse path holds and dense_mode is 'never'")
+            model._regime = (model._weights_key(), "dense")
+    if r is None:
+        r = model.forward_dense_active(x)
+    model._train_l0_over_h = float(r["level_counts"].sum()) / max(1, x.shape[0] * H)
+    return r
+
+
 def qsae_trainer_decoder_grads(model, x, active_cap: int = 256):
     """One q_sae step of the reference trainer as far as the decoder is concerned (training/trainer.py:88-113):
-    forward, recon_loss = sum_i 0.5 * mse(result_i, x), decoder gradients of it, apply_secant_grad.
-    -> dict(recon_losses [n_bits] device tensor, latent_groups, reconstruction_levels)."""
-    out = model.forward_active(x, active_cap)
+    forward, recon_loss = sum_i 0.5 * mse(result_i, x), decoder gradients of it, apply_secant_grad. Any activity: the
+    route (active lists and a scatter, or an activity mask and a tensor-core product) follows the activity, and
+    model.last_path records which forward ran. -> dict(recon_losses [n_bits] device tensor, latent_groups,
+    reconstruction_levels)."""
+    x = x.contiguous().float()
+    out = _qsae_train_active(model, x, active_cap)
     B, D = x.shape
     levels = out["reconstruction_levels"]
     grads = [(r - x) / float(B * D) for r in levels]
-    qsae_ste_backward(model.decoder, out["active_idx"], grads, B)
+    active = out["active_mask"] if "active_mask" in out else out["active_idx"]
+    qsae_ste_backward(model.decoder, active, grads, B, exact=model.exact)
     qsae_apply_secant_grad(model.decoder)
     losses = torch.stack([0.5 * ((r - x) ** 2).mean() for r in levels])
     return {"recon_losses": losses, "latent_groups": out["latent_groups"], "reconstruction_levels": levels}
