@@ -418,6 +418,25 @@ int qsae_tsae_backward(const float* x /* [B, D] */, const float* h /* [B, H] for
                        float* grad_w_dec /* [D, H] */, float* grad_x /* [B, D] or NULL */, void* workspace,
                        size_t workspace_bytes, void* stream);
 
+/* Backward of BaselineSparseAutoencoder.forward (Linear -> top-k -> scatter -> Linear; what torch autograd computes on
+ * the reference). With g = d loss / d recon [B, D], the forward's top-k (vals, idx) [B, k] and
+ *   gv[b,j] = <g[b,:], W_dec[:, idx[b,j]]> + g_h[b, idx[b,j]]    (g_h: dense [B, H], or g_vals [B, k]; at most one)
+ *   grad_w_enc[h,:] = sum gv x[b,:] [H, D]   grad_b_enc[h] = sum gv [H]   grad_w_dec[:,h] = sum v g[b,:] [D, H]
+ * over the rows b that selected h; grad_b_dec = sum_b g [D]; grad_x = gv W_enc [B, D] over the kept entries (NULL: not
+ * computed, w_enc unused). dec_rows [H, D] = W_dec^T (qsae_transpose_f32). The entries are grouped by latent with a
+ * stable sort, so each output element has one writer and a fixed summation order: every output is bit-deterministic.
+ * Latents no row selected get exact zeros. Outputs are overwritten. Caller workspace, one stream, no host
+ * synchronisation (CUDA-graph capturable). Same shape rules as qsae_encode_topk (D a multiple of 8 in [8, 512],
+ * 1 <= k <= H), B k < 2^31; B may be 0 (zero gradients). x, g_recon, w_enc, dec_rows, grad_w_enc, grad_x and the
+ * workspace 16-byte aligned. */
+int qsae_baseline_backward_workspace_bytes(int B, int H, int D, int k, size_t* bytes);
+int qsae_baseline_backward(const float* x /* [B, D] */, const float* vals, const int32_t* idx /* [B, k] */,
+                           const float* g_recon /* [B, D] */, const float* g_h /* [B, H] or NULL */,
+                           const float* g_vals /* [B, k] or NULL */, const float* w_enc /* [H, D], grad_x only */,
+                           const float* dec_rows /* [H, D] */, int B, int H, int D, int k, float* grad_w_enc /* [H, D] */,
+                           float* grad_b_enc /* [H] */, float* grad_w_dec /* [D, H] */, float* grad_b_dec /* [D] */,
+                           float* grad_x /* [B, D] or NULL */, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Dictionary-sharded b_sae (2^20-latent dictionaries over G GPUs; SURVEY.md 8e). Shard g owns the
  * latents [g * shard_latents, (g + 1) * shard_latents) of nn.Linear / binary_decoder

@@ -113,6 +113,9 @@ SYMBOLS = {
     "qsae_wgrad": (_i, [C.POINTER(_vp), C.POINTER(_vp), _i, _i, _i, _i, _i, _vp, _vp]),
     "qsae_tsae_backward_workspace_bytes": (_i, [_i, _i, _i, _i, C.POINTER(_sz)]),
     "qsae_tsae_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "qsae_baseline_backward_workspace_bytes": (_i, [_i, _i, _i, _i, C.POINTER(_sz)]),
+    "qsae_baseline_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                                    _vp]),
 }
 
 
@@ -806,6 +809,43 @@ def tsae_backward(x: torch.Tensor, h: torch.Tensor, g_recon: torch.Tensor, g_h: 
                                     _ptr(w[0]), _ptr(w[1]), _ptr(w[2]), B, H, D, 1 if exact else 0, gwe.data_ptr(),
                                     gbe.data_ptr(), gwd.data_ptr(), _ptr(gx), ws.data_ptr(), ws.numel(), _stream()))
     return gwe, gbe, gwd, gx
+
+
+def baseline_backward_workspace_bytes(B: int, H: int, D: int, k: int) -> int:
+    n = _sz(0)
+    check(load().qsae_baseline_backward_workspace_bytes(B, H, D, k, C.byref(n)))
+    return int(n.value)
+
+
+def baseline_backward(x: torch.Tensor, vals: torch.Tensor, idx: torch.Tensor, g_recon: torch.Tensor,
+                      g_h: torch.Tensor | None, g_vals: torch.Tensor | None, w_enc: torch.Tensor | None,
+                      dec_rows: torch.Tensor, want_grad_x: bool):
+    """Backward of baseline_sae's forward (qsae_baseline_backward): g_h = d loss / d h dense [B, H] or g_vals over the
+    kept values [B, k] (at most one). dec_rows: decoder.weight^T [H, D]. Bit-deterministic.
+    -> (grad W_enc [H, D], grad b_enc [H], grad W_dec [D, H], grad b_dec [D], grad x [B, D] | None)"""
+    _need_cuda(x, vals, idx, g_recon, g_h, g_vals, w_enc, dec_rows)
+    _f32c(x, vals, g_recon, g_h, g_vals, w_enc, dec_rows)
+    B, D = x.shape
+    H = dec_rows.shape[0]
+    k = idx.shape[1]
+    assert vals.shape == (B, k) and idx.shape == (B, k) and idx.dtype == torch.int32 and g_recon.shape == (B, D)
+    assert dec_rows.shape == (H, D) and (w_enc is None or w_enc.shape == (H, D))
+    assert g_h is None or g_h.shape == (B, H)
+    assert g_vals is None or g_vals.shape == (B, k)
+    if want_grad_x and w_enc is None:
+        raise ValueError("baseline_backward: grad_x needs the encoder weight")
+    dev = x.device
+    gwe = torch.empty((H, D), dtype=torch.float32, device=dev)
+    gbe = torch.empty((H,), dtype=torch.float32, device=dev)
+    gwd = torch.empty((D, H), dtype=torch.float32, device=dev)
+    gbd = torch.empty((D,), dtype=torch.float32, device=dev)
+    gx = torch.empty((B, D), dtype=torch.float32, device=dev) if want_grad_x else None
+    ws = _workspace(dev, baseline_backward_workspace_bytes(B, H, D, k))
+    check(load().qsae_baseline_backward(x.data_ptr(), vals.data_ptr(), idx.data_ptr(), g_recon.data_ptr(), _ptr(g_h),
+                                        _ptr(g_vals), _ptr(w_enc) if want_grad_x else None, dec_rows.data_ptr(), B, H, D, k,
+                                        gwe.data_ptr(), gbe.data_ptr(), gwd.data_ptr(), gbd.data_ptr(), _ptr(gx),
+                                        ws.data_ptr(), ws.numel(), _stream()))
+    return gwe, gbe, gwd, gbd, gx
 
 
 def pack_candidates(vals: torch.Tensor, idx: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:

@@ -337,6 +337,12 @@ const char* rigl_update_mask_launch(float* weight, float* mask, const float* ame
                                     unsigned long long n_drop, unsigned long long n_grow, void* ws, int sms,
                                     cudaStream_t stream);
 const char* mul_inplace_launch(float* a, const float* b, size_t n, cudaStream_t stream);
+// baseline_sae backward (deterministic, latent-major): gradients of both Linear layers, b_dec and (gx != null) x
+size_t baseline_backward_workspace_bytes(int B, int H, int D, int k);
+const char* baseline_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g,
+                                     const float* g_h, const float* g_vals, const float* w_enc, const float* dec_rows, int B,
+                                     int H, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx, void* workspace,
+                                     cudaStream_t stream);
 
 // peer.cu: flag-based exchange over CUDA IPC peer memory (dictionary-sharded forward)
 const char* peer_signal_launch(unsigned* const* targets, int n, unsigned value, cudaStream_t stream);

@@ -1412,6 +1412,61 @@ int qsae_tsae_backward(const float* x, const float* h, const float* g_recon, con
   return rc;
 }
 
+// ---- baseline_sae backward: deterministic, latent-major (csrc/train.cu)
+namespace {
+int check_baseline_backward(int B, int H, int D, int k) {
+  if (B < 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward: negative batch");
+  const int rc = check_encode_shape(B > 0 ? B : 1, H, D);   // the forward's shape rules
+  if (rc != QSAE_OK) return rc;
+  if (k < 1) return fail(QSAE_ERR_INVALID_ARGUMENT, "k must be >= 1, got %d", k);
+  if (k > H) return fail(QSAE_ERR_K_OUT_OF_RANGE, "selected index k out of range (k=%d > H=%d)", k, H);
+  if (static_cast<long long>(B) * k > 0x7fffffffLL)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward: B k = %lld entries exceed 2^31 - 1", static_cast<long long>(B) * k);
+  return QSAE_OK;
+}
+}  // namespace
+
+int qsae_baseline_backward_workspace_bytes(int B, int H, int D, int k, size_t* bytes) {
+  if (!bytes) return fail(QSAE_ERR_INVALID_ARGUMENT, "workspace query: null pointer");
+  const int rc = check_baseline_backward(B, H, D, k);
+  if (rc != QSAE_OK) return rc;
+  *bytes = baseline_backward_workspace_bytes(B, H, D, k);
+  return QSAE_OK;
+}
+
+int qsae_baseline_backward(const float* x, const float* vals, const int32_t* idx, const float* g_recon, const float* g_h,
+                           const float* g_vals, const float* w_enc, const float* dec_rows, int B, int H, int D, int k,
+                           float* grad_w_enc, float* grad_b_enc, float* grad_w_dec, float* grad_b_dec, float* grad_x,
+                           void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_baseline_backward(B, H, D, k);
+  if (rc != QSAE_OK) return rc;
+  if (g_h && g_vals) return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward: pass the latent gradient as g_h or g_vals, not both");
+  if (!grad_w_enc || !grad_b_enc || !grad_w_dec || !grad_b_dec)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward: null gradient pointer");
+  cudaStream_t st = S(stream);
+  const size_t nhd = static_cast<size_t>(H) * D;
+  if (B == 0) {   // nothing selected: zero gradients
+    cudaError_t e = cudaMemsetAsync(grad_w_enc, 0, nhd * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_b_enc, 0, static_cast<size_t>(H) * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_w_dec, 0, nhd * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_b_dec, 0, static_cast<size_t>(D) * 4, st);
+    return e == cudaSuccess ? QSAE_OK : fail(QSAE_ERR_CUDA, "baseline_backward: %s", cudaGetErrorString(e));
+  }
+  if (!x || !vals || !idx || !g_recon || !dec_rows || !workspace) return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward: null pointer");
+  if (grad_x && !w_enc) return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward: grad_x needs W_enc");
+  const size_t need = baseline_backward_workspace_bytes(B, H, D, k);
+  if (workspace_bytes < need)
+    return fail(QSAE_ERR_WORKSPACE_TOO_SMALL, "baseline_backward: workspace %zu < %zu bytes", workspace_bytes, need);
+  const uintptr_t align16 = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(g_recon) |
+                            reinterpret_cast<uintptr_t>(w_enc) | reinterpret_cast<uintptr_t>(dec_rows) |
+                            reinterpret_cast<uintptr_t>(grad_w_enc) | reinterpret_cast<uintptr_t>(grad_x) |
+                            reinterpret_cast<uintptr_t>(workspace);
+  if ((align16 & 15) != 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward: workspace and row-major tensors must be 16-byte aligned");
+  const char* err = baseline_backward_launch(x, vals, idx, g_recon, g_h, g_vals, w_enc, dec_rows, B, H, D, k, grad_w_enc,
+                                             grad_b_enc, grad_w_dec, grad_b_dec, grad_x, workspace, st);
+  return err == nullptr ? QSAE_OK : fail(QSAE_ERR_CUDA, "baseline_backward: %s", err);
+}
+
 // ---- q_sae dense fallback: any activity level (an untrained model is ~50 % active), level sums as GEMMs
 int qsae_unpack_matryoshka_t(const uint32_t* packed, int H, int D, uint16_t* t_bf16, void* stream) {
   if (!packed || !t_bf16 || H <= 0 || D <= 0 || (D % 16) != 0)

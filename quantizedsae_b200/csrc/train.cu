@@ -9,7 +9,8 @@
 //   * mask_column_count: z2 of the same backward from a dense activity mask (the product itself runs on the tensor
 //     cores, wgrad_sm100.cu);
 //   * radix select + apply kernels: STEWeights.init_mask / update_mask (RigL drop / grow, sae/ternary.py:27-87) and
-//     mask_grad (:89-90).
+//     mask_grad (:89-90);
+//   * bwd_* kernels: the deterministic latent-major backward of baseline_sae (sae/baseline.py:17-40).
 // All HBM-bound elementwise / scatter work: no tensor cores. Compiled without fast-math: the logistic is the literal
 // 1 / (1 + expf(-w)) the packing kernels use, so Bsign here equals the sign packed for the forward.
 #include <cuda_runtime.h>
@@ -815,6 +816,472 @@ const char* rigl_update_mask_launch(float* weight, float* mask, const float* ame
 const char* mul_inplace_launch(float* a, const float* b, size_t n, cudaStream_t stream) {
   if (n == 0) return nullptr;
   mul_inplace_kernel<<<grid_for(n, 256 * 4, 148 * 8), 256, 0, stream>>>(a, b, n);
+  return cuda_err(cudaGetLastError());
+}
+
+// ---------------------------------------------------------------------------------------------
+// baseline_sae backward (sae/baseline.py:17-40 under loss.backward(): Linear -> top-k -> scatter -> Linear).
+// With g = d loss / d recon and gv[b,j] = <g[b,:], W_dec[:, idx[b,j]]> + g_h[b, idx[b,j]]:
+//   grad W_enc[h,:] = sum gv x[b,:],  grad b_enc[h] = sum gv,  grad W_dec[:,h] = sum v g[b,:]
+// over the rows b that selected h; grad b_dec = column sums of g; grad x = gv W_enc (decode_rows_f32).
+// The B k entries are grouped by latent with a stable radix sort of the row-major entries (b ascends inside a
+// latent), so every gradient element has one writer and a summation order fixed by the inputs alone: the whole
+// backward is bit-deterministic, with no float atomics and no [H, D] scratch matrices.
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+constexpr int kBwdChunk = 256;   // entries one warp reduces directly; longer latents are split into chunks of this size
+constexpr int kBwdTile = 32;     // consecutive latents per block of the reduction: grad W_dec leaves in [D, 32] segments
+constexpr int kSortThreads = 256, kSortItems = 16, kSortTile = kSortThreads * kSortItems, kRadix = 256;
+constexpr int kColParts = 256;   // most partial rows of the two-level column sum
+
+__device__ __forceinline__ int clamp_key(int h, int H) { return static_cast<unsigned>(h) < static_cast<unsigned>(H) ? h : H; }
+
+// gv[b,j] = <g[b,:], rows[idx[b,j],:]> + g_h term (0 for an index outside [0, H)); cnt[h] += 1 per selection.
+// Warp per row, the row of g in registers, butterfly reductions: the same bits in every lane and on every run.
+template <int NCH>
+__global__ void __launch_bounds__(256)
+bwd_latent_grad_kernel(const float* __restrict__ g, const float* __restrict__ rows, const int32_t* __restrict__ idx,
+                       const float* __restrict__ gh_dense, const float* __restrict__ gh_vals, int B, int k, int D, int H,
+                       float* __restrict__ gv, int* __restrict__ cnt) {
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int nwarps = (gridDim.x * blockDim.x) >> 5;
+  const int nchunk = D >> 2;
+  for (int row = warp; row < B; row += nwarps) {
+    float4 gr[NCH];
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) {
+      const int q = lane + 32 * c;
+      gr[c] = q < nchunk ? reinterpret_cast<const float4*>(g + static_cast<size_t>(row) * D)[q] : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    for (int j0 = 0; j0 < k; j0 += 32) {
+      const int jl = j0 + lane;
+      const size_t e = static_cast<size_t>(row) * k + jl;
+      const int my_h = jl < k ? idx[e] : -1;
+      const bool ok = static_cast<unsigned>(my_h) < static_cast<unsigned>(H);
+      float my_gh = 0.f;
+      if (ok && gh_vals != nullptr) my_gh = gh_vals[e];
+      else if (ok && gh_dense != nullptr) my_gh = gh_dense[static_cast<size_t>(row) * H + my_h];
+      float my_dot = 0.f;
+      const int nj = min(32, k - j0);
+      for (int j = 0; j < nj; ++j) {
+        const int h = __shfl_sync(0xffffffffu, my_h, j);
+        if (static_cast<unsigned>(h) >= static_cast<unsigned>(H)) continue;
+        const float4* r = reinterpret_cast<const float4*>(rows + static_cast<size_t>(h) * D);
+        float acc = 0.f;
+#pragma unroll
+        for (int c = 0; c < NCH; ++c) {
+          const int q = lane + 32 * c;
+          if (q < nchunk) {
+            const float4 w = r[q];
+            acc += gr[c].x * w.x + gr[c].y * w.y + gr[c].z * w.z + gr[c].w * w.w;
+          }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+        if (lane == j) my_dot = acc;
+      }
+      if (jl < k) {
+        gv[e] = ok ? my_dot + my_gh : 0.f;
+        if (ok) atomicAdd(cnt + my_h, 1);     // integer counts: exact in any order
+      }
+    }
+  }
+}
+
+// Exclusive prefix sums by one block of 1024 threads (each owns a contiguous run): out[0..n], out[n] = total.
+// CHUNKED: the values are the chunk counts of the per-latent entry counts in[] (latents longer than kBwdChunk only).
+// May run in place (in == out): every thread reads and writes only its own run.
+template <bool CHUNKED>
+__global__ void __launch_bounds__(1024) bwd_scan_kernel(const int* in, int n, int* out) {
+  __shared__ int warp_tot[32];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int per = (n + 1023) / 1024;
+  const int lo = min(n, threadIdx.x * per), hi = min(n, lo + per);
+  auto value = [&](int i) {
+    const int c = in[i];
+    return CHUNKED ? (c > kBwdChunk ? (c + kBwdChunk - 1) / kBwdChunk : 0) : c;
+  };
+  int local = 0;
+  for (int i = lo; i < hi; ++i) local += value(i);
+  int incl = local;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  if (lane == 31) warp_tot[wid] = incl;
+  __syncthreads();
+  int base = 0, all = 0;
+  for (int w = 0; w < 32; ++w) {
+    if (w < wid) base += warp_tot[w];
+    all += warp_tot[w];
+  }
+  int run = base + incl - local;
+  for (int i = lo; i < hi; ++i) {
+    const int v = value(i);
+    out[i] = run;
+    run += v;
+  }
+  if (threadIdx.x == 0) out[n] = all;
+}
+
+// radix sort of the entries by latent, 8 bits per pass: digit counts of one tile of kSortTile entries, digit-major
+// [kRadix][ntiles] so that one exclusive scan gives every (digit, tile) its first output position
+__global__ void __launch_bounds__(kSortThreads)
+bwd_sort_hist_kernel(const int32_t* __restrict__ keys, int n, int H, int shift, int ntiles, int* __restrict__ hist) {
+  __shared__ int h[kRadix];
+  h[threadIdx.x] = 0;
+  __syncthreads();
+  const int base = blockIdx.x * kSortTile;
+  for (int i = threadIdx.x; i < kSortTile; i += kSortThreads)
+    if (base + i < n) atomicAdd(&h[(clamp_key(keys[base + i], H) >> shift) & (kRadix - 1)], 1);
+  __syncthreads();
+  hist[threadIdx.x * ntiles + blockIdx.x] = h[threadIdx.x];
+}
+
+// Stable scatter of one tile: rounds of 256 consecutive entries in order; inside a round the rank of an entry among
+// its digit's is its warp's earlier lanes (match_any) plus the earlier warps' counts. Intermediate passes move
+// (key, entry); the last one writes the records {b, v, gv} the reduction reads.
+template <bool LAST>
+__global__ void __launch_bounds__(kSortThreads)
+bwd_sort_scatter_kernel(const int32_t* __restrict__ keys, const int* __restrict__ src_e, int n, int H, int shift, int ntiles,
+                        const int* __restrict__ hist_off, int* __restrict__ keys_out, int* __restrict__ e_out, int k,
+                        const float* __restrict__ vals, const float* __restrict__ gv, int* __restrict__ ent_b,
+                        float* __restrict__ ent_v, float* __restrict__ ent_g) {
+  constexpr int kWarps = kSortThreads / 32;
+  __shared__ int run[kRadix];
+  __shared__ int wcnt[kWarps][kRadix];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  run[threadIdx.x] = hist_off[threadIdx.x * ntiles + blockIdx.x];
+#pragma unroll
+  for (int w = 0; w < kWarps; ++w) wcnt[w][threadIdx.x] = 0;
+  __syncthreads();
+  const int base = blockIdx.x * kSortTile;
+  for (int r = 0; r < kSortItems; ++r) {
+    const int i = base + r * kSortThreads + threadIdx.x;
+    const bool valid = i < n;
+    const int key = valid ? clamp_key(keys[i], H) : 0;
+    const int d = valid ? (key >> shift) & (kRadix - 1) : -1;
+    const unsigned peers = __match_any_sync(0xffffffffu, d);
+    const int lt = __popc(peers & ((1u << lane) - 1u));
+    if (valid && lt == 0) wcnt[wid][d] = __popc(peers);
+    __syncthreads();
+    if (valid) {
+      int pos = run[d] + lt;
+      for (int w = 0; w < wid; ++w) pos += wcnt[w][d];
+      const int e = src_e != nullptr ? src_e[i] : i;
+      if (LAST) {
+        ent_b[pos] = e / k;
+        ent_v[pos] = vals[e];
+        ent_g[pos] = gv[e];
+      } else {
+        keys_out[pos] = key;
+        e_out[pos] = e;
+      }
+    }
+    __syncthreads();
+    int s = 0;
+#pragma unroll
+    for (int w = 0; w < kWarps; ++w) {
+      s += wcnt[w][threadIdx.x];
+      wcnt[w][threadIdx.x] = 0;
+    }
+    run[threadIdx.x] += s;
+    __syncthreads();
+  }
+}
+
+// aWe += sum gv x[b,:], aWd += sum v g[b,:], sbe += sum gv over the records [lo, hi), in record order
+template <int NCH>
+__device__ __forceinline__ void bwd_reduce_entries(int lo, int hi, const int* __restrict__ ent_b, const float* __restrict__ ent_v,
+                                                   const float* __restrict__ ent_g, const float4* __restrict__ x4,
+                                                   const float4* __restrict__ g4, int nchunk, int lane, float4 (&aWe)[NCH],
+                                                   float4 (&aWd)[NCH], float& sbe) {
+  for (int e0 = lo; e0 < hi; e0 += 32) {
+    const int my = e0 + lane;
+    const int my_b = my < hi ? ent_b[my] : 0;
+    const float my_v = my < hi ? ent_v[my] : 0.f;
+    const float my_g = my < hi ? ent_g[my] : 0.f;
+    const int n = min(32, hi - e0);
+#pragma unroll 4
+    for (int j = 0; j < n; ++j) {
+      const int b = __shfl_sync(0xffffffffu, my_b, j);
+      const float v = __shfl_sync(0xffffffffu, my_v, j);
+      const float gg = __shfl_sync(0xffffffffu, my_g, j);
+      sbe += gg;
+#pragma unroll
+      for (int c = 0; c < NCH; ++c) {
+        const int q = lane + 32 * c;
+        if (q < nchunk) {
+          const float4 xr = x4[static_cast<size_t>(b) * nchunk + q];
+          const float4 gr = g4[static_cast<size_t>(b) * nchunk + q];
+          aWe[c].x = fmaf(gg, xr.x, aWe[c].x); aWe[c].y = fmaf(gg, xr.y, aWe[c].y);
+          aWe[c].z = fmaf(gg, xr.z, aWe[c].z); aWe[c].w = fmaf(gg, xr.w, aWe[c].w);
+          aWd[c].x = fmaf(v, gr.x, aWd[c].x); aWd[c].y = fmaf(v, gr.y, aWd[c].y);
+          aWd[c].z = fmaf(v, gr.z, aWd[c].z); aWd[c].w = fmaf(v, gr.w, aWd[c].w);
+        }
+      }
+    }
+  }
+}
+
+__device__ __forceinline__ void add4(float4& a, const float4 b) { a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w; }
+
+// Partials of the latents with more than kBwdChunk entries: warp per chunk q (chunks of latent h are
+// [coff[h], coff[h+1]), entries [off[h] + c kBwdChunk, ...)). part[q] = {We partial [D], Wd partial [D], be, pad}.
+template <int NCH>
+__global__ void __launch_bounds__(256)
+bwd_chunk_kernel(const int* __restrict__ off, const int* __restrict__ coff, int H, const int* __restrict__ ent_b,
+                 const float* __restrict__ ent_v, const float* __restrict__ ent_g, const float* __restrict__ x,
+                 const float* __restrict__ g, int D, float* __restrict__ part) {
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int nwarps = (gridDim.x * blockDim.x) >> 5;
+  const int nchunk = D >> 2;
+  const size_t pitch = 2 * static_cast<size_t>(D) + 4;
+  const int total = coff[H];
+  for (int q = warp; q < total; q += nwarps) {
+    int lo_h = 0, hi_h = H;                    // the last h with coff[h] <= q
+    while (hi_h - lo_h > 1) {
+      const int mid = (lo_h + hi_h) >> 1;
+      if (coff[mid] <= q) lo_h = mid;
+      else hi_h = mid;
+    }
+    const int h = lo_h;
+    const int lo = off[h] + (q - coff[h]) * kBwdChunk;
+    const int hi = min(off[h + 1], lo + kBwdChunk);
+    float4 aWe[NCH], aWd[NCH];
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) aWe[c] = aWd[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+    float sbe = 0.f;
+    bwd_reduce_entries<NCH>(lo, hi, ent_b, ent_v, ent_g, reinterpret_cast<const float4*>(x), reinterpret_cast<const float4*>(g),
+                            nchunk, lane, aWe, aWd, sbe);
+    float* p = part + static_cast<size_t>(q) * pitch;
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) {
+      const int q4 = lane + 32 * c;
+      if (q4 < nchunk) {
+        reinterpret_cast<float4*>(p)[q4] = aWe[c];
+        reinterpret_cast<float4*>(p + D)[q4] = aWd[c];
+      }
+    }
+    if (lane == 0) p[2 * D] = sbe;
+  }
+}
+
+// Latent-major reduction: block of 8 warps over kBwdTile consecutive latents, warp per latent. A latent with at most
+// kBwdChunk entries is reduced from its records, a longer one sums its chunk partials in chunk order. grad W_enc rows
+// and grad b_enc leave directly; the grad W_dec columns are staged in shared memory [kBwdTile][D + 1] and leave as
+// [D, kBwdTile] row segments. Latents nobody selected get exact zeros.
+template <int NCH>
+__global__ void __launch_bounds__(256)
+bwd_latent_reduce_kernel(const int* __restrict__ off, const int* __restrict__ coff, int H, const int* __restrict__ ent_b,
+                         const float* __restrict__ ent_v, const float* __restrict__ ent_g, const float* __restrict__ x,
+                         const float* __restrict__ g, int D, const float* __restrict__ part, float* __restrict__ gWe,
+                         float* __restrict__ gbe, float* __restrict__ gWd) {
+  extern __shared__ float stage[];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int nchunk = D >> 2;
+  const size_t pitch = 2 * static_cast<size_t>(D) + 4;
+  const int h0 = blockIdx.x * kBwdTile;
+  const int nl = min(kBwdTile, H - h0);
+  for (int l = wid; l < nl; l += blockDim.x >> 5) {
+    const int h = h0 + l;
+    float4 aWe[NCH], aWd[NCH];
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) aWe[c] = aWd[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+    float sbe = 0.f;
+    const int lo = off[h], hi = off[h + 1];
+    if (hi - lo <= kBwdChunk) {
+      bwd_reduce_entries<NCH>(lo, hi, ent_b, ent_v, ent_g, reinterpret_cast<const float4*>(x),
+                              reinterpret_cast<const float4*>(g), nchunk, lane, aWe, aWd, sbe);
+    } else {
+      for (int q = coff[h]; q < coff[h + 1]; ++q) {
+        const float* p = part + static_cast<size_t>(q) * pitch;
+#pragma unroll
+        for (int c = 0; c < NCH; ++c) {
+          const int q4 = lane + 32 * c;
+          if (q4 < nchunk) {
+            add4(aWe[c], reinterpret_cast<const float4*>(p)[q4]);
+            add4(aWd[c], reinterpret_cast<const float4*>(p + D)[q4]);
+          }
+        }
+        sbe += p[2 * D];
+      }
+    }
+    float* srow = stage + static_cast<size_t>(l) * (D + 1);
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) {
+      const int q4 = lane + 32 * c;
+      if (q4 < nchunk) {
+        reinterpret_cast<float4*>(gWe + static_cast<size_t>(h) * D)[q4] = aWe[c];
+        srow[4 * q4] = aWd[c].x; srow[4 * q4 + 1] = aWd[c].y; srow[4 * q4 + 2] = aWd[c].z; srow[4 * q4 + 3] = aWd[c].w;
+      }
+    }
+    if (lane == 0) gbe[h] = sbe;
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < D * kBwdTile; i += blockDim.x) {
+    const int d = i / kBwdTile, l = i - d * kBwdTile;
+    if (l < nl) gWd[static_cast<size_t>(d) * H + h0 + l] = stage[static_cast<size_t>(l) * (D + 1) + d];
+  }
+}
+
+// grad b_dec = column sums of g [B, D] in a fixed order: partial sums over fixed row slices, then the partials in order
+__global__ void __launch_bounds__(128)
+bwd_colsum_part_kernel(const float* __restrict__ g, int B, int D, int rows_per, float* __restrict__ part) {
+  const int t = threadIdx.x, nchunk = D >> 2;
+  if (t >= nchunk) return;
+  const int r0 = blockIdx.x * rows_per, r1 = min(B, r0 + rows_per);
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int r = r0; r < r1; ++r) add4(acc, reinterpret_cast<const float4*>(g)[static_cast<size_t>(r) * nchunk + t]);
+  reinterpret_cast<float4*>(part)[static_cast<size_t>(blockIdx.x) * nchunk + t] = acc;
+}
+
+__global__ void __launch_bounds__(128) bwd_colsum_final_kernel(const float* __restrict__ part, int nparts, int D, float* __restrict__ out) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= D) return;
+  float s = 0.f;
+#pragma unroll 8
+  for (int p = 0; p < nparts; ++p) s += part[static_cast<size_t>(p) * D + c];
+  out[c] = s;
+}
+
+struct BaselineBwdLayout {
+  int n, ntiles, npasses, max_chunks, col_rows, col_parts;
+  size_t gv, cnt, off, coff, hist, keys[2], ent[2], eb, ev, eg, part, colpart, total;
+};
+
+BaselineBwdLayout baseline_bwd_layout(int B, int H, int D, int k) {
+  BaselineBwdLayout L{};
+  L.n = B * k;
+  L.ntiles = (L.n + kSortTile - 1) / kSortTile;
+  const int key_bits = 32 - __builtin_clz(static_cast<unsigned>(H));    // keys run over [0, H]: H marks a bad index
+  L.npasses = (key_bits + 7) / 8;
+  // a latent with c > kBwdChunk entries has ceil(c / kBwdChunk) < 2 c / kBwdChunk chunks
+  L.max_chunks = static_cast<int>(2 * (static_cast<long long>(L.n) / kBwdChunk) + 1);
+  L.col_rows = B > 0 ? (B + kColParts - 1) / kColParts : 1;
+  if (L.col_rows < 32) L.col_rows = 32;
+  L.col_parts = B > 0 ? (B + L.col_rows - 1) / L.col_rows : 0;
+  const size_t n = static_cast<size_t>(L.n);
+  size_t o = 0;
+  auto take = [&](size_t bytes) {
+    const size_t s = o;
+    o = (o + bytes + 255) / 256 * 256;
+    return s;
+  };
+  L.gv = take(n * 4);
+  L.cnt = take((static_cast<size_t>(H) + 1) * 4);
+  L.off = take((static_cast<size_t>(H) + 1) * 4);
+  L.coff = take((static_cast<size_t>(H) + 1) * 4);
+  L.hist = take((static_cast<size_t>(kRadix) * L.ntiles + 1) * 4);
+  for (int i = 0; i < 2; ++i) {
+    L.keys[i] = take(n * 4);
+    L.ent[i] = take(n * 4);
+  }
+  L.eb = take(n * 4);
+  L.ev = take(n * 4);
+  L.eg = take(n * 4);
+  L.part = take(static_cast<size_t>(L.max_chunks) * (2 * static_cast<size_t>(D) + 4) * 4);
+  L.colpart = take(static_cast<size_t>(L.col_parts) * D * 4);
+  L.total = o;
+  return L;
+}
+
+template <int NCH>
+void bwd_reduce_launches(const BaselineBwdLayout& L, uint8_t* ws, int H, int D, const float* x, const float* g, float* gWe,
+                         float* gbe, float* gWd, cudaStream_t stream) {
+  const int* off = reinterpret_cast<const int*>(ws + L.off);
+  const int* coff = reinterpret_cast<const int*>(ws + L.coff);
+  const int* eb = reinterpret_cast<const int*>(ws + L.eb);
+  const float* ev = reinterpret_cast<const float*>(ws + L.ev);
+  const float* eg = reinterpret_cast<const float*>(ws + L.eg);
+  float* part = reinterpret_cast<float*>(ws + L.part);
+  // one warp per possible chunk (the device-side total decides which run): no host synchronisation
+  bwd_chunk_kernel<NCH><<<grid_for(static_cast<size_t>(L.max_chunks) * 32, 256, 148 * 8), 256, 0, stream>>>(
+      off, coff, H, eb, ev, eg, x, g, D, part);
+  const size_t smem = static_cast<size_t>(kBwdTile) * (D + 1) * sizeof(float);
+  cudaFuncSetAttribute(bwd_latent_reduce_kernel<NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+  bwd_latent_reduce_kernel<NCH><<<(H + kBwdTile - 1) / kBwdTile, 256, smem, stream>>>(off, coff, H, eb, ev, eg, x, g, D, part,
+                                                                                         gWe, gbe, gWd);
+}
+
+}  // namespace
+
+size_t baseline_backward_workspace_bytes(int B, int H, int D, int k) { return baseline_bwd_layout(B, H, D, k).total; }
+
+const char* baseline_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g,
+                                     const float* g_h, const float* g_vals, const float* w_enc, const float* dec_rows, int B,
+                                     int H, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx, void* workspace,
+                                     cudaStream_t stream) {
+  const BaselineBwdLayout L = baseline_bwd_layout(B, H, D, k);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  float* gv = reinterpret_cast<float*>(ws + L.gv);
+  int* cnt = reinterpret_cast<int*>(ws + L.cnt);
+  int* off = reinterpret_cast<int*>(ws + L.off);
+  int* coff = reinterpret_cast<int*>(ws + L.coff);
+  int* hist = reinterpret_cast<int*>(ws + L.hist);
+  const int nch = (D / 4 + 31) / 32;
+  int launches = 0;
+  cudaError_t e = cudaMemsetAsync(cnt, 0, static_cast<size_t>(H) * 4, stream);
+  if (e != cudaSuccess) return cudaGetErrorString(e);
+  // 1. gv and the per-latent counts
+  const int grid_rows = grid_for(static_cast<size_t>(B) * 32, 256, 148 * 8);
+  switch (nch) {
+    case 1: bwd_latent_grad_kernel<1><<<grid_rows, 256, 0, stream>>>(g, dec_rows, idx, g_h, g_vals, B, k, D, H, gv, cnt); break;
+    case 2: bwd_latent_grad_kernel<2><<<grid_rows, 256, 0, stream>>>(g, dec_rows, idx, g_h, g_vals, B, k, D, H, gv, cnt); break;
+    case 3: bwd_latent_grad_kernel<3><<<grid_rows, 256, 0, stream>>>(g, dec_rows, idx, g_h, g_vals, B, k, D, H, gv, cnt); break;
+    default: bwd_latent_grad_kernel<4><<<grid_rows, 256, 0, stream>>>(g, dec_rows, idx, g_h, g_vals, B, k, D, H, gv, cnt); break;
+  }
+  // 2. CSC offsets of the entries and of the chunks of long latents
+  bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(cnt, H, off);
+  bwd_scan_kernel<true><<<1, 1024, 0, stream>>>(cnt, H, coff);
+  launches += 3;
+  // 3. stable radix sort of the row-major entries by latent -> records {b, v, gv}, latent-major
+  const int32_t* keys_in = idx;
+  const int* e_in = nullptr;
+  for (int p = 0; p < L.npasses; ++p) {
+    const int shift = 8 * p;
+    const bool last = p == L.npasses - 1;
+    bwd_sort_hist_kernel<<<L.ntiles, kSortThreads, 0, stream>>>(keys_in, L.n, H, shift, L.ntiles, hist);
+    bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(hist, kRadix * L.ntiles, hist);
+    int* keys_out = reinterpret_cast<int*>(ws + L.keys[p & 1]);
+    int* e_out = reinterpret_cast<int*>(ws + L.ent[p & 1]);
+    if (last)
+      bwd_sort_scatter_kernel<true><<<L.ntiles, kSortThreads, 0, stream>>>(
+          keys_in, e_in, L.n, H, shift, L.ntiles, hist, nullptr, nullptr, k, vals, gv, reinterpret_cast<int*>(ws + L.eb),
+          reinterpret_cast<float*>(ws + L.ev), reinterpret_cast<float*>(ws + L.eg));
+    else
+      bwd_sort_scatter_kernel<false><<<L.ntiles, kSortThreads, 0, stream>>>(
+          keys_in, e_in, L.n, H, shift, L.ntiles, hist, keys_out, e_out, k, nullptr, nullptr, nullptr, nullptr, nullptr);
+    keys_in = keys_out;
+    e_in = e_out;
+    launches += 3;
+  }
+  // 4. latent-major reduction: grad W_enc, grad b_enc, grad W_dec
+  switch (nch) {
+    case 1: bwd_reduce_launches<1>(L, ws, H, D, x, g, gWe, gbe, gWd, stream); break;
+    case 2: bwd_reduce_launches<2>(L, ws, H, D, x, g, gWe, gbe, gWd, stream); break;
+    case 3: bwd_reduce_launches<3>(L, ws, H, D, x, g, gWe, gbe, gWd, stream); break;
+    default: bwd_reduce_launches<4>(L, ws, H, D, x, g, gWe, gbe, gWd, stream); break;
+  }
+  launches += 2;
+  // 5. grad b_dec
+  float* colpart = reinterpret_cast<float*>(ws + L.colpart);
+  bwd_colsum_part_kernel<<<L.col_parts, 128, 0, stream>>>(g, B, D, L.col_rows, colpart);
+  bwd_colsum_final_kernel<<<(D + 127) / 128, 128, 0, stream>>>(colpart, L.col_parts, D, gbd);
+  launches += 2;
+  // 6. grad x = gv W_enc over the kept entries: the sparse decoder over the encoder rows
+  if (gx != nullptr) {
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return cudaGetErrorString(e);
+    const char* err = decode_f32_launch(gv, idx, B, k, w_enc, H, D, 1.0f, nullptr, gx, 0, stream);
+    if (err != nullptr) return err;
+    ++launches;
+  }
+  count_launches(launches);
   return cuda_err(cudaGetLastError());
 }
 

@@ -4,6 +4,9 @@ forward(x) -> (h_sparse, recon): Linear (no ReLU, sae/baseline.py:8-10) -> top-`
 pre-activations (:35) -> Linear decode (:29). The encoder + top-k is the same fused tcgen05
 kernel as b_sae; the decoder gathers the selected columns of decoder.weight [D, H] from a
 transposed [H, D] float32 copy cached per weight version.
+
+`autograd = True` (training): the same forward behind one autograd node whose backward is the deterministic
+latent-major kernel set of csrc/train.cu (training.py, `baseline_forward`).
 """
 from __future__ import annotations
 
@@ -25,6 +28,9 @@ class BaselineSparseAutoencoder(nn.Module):
         self.hidden_dim = hidden_dim
         self.return_dense = True
         self.exact = True
+        # True: forward builds one autograd node (training.py, _BaselineSAEFn) whenever grad mode is on, so the
+        # trainer's loss.backward() fills encoder.0.weight / .bias, decoder.weight / .bias (and x) .grad
+        self.autograd = False
         self.last_flags = None
         self._prep = PreparedCache()
 
@@ -67,6 +73,9 @@ class BaselineSparseAutoencoder(nn.Module):
         return _lib.densify(vals, idx, h.shape[1])
 
     def forward(self, x):
+        if self.autograd and torch.is_grad_enabled():
+            from .. import training
+            return training.baseline_forward(self, x)
         latents = self.encode_topk(x)
         recon = _lib.decode_rows_f32(latents.values, latents.indices, self._dec_rows(), self.hidden_dim,
                                      self.input_dim, 1.0, self.decoder.bias.detach())

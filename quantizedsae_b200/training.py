@@ -36,6 +36,16 @@ t_sae   `tsae_forward(model, x)` (what `TernarySparseAutoencoder.forward` runs w
         exact = False one bf16 product per GEMM.
         `STEWeights.init_mask / update_mask / mask_grad` (sae/ternary.py:27-90): exact RigL drop / grow by radix
         select on the device.
+baseline_sae  `baseline_forward(model, x)` (what `BaselineSparseAutoencoder.forward` runs when `model.autograd = True` and
+        grad mode is on): the same (h_sparse, recon) bits as the plain forward behind ONE autograd node (h_sparse, or
+        latents.values when return_dense is off, is differentiable), so the reference trainer's baseline loop
+        (training/trainer.py:168-173) runs as written: loss.backward() fills .grad of encoder.0.weight / encoder.0.bias /
+        decoder.weight / decoder.bias (and of x when it requires grad). With g = d loss / d recon, g_h = d loss / d h and
+        gv = <g, W_dec[:, h]> + g_h at each kept entry (qsae_baseline_backward, csrc/train.cu):
+            grad W_enc[h] = sum gv x, grad b_enc[h] = sum gv, grad W_dec[:, h] = sum v g over the rows that selected h,
+            from one latent-major pass over the entries grouped by latent (one writer per element, no atomics);
+            grad b_dec = column sums of g (two fixed-order levels); grad x = gv W_enc (the sparse row decoder).
+        Every gradient is bit-deterministic.
 No CPU fallback: CUDA tensors only.
 """
 from __future__ import annotations
@@ -241,6 +251,48 @@ def tsae_forward(model, x):
     h, recon = _TernarySAEFn.apply(x, lin.weight, lin.bias, model.decoder.weight, model)
     model.decoder.input_activations = h.detach()  # the reference's forward hook (sae/ternary.py:21-22)
     return h, recon
+
+
+# ---- baseline_sae: autograd node ------------------------------------------------------------------------
+
+class _BaselineSAEFn(torch.autograd.Function):
+    """(x, W_enc, b_enc, W_dec, b_dec) -> (h_sparse [B, H] or values [B, k], indices, recon)."""
+
+    @staticmethod
+    def forward(ctx, x, w_enc, b_enc, w_dec, b_dec, model):
+        ctx.set_materialize_grads(False)
+        lat = model.encode_topk(x.detach())
+        rows = model._dec_rows()
+        recon = _lib.decode_rows_f32(lat.values, lat.indices, rows, model.hidden_dim, model.input_dim, 1.0, b_dec.detach())
+        ctx.dense = bool(model.return_dense)
+        ctx.rows = rows
+        ctx.save_for_backward(x, lat.values, lat.indices, w_enc)
+        ctx.mark_non_differentiable(lat.indices)
+        return (lat.to_dense() if ctx.dense else lat.values), lat.indices, recon
+
+    @staticmethod
+    def backward(ctx, g_lat, _g_idx, g_recon):
+        x, vals, idx, w_enc = ctx.saved_tensors
+        B, D = x.shape
+        g = (torch.zeros((B, D), dtype=torch.float32, device=x.device) if g_recon is None
+             else g_recon.detach().contiguous().float())
+        gl = None if g_lat is None else g_lat.detach().contiguous().float()
+        gwe, gbe, gwd, gbd, gx = _lib.baseline_backward(x.detach(), vals, idx, g, gl if ctx.dense else None,
+                                                        None if ctx.dense else gl, w_enc.detach().contiguous(), ctx.rows,
+                                                        want_grad_x=ctx.needs_input_grad[0])
+        return gx, gwe, gbe, gwd, gbd, None
+
+
+def baseline_forward(model, x):
+    """BaselineSparseAutoencoder.forward with an autograd node behind (h_sparse, recon) (see module docstring)."""
+    from .sae.base import require_cuda_input
+
+    x = require_cuda_input(x, model)
+    lin, dec = model.encoder[0], model.decoder
+    h, idx, recon = _BaselineSAEFn.apply(x, lin.weight, lin.bias, dec.weight, dec.bias, model)
+    if model.return_dense:
+        return h, recon
+    return SparseLatents(h, idx, (x.shape[0], model.hidden_dim)), recon
 
 
 # ---- t_sae: RigL mask maintenance ---------------------------------------------------------------------
