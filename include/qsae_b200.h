@@ -437,6 +437,29 @@ int qsae_baseline_backward(const float* x /* [B, D] */, const float* vals, const
                            float* grad_b_enc /* [H] */, float* grad_w_dec /* [D, H] */, float* grad_b_dec /* [D] */,
                            float* grad_x /* [B, D] or NULL */, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Bit-deterministic backward of BinarySAE.forward under its soft (sigmoid) dictionary (sae/binary.py:24-47, 91-103).
+ * With g = d loss / d recon [B, D], the forward's top-k (vals, idx) [B, k], q the quantization step and
+ *   gv[b,j] = q <g[b,:], soft_rows[idx[b,j], :]>,   G[h,:] = q sum v g[b,:]   (d loss / d int_w)
+ *   grad_w_enc[h,:] = sum gv x[b,:] [H, D]   grad_b_enc[h] = sum gv [H]   over the rows b that selected h;
+ *   grad_logits[h, d n + i] = (G[h,d] c_i + gp 2^i (1 - 2p) / (H D n)) p (1 - p)   [H, D n]   (qsae_bsae_logit_grad's
+ *   formula and bits for the same G; gp_dev / gp_host as there);   grad_b_dec = sum_b g [D];
+ *   grad_x = gv W_enc [B, D] over the kept entries (NULL: not computed, w_enc unused).
+ * soft_rows [H, D] is the soft dictionary (qsae_dequant_soft of logits). The entries are grouped by latent with a stable
+ * sort; each output element has one writer and a fixed summation order, so every output is bit-deterministic. G never
+ * reaches memory. Latents no row selected get exact zeros in grad_w_enc / grad_b_enc and the polarize-only logit
+ * gradient. Outputs are overwritten. Caller workspace, one stream, no host synchronisation (CUDA-graph capturable).
+ * Shape rules of qsae_encode_topk (D a multiple of 8 in [8, 512], 1 <= k <= min(H, QSAE_MAX_K_LARGE)), 1 <= n_bits <= 8,
+ * B k < 2^31; B may be 0. x, g_recon, soft_rows, logits, w_enc, grad_w_enc, grad_logits, grad_x and the workspace
+ * 16-byte aligned. */
+int qsae_bsae_backward_workspace_bytes(int B, int H, int D, int k, int n_bits, size_t* bytes);
+int qsae_bsae_backward(const float* x /* [B, D] */, const float* vals, const int32_t* idx /* [B, k] */,
+                       const float* g_recon /* [B, D] */, const float* soft_rows /* [H, D] */,
+                       const float* logits /* [H, D*n_bits] */, float q, const float* gp_dev, float gp_host,
+                       const float* w_enc /* [H, D], grad_x only */, int B, int H, int D, int k, int n_bits,
+                       float* grad_w_enc /* [H, D] */, float* grad_b_enc /* [H] */, float* grad_logits /* [H, D*n_bits] */,
+                       float* grad_b_dec /* [D] */, float* grad_x /* [B, D] or NULL */, void* workspace,
+                       size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Dictionary-sharded b_sae (2^20-latent dictionaries over G GPUs; SURVEY.md 8e). Shard g owns the
  * latents [g * shard_latents, (g + 1) * shard_latents) of nn.Linear / binary_decoder

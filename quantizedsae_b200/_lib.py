@@ -116,6 +116,9 @@ SYMBOLS = {
     "qsae_baseline_backward_workspace_bytes": (_i, [_i, _i, _i, _i, C.POINTER(_sz)]),
     "qsae_baseline_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
                                     _vp]),
+    "qsae_bsae_backward_workspace_bytes": (_i, [_i, _i, _i, _i, _i, C.POINTER(_sz)]),
+    "qsae_bsae_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _f, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp,
+                                _sz, _vp]),
 }
 
 
@@ -846,6 +849,47 @@ def baseline_backward(x: torch.Tensor, vals: torch.Tensor, idx: torch.Tensor, g_
                                         gwe.data_ptr(), gbe.data_ptr(), gwd.data_ptr(), gbd.data_ptr(), _ptr(gx),
                                         ws.data_ptr(), ws.numel(), _stream()))
     return gwe, gbe, gwd, gbd, gx
+
+
+def bsae_backward_workspace_bytes(B: int, H: int, D: int, k: int, n_bits: int) -> int:
+    n = _sz(0)
+    check(load().qsae_bsae_backward_workspace_bytes(B, H, D, k, n_bits, C.byref(n)))
+    return int(n.value)
+
+
+def bsae_backward(x: torch.Tensor, vals: torch.Tensor, idx: torch.Tensor, g_recon: torch.Tensor, soft_rows: torch.Tensor,
+                  logits: torch.Tensor, q: float, grad_polarize, w_enc: torch.Tensor | None, n_bits: int, want_grad_x: bool):
+    """Bit-deterministic backward of b_sae's soft forward (qsae_bsae_backward). soft_rows: the soft dictionary [H, D];
+    grad_polarize: python float or 0-d device tensor (read on the device, no host synchronisation).
+    -> (grad W_enc [H, D], grad b_enc [H], grad logits [H, D n_bits], grad b_dec [D], grad x [B, D] | None)"""
+    _need_cuda(x, vals, idx, g_recon, soft_rows, logits, w_enc)
+    _f32c(x, vals, g_recon, soft_rows, logits, w_enc)
+    B, D = x.shape
+    H = soft_rows.shape[0]
+    k = idx.shape[1]
+    assert vals.shape == (B, k) and idx.shape == (B, k) and idx.dtype == torch.int32 and g_recon.shape == (B, D)
+    assert soft_rows.shape == (H, D) and logits.shape == (H, D * n_bits) and (w_enc is None or w_enc.shape == (H, D))
+    if want_grad_x and w_enc is None:
+        raise ValueError("bsae_backward: grad_x needs the encoder weight")
+    gp_dev, gp_host = None, 0.0
+    if isinstance(grad_polarize, torch.Tensor):
+        _need_cuda(grad_polarize)
+        assert grad_polarize.dtype == torch.float32 and grad_polarize.numel() == 1
+        gp_dev = grad_polarize
+    else:
+        gp_host = float(grad_polarize)
+    dev = x.device
+    gwe = torch.empty((H, D), dtype=torch.float32, device=dev)
+    gbe = torch.empty((H,), dtype=torch.float32, device=dev)
+    glog = torch.empty((H, D * n_bits), dtype=torch.float32, device=dev)
+    gbd = torch.empty((D,), dtype=torch.float32, device=dev)
+    gx = torch.empty((B, D), dtype=torch.float32, device=dev) if want_grad_x else None
+    ws = _workspace(dev, bsae_backward_workspace_bytes(B, H, D, k, n_bits))
+    check(load().qsae_bsae_backward(x.data_ptr(), vals.data_ptr(), idx.data_ptr(), g_recon.data_ptr(), soft_rows.data_ptr(),
+                                    logits.data_ptr(), float(q), _ptr(gp_dev), gp_host, _ptr(w_enc) if want_grad_x else None,
+                                    B, H, D, k, n_bits, gwe.data_ptr(), gbe.data_ptr(), glog.data_ptr(), gbd.data_ptr(),
+                                    _ptr(gx), ws.data_ptr(), ws.numel(), _stream()))
+    return gwe, gbe, glog, gbd, gx
 
 
 def pack_candidates(vals: torch.Tensor, idx: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:

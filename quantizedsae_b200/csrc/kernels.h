@@ -343,6 +343,12 @@ const char* baseline_backward_launch(const float* x, const float* vals, const in
                                      const float* g_h, const float* g_vals, const float* w_enc, const float* dec_rows, int B,
                                      int H, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx, void* workspace,
                                      cudaStream_t stream);
+// b_sae backward (deterministic, latent-major, the logit chain rule fused in): gradients of the encoder Linear, the bit
+// logits, b_dec and (gx != null) x; workspace of baseline_backward_workspace_bytes(B, H, D, k)
+const char* bsae_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g, const float* soft_rows,
+                                 const float* logits, float q, const float* gp_dev, float gp_host, const float* w_enc, int B,
+                                 int H, int D, int k, int n_bits, float* gWe, float* gbe, float* glog, float* gbd, float* gx,
+                                 void* workspace, cudaStream_t stream);
 
 // peer.cu: flag-based exchange over CUDA IPC peer memory (dictionary-sharded forward)
 const char* peer_signal_launch(unsigned* const* targets, int n, unsigned value, cudaStream_t stream);

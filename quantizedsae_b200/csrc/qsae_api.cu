@@ -1467,6 +1467,64 @@ int qsae_baseline_backward(const float* x, const float* vals, const int32_t* idx
   return err == nullptr ? QSAE_OK : fail(QSAE_ERR_CUDA, "baseline_backward: %s", err);
 }
 
+// ---- b_sae backward: deterministic, latent-major, the logit chain rule fused in (csrc/train.cu)
+namespace {
+int check_bsae_backward(int B, int H, int D, int k, int n_bits) {
+  if (B < 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "bsae_backward: negative batch");
+  const int rc = check_encode_shape(B > 0 ? B : 1, H, D);   // the forward's shape rules
+  if (rc != QSAE_OK) return rc;
+  if (n_bits < 1 || n_bits > 8) return fail(QSAE_ERR_INVALID_ARGUMENT, "bsae_backward: 1 <= n_bits <= 8, got %d", n_bits);
+  if (k < 1) return fail(QSAE_ERR_INVALID_ARGUMENT, "k must be >= 1, got %d", k);
+  if (k > H) return fail(QSAE_ERR_K_OUT_OF_RANGE, "selected index k out of range (k=%d > H=%d)", k, H);
+  if (k > kMaxKLarge) return fail(QSAE_ERR_INVALID_ARGUMENT, "k=%d exceeds QSAE_MAX_K_LARGE=%d", k, kMaxKLarge);
+  if (static_cast<long long>(B) * k > 0x7fffffffLL)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "bsae_backward: B k = %lld entries exceed 2^31 - 1", static_cast<long long>(B) * k);
+  return QSAE_OK;
+}
+}  // namespace
+
+int qsae_bsae_backward_workspace_bytes(int B, int H, int D, int k, int n_bits, size_t* bytes) {
+  if (!bytes) return fail(QSAE_ERR_INVALID_ARGUMENT, "workspace query: null pointer");
+  const int rc = check_bsae_backward(B, H, D, k, n_bits);
+  if (rc != QSAE_OK) return rc;
+  *bytes = baseline_backward_workspace_bytes(B, H, D, k);   // the same regions as the baseline_sae backward
+  return QSAE_OK;
+}
+
+int qsae_bsae_backward(const float* x, const float* vals, const int32_t* idx, const float* g_recon, const float* soft_rows,
+                       const float* logits, float q, const float* gp_dev, float gp_host, const float* w_enc, int B, int H,
+                       int D, int k, int n_bits, float* grad_w_enc, float* grad_b_enc, float* grad_logits, float* grad_b_dec,
+                       float* grad_x, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_bsae_backward(B, H, D, k, n_bits);
+  if (rc != QSAE_OK) return rc;
+  if (!grad_w_enc || !grad_b_enc || !grad_logits || !grad_b_dec)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "bsae_backward: null gradient pointer");
+  if (!logits) return fail(QSAE_ERR_INVALID_ARGUMENT, "bsae_backward: null pointer");
+  const uintptr_t align16 = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(g_recon) |
+                            reinterpret_cast<uintptr_t>(soft_rows) | reinterpret_cast<uintptr_t>(logits) |
+                            reinterpret_cast<uintptr_t>(w_enc) | reinterpret_cast<uintptr_t>(grad_w_enc) |
+                            reinterpret_cast<uintptr_t>(grad_logits) | reinterpret_cast<uintptr_t>(grad_x) |
+                            reinterpret_cast<uintptr_t>(workspace);
+  if ((align16 & 15) != 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "bsae_backward: workspace and row-major tensors must be 16-byte aligned");
+  cudaStream_t st = S(stream);
+  if (B == 0) {   // nothing selected: zero encoder / bias gradients, the polarize-only logit gradient
+    const size_t nhd = static_cast<size_t>(H) * D;
+    cudaError_t e = cudaMemsetAsync(grad_w_enc, 0, nhd * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_b_enc, 0, static_cast<size_t>(H) * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_b_dec, 0, static_cast<size_t>(D) * 4, st);
+    if (e != cudaSuccess) return fail(QSAE_ERR_CUDA, "bsae_backward: %s", cudaGetErrorString(e));
+    return launch_status("bsae_backward", bsae_logit_grad_launch(logits, nullptr, H, D, n_bits, gp_dev, gp_host, 0, grad_logits, st));
+  }
+  if (!x || !vals || !idx || !g_recon || !soft_rows || !workspace) return fail(QSAE_ERR_INVALID_ARGUMENT, "bsae_backward: null pointer");
+  if (grad_x && !w_enc) return fail(QSAE_ERR_INVALID_ARGUMENT, "bsae_backward: grad_x needs W_enc");
+  const size_t need = baseline_backward_workspace_bytes(B, H, D, k);
+  if (workspace_bytes < need)
+    return fail(QSAE_ERR_WORKSPACE_TOO_SMALL, "bsae_backward: workspace %zu < %zu bytes", workspace_bytes, need);
+  const char* err = bsae_backward_launch(x, vals, idx, g_recon, soft_rows, logits, q, gp_dev, gp_host, w_enc, B, H, D, k, n_bits,
+                                         grad_w_enc, grad_b_enc, grad_logits, grad_b_dec, grad_x, workspace, st);
+  return err == nullptr ? QSAE_OK : fail(QSAE_ERR_CUDA, "bsae_backward: %s", err);
+}
+
 // ---- q_sae dense fallback: any activity level (an untrained model is ~50 % active), level sums as GEMMs
 int qsae_unpack_matryoshka_t(const uint32_t* packed, int H, int D, uint16_t* t_bf16, void* stream) {
   if (!packed || !t_bf16 || H <= 0 || D <= 0 || (D % 16) != 0)

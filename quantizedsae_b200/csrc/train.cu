@@ -10,7 +10,8 @@
 //     cores, wgrad_sm100.cu);
 //   * radix select + apply kernels: STEWeights.init_mask / update_mask (RigL drop / grow, sae/ternary.py:27-87) and
 //     mask_grad (:89-90);
-//   * bwd_* kernels: the deterministic latent-major backward of baseline_sae (sae/baseline.py:17-40).
+//   * bwd_* kernels: the deterministic latent-major backward of baseline_sae (sae/baseline.py:17-40), and with
+//     bsae_latent_reduce_kernel the deterministic b_sae backward (the logit chain rule fused into the reduction).
 // All HBM-bound elementwise / scatter work: no tensor cores. Compiled without fast-math: the logistic is the literal
 // 1 / (1 + expf(-w)) the packing kernels use, so Bsign here equals the sign packed for the forward.
 #include <cuda_runtime.h>
@@ -132,9 +133,28 @@ column_sum_kernel(const float* __restrict__ src, int R, int C, float scale, floa
 // rows because D n_bits % 4 == 0 on this path; the launcher falls back to VEC = 1 otherwise).
 // gp: device scalar (upstream gradient of polarize_loss, e.g. polarize_lambda) or NULL = gp_host.
 // ---------------------------------------------------------------------------------------------
-// blockIdx.x / threadIdx.x pick the group of VEC consecutive logits of a row, blockIdx.y strides over the rows: bit
-// index, bit weight and dictionary column are per-thread constants. The logistic uses the fast exponential /
+// The three helpers below are the whole per-element formula; bsae_latent_reduce_kernel (the deterministic backward)
+// calls the same ones, so both paths give the same bits for the same G. The logistic uses the fast exponential /
 // reciprocal (relative error ~1e-6: a gradient, not a thresholded bit -- the packing kernels keep the exact form).
+// gp / N, N = H D n_bits: the polarize gradient's scale, divided once per thread
+__device__ __forceinline__ float bsae_polarize_scale(const float* gp_dev, float gp_host, int H, int cols) {
+  return (gp_dev != nullptr ? *gp_dev : gp_host) / static_cast<float>(static_cast<double>(H) * cols);
+}
+
+// bit i of n: its coefficient c_i (2^i, the sign bit -2^(n-1)) and gp 2^i
+__device__ __forceinline__ void bsae_bit_consts(int i, int n_bits, float gp, float& ci, float& gpw) {
+  const float pw = static_cast<float>(1u << i);
+  ci = (i == n_bits - 1) ? -pw : pw;
+  gpw = gp * pw;
+}
+
+__device__ __forceinline__ float bsae_logit_grad_value(float w, float up, float ci, float gpw) {
+  const float p = __frcp_rn(1.0f + __expf(-w));
+  return (up * ci + gpw * (1.f - 2.f * p)) * (p * (1.f - p));
+}
+
+// blockIdx.x / threadIdx.x pick the group of VEC consecutive logits of a row, blockIdx.y strides over the rows: bit
+// index, bit weight and dictionary column are per-thread constants.
 template <int VEC>
 __global__ void __launch_bounds__(256)
 bsae_logit_grad_kernel(const float* __restrict__ logits, const float* __restrict__ G, int H, int D, int n_bits,
@@ -143,17 +163,14 @@ bsae_logit_grad_kernel(const float* __restrict__ logits, const float* __restrict
   const int groups = cols / VEC;
   const int cg = blockIdx.x * blockDim.x + threadIdx.x;
   if (cg >= groups) return;
-  const float gp = (gp_dev != nullptr ? *gp_dev : gp_host) / static_cast<float>(static_cast<double>(H) * cols);
+  const float gp = bsae_polarize_scale(gp_dev, gp_host, H, cols);
   int dcol[VEC];
   float ci[VEC], gpw[VEC];
 #pragma unroll
   for (int u = 0; u < VEC; ++u) {
     const int col = cg * VEC + u;
     dcol[u] = col / n_bits;
-    const int i = col - dcol[u] * n_bits;
-    const float pw = static_cast<float>(1u << i);
-    ci[u] = (i == n_bits - 1) ? -pw : pw;
-    gpw[u] = gp * pw;
+    bsae_bit_consts(col - dcol[u] * n_bits, n_bits, gp, ci[u], gpw[u]);
   }
   constexpr int R = 2;                                // rows in flight per thread
   for (int h0 = blockIdx.y; h0 < H; h0 += R * gridDim.y) {
@@ -185,8 +202,7 @@ bsae_logit_grad_kernel(const float* __restrict__ logits, const float* __restrict
       float o[VEC];
 #pragma unroll
       for (int u = 0; u < VEC; ++u) {
-        const float p = __frcp_rn(1.0f + __expf(-w[r][u]));
-        o[u] = (up0[r][u] * ci[u] + gpw[u] * (1.f - 2.f * p)) * (p * (1.f - p));
+        o[u] = bsae_logit_grad_value(w[r][u], up0[r][u], ci[u], gpw[u]);
         if (accumulate) o[u] += old[r][u];
       }
       if (VEC == 4) reinterpret_cast<float4*>(grad)[e] = make_float4(o[0], o[1 % VEC], o[2 % VEC], o[3 % VEC]);
@@ -837,13 +853,14 @@ constexpr int kColParts = 256;   // most partial rows of the two-level column su
 
 __device__ __forceinline__ int clamp_key(int h, int H) { return static_cast<unsigned>(h) < static_cast<unsigned>(H) ? h : H; }
 
-// gv[b,j] = <g[b,:], rows[idx[b,j],:]> + g_h term (0 for an index outside [0, H)); cnt[h] += 1 per selection.
+// gv[b,j] = scale <g[b,:], rows[idx[b,j],:]> + g_h term (0 for an index outside [0, H)); cnt[h] += 1 per selection.
 // Warp per row, the row of g in registers, butterfly reductions: the same bits in every lane and on every run.
+// baseline_sae passes scale 1 (the product is exact, so its bits are those of the plain dot), b_sae the step q.
 template <int NCH>
 __global__ void __launch_bounds__(256)
 bwd_latent_grad_kernel(const float* __restrict__ g, const float* __restrict__ rows, const int32_t* __restrict__ idx,
                        const float* __restrict__ gh_dense, const float* __restrict__ gh_vals, int B, int k, int D, int H,
-                       float* __restrict__ gv, int* __restrict__ cnt) {
+                       float scale, float* __restrict__ gv, int* __restrict__ cnt) {
   const int lane = threadIdx.x & 31;
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int nwarps = (gridDim.x * blockDim.x) >> 5;
@@ -883,7 +900,7 @@ bwd_latent_grad_kernel(const float* __restrict__ g, const float* __restrict__ ro
         if (lane == j) my_dot = acc;
       }
       if (jl < k) {
-        gv[e] = ok ? my_dot + my_gh : 0.f;
+        gv[e] = ok ? scale * my_dot + my_gh : 0.f;
         if (ok) atomicAdd(cnt + my_h, 1);     // integer counts: exact in any order
       }
     }
@@ -1071,10 +1088,43 @@ bwd_chunk_kernel(const int* __restrict__ off, const int* __restrict__ coff, int 
   }
 }
 
-// Latent-major reduction: block of 8 warps over kBwdTile consecutive latents, warp per latent. A latent with at most
-// kBwdChunk entries is reduced from its records, a longer one sums its chunk partials in chunk order. grad W_enc rows
+// One warp's sums for latent h: aWe = sum gv x, aWd = sum v g, sbe = sum gv over the rows that selected h. A latent
+// with at most kBwdChunk entries is reduced from its records, a longer one sums its chunk partials in chunk order;
+// a latent nobody selected gets exact zeros.
+template <int NCH>
+__device__ __forceinline__ void bwd_latent_sums(int h, const int* __restrict__ off, const int* __restrict__ coff,
+                                                const int* __restrict__ ent_b, const float* __restrict__ ent_v,
+                                                const float* __restrict__ ent_g, const float* __restrict__ x,
+                                                const float* __restrict__ g, int D, const float* __restrict__ part, int lane,
+                                                float4 (&aWe)[NCH], float4 (&aWd)[NCH], float& sbe) {
+  const int nchunk = D >> 2;
+  const size_t pitch = 2 * static_cast<size_t>(D) + 4;
+#pragma unroll
+  for (int c = 0; c < NCH; ++c) aWe[c] = aWd[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+  sbe = 0.f;
+  const int lo = off[h], hi = off[h + 1];
+  if (hi - lo <= kBwdChunk) {
+    bwd_reduce_entries<NCH>(lo, hi, ent_b, ent_v, ent_g, reinterpret_cast<const float4*>(x),
+                            reinterpret_cast<const float4*>(g), nchunk, lane, aWe, aWd, sbe);
+  } else {
+    for (int q = coff[h]; q < coff[h + 1]; ++q) {
+      const float* p = part + static_cast<size_t>(q) * pitch;
+#pragma unroll
+      for (int c = 0; c < NCH; ++c) {
+        const int q4 = lane + 32 * c;
+        if (q4 < nchunk) {
+          add4(aWe[c], reinterpret_cast<const float4*>(p)[q4]);
+          add4(aWd[c], reinterpret_cast<const float4*>(p + D)[q4]);
+        }
+      }
+      sbe += p[2 * D];
+    }
+  }
+}
+
+// Latent-major reduction: block of 8 warps over kBwdTile consecutive latents, warp per latent. grad W_enc rows
 // and grad b_enc leave directly; the grad W_dec columns are staged in shared memory [kBwdTile][D + 1] and leave as
-// [D, kBwdTile] row segments. Latents nobody selected get exact zeros.
+// [D, kBwdTile] row segments.
 template <int NCH>
 __global__ void __launch_bounds__(256)
 bwd_latent_reduce_kernel(const int* __restrict__ off, const int* __restrict__ coff, int H, const int* __restrict__ ent_b,
@@ -1084,33 +1134,13 @@ bwd_latent_reduce_kernel(const int* __restrict__ off, const int* __restrict__ co
   extern __shared__ float stage[];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int nchunk = D >> 2;
-  const size_t pitch = 2 * static_cast<size_t>(D) + 4;
   const int h0 = blockIdx.x * kBwdTile;
   const int nl = min(kBwdTile, H - h0);
   for (int l = wid; l < nl; l += blockDim.x >> 5) {
     const int h = h0 + l;
     float4 aWe[NCH], aWd[NCH];
-#pragma unroll
-    for (int c = 0; c < NCH; ++c) aWe[c] = aWd[c] = make_float4(0.f, 0.f, 0.f, 0.f);
-    float sbe = 0.f;
-    const int lo = off[h], hi = off[h + 1];
-    if (hi - lo <= kBwdChunk) {
-      bwd_reduce_entries<NCH>(lo, hi, ent_b, ent_v, ent_g, reinterpret_cast<const float4*>(x),
-                              reinterpret_cast<const float4*>(g), nchunk, lane, aWe, aWd, sbe);
-    } else {
-      for (int q = coff[h]; q < coff[h + 1]; ++q) {
-        const float* p = part + static_cast<size_t>(q) * pitch;
-#pragma unroll
-        for (int c = 0; c < NCH; ++c) {
-          const int q4 = lane + 32 * c;
-          if (q4 < nchunk) {
-            add4(aWe[c], reinterpret_cast<const float4*>(p)[q4]);
-            add4(aWd[c], reinterpret_cast<const float4*>(p + D)[q4]);
-          }
-        }
-        sbe += p[2 * D];
-      }
-    }
+    float sbe;
+    bwd_latent_sums<NCH>(h, off, coff, ent_b, ent_v, ent_g, x, g, D, part, lane, aWe, aWd, sbe);
     float* srow = stage + static_cast<size_t>(l) * (D + 1);
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
@@ -1126,6 +1156,72 @@ bwd_latent_reduce_kernel(const int* __restrict__ off, const int* __restrict__ co
   for (int i = threadIdx.x; i < D * kBwdTile; i += blockDim.x) {
     const int d = i / kBwdTile, l = i - d * kBwdTile;
     if (l < nl) gWd[static_cast<size_t>(d) * H + h0 + l] = stage[static_cast<size_t>(l) * (D + 1) + d];
+  }
+}
+
+// b_sae latent-major pass: warp per latent h, 8 latents per block. From the sums of bwd_latent_sums:
+//   grad W_enc[h,:] = sum gv x, grad b_enc[h] = sum gv,  G[h,:] = q sum v g  (d loss / d int_w, never in memory)
+//   grad_logits[h, d n + i] = (G[h,d] c_i + gp 2^i (1 - 2p) / N) p (1 - p)   (the bsae_logit_grad formula)
+// G's row is staged in the warp's slice of shared memory so that the logit row streams in coalesced 16-byte groups,
+// exactly as bsae_logit_grad reads it. Each logit is read once and each output element has one writer; a latent
+// nobody selected has G = 0 and gets the polarize-only gradient and exact zeros in grad W_enc / grad b_enc.
+constexpr int kBsaeWarps = 8;
+constexpr int kBsaeUnroll = 4;   // 16-byte logit loads in flight per lane
+
+template <int NCH>
+__global__ void __launch_bounds__(32 * kBsaeWarps)
+bsae_latent_reduce_kernel(const int* __restrict__ off, const int* __restrict__ coff, int H, const int* __restrict__ ent_b,
+                          const float* __restrict__ ent_v, const float* __restrict__ ent_g, const float* __restrict__ x,
+                          const float* __restrict__ g, int D, const float* __restrict__ part, float q,
+                          const float* __restrict__ logits, int n_bits, const float* __restrict__ gp_dev, float gp_host,
+                          float* __restrict__ gWe, float* __restrict__ gbe, float* __restrict__ glog) {
+  __shared__ float4 sG[kBsaeWarps][NCH * 32];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int h = blockIdx.x * kBsaeWarps + wid;
+  if (h >= H) return;                             // warp-uniform; the block never synchronises
+  const int nchunk = D >> 2;
+  float4 aWe[NCH], aWd[NCH];
+  float sbe;
+  bwd_latent_sums<NCH>(h, off, coff, ent_b, ent_v, ent_g, x, g, D, part, lane, aWe, aWd, sbe);
+#pragma unroll
+  for (int c = 0; c < NCH; ++c) {
+    const int q4 = lane + 32 * c;
+    if (q4 < nchunk) {
+      reinterpret_cast<float4*>(gWe + static_cast<size_t>(h) * D)[q4] = aWe[c];
+      sG[wid][q4] = make_float4(q * aWd[c].x, q * aWd[c].y, q * aWd[c].z, q * aWd[c].w);
+    }
+  }
+  if (lane == 0) gbe[h] = sbe;
+  __syncwarp();
+  const float* Gs = reinterpret_cast<const float*>(sG[wid]);
+  const int cols = D * n_bits, groups = cols >> 2;     // D % 8 == 0: a row is whole 16-byte groups
+  const float gp = bsae_polarize_scale(gp_dev, gp_host, H, cols);
+  const float4* lrow = reinterpret_cast<const float4*>(logits + static_cast<size_t>(h) * cols);
+  float4* grow = reinterpret_cast<float4*>(glog + static_cast<size_t>(h) * cols);
+  for (int c0 = lane; c0 < groups; c0 += 32 * kBsaeUnroll) {
+    float4 w[kBsaeUnroll];
+#pragma unroll
+    for (int u = 0; u < kBsaeUnroll; ++u) {
+      const int cg = c0 + 32 * u;
+      if (cg < groups) w[u] = lrow[cg];
+    }
+#pragma unroll
+    for (int u = 0; u < kBsaeUnroll; ++u) {
+      const int cg = c0 + 32 * u;
+      if (cg >= groups) continue;
+      const int col = 4 * cg;
+      int d = col / n_bits, i = col - d * n_bits;
+      const float wv[4] = {w[u].x, w[u].y, w[u].z, w[u].w};
+      float o[4];
+#pragma unroll
+      for (int t = 0; t < 4; ++t) {
+        float ci, gpw;
+        bsae_bit_consts(i, n_bits, gp, ci, gpw);
+        o[t] = bsae_logit_grad_value(wv[t], Gs[d], ci, gpw);
+        if (++i == n_bits) { i = 0; ++d; }
+      }
+      grow[cg] = make_float4(o[0], o[1], o[2], o[3]);
+    }
   }
 }
 
@@ -1149,6 +1245,7 @@ __global__ void __launch_bounds__(128) bwd_colsum_final_kernel(const float* __re
   out[c] = s;
 }
 
+// workspace of both latent-major backwards (baseline_sae and b_sae need the same regions)
 struct BaselineBwdLayout {
   int n, ntiles, npasses, max_chunks, col_rows, col_parts;
   size_t gv, cnt, off, coff, hist, keys[2], ent[2], eb, ev, eg, part, colpart, total;
@@ -1190,56 +1287,61 @@ BaselineBwdLayout baseline_bwd_layout(int B, int H, int D, int k) {
   return L;
 }
 
+// one warp per possible chunk (the device-side total decides which run): no host synchronisation
+template <int NCH>
+void bwd_chunk_launch(const BaselineBwdLayout& L, uint8_t* ws, int H, int D, const float* x, const float* g, cudaStream_t stream) {
+  bwd_chunk_kernel<NCH><<<grid_for(static_cast<size_t>(L.max_chunks) * 32, 256, 148 * 8), 256, 0, stream>>>(
+      reinterpret_cast<const int*>(ws + L.off), reinterpret_cast<const int*>(ws + L.coff), H,
+      reinterpret_cast<const int*>(ws + L.eb), reinterpret_cast<const float*>(ws + L.ev),
+      reinterpret_cast<const float*>(ws + L.eg), x, g, D, reinterpret_cast<float*>(ws + L.part));
+}
+
 template <int NCH>
 void bwd_reduce_launches(const BaselineBwdLayout& L, uint8_t* ws, int H, int D, const float* x, const float* g, float* gWe,
                          float* gbe, float* gWd, cudaStream_t stream) {
-  const int* off = reinterpret_cast<const int*>(ws + L.off);
-  const int* coff = reinterpret_cast<const int*>(ws + L.coff);
-  const int* eb = reinterpret_cast<const int*>(ws + L.eb);
-  const float* ev = reinterpret_cast<const float*>(ws + L.ev);
-  const float* eg = reinterpret_cast<const float*>(ws + L.eg);
-  float* part = reinterpret_cast<float*>(ws + L.part);
-  // one warp per possible chunk (the device-side total decides which run): no host synchronisation
-  bwd_chunk_kernel<NCH><<<grid_for(static_cast<size_t>(L.max_chunks) * 32, 256, 148 * 8), 256, 0, stream>>>(
-      off, coff, H, eb, ev, eg, x, g, D, part);
+  bwd_chunk_launch<NCH>(L, ws, H, D, x, g, stream);
   const size_t smem = static_cast<size_t>(kBwdTile) * (D + 1) * sizeof(float);
   cudaFuncSetAttribute(bwd_latent_reduce_kernel<NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
-  bwd_latent_reduce_kernel<NCH><<<(H + kBwdTile - 1) / kBwdTile, 256, smem, stream>>>(off, coff, H, eb, ev, eg, x, g, D, part,
-                                                                                         gWe, gbe, gWd);
+  bwd_latent_reduce_kernel<NCH><<<(H + kBwdTile - 1) / kBwdTile, 256, smem, stream>>>(
+      reinterpret_cast<const int*>(ws + L.off), reinterpret_cast<const int*>(ws + L.coff), H,
+      reinterpret_cast<const int*>(ws + L.eb), reinterpret_cast<const float*>(ws + L.ev),
+      reinterpret_cast<const float*>(ws + L.eg), x, g, D, reinterpret_cast<const float*>(ws + L.part), gWe, gbe, gWd);
 }
 
-}  // namespace
+template <int NCH>
+void bsae_reduce_launches(const BaselineBwdLayout& L, uint8_t* ws, int H, int D, const float* x, const float* g, float q,
+                          const float* logits, int n_bits, const float* gp_dev, float gp_host, float* gWe, float* gbe,
+                          float* glog, cudaStream_t stream) {
+  bwd_chunk_launch<NCH>(L, ws, H, D, x, g, stream);
+  bsae_latent_reduce_kernel<NCH><<<(H + kBsaeWarps - 1) / kBsaeWarps, 32 * kBsaeWarps, 0, stream>>>(
+      reinterpret_cast<const int*>(ws + L.off), reinterpret_cast<const int*>(ws + L.coff), H,
+      reinterpret_cast<const int*>(ws + L.eb), reinterpret_cast<const float*>(ws + L.ev),
+      reinterpret_cast<const float*>(ws + L.eg), x, g, D, reinterpret_cast<const float*>(ws + L.part), q, logits, n_bits,
+      gp_dev, gp_host, gWe, gbe, glog);
+}
 
-size_t baseline_backward_workspace_bytes(int B, int H, int D, int k) { return baseline_bwd_layout(B, H, D, k).total; }
-
-const char* baseline_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g,
-                                     const float* g_h, const float* g_vals, const float* w_enc, const float* dec_rows, int B,
-                                     int H, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx, void* workspace,
-                                     cudaStream_t stream) {
-  const BaselineBwdLayout L = baseline_bwd_layout(B, H, D, k);
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
+// The first steps of both latent-major backwards:
+//   1. gv = scale <g, rows[h]> + g_h term at each kept entry, and the per-latent counts;
+//   2. CSC offsets of the entries and of the chunks of long latents;
+//   3. stable radix sort of the row-major entries by latent -> records {b, v, gv}, latent-major.
+const char* bwd_group_by_latent(const BaselineBwdLayout& L, uint8_t* ws, const float* g, const float* rows, const int32_t* idx,
+                                const float* vals, const float* g_h, const float* g_vals, int B, int H, int D, int k,
+                                float scale, int* launches, cudaStream_t stream) {
   float* gv = reinterpret_cast<float*>(ws + L.gv);
   int* cnt = reinterpret_cast<int*>(ws + L.cnt);
-  int* off = reinterpret_cast<int*>(ws + L.off);
-  int* coff = reinterpret_cast<int*>(ws + L.coff);
   int* hist = reinterpret_cast<int*>(ws + L.hist);
-  const int nch = (D / 4 + 31) / 32;
-  int launches = 0;
-  cudaError_t e = cudaMemsetAsync(cnt, 0, static_cast<size_t>(H) * 4, stream);
+  const cudaError_t e = cudaMemsetAsync(cnt, 0, static_cast<size_t>(H) * 4, stream);
   if (e != cudaSuccess) return cudaGetErrorString(e);
-  // 1. gv and the per-latent counts
   const int grid_rows = grid_for(static_cast<size_t>(B) * 32, 256, 148 * 8);
-  switch (nch) {
-    case 1: bwd_latent_grad_kernel<1><<<grid_rows, 256, 0, stream>>>(g, dec_rows, idx, g_h, g_vals, B, k, D, H, gv, cnt); break;
-    case 2: bwd_latent_grad_kernel<2><<<grid_rows, 256, 0, stream>>>(g, dec_rows, idx, g_h, g_vals, B, k, D, H, gv, cnt); break;
-    case 3: bwd_latent_grad_kernel<3><<<grid_rows, 256, 0, stream>>>(g, dec_rows, idx, g_h, g_vals, B, k, D, H, gv, cnt); break;
-    default: bwd_latent_grad_kernel<4><<<grid_rows, 256, 0, stream>>>(g, dec_rows, idx, g_h, g_vals, B, k, D, H, gv, cnt); break;
+  switch ((D / 4 + 31) / 32) {
+    case 1: bwd_latent_grad_kernel<1><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, scale, gv, cnt); break;
+    case 2: bwd_latent_grad_kernel<2><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, scale, gv, cnt); break;
+    case 3: bwd_latent_grad_kernel<3><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, scale, gv, cnt); break;
+    default: bwd_latent_grad_kernel<4><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, scale, gv, cnt); break;
   }
-  // 2. CSC offsets of the entries and of the chunks of long latents
-  bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(cnt, H, off);
-  bwd_scan_kernel<true><<<1, 1024, 0, stream>>>(cnt, H, coff);
-  launches += 3;
-  // 3. stable radix sort of the row-major entries by latent -> records {b, v, gv}, latent-major
+  bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(cnt, H, reinterpret_cast<int*>(ws + L.off));
+  bwd_scan_kernel<true><<<1, 1024, 0, stream>>>(cnt, H, reinterpret_cast<int*>(ws + L.coff));
+  *launches += 3;
   const int32_t* keys_in = idx;
   const int* e_in = nullptr;
   for (int p = 0; p < L.npasses; ++p) {
@@ -1258,29 +1360,76 @@ const char* baseline_backward_launch(const float* x, const float* vals, const in
           keys_in, e_in, L.n, H, shift, L.ntiles, hist, keys_out, e_out, k, nullptr, nullptr, nullptr, nullptr, nullptr);
     keys_in = keys_out;
     e_in = e_out;
-    launches += 3;
+    *launches += 3;
   }
+  return nullptr;
+}
+
+// grad b_dec = column sums of g, then grad x = gv W_enc over the kept entries (the sparse decoder over the encoder rows)
+const char* bwd_tail_launches(const BaselineBwdLayout& L, uint8_t* ws, const float* g, const int32_t* idx, const float* w_enc,
+                              int B, int H, int D, int k, float* gbd, float* gx, int* launches, cudaStream_t stream) {
+  float* colpart = reinterpret_cast<float*>(ws + L.colpart);
+  bwd_colsum_part_kernel<<<L.col_parts, 128, 0, stream>>>(g, B, D, L.col_rows, colpart);
+  bwd_colsum_final_kernel<<<(D + 127) / 128, 128, 0, stream>>>(colpart, L.col_parts, D, gbd);
+  *launches += 2;
+  if (gx != nullptr) {
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cudaGetErrorString(e);
+    const char* err = decode_f32_launch(reinterpret_cast<const float*>(ws + L.gv), idx, B, k, w_enc, H, D, 1.0f, nullptr, gx, 0, stream);
+    if (err != nullptr) return err;
+    ++*launches;
+  }
+  return nullptr;
+}
+
+}  // namespace
+
+size_t baseline_backward_workspace_bytes(int B, int H, int D, int k) { return baseline_bwd_layout(B, H, D, k).total; }
+
+const char* baseline_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g,
+                                     const float* g_h, const float* g_vals, const float* w_enc, const float* dec_rows, int B,
+                                     int H, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx, void* workspace,
+                                     cudaStream_t stream) {
+  const BaselineBwdLayout L = baseline_bwd_layout(B, H, D, k);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  int launches = 0;
+  const char* err = bwd_group_by_latent(L, ws, g, dec_rows, idx, vals, g_h, g_vals, B, H, D, k, 1.0f, &launches, stream);
+  if (err != nullptr) return err;
   // 4. latent-major reduction: grad W_enc, grad b_enc, grad W_dec
-  switch (nch) {
+  switch ((D / 4 + 31) / 32) {
     case 1: bwd_reduce_launches<1>(L, ws, H, D, x, g, gWe, gbe, gWd, stream); break;
     case 2: bwd_reduce_launches<2>(L, ws, H, D, x, g, gWe, gbe, gWd, stream); break;
     case 3: bwd_reduce_launches<3>(L, ws, H, D, x, g, gWe, gbe, gWd, stream); break;
     default: bwd_reduce_launches<4>(L, ws, H, D, x, g, gWe, gbe, gWd, stream); break;
   }
   launches += 2;
-  // 5. grad b_dec
-  float* colpart = reinterpret_cast<float*>(ws + L.colpart);
-  bwd_colsum_part_kernel<<<L.col_parts, 128, 0, stream>>>(g, B, D, L.col_rows, colpart);
-  bwd_colsum_final_kernel<<<(D + 127) / 128, 128, 0, stream>>>(colpart, L.col_parts, D, gbd);
-  launches += 2;
-  // 6. grad x = gv W_enc over the kept entries: the sparse decoder over the encoder rows
-  if (gx != nullptr) {
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return cudaGetErrorString(e);
-    const char* err = decode_f32_launch(gv, idx, B, k, w_enc, H, D, 1.0f, nullptr, gx, 0, stream);
-    if (err != nullptr) return err;
-    ++launches;
+  // 5, 6. grad b_dec, grad x
+  err = bwd_tail_launches(L, ws, g, idx, w_enc, B, H, D, k, gbd, gx, &launches, stream);
+  if (err != nullptr) return err;
+  count_launches(launches);
+  return cuda_err(cudaGetLastError());
+}
+
+// b_sae (sae/binary.py:24-47, 91-103): the baseline's steps with gv = q <g, soft_rows[h]>, the soft rows in place of
+// W_dec^T, and the b_sae pass in place of the grad W_dec reduction; the same workspace layout.
+const char* bsae_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g, const float* soft_rows,
+                                 const float* logits, float q, const float* gp_dev, float gp_host, const float* w_enc, int B,
+                                 int H, int D, int k, int n_bits, float* gWe, float* gbe, float* glog, float* gbd, float* gx,
+                                 void* workspace, cudaStream_t stream) {
+  const BaselineBwdLayout L = baseline_bwd_layout(B, H, D, k);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  int launches = 0;
+  const char* err = bwd_group_by_latent(L, ws, g, soft_rows, idx, vals, nullptr, nullptr, B, H, D, k, q, &launches, stream);
+  if (err != nullptr) return err;
+  switch ((D / 4 + 31) / 32) {
+    case 1: bsae_reduce_launches<1>(L, ws, H, D, x, g, q, logits, n_bits, gp_dev, gp_host, gWe, gbe, glog, stream); break;
+    case 2: bsae_reduce_launches<2>(L, ws, H, D, x, g, q, logits, n_bits, gp_dev, gp_host, gWe, gbe, glog, stream); break;
+    case 3: bsae_reduce_launches<3>(L, ws, H, D, x, g, q, logits, n_bits, gp_dev, gp_host, gWe, gbe, glog, stream); break;
+    default: bsae_reduce_launches<4>(L, ws, H, D, x, g, q, logits, n_bits, gp_dev, gp_host, gWe, gbe, glog, stream); break;
   }
+  launches += 2;
+  err = bwd_tail_launches(L, ws, g, idx, w_enc, B, H, D, k, gbd, gx, &launches, stream);
+  if (err != nullptr) return err;
   count_launches(launches);
   return cuda_err(cudaGetLastError());
 }

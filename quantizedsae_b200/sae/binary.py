@@ -147,6 +147,7 @@ class BinarySAE(SparseAutoencoder):
         self.exact = True                    # fp32 re-scoring of the tensor-core candidates
         self.last_flags = None               # rows whose selection was not certified (exact mode)
         self.autograd = False                # True: forward attaches the sparse backward (quantizedsae_b200/training.py)
+        self.deterministic = False           # with autograd: the bit-deterministic latent-major backward (qsae_bsae_backward)
         self.ordered_latents = True          # False (fast mode, k > QSAE_MAX_K): sparse latents as unordered winner sets
         self._prep = PreparedCache()
 

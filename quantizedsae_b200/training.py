@@ -11,6 +11,9 @@ b_sae   `bsae_forward(model, x)` (what `BinarySAE.forward` runs when `model.auto
         decoder.bias. Backward of sae/binary.py:24-47 and :91-99: sparse outer products (16-byte vector reductions),
         row dots against the soft dictionary, one streaming pass over the bit logits that applies the sigmoid chain
         rule and adds the polarize gradient. The returned latent carries no gradient (the trainer only logs it).
+        With model.deterministic = True the backward is qsae_bsae_backward instead: the baseline_sae latent-major
+        pass below with gv = q <g, soft_rows[h]>, G[h] = q sum v g built per latent and the logit chain rule applied
+        while G's row is in shared memory (G never reaches memory). Every gradient is then bit-deterministic.
 q_sae   `QuantizedMatryoshkaDecoder.ste_backward(active, grad_levels)`: what loss.backward() leaves in
         decoder.weight.grad, weight_mirror.grad and bias.grad (STE through the sign, sae/quantized_matryoshka.py:94-124,
         joint_gradient = False), at any activity: from the active lists of `QuantizedMatryoshkaSAE.forward_active`
@@ -75,6 +78,7 @@ class _BinarySAEFn(torch.autograd.Function):
         pol = dec.polarize_loss().detach().clone()
         ctx.save_for_backward(x, lat.values, lat.indices, logits, w_enc, rows)
         ctx.dims = (H, D, dec.n_bits, float(dec.quantization_step))
+        ctx.deterministic = bool(model.deterministic)
         ctx.mark_non_differentiable(lat.values, lat.indices)
         return lat.values, lat.indices, recon, pol
 
@@ -87,6 +91,12 @@ class _BinarySAEFn(torch.autograd.Function):
         g = (torch.zeros((B, D), dtype=torch.float32, device=dev) if g_recon is None
              else g_recon.contiguous().float())
         gp = 0.0 if g_pol is None else g_pol.detach().reshape(()).float().contiguous()
+        if ctx.deterministic:
+            want_x = ctx.needs_input_grad[0]
+            gwe, gbe, glog, gbd, gx = _lib.bsae_backward(x.detach().contiguous(), vals, idx, g, rows,
+                                                         logits.detach().contiguous(), q, gp,
+                                                         w_enc.detach().contiguous() if want_x else None, n_bits, want_x)
+            return gx, gwe, gbe, glog, gbd, None
         G = torch.zeros((H, D), dtype=torch.float32, device=dev)
         _lib.rows_scatter_add(vals, idx, g, G, scale=q)                       # d / d int_w
         grad_logits = torch.empty_like(logits, memory_format=torch.contiguous_format)
