@@ -520,6 +520,12 @@ int qsae_decode_int4_range(const float* vals, const int32_t* idx, int B, int k, 
 int qsae_decode_int8_range(const float* vals, const int32_t* idx, int B, int k, const int8_t* rows_shard,
                            int shard_latents, int idx_begin, int D, float scale, const float* bias,
                            float* recon, void* stream);
+/* qsae_decode_rows_f32 restricted to the latents [idx_begin, idx_begin + shard_latents) whose fp32 rows
+ * [shard_latents, D] are in `rows_shard` (the dictionary-sharded baseline_sae's transposed decoder columns).
+ * rows_shard, bias and recon must be 16-byte aligned (recon may be a slot of a peer-exchange buffer). */
+int qsae_decode_rows_f32_range(const float* vals, const int32_t* idx, int B, int k, const float* rows_shard,
+                               int shard_latents, int idx_begin, int D, float scale, const float* bias,
+                               float* recon, void* stream);
 
 /* latent * mask (sae/binary.py:96-99) / zeros_like + scatter_ (sae/baseline.py:38-39):
  * dense [B, H] float32 from the sparse form. Zero-fills `dense` first. */

@@ -89,6 +89,7 @@ SYMBOLS = {
     "qsae_reduce_partials_peer": (_i, [_vp, _i, _i, _i, _i, _vp, _vp]),
     "qsae_decode_int4_range": (_i, [_vp, _vp, _i, _i, _vp, _i, _i, _i, _f, _vp, _vp, _vp]),
     "qsae_decode_int8_range": (_i, [_vp, _vp, _i, _i, _vp, _i, _i, _i, _f, _vp, _vp, _vp]),
+    "qsae_decode_rows_f32_range": (_i, [_vp, _vp, _i, _i, _vp, _i, _i, _i, _f, _vp, _vp, _vp]),
     "qsae_densify": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "qsae_bsae_plan_create": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _f, _i, _i, C.POINTER(_vp)]),
     "qsae_bsae_plan_destroy": (None, [_vp]),
@@ -933,6 +934,20 @@ def decode_range(vals, idx, dict_shard, shard_latents: int, idx_begin: int, D: i
     fn = load().qsae_decode_int4_range if n_bits <= 4 else load().qsae_decode_int8_range
     check(fn(vals.data_ptr(), idx.data_ptr(), B, k, dict_shard.data_ptr(), shard_latents, idx_begin, D, float(scale),
              _ptr(bias), recon.data_ptr(), _stream()))
+    return recon
+
+
+def decode_rows_f32_range(vals, idx, rows_shard, idx_begin: int, scale: float, bias, out: torch.Tensor | None = None):
+    """Partial reconstruction from the winners inside [idx_begin, idx_begin + rows_shard.shape[0]) of an fp32 [H/G, D]
+    row dictionary (the dictionary-sharded baseline_sae)."""
+    _need_cuda(vals, idx, rows_shard, bias, out)
+    B, k = vals.shape
+    shard_latents, D = rows_shard.shape
+    assert rows_shard.dtype == torch.float32
+    recon = torch.empty((B, D), dtype=torch.float32, device=vals.device) if out is None else out
+    assert recon.dtype == torch.float32 and tuple(recon.shape) == (B, D)
+    check(load().qsae_decode_rows_f32_range(vals.data_ptr(), idx.data_ptr(), B, k, rows_shard.data_ptr(), shard_latents,
+                                            idx_begin, D, float(scale), _ptr(bias), recon.data_ptr(), _stream()))
     return recon
 
 

@@ -1897,6 +1897,18 @@ int qsae_decode_int8_range(const float* vals, const int32_t* idx, int B, int k, 
                                                          idx_begin, S(stream)));
 }
 
+int qsae_decode_rows_f32_range(const float* vals, const int32_t* idx, int B, int k, const float* rows_shard,
+                               int shard_latents, int idx_begin, int D, float scale, const float* bias, float* recon,
+                               void* stream) {
+  int rc = check_decode("decode_rows_f32_range", vals, idx, rows_shard, recon, B, k, shard_latents, D, 4);
+  if (rc != QSAE_OK || B == 0) return rc;
+  // the kernel moves rows, bias and recon in float4 groups
+  if ((reinterpret_cast<uintptr_t>(rows_shard) | reinterpret_cast<uintptr_t>(bias) | reinterpret_cast<uintptr_t>(recon)) & 15)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "decode_rows_f32_range: rows, bias and recon must be 16-byte aligned");
+  return launch_status("decode_rows_f32", decode_f32_launch(vals, idx, B, k, rows_shard, shard_latents, D, scale, bias, recon,
+                                                            idx_begin, S(stream)));
+}
+
 int qsae_densify(const float* vals, const int32_t* idx, int B, int k, int H, float* dense, void* stream) {
   if (B == 0) return QSAE_OK;
   if (!vals || !idx || !dense || B < 0 || k < 0 || H <= 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "densify: bad argument");

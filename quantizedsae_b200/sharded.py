@@ -15,6 +15,12 @@ logits decoder.weight; decoder.bias and the input batch x are replicated. One fo
 which equals the reference forward on the concatenated dictionary: topk over all H latents
 (:94) and latent.matmul(int_weights) (:38) split by rows of int_weights.
 
+DictionaryShardedBaselineSAE runs the same choreography for the top-k baseline (sae/baseline.py): its encoder is the
+same fused encoder + top-k on raw pre-activations, and a shard decodes its winners from its columns of the
+nn.Linear(H, D) decoder. Everything between the local top-k and the decode (the exchange rounds, the large-k retry,
+the peer-exchange lifecycle, gather_output) lives once, in _DictionaryShardedForward; the ops object owns the
+model-specific steps.
+
 The collectives go through torch.distributed (NCCL over NVLink on the B200 box; gloo in the CPU
 tests). The compute steps are injected as `ops`: `CudaShardOps` (libqsae_b200.so, the product) is the
 default; the CPU tests pass a numpy implementation to exercise the choreography under gloo. There is
@@ -91,13 +97,27 @@ class ShardPlan:
                 "decoder.weight": full["decoder.weight"][a:b].clone(),
                 "decoder.bias": full["decoder.bias"].clone()}
 
+    def shard_baseline_state_dict(self, full: dict) -> dict:
+        """Slice a full BaselineSparseAutoencoder state_dict (sae/baseline.py layout) down to this rank's shard. The
+        decoder is nn.Linear(H, D): its weight [D, H] is sliced by columns."""
+        a, b = self.latent_range()
+        return {"encoder.0.weight": full["encoder.0.weight"][a:b].clone(),
+                "encoder.0.bias": full["encoder.0.bias"][a:b].clone(),
+                "decoder.weight": full["decoder.weight"][:, a:b].clone(memory_format=torch.contiguous_format),
+                "decoder.bias": full["decoder.bias"].clone()}
 
-class CudaShardOps:
-    """The compute steps on libqsae_b200.so."""
 
-    def __init__(self, module: "DictionaryShardedBinarySAE"):
+class _CudaEncoderOps:
+    """The shard-local encoder + top-k and the candidate merge on libqsae_b200.so: the steps every dictionary-sharded
+    module shares (the encoder is nn.Linear(D, H/G) on raw pre-activations in both)."""
+
+    def __init__(self, module):
         self.m = module
         self._prep = PreparedCache()
+
+    def _require_cuda(self, t: torch.Tensor) -> None:
+        if not t.is_cuda:
+            raise RuntimeError(f"{type(self.m).__name__} runs only on CUDA (no CPU fallback)")
 
     def _w_bf16(self):
         w = self.m.encoder[0].weight
@@ -108,39 +128,60 @@ class CudaShardOps:
         return self._prep.get("sample", param_key(lin.weight, lin.bias),
                               lambda: _lib.prepare_sample(self._w_bf16(), lin.bias.detach()))
 
-    def _packed(self):
-        w = self.m.decoder_weight
-        if not w.is_cuda:
-            raise RuntimeError("DictionaryShardedBinarySAE runs only on CUDA (no CPU fallback)")
-        return self._prep.get("packed", param_key(w),
-                              lambda: _lib.pack_bitplanes(w.detach(), self.m.input_dim, self.m.n_bits))
-
-    def local_candidates(self, x: torch.Tensor, k_local: int) -> torch.Tensor:
-        """-> [B, k_local, 2] int32 entries {value bits, shard-local index}"""
-        if not x.is_cuda:
-            raise RuntimeError("DictionaryShardedBinarySAE runs only on CUDA (no CPU fallback)")
+    def local_topk(self, x: torch.Tensor, k_local: int):
+        """-> (vals [B, k_local] f32, shard-local idx [B, k_local] i32)"""
+        self._require_cuda(x)
         lin = self.m.encoder[0]
         w32 = lin.weight.detach().contiguous()
         vals, idx, _ = _lib.encode_topk(x, self._w_bf16(), w32 if self.m.exact else None, lin.bias.detach(), k_local,
                                         _lib.ACT_NONE, self.m.exact, sample=self._sample())
-        return _lib.pack_candidates(vals, idx)
+        return vals, idx
+
+    def local_candidates(self, x: torch.Tensor, k_local: int) -> torch.Tensor:
+        """-> [B, k_local, 2] int32 entries {value bits, shard-local index}"""
+        return _lib.pack_candidates(*self.local_topk(x, k_local))
 
     def merge(self, cand_all: torch.Tensor, shard_latents: int, k: int, truncated: bool = False):
         return _lib.merge_candidates(cand_all, shard_latents, k, truncated=truncated)
 
-    def decode_partial(self, vals, idx, plan: ShardPlan, with_bias: bool) -> torch.Tensor:
+
+class CudaShardOps(_CudaEncoderOps):
+    """The compute steps of the dictionary-sharded b_sae on libqsae_b200.so."""
+
+    def _packed(self):
+        w = self.m.decoder_weight
+        self._require_cuda(w)
+        return self._prep.get("packed", param_key(w),
+                              lambda: _lib.pack_bitplanes(w.detach(), self.m.input_dim, self.m.n_bits))
+
+    def decode_partial(self, vals, idx, plan: ShardPlan, with_bias: bool, out: torch.Tensor | None = None) -> torch.Tensor:
         packed, _, gap = self._packed()
         if gap > self.m.polar_tol:
             raise RuntimeError("dictionary-sharded b_sae serves the packed (polarised / hard) dictionary only; "
                                f"max |sigmoid(w) - bit| = {gap:.3g} on this shard")
         return _lib.decode_range(vals, idx, packed, plan.shard_latents, plan.latent_begin, self.m.input_dim,
                                  self.m.quantization_step, self.m.decoder_bias.detach() if with_bias else None,
-                                 self.m.n_bits)
+                                 self.m.n_bits, out=out)
 
     def polarize_numerator(self) -> float:
         """sum over the shard of p (1 - p) 2^i (sae/binary.py:41-42 before the mean)."""
         w = self.m.decoder_weight
         return self._packed()[1] * w.numel()
+
+
+class CudaBaselineShardOps(_CudaEncoderOps):
+    """The compute steps of the dictionary-sharded baseline_sae on libqsae_b200.so: the shared encoder and merge, and
+    the decode of this shard's winners from its transposed fp32 decoder columns [H/G, D], cached per weight version
+    as BaselineSparseAutoencoder._dec_rows does."""
+
+    def _dec_rows(self):
+        w = self.m.decoder.weight                     # [D, H/G]: feature vectors are columns
+        self._require_cuda(w)
+        return self._prep.get("dec_rows", param_key(w), lambda: _lib.transpose(w.detach().contiguous()))
+
+    def decode_partial(self, vals, idx, plan: ShardPlan, with_bias: bool, out: torch.Tensor | None = None) -> torch.Tensor:
+        return _lib.decode_rows_f32_range(vals, idx, self._dec_rows(), plan.latent_begin, 1.0,
+                                          self.m.decoder.bias.detach() if with_bias else None, out=out)
 
 
 class PeerExchange:
@@ -250,16 +291,12 @@ class PeerExchange:
         _lib.peer_free(self.ptr)
 
 
-class DictionaryShardedBinarySAE(nn.Module):
-    """Rank-local shard of BinarySAE(input_dim, hidden_dim, gamma, n_bits) (sae/binary.py:73).
+class _DictionaryShardedForward(nn.Module):
+    """The forward choreography shared by the dictionary-sharded modules: local top-k, candidate exchange (truncated
+    round + full retry for large k), global merge, owner decode through `ops.decode_partial`, reduce of the partial
+    rows, over NCCL collectives or peer memory. Subclasses own the parameters, `top_k()` and `ops`."""
 
-    state_dict keys are the reference's, with the latent axis sliced: encoder.0.weight [H/G, D],
-    encoder.0.bias [H/G], decoder.weight [H/G, D*n_bits], decoder.bias [D] (replicated).
-    forward(x) -> (SparseLatents over all H latents, recon rows owned by this rank [B/G, D] or the
-    gathered [B, D] when `gather_output`, polarize_loss)."""
-
-    def __init__(self, input_dim, hidden_dim, gamma=4.0, n_bits=8, *, rank=None, world_size=None,
-                 process_group=None, ops=None):
+    def __init__(self, hidden_dim, rank, world_size, process_group):
         super().__init__()
         import torch.distributed as dist
 
@@ -270,20 +307,9 @@ class DictionaryShardedBinarySAE(nn.Module):
         if rank is None:
             rank = dist.get_rank(process_group) if dist.is_initialized() else 0
         self.plan = ShardPlan(hidden_dim, world_size, rank)
-        self.input_dim, self.hidden_dim, self.n_bits, self.gamma = input_dim, hidden_dim, n_bits, gamma
-        self.quantization_step = gamma / (2 ** (n_bits - 1))
-        self.k = 0.002
-        hs = self.plan.shard_latents
-        self.encoder = nn.Sequential(nn.Linear(input_dim, hs))
-        self.decoder = nn.Module()
-        self.decoder.weight = nn.Parameter(torch.empty(hs, input_dim * n_bits))
-        self.decoder.bias = nn.Parameter(torch.zeros(input_dim))
-        nn.init.xavier_uniform_(self.encoder[0].weight, gain=1)
-        nn.init.zeros_(self.encoder[0].bias)
-        nn.init.kaiming_normal_(self.decoder.weight)
+        self.hidden_dim = hidden_dim
         self.exact = True
         self.gather_output = False
-        self.polar_tol = 1e-6
         self.trim_min_k = 256                # k below this: every shard sends its full top-k (tiny anyway)
         self.last_exchange = None            # "truncated" / "full": which candidate exchange produced the last forward
         self.last_k_send = None              # candidates per shard and row of the last (successful) exchange round
@@ -293,20 +319,6 @@ class DictionaryShardedBinarySAE(nn.Module):
         # selection's instructions. Fast mode (exact = False) only; exact mode always sorts.
         self.ordered_latents = True
         self._peer = None
-        self._pol_cache = None
-        # ops=False defers the choice (tests install their own backend after construction)
-        self.ops = CudaShardOps(self) if ops is None else (ops or None)
-
-    @property
-    def decoder_weight(self):
-        return self.decoder.weight
-
-    @property
-    def decoder_bias(self):
-        return self.decoder.bias
-
-    def top_k(self) -> int:
-        return int(self.hidden_dim * self.k)          # over the FULL dictionary, as sae/binary.py:94
 
     def invalidate(self) -> None:
         """Forget the prepared copies of this shard's weights (needed after in-place edits through `.data`)."""
@@ -334,70 +346,76 @@ class DictionaryShardedBinarySAE(nn.Module):
         a, b = self.plan.row_range(B)
         return out[: b - a]
 
-    def polarize_loss(self, like: torch.Tensor) -> torch.Tensor:
-        """mean over the FULL dictionary of p (1 - p) 2^i (sae/binary.py:41-42): weight-only, so the
-        all-reduce of the per-shard numerators runs once per weight version, not per forward."""
-        key = param_key(self.decoder.weight) + (str(like.device),)
-        if self._pol_cache is None or self._pol_cache[0] != key:
-            num = torch.tensor([self.ops.polarize_numerator()], dtype=torch.float64, device=like.device)
-            if self.plan.world_size > 1:
-                self._dist.all_reduce(num, group=self.group)
-            total = self.hidden_dim * self.input_dim * self.n_bits
-            self._pol_cache = (key, (num[0] / total).to(torch.float32))
-        return self._pol_cache[1]
+    def _gather_rows(self, rows: torch.Tensor, B: int) -> torch.Tensor:
+        per = self.plan.padded_batch(B) // self.plan.world_size
+        if rows.shape[0] != per:
+            rows = torch.cat([rows, rows.new_zeros((per - rows.shape[0], rows.shape[1]))], 0)
+        return self._all_gather(rows).reshape(-1, rows.shape[1])[:B]
 
     # ---- forward ------------------------------------------------------------------------------
-    def forward(self, x: torch.Tensor):
+    def _sharded_forward(self, x: torch.Tensor):
+        """-> (SparseLatents over all H latents, this rank's reconstruction rows or all of them with gather_output)"""
         if x.dim() != 2 or x.shape[1] != self.input_dim:
             raise RuntimeError(f"expected a [batch, {self.input_dim}] matrix, got shape {tuple(x.shape)}")
         x = x.contiguous().float()
         k = self.top_k()
         if k > self.hidden_dim:
             raise RuntimeError(f"selected index k out of range (k={k} > H={self.hidden_dim})")
-        plan = self.plan
-        if not self.ordered_latents and not self.exact and isinstance(self.ops, CudaShardOps):
+        if not self.ordered_latents and not self.exact and isinstance(self.ops, _CudaEncoderOps):
             with _lib.unordered_topk():
                 return self._forward_impl(x, k)
         return self._forward_impl(x, k)
 
     def _forward_impl(self, x: torch.Tensor, k: int):
-        plan = self.plan
-        if self.transport == "p2p" and plan.world_size > 1:
-            return self._forward_p2p(x, k)
+        plan, ops = self.plan, self.ops
+        B = x.shape[0]
         k_loc, k_snd = plan.k_local(k), plan.k_send(k, self.trim_min_k)
+        px = None
+        if self.transport == "p2p" and plan.world_size > 1:
+            px = self._peer_exchange(B, k_loc)
+            px.check_previous()                # a flag wait of the previous forward timed out: raise before going on
+
+        def exchange_and_merge(kk, truncated=False):
+            if px is not None:
+                bases = px.publish_candidates(*ops.local_topk(x, kk))
+                return _lib.merge_candidates_peer(bases, B, kk, plan.shard_latents, k, truncated=truncated)
+            cand_all = self._all_gather(ops.local_candidates(x, kk))         # [G, B, kk, 2]
+            return ops.merge(cand_all, plan.shard_latents, k, truncated=truncated)  # global top-k, same on all ranks
+
         self.last_exchange = "full"
         vals = None
         if k_snd < k_loc:
-            # round 1: truncated lists; every rank merges the same tensor and therefore sees the same verdict
-            cand_all = self._all_gather(self.ops.local_candidates(x, k_snd))  # [G, B, k_snd, 2]
-            vals, idx, incomplete = self.ops.merge(cand_all, plan.shard_latents, k, truncated=True)
+            # round 1: truncated lists; every rank merges the same candidates and therefore sees the same verdict
+            vals, idx, incomplete = exchange_and_merge(k_snd, truncated=True)
             if int(incomplete.item()) != 0:
                 vals = None                                                   # some shard ran out of candidates
             else:
                 self.last_exchange = "truncated"
+            if px is not None:
+                px.check()                     # the forward has synchronised anyway: a stale merge must not be used
         self.last_k_send = k_snd if vals is not None else k_loc
         if vals is None:
-            cand = self.ops.local_candidates(x, k_loc)                        # [B, k_loc, 2]
-            cand_all = self._all_gather(cand)                                 # [G, B, k_loc, 2]
-            vals, idx = self.ops.merge(cand_all, plan.shard_latents, k)       # global top-k, same on all ranks
-        partial = self.ops.decode_partial(vals, idx, plan, with_bias=(plan.rank == 0))
-        rows = self._reduce_scatter_rows(partial)
+            vals, idx = exchange_and_merge(k_loc)
+        with_bias = plan.rank == 0
+        if px is not None:
+            ops.decode_partial(vals, idx, plan, with_bias, out=px.partial_view(B))
+            a, b = plan.row_range(B)
+            rows = px.reduce_rows(a, b - a)
+        else:
+            rows = self._reduce_scatter_rows(ops.decode_partial(vals, idx, plan, with_bias))
         if self.gather_output and plan.world_size > 1:
-            B = x.shape[0]
-            per = plan.padded_batch(B) // plan.world_size
-            if rows.shape[0] != per:
-                rows = torch.cat([rows, rows.new_zeros((per - rows.shape[0], rows.shape[1]))], 0)
-            rows = self._all_gather(rows).reshape(-1, rows.shape[1])[:B]
-        latents = SparseLatents(vals, idx, (x.shape[0], self.hidden_dim))
-        return latents, rows, self.polarize_loss(x)
+            rows = self._gather_rows(rows, B)
+        if px is not None:
+            px.note_forward_done()
+        return SparseLatents(vals, idx, (B, self.hidden_dim)), rows
 
-    # ---- the same forward with both exchanges over peer memory --------------------------------------------------
     def local_candidates(self, x: torch.Tensor) -> torch.Tensor:
         """The rank-local stage alone (fused encoder sweep + top-k over this shard, candidates of the first exchange
         round): what bench.py times to split a step into local compute and exchange + merge + decode."""
         k = self.top_k()
         return self.ops.local_candidates(x.contiguous().float(), self.plan.k_send(k, self.trim_min_k))
 
+    # ---- the same forward with both exchanges over peer memory --------------------------------------------------
     def _peer_exchange(self, rows: int, k: int) -> PeerExchange:
         if self._peer is not None and self._peer.broken:
             self._peer.close(collective=False)
@@ -411,48 +429,95 @@ class DictionaryShardedBinarySAE(nn.Module):
                                       rows, k, self.input_dim)
         return self._peer
 
-    def _forward_p2p(self, x: torch.Tensor, k: int):
-        plan = self.plan
-        ops = self.ops
-        B = x.shape[0]
-        k_loc, k_snd = plan.k_local(k), plan.k_send(k, self.trim_min_k)
-        px = self._peer_exchange(B, k_loc)
-        px.check_previous()                    # a flag wait of the previous forward timed out: raise before going on
-        lin = self.encoder[0]
-        w32 = lin.weight.detach().contiguous()
 
-        def local_topk(kk):
-            v, i, _ = _lib.encode_topk(x, ops._w_bf16(), w32 if self.exact else None, lin.bias.detach(), kk, _lib.ACT_NONE,
-                                       self.exact, sample=ops._sample())
-            return v, i
+class DictionaryShardedBinarySAE(_DictionaryShardedForward):
+    """Rank-local shard of BinarySAE(input_dim, hidden_dim, gamma, n_bits) (sae/binary.py:73).
 
-        self.last_exchange = "full"
-        vals = None
-        if k_snd < k_loc:
-            bases = px.publish_candidates(*local_topk(k_snd))
-            vals, idx, incomplete = _lib.merge_candidates_peer(bases, B, k_snd, plan.shard_latents, k, truncated=True)
-            if int(incomplete.item()) != 0:
-                vals = None
-            else:
-                self.last_exchange = "truncated"
-            px.check()                         # the forward has synchronised anyway: a stale merge must not be used
-        self.last_k_send = k_snd if vals is not None else k_loc
-        if vals is None:
-            bases = px.publish_candidates(*local_topk(k_loc))
-            vals, idx = _lib.merge_candidates_peer(bases, B, k_loc, plan.shard_latents, k)
-        packed, _, gap = ops._packed()
-        if gap > self.polar_tol:
-            raise RuntimeError("dictionary-sharded b_sae serves the packed (polarised / hard) dictionary only; "
-                               f"max |sigmoid(w) - bit| = {gap:.3g} on this shard")
-        _lib.decode_range(vals, idx, packed, plan.shard_latents, plan.latent_begin, self.input_dim, self.quantization_step,
-                          self.decoder.bias.detach() if plan.rank == 0 else None, self.n_bits, out=px.partial_view(B))
-        a, b = plan.row_range(B)
-        rows = px.reduce_rows(a, b - a)
-        if self.gather_output:
-            per = plan.padded_batch(B) // plan.world_size
-            if rows.shape[0] != per:
-                rows = torch.cat([rows, rows.new_zeros((per - rows.shape[0], rows.shape[1]))], 0)
-            rows = self._all_gather(rows).reshape(-1, rows.shape[1])[:B]
-        px.note_forward_done()
-        latents = SparseLatents(vals, idx, (B, self.hidden_dim))
+    state_dict keys are the reference's, with the latent axis sliced: encoder.0.weight [H/G, D],
+    encoder.0.bias [H/G], decoder.weight [H/G, D*n_bits], decoder.bias [D] (replicated).
+    forward(x) -> (SparseLatents over all H latents, recon rows owned by this rank [B/G, D] or the
+    gathered [B, D] when `gather_output`, polarize_loss)."""
+
+    def __init__(self, input_dim, hidden_dim, gamma=4.0, n_bits=8, *, rank=None, world_size=None,
+                 process_group=None, ops=None):
+        super().__init__(hidden_dim, rank, world_size, process_group)
+        self.input_dim, self.n_bits, self.gamma = input_dim, n_bits, gamma
+        self.quantization_step = gamma / (2 ** (n_bits - 1))
+        self.k = 0.002
+        hs = self.plan.shard_latents
+        self.encoder = nn.Sequential(nn.Linear(input_dim, hs))
+        self.decoder = nn.Module()
+        self.decoder.weight = nn.Parameter(torch.empty(hs, input_dim * n_bits))
+        self.decoder.bias = nn.Parameter(torch.zeros(input_dim))
+        nn.init.xavier_uniform_(self.encoder[0].weight, gain=1)
+        nn.init.zeros_(self.encoder[0].bias)
+        nn.init.kaiming_normal_(self.decoder.weight)
+        self.polar_tol = 1e-6
+        self._pol_cache = None
+        # ops=False defers the choice (tests install their own backend after construction)
+        self.ops = CudaShardOps(self) if ops is None else (ops or None)
+
+    @property
+    def decoder_weight(self):
+        return self.decoder.weight
+
+    @property
+    def decoder_bias(self):
+        return self.decoder.bias
+
+    def top_k(self) -> int:
+        return int(self.hidden_dim * self.k)          # over the FULL dictionary, as sae/binary.py:94
+
+    def polarize_loss(self, like: torch.Tensor) -> torch.Tensor:
+        """mean over the FULL dictionary of p (1 - p) 2^i (sae/binary.py:41-42): weight-only, so the
+        all-reduce of the per-shard numerators runs once per weight version, not per forward."""
+        key = param_key(self.decoder.weight) + (str(like.device),)
+        if self._pol_cache is None or self._pol_cache[0] != key:
+            num = torch.tensor([self.ops.polarize_numerator()], dtype=torch.float64, device=like.device)
+            if self.plan.world_size > 1:
+                self._dist.all_reduce(num, group=self.group)
+            total = self.hidden_dim * self.input_dim * self.n_bits
+            self._pol_cache = (key, (num[0] / total).to(torch.float32))
+        return self._pol_cache[1]
+
+    def forward(self, x: torch.Tensor):
+        latents, rows = self._sharded_forward(x)
         return latents, rows, self.polarize_loss(x)
+
+
+class DictionaryShardedBaselineSAE(_DictionaryShardedForward):
+    """Rank-local shard of BaselineSparseAutoencoder(input_dim, hidden_dim) (sae/baseline.py): the top-k baseline at
+    2^20 latents, split over G ranks by latents.
+
+    state_dict keys are the baseline's, with the latent axis sliced: encoder.0.weight [H/G, D], encoder.0.bias [H/G],
+    decoder.weight [D, H/G] (the decoder is nn.Linear(H, D), so a shard holds a column slice), decoder.bias [D]
+    (replicated, added by rank 0 only). ShardPlan.shard_baseline_state_dict slices a full checkpoint.
+
+    forward(x) -> (SparseLatents over all H latents with global indices, recon rows): this rank's [B/G, D] rows after
+    the reduce-scatter, or the gathered [B, D] with `gather_output`. There is no dense [B, H] latent (the single-GPU
+    module's `return_dense`): at H = 2^20 and B = 4096 it would take 17 GB. `SparseLatents.to_dense()` builds it on
+    request. Inference and analysis only: there is no backward."""
+
+    def __init__(self, input_dim, hidden_dim, *, rank=None, world_size=None, process_group=None, ops=None):
+        super().__init__(hidden_dim, rank, world_size, process_group)
+        self.input_dim = input_dim
+        hs = self.plan.shard_latents
+        # nn.Linear's own initialisation of the shard; load a full checkpoint through shard_baseline_state_dict
+        self.encoder = nn.Sequential(nn.Linear(input_dim, hs))
+        self.decoder = nn.Linear(hs, input_dim)
+        self.topk = 32
+        # ops=False defers the choice (tests install their own backend after construction)
+        self.ops = CudaBaselineShardOps(self) if ops is None else (ops or None)
+
+    def top_k(self) -> int:
+        return int(self.topk)                         # a count over the FULL dictionary, as sae/baseline.py:35
+
+    def forward(self, x: torch.Tensor):
+        return self._sharded_forward(x)
+
+    def normalize_decoder_weights(self):
+        """Unit-norm decoder columns (sae/baseline.py:42-50). A column is one latent, so every norm is local to the
+        shard that holds it: the single-GPU formula on the shard, with no collective."""
+        with torch.no_grad():
+            w = self.decoder.weight.data
+            self.decoder.weight.data = w / torch.clamp(torch.norm(w, dim=0, keepdim=True), min=1e-8)
