@@ -122,6 +122,8 @@ def _check(name, m, x, lat, g, g_lat, x_grad=None):
 ODD = {
     "b37_d8_h1000": dict(D=8, H=1000, B=37, bf16=False, seed=81),
     "b300_d256_h2056": dict(D=256, H=2056, B=300, bf16=False, seed=82),
+    "b300_d136_h4096": dict(D=136, H=4096, B=300, bf16=False, seed=83),     # 3 K chunks, the last one partial
+    "b300_d456_h4096": dict(D=456, H=4096, B=300, bf16=False, seed=84),     # 8 K chunks above D = 448, the last partial
 }
 STEP_CASES = {**cases.BASELINE_CASES, **ODD}
 

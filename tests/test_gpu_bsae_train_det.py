@@ -208,6 +208,8 @@ BOUND_CASES = {   # name: (D, H, n_bits, k, B, gamma, skew)
     "d512_h32768_4b_k32": (512, 32768, 4, 32, 4096, 4.0, False),
     "d512_h32768_4b_skew": (512, 32768, 4, 32, 4096, 4.0, True),
     "d64_h1m_4b_k16": (64, 1 << 20, 4, 16, 1024, 4.0, False),          # keys over [0, 2^20]: three radix passes
+    "d136_h4096_3b_k32": (136, 4096, 3, 32, 300, 4.0, False),          # 3 K chunks, the last one partial
+    "d456_h32768_4b_k32": (456, 32768, 4, 32, 4096, 4.0, False),       # 8 K chunks (pair schedule), the last partial
 }
 
 

@@ -60,6 +60,7 @@ SHAPES = [
     (8, 32768, 512, 130),                                                        # headline size
     (8, 1000, 512, 130), (5, 1000, 16, 33),                                      # boundaries off the 8-grid
     (4, 2056, 48, 33), (4, 32776, 512, 1),                                       # one level boundary off the 8-grid
+    (4, 4096, 144, 130), (6, 4096, 336, 33), (3, 2056, 400, 130), (8, 4096, 464, 130),   # 3, 6, 7, 8 K chunks, the last partial
 ]
 IDS = [f"nb{nb}-h{H}-d{D}-b{B}" for nb, H, D, B in SHAPES]
 LEVEL_SIZES = {

@@ -82,6 +82,8 @@ ODD_CASES = {
     "b37_d64_h1000": dict(D=64, H=1000, B=37, bf16=False, seed=71),     # H % 128 != 0, B not a multiple of 128
     "b130_d8_h264": dict(D=8, H=264, B=130, bf16=False, seed=72),       # D = 8
     "b300_d512_h2056": dict(D=512, H=2056, B=300, bf16=True, seed=73),
+    "b130_d392_h1000": dict(D=392, H=1000, B=130, bf16=False, seed=74),     # 7 K chunks, the last one partial
+    "b300_d456_h2056": dict(D=456, H=2056, B=300, bf16=True, seed=75),      # 8 K chunks above D = 448, the last partial
 }
 STEP_CASES = {**cases.TSAE_CASES, **ODD_CASES}
 
