@@ -437,6 +437,24 @@ int qsae_baseline_backward(const float* x /* [B, D] */, const float* vals, const
                            float* grad_b_enc /* [H] */, float* grad_w_dec /* [D, H] */, float* grad_b_dec /* [D] */,
                            float* grad_x /* [B, D] or NULL */, void* workspace, size_t workspace_bytes, void* stream);
 
+/* One shard's part of qsae_baseline_backward in the dictionary-sharded baseline_sae: the shard owns the latents
+ * [idx_begin, idx_begin + H_shard) and holds their decoder rows rows_shard [H_shard, D] (its decoder.weight^T); idx
+ * holds global indices, and an entry outside the range is skipped. The owned entries are compacted in row-major order
+ * before they are grouped by latent, so every latent's sums run over the same entries in the same order as in
+ * qsae_baseline_backward: grad_w_enc [H_shard, D], grad_b_enc [H_shard] and grad_w_dec [D, H_shard] (row stride
+ * H_shard) are bit-equal to the matching slices of its outputs for the same (vals, idx, g_recon, g_vals), and
+ * grad_b_dec [D] (over all of g_recon) to its grad_b_dec. No g_h, no grad_x. k counts winners over the whole
+ * dictionary and may exceed H_shard (1 <= k <= QSAE_MAX_K_LARGE); B k < 2^31; idx_begin >= 0; H_shard >= 1 and D as
+ * in qsae_encode_topk; B may be 0 (zero gradients). x, g_recon, rows_shard, grad_w_enc and the workspace 16-byte
+ * aligned. Caller workspace, one stream, no host synchronisation. */
+int qsae_baseline_backward_range_workspace_bytes(int B, int H_shard, int D, int k, size_t* bytes);
+int qsae_baseline_backward_range(const float* x /* [B, D] */, const float* vals, const int32_t* idx /* [B, k] */,
+                                 const float* g_recon /* [B, D] */, const float* g_vals /* [B, k] or NULL */,
+                                 const float* rows_shard /* [H_shard, D] */, int B, int H_shard, int idx_begin, int D, int k,
+                                 float* grad_w_enc /* [H_shard, D] */, float* grad_b_enc /* [H_shard] */,
+                                 float* grad_w_dec /* [D, H_shard] */, float* grad_b_dec /* [D] */, void* workspace,
+                                 size_t workspace_bytes, void* stream);
+
 /* Bit-deterministic backward of BinarySAE.forward under its soft (sigmoid) dictionary (sae/binary.py:24-47, 91-103).
  * With g = d loss / d recon [B, D], the forward's top-k (vals, idx) [B, k], q the quantization step and
  *   gv[b,j] = q <g[b,:], soft_rows[idx[b,j], :]>,   G[h,:] = q sum v g[b,:]   (d loss / d int_w)

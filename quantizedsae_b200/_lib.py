@@ -117,6 +117,8 @@ SYMBOLS = {
     "qsae_baseline_backward_workspace_bytes": (_i, [_i, _i, _i, _i, C.POINTER(_sz)]),
     "qsae_baseline_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
                                     _vp]),
+    "qsae_baseline_backward_range_workspace_bytes": (_i, [_i, _i, _i, _i, C.POINTER(_sz)]),
+    "qsae_baseline_backward_range": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "qsae_bsae_backward_workspace_bytes": (_i, [_i, _i, _i, _i, _i, C.POINTER(_sz)]),
     "qsae_bsae_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _f, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp,
                                 _sz, _vp]),
@@ -850,6 +852,38 @@ def baseline_backward(x: torch.Tensor, vals: torch.Tensor, idx: torch.Tensor, g_
                                         gwe.data_ptr(), gbe.data_ptr(), gwd.data_ptr(), gbd.data_ptr(), _ptr(gx),
                                         ws.data_ptr(), ws.numel(), _stream()))
     return gwe, gbe, gwd, gbd, gx
+
+
+def baseline_backward_range_workspace_bytes(B: int, H_shard: int, D: int, k: int) -> int:
+    n = _sz(0)
+    check(load().qsae_baseline_backward_range_workspace_bytes(B, H_shard, D, k, C.byref(n)))
+    return int(n.value)
+
+
+def baseline_backward_range(x: torch.Tensor, vals: torch.Tensor, idx: torch.Tensor, g_recon: torch.Tensor,
+                            g_vals: torch.Tensor | None, rows_shard: torch.Tensor, idx_begin: int):
+    """One shard's part of baseline_backward (qsae_baseline_backward_range): the shard owns the latents [idx_begin,
+    idx_begin + H_shard) and holds rows_shard = its decoder.weight^T [H_shard, D]; idx holds global indices. The outputs
+    are bit-equal to the matching slices of baseline_backward's for the same inputs.
+    -> (grad W_enc [H_shard, D], grad b_enc [H_shard], grad W_dec [D, H_shard], grad b_dec [D])"""
+    _need_cuda(x, vals, idx, g_recon, g_vals, rows_shard)
+    _f32c(x, vals, g_recon, g_vals, rows_shard)
+    B, D = x.shape
+    H = rows_shard.shape[0]
+    k = idx.shape[1]
+    assert vals.shape == (B, k) and idx.shape == (B, k) and idx.dtype == torch.int32 and g_recon.shape == (B, D)
+    assert rows_shard.shape == (H, D) and (g_vals is None or g_vals.shape == (B, k))
+    dev = x.device
+    gwe = torch.empty((H, D), dtype=torch.float32, device=dev)
+    gbe = torch.empty((H,), dtype=torch.float32, device=dev)
+    gwd = torch.empty((D, H), dtype=torch.float32, device=dev)
+    gbd = torch.empty((D,), dtype=torch.float32, device=dev)
+    ws = _workspace(dev, baseline_backward_range_workspace_bytes(B, H, D, k))
+    check(load().qsae_baseline_backward_range(x.data_ptr(), vals.data_ptr(), idx.data_ptr(), g_recon.data_ptr(),
+                                              _ptr(g_vals), rows_shard.data_ptr(), B, H, int(idx_begin), D, k,
+                                              gwe.data_ptr(), gbe.data_ptr(), gwd.data_ptr(), gbd.data_ptr(),
+                                              ws.data_ptr(), ws.numel(), _stream()))
+    return gwe, gbe, gwd, gbd
 
 
 def bsae_backward_workspace_bytes(B: int, H: int, D: int, k: int, n_bits: int) -> int:

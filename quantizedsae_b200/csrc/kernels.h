@@ -343,6 +343,12 @@ const char* baseline_backward_launch(const float* x, const float* vals, const in
                                      const float* g_h, const float* g_vals, const float* w_enc, const float* dec_rows, int B,
                                      int H, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx, void* workspace,
                                      cudaStream_t stream);
+// the same over one shard's latents [idx_begin, idx_begin + H_shard) (no g_h, no grad x); grad b_dec over all of g;
+// workspace of baseline_backward_workspace_bytes(B, H_shard, D, k)
+const char* baseline_backward_range_launch(const float* x, const float* vals, const int32_t* idx, const float* g,
+                                           const float* g_vals, const float* rows_shard, int B, int H_shard, int idx_begin, int D,
+                                           int k, float* gWe, float* gbe, float* gWd, float* gbd, void* workspace,
+                                           cudaStream_t stream);
 // b_sae backward (deterministic, latent-major, the logit chain rule fused in): gradients of the encoder Linear, the bit
 // logits, b_dec and (gx != null) x; workspace of baseline_backward_workspace_bytes(B, H, D, k)
 const char* bsae_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g, const float* soft_rows,

@@ -1467,6 +1467,66 @@ int qsae_baseline_backward(const float* x, const float* vals, const int32_t* idx
   return err == nullptr ? QSAE_OK : fail(QSAE_ERR_CUDA, "baseline_backward: %s", err);
 }
 
+// ---- dictionary-sharded baseline_sae backward: one shard's latent range of the above (csrc/train.cu)
+namespace {
+// k counts winners over the whole dictionary, so it may exceed the shard (k = 1000 of 512-latent shards is legal)
+int check_baseline_backward_range(int B, int H_shard, int D, int k) {
+  if (B < 0) return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward_range: negative batch");
+  if (H_shard < 1) return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward_range: H_shard must be >= 1, got %d", H_shard);
+  const int rc = check_encode_shape(B > 0 ? B : 1, H_shard, D);
+  if (rc != QSAE_OK) return rc;
+  if (k < 1) return fail(QSAE_ERR_INVALID_ARGUMENT, "k must be >= 1, got %d", k);
+  if (k > kMaxKLarge) return fail(QSAE_ERR_INVALID_ARGUMENT, "k=%d exceeds QSAE_MAX_K_LARGE=%d", k, kMaxKLarge);
+  if (static_cast<long long>(B) * k > 0x7fffffffLL)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward_range: B k = %lld entries exceed 2^31 - 1",
+                static_cast<long long>(B) * k);
+  return QSAE_OK;
+}
+}  // namespace
+
+int qsae_baseline_backward_range_workspace_bytes(int B, int H_shard, int D, int k, size_t* bytes) {
+  if (!bytes) return fail(QSAE_ERR_INVALID_ARGUMENT, "workspace query: null pointer");
+  const int rc = check_baseline_backward_range(B, H_shard, D, k);
+  if (rc != QSAE_OK) return rc;
+  *bytes = baseline_backward_workspace_bytes(B, H_shard, D, k);
+  return QSAE_OK;
+}
+
+int qsae_baseline_backward_range(const float* x, const float* vals, const int32_t* idx, const float* g_recon,
+                                 const float* g_vals, const float* rows_shard, int B, int H_shard, int idx_begin, int D, int k,
+                                 float* grad_w_enc, float* grad_b_enc, float* grad_w_dec, float* grad_b_dec, void* workspace,
+                                 size_t workspace_bytes, void* stream) {
+  int rc = check_baseline_backward_range(B, H_shard, D, k);
+  if (rc != QSAE_OK) return rc;
+  if (idx_begin < 0 || static_cast<long long>(idx_begin) + H_shard > 0x7fffffffLL)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward_range: latent range [%d, %d + %d) out of int32", idx_begin,
+                idx_begin, H_shard);
+  if (!grad_w_enc || !grad_b_enc || !grad_w_dec || !grad_b_dec)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward_range: null gradient pointer");
+  cudaStream_t st = S(stream);
+  const size_t nhd = static_cast<size_t>(H_shard) * D;
+  if (B == 0) {   // nothing selected: zero gradients
+    cudaError_t e = cudaMemsetAsync(grad_w_enc, 0, nhd * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_b_enc, 0, static_cast<size_t>(H_shard) * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_w_dec, 0, nhd * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(grad_b_dec, 0, static_cast<size_t>(D) * 4, st);
+    return e == cudaSuccess ? QSAE_OK : fail(QSAE_ERR_CUDA, "baseline_backward_range: %s", cudaGetErrorString(e));
+  }
+  if (!x || !vals || !idx || !g_recon || !rows_shard || !workspace)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward_range: null pointer");
+  const size_t need = baseline_backward_workspace_bytes(B, H_shard, D, k);
+  if (workspace_bytes < need)
+    return fail(QSAE_ERR_WORKSPACE_TOO_SMALL, "baseline_backward_range: workspace %zu < %zu bytes", workspace_bytes, need);
+  const uintptr_t align16 = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(g_recon) |
+                            reinterpret_cast<uintptr_t>(rows_shard) | reinterpret_cast<uintptr_t>(grad_w_enc) |
+                            reinterpret_cast<uintptr_t>(workspace);
+  if ((align16 & 15) != 0)
+    return fail(QSAE_ERR_INVALID_ARGUMENT, "baseline_backward_range: workspace and row-major tensors must be 16-byte aligned");
+  const char* err = baseline_backward_range_launch(x, vals, idx, g_recon, g_vals, rows_shard, B, H_shard, idx_begin, D, k,
+                                                   grad_w_enc, grad_b_enc, grad_w_dec, grad_b_dec, workspace, st);
+  return err == nullptr ? QSAE_OK : fail(QSAE_ERR_CUDA, "baseline_backward_range: %s", err);
+}
+
 // ---- b_sae backward: deterministic, latent-major, the logit chain rule fused in (csrc/train.cu)
 namespace {
 int check_bsae_backward(int B, int H, int D, int k, int n_bits) {

@@ -853,14 +853,21 @@ constexpr int kColParts = 256;   // most partial rows of the two-level column su
 
 __device__ __forceinline__ int clamp_key(int h, int H) { return static_cast<unsigned>(h) < static_cast<unsigned>(H) ? h : H; }
 
-// gv[b,j] = scale <g[b,:], rows[idx[b,j],:]> + g_h term (0 for an index outside [0, H)); cnt[h] += 1 per selection.
-// Warp per row, the row of g in registers, butterfly reductions: the same bits in every lane and on every run.
-// baseline_sae passes scale 1 (the product is exact, so its bits are those of the plain dot), b_sae the step q.
+// The latent an entry selects, relative to the first latent of the range [idx_begin, idx_begin + H) a backward owns;
+// unsigned, so that an index below the range (or a negative one) lands outside [0, H) as well.
+__device__ __forceinline__ int local_latent(int32_t i, int idx_begin) {
+  return static_cast<int>(static_cast<unsigned>(i) - static_cast<unsigned>(idx_begin));
+}
+
+// gv[b,j] = scale <g[b,:], rows[h,:]> + g_h term with h = idx[b,j] - idx_begin (0 for an entry outside the range
+// [0, H)); cnt[h] += 1 per selection. Warp per row, the row of g in registers, butterfly reductions: the same bits in
+// every lane and on every run. baseline_sae passes scale 1 (the product is exact, so its bits are those of the plain
+// dot), b_sae the step q.
 template <int NCH>
 __global__ void __launch_bounds__(256)
 bwd_latent_grad_kernel(const float* __restrict__ g, const float* __restrict__ rows, const int32_t* __restrict__ idx,
                        const float* __restrict__ gh_dense, const float* __restrict__ gh_vals, int B, int k, int D, int H,
-                       float scale, float* __restrict__ gv, int* __restrict__ cnt) {
+                       int idx_begin, float scale, float* __restrict__ gv, int* __restrict__ cnt) {
   const int lane = threadIdx.x & 31;
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int nwarps = (gridDim.x * blockDim.x) >> 5;
@@ -875,7 +882,7 @@ bwd_latent_grad_kernel(const float* __restrict__ g, const float* __restrict__ ro
     for (int j0 = 0; j0 < k; j0 += 32) {
       const int jl = j0 + lane;
       const size_t e = static_cast<size_t>(row) * k + jl;
-      const int my_h = jl < k ? idx[e] : -1;
+      const int my_h = jl < k ? local_latent(idx[e], idx_begin) : -1;
       const bool ok = static_cast<unsigned>(my_h) < static_cast<unsigned>(H);
       float my_gh = 0.f;
       if (ok && gh_vals != nullptr) my_gh = gh_vals[e];
@@ -907,13 +914,70 @@ bwd_latent_grad_kernel(const float* __restrict__ g, const float* __restrict__ ro
   }
 }
 
+__device__ __forceinline__ int sort_tiles(int n) { return (n + kSortTile - 1) / kSortTile; }
+
+// Stable compaction of the entries inside a latent range (the dictionary-sharded backward), so that the scans, the
+// sort and the chunk grid run on the owned entries only. Tiles of kSortTile row-major entries: the owned count of
+// each tile, an exclusive scan of those, then an in-order scatter of {local latent, entry}.
+__global__ void __launch_bounds__(kSortThreads)
+bwd_own_count_kernel(const int32_t* __restrict__ idx, int n, int idx_begin, int H, int* __restrict__ tile_cnt) {
+  __shared__ int wsum[kSortThreads / 32];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int base = blockIdx.x * kSortTile;
+  int c = 0;
+  for (int i = threadIdx.x; i < kSortTile; i += kSortThreads)
+    if (base + i < n && static_cast<unsigned>(local_latent(idx[base + i], idx_begin)) < static_cast<unsigned>(H)) ++c;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+  if (lane == 0) wsum[wid] = c;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int t = 0;
+#pragma unroll
+    for (int w = 0; w < kSortThreads / 32; ++w) t += wsum[w];
+    tile_cnt[blockIdx.x] = t;
+  }
+}
+
+__global__ void __launch_bounds__(kSortThreads)
+bwd_own_scatter_kernel(const int32_t* __restrict__ idx, int n, int idx_begin, int H, const int* __restrict__ tile_off,
+                       int* __restrict__ keys_out, int* __restrict__ e_out) {
+  constexpr int kWarps = kSortThreads / 32;
+  __shared__ int wcnt[kWarps];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  int run = tile_off[blockIdx.x];                    // every thread keeps the tile's running output position
+  const int base = blockIdx.x * kSortTile;
+  for (int r = 0; r < kSortItems; ++r) {
+    const int i = base + r * kSortThreads + threadIdx.x;
+    const int h = i < n ? local_latent(idx[i], idx_begin) : -1;
+    const bool own = static_cast<unsigned>(h) < static_cast<unsigned>(H);
+    const unsigned mask = __ballot_sync(0xffffffffu, own);
+    if (lane == 0) wcnt[wid] = __popc(mask);
+    __syncthreads();
+    int pos = run + __popc(mask & ((1u << lane) - 1u)), all = 0;
+#pragma unroll
+    for (int w = 0; w < kWarps; ++w) {
+      if (w < wid) pos += wcnt[w];
+      all += wcnt[w];
+    }
+    if (own) {
+      keys_out[pos] = h;
+      e_out[pos] = i;
+    }
+    run += all;
+    __syncthreads();                                 // wcnt is rewritten by the next round
+  }
+}
+
 // Exclusive prefix sums by one block of 1024 threads (each owns a contiguous run): out[0..n], out[n] = total.
 // CHUNKED: the values are the chunk counts of the per-latent entry counts in[] (latents longer than kBwdChunk only).
+// sort_n != null: in[] is the digit histogram of a sort whose entry count is on the device, n = kRadix tiles of it.
 // May run in place (in == out): every thread reads and writes only its own run.
 template <bool CHUNKED>
-__global__ void __launch_bounds__(1024) bwd_scan_kernel(const int* in, int n, int* out) {
+__global__ void __launch_bounds__(1024) bwd_scan_kernel(const int* in, int n, int* out, const int* sort_n) {
   __shared__ int warp_tot[32];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  if (sort_n != nullptr) n = kRadix * sort_tiles(*sort_n);
   const int per = (n + 1023) / 1024;
   const int lo = min(n, threadIdx.x * per), hi = min(n, lo + per);
   auto value = [&](int i) {
@@ -945,10 +1009,17 @@ __global__ void __launch_bounds__(1024) bwd_scan_kernel(const int* in, int n, in
 }
 
 // radix sort of the entries by latent, 8 bits per pass: digit counts of one tile of kSortTile entries, digit-major
-// [kRadix][ntiles] so that one exclusive scan gives every (digit, tile) its first output position
+// [kRadix][ntiles] so that one exclusive scan gives every (digit, tile) its first output position.
+// n_dev != null: the entry count is on the device (n and ntiles are upper bounds, the tiles past it exit).
 __global__ void __launch_bounds__(kSortThreads)
-bwd_sort_hist_kernel(const int32_t* __restrict__ keys, int n, int H, int shift, int ntiles, int* __restrict__ hist) {
+bwd_sort_hist_kernel(const int32_t* __restrict__ keys, int n, int H, int shift, int ntiles, int* __restrict__ hist,
+                     const int* __restrict__ n_dev) {
   __shared__ int h[kRadix];
+  if (n_dev != nullptr) {
+    n = *n_dev;
+    ntiles = sort_tiles(n);
+    if (static_cast<int>(blockIdx.x) >= ntiles) return;      // block-uniform
+  }
   h[threadIdx.x] = 0;
   __syncthreads();
   const int base = blockIdx.x * kSortTile;
@@ -966,11 +1037,16 @@ __global__ void __launch_bounds__(kSortThreads)
 bwd_sort_scatter_kernel(const int32_t* __restrict__ keys, const int* __restrict__ src_e, int n, int H, int shift, int ntiles,
                         const int* __restrict__ hist_off, int* __restrict__ keys_out, int* __restrict__ e_out, int k,
                         const float* __restrict__ vals, const float* __restrict__ gv, int* __restrict__ ent_b,
-                        float* __restrict__ ent_v, float* __restrict__ ent_g) {
+                        float* __restrict__ ent_v, float* __restrict__ ent_g, const int* __restrict__ n_dev) {
   constexpr int kWarps = kSortThreads / 32;
   __shared__ int run[kRadix];
   __shared__ int wcnt[kWarps][kRadix];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  if (n_dev != nullptr) {
+    n = *n_dev;
+    ntiles = sort_tiles(n);
+    if (static_cast<int>(blockIdx.x) >= ntiles) return;      // block-uniform
+  }
   run[threadIdx.x] = hist_off[threadIdx.x * ntiles + blockIdx.x];
 #pragma unroll
   for (int w = 0; w < kWarps; ++w) wcnt[w][threadIdx.x] = 0;
@@ -1320,13 +1396,18 @@ void bsae_reduce_launches(const BaselineBwdLayout& L, uint8_t* ws, int H, int D,
       gp_dev, gp_host, gWe, gbe, glog);
 }
 
-// The first steps of both latent-major backwards:
+// The first steps of both latent-major backwards over the latents [idx_begin, idx_begin + H) (rows: theirs, [H, D]):
 //   1. gv = scale <g, rows[h]> + g_h term at each kept entry, and the per-latent counts;
 //   2. CSC offsets of the entries and of the chunks of long latents;
-//   3. stable radix sort of the row-major entries by latent -> records {b, v, gv}, latent-major.
+//   3. compact: stable compaction of the entries inside the range (their count, off[H], stays on the device; the
+//      sort's grids are sized for all B k entries and the tiles past it exit). The whole dictionary (compact = false)
+//      sorts the entries in place, an index outside [0, H) keyed H, past every latent;
+//   4. stable radix sort of the row-major entries by latent -> records {b, v, gv}, latent-major.
+// Each latent's records come out in the same order either way (rows ascending), so a range's sums are bit-equal to
+// those of the whole dictionary.
 const char* bwd_group_by_latent(const BaselineBwdLayout& L, uint8_t* ws, const float* g, const float* rows, const int32_t* idx,
-                                const float* vals, const float* g_h, const float* g_vals, int B, int H, int D, int k,
-                                float scale, int* launches, cudaStream_t stream) {
+                                const float* vals, const float* g_h, const float* g_vals, int B, int H, int idx_begin,
+                                bool compact, int D, int k, float scale, int* launches, cudaStream_t stream) {
   float* gv = reinterpret_cast<float*>(ws + L.gv);
   int* cnt = reinterpret_cast<int*>(ws + L.cnt);
   int* hist = reinterpret_cast<int*>(ws + L.hist);
@@ -1334,30 +1415,44 @@ const char* bwd_group_by_latent(const BaselineBwdLayout& L, uint8_t* ws, const f
   if (e != cudaSuccess) return cudaGetErrorString(e);
   const int grid_rows = grid_for(static_cast<size_t>(B) * 32, 256, 148 * 8);
   switch ((D / 4 + 31) / 32) {
-    case 1: bwd_latent_grad_kernel<1><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, scale, gv, cnt); break;
-    case 2: bwd_latent_grad_kernel<2><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, scale, gv, cnt); break;
-    case 3: bwd_latent_grad_kernel<3><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, scale, gv, cnt); break;
-    default: bwd_latent_grad_kernel<4><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, scale, gv, cnt); break;
+    case 1: bwd_latent_grad_kernel<1><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, idx_begin, scale, gv, cnt); break;
+    case 2: bwd_latent_grad_kernel<2><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, idx_begin, scale, gv, cnt); break;
+    case 3: bwd_latent_grad_kernel<3><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, idx_begin, scale, gv, cnt); break;
+    default: bwd_latent_grad_kernel<4><<<grid_rows, 256, 0, stream>>>(g, rows, idx, g_h, g_vals, B, k, D, H, idx_begin, scale, gv, cnt); break;
   }
-  bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(cnt, H, reinterpret_cast<int*>(ws + L.off));
-  bwd_scan_kernel<true><<<1, 1024, 0, stream>>>(cnt, H, reinterpret_cast<int*>(ws + L.coff));
+  const int* off = reinterpret_cast<const int*>(ws + L.off);
+  bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(cnt, H, reinterpret_cast<int*>(ws + L.off), nullptr);
+  bwd_scan_kernel<true><<<1, 1024, 0, stream>>>(cnt, H, reinterpret_cast<int*>(ws + L.coff), nullptr);
   *launches += 3;
   const int32_t* keys_in = idx;
   const int* e_in = nullptr;
+  const int* n_dev = nullptr;
+  if (compact) {
+    // into the second ping-pong buffers, which the first sort pass does not write; the tile offsets use the histogram
+    int* keys_c = reinterpret_cast<int*>(ws + L.keys[1]);
+    int* e_c = reinterpret_cast<int*>(ws + L.ent[1]);
+    bwd_own_count_kernel<<<L.ntiles, kSortThreads, 0, stream>>>(idx, L.n, idx_begin, H, hist);
+    bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(hist, L.ntiles, hist, nullptr);
+    bwd_own_scatter_kernel<<<L.ntiles, kSortThreads, 0, stream>>>(idx, L.n, idx_begin, H, hist, keys_c, e_c);
+    *launches += 3;
+    keys_in = keys_c;
+    e_in = e_c;
+    n_dev = off + H;                                   // the owned entries: every one is counted in cnt
+  }
   for (int p = 0; p < L.npasses; ++p) {
     const int shift = 8 * p;
     const bool last = p == L.npasses - 1;
-    bwd_sort_hist_kernel<<<L.ntiles, kSortThreads, 0, stream>>>(keys_in, L.n, H, shift, L.ntiles, hist);
-    bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(hist, kRadix * L.ntiles, hist);
+    bwd_sort_hist_kernel<<<L.ntiles, kSortThreads, 0, stream>>>(keys_in, L.n, H, shift, L.ntiles, hist, n_dev);
+    bwd_scan_kernel<false><<<1, 1024, 0, stream>>>(hist, kRadix * L.ntiles, hist, n_dev);
     int* keys_out = reinterpret_cast<int*>(ws + L.keys[p & 1]);
     int* e_out = reinterpret_cast<int*>(ws + L.ent[p & 1]);
     if (last)
       bwd_sort_scatter_kernel<true><<<L.ntiles, kSortThreads, 0, stream>>>(
           keys_in, e_in, L.n, H, shift, L.ntiles, hist, nullptr, nullptr, k, vals, gv, reinterpret_cast<int*>(ws + L.eb),
-          reinterpret_cast<float*>(ws + L.ev), reinterpret_cast<float*>(ws + L.eg));
+          reinterpret_cast<float*>(ws + L.ev), reinterpret_cast<float*>(ws + L.eg), n_dev);
     else
       bwd_sort_scatter_kernel<false><<<L.ntiles, kSortThreads, 0, stream>>>(
-          keys_in, e_in, L.n, H, shift, L.ntiles, hist, keys_out, e_out, k, nullptr, nullptr, nullptr, nullptr, nullptr);
+          keys_in, e_in, L.n, H, shift, L.ntiles, hist, keys_out, e_out, k, nullptr, nullptr, nullptr, nullptr, nullptr, n_dev);
     keys_in = keys_out;
     e_in = e_out;
     *launches += 3;
@@ -1386,14 +1481,18 @@ const char* bwd_tail_launches(const BaselineBwdLayout& L, uint8_t* ws, const flo
 
 size_t baseline_backward_workspace_bytes(int B, int H, int D, int k) { return baseline_bwd_layout(B, H, D, k).total; }
 
-const char* baseline_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g,
-                                     const float* g_h, const float* g_vals, const float* w_enc, const float* dec_rows, int B,
-                                     int H, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx, void* workspace,
-                                     cudaStream_t stream) {
+namespace {
+// the baseline backward over the latents [idx_begin, idx_begin + H); the whole dictionary is idx_begin = 0 without
+// the compaction
+const char* baseline_backward_impl(const float* x, const float* vals, const int32_t* idx, const float* g, const float* g_h,
+                                   const float* g_vals, const float* w_enc, const float* dec_rows, int B, int H, int idx_begin,
+                                   bool compact, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx,
+                                   void* workspace, cudaStream_t stream) {
   const BaselineBwdLayout L = baseline_bwd_layout(B, H, D, k);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   int launches = 0;
-  const char* err = bwd_group_by_latent(L, ws, g, dec_rows, idx, vals, g_h, g_vals, B, H, D, k, 1.0f, &launches, stream);
+  const char* err = bwd_group_by_latent(L, ws, g, dec_rows, idx, vals, g_h, g_vals, B, H, idx_begin, compact, D, k, 1.0f,
+                                        &launches, stream);
   if (err != nullptr) return err;
   // 4. latent-major reduction: grad W_enc, grad b_enc, grad W_dec
   switch ((D / 4 + 31) / 32) {
@@ -1409,6 +1508,25 @@ const char* baseline_backward_launch(const float* x, const float* vals, const in
   count_launches(launches);
   return cuda_err(cudaGetLastError());
 }
+}  // namespace
+
+const char* baseline_backward_launch(const float* x, const float* vals, const int32_t* idx, const float* g,
+                                     const float* g_h, const float* g_vals, const float* w_enc, const float* dec_rows, int B,
+                                     int H, int D, int k, float* gWe, float* gbe, float* gWd, float* gbd, float* gx, void* workspace,
+                                     cudaStream_t stream) {
+  return baseline_backward_impl(x, vals, idx, g, g_h, g_vals, w_enc, dec_rows, B, H, 0, false, D, k, gWe, gbe, gWd, gbd, gx,
+                                workspace, stream);
+}
+
+// One shard's part of the dictionary-sharded backward: the same steps on the entries inside [idx_begin, idx_begin +
+// H_shard), rows_shard and the outputs the shard's; grad b_dec over all of g as above; no grad x.
+const char* baseline_backward_range_launch(const float* x, const float* vals, const int32_t* idx, const float* g,
+                                           const float* g_vals, const float* rows_shard, int B, int H_shard, int idx_begin, int D,
+                                           int k, float* gWe, float* gbe, float* gWd, float* gbd, void* workspace,
+                                           cudaStream_t stream) {
+  return baseline_backward_impl(x, vals, idx, g, nullptr, g_vals, nullptr, rows_shard, B, H_shard, idx_begin, true, D, k, gWe,
+                                gbe, gWd, gbd, nullptr, workspace, stream);
+}
 
 // b_sae (sae/binary.py:24-47, 91-103): the baseline's steps with gv = q <g, soft_rows[h]>, the soft rows in place of
 // W_dec^T, and the b_sae pass in place of the grad W_dec reduction; the same workspace layout.
@@ -1419,7 +1537,8 @@ const char* bsae_backward_launch(const float* x, const float* vals, const int32_
   const BaselineBwdLayout L = baseline_bwd_layout(B, H, D, k);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   int launches = 0;
-  const char* err = bwd_group_by_latent(L, ws, g, soft_rows, idx, vals, nullptr, nullptr, B, H, D, k, q, &launches, stream);
+  const char* err = bwd_group_by_latent(L, ws, g, soft_rows, idx, vals, nullptr, nullptr, B, H, 0, false, D, k, q, &launches,
+                                        stream);
   if (err != nullptr) return err;
   switch ((D / 4 + 31) / 32) {
     case 1: bsae_reduce_launches<1>(L, ws, H, D, x, g, q, logits, n_bits, gp_dev, gp_host, gWe, gbe, glog, stream); break;

@@ -21,6 +21,17 @@ nn.Linear(H, D) decoder. Everything between the local top-k and the decode (the 
 the peer-exchange lifecycle, gather_output) lives once, in _DictionaryShardedForward; the ops object owns the
 model-specific steps.
 
+The baseline also trains sharded (`autograd = True`, _ShardedBaselineFn). Its gradients split by latent: grad W_enc[h],
+grad b_enc[h] and grad W_dec[:, h] read only the entries that selected h, which the shard owning h can compute from the
+global winners every rank holds. The backward is
+
+    all-gather of d loss / d rows               -> g [B, D] on every rank           (the forward's reduce-scatter, adjointed)
+    all-gather of d loss / d values, summed in rank order -> [B, k], the same bits on every rank
+    the latent-major backward over this shard's latent range (qsae_baseline_backward_range)
+
+and every shard gradient is bit-equal to the matching slice of the single-GPU backward; grad b_dec (the column sums of
+g) is the full gradient, the same bits on every rank.
+
 The collectives go through torch.distributed (NCCL over NVLink on the B200 box; gloo in the CPU
 tests). The compute steps are injected as `ops`: `CudaShardOps` (libqsae_b200.so, the product) is the
 default; the CPU tests pass a numpy implementation to exercise the choreography under gloo. There is
@@ -96,6 +107,25 @@ class ShardPlan:
                 "encoder.0.bias": full["encoder.0.bias"][a:b].clone(),
                 "decoder.weight": full["decoder.weight"][a:b].clone(),
                 "decoder.bias": full["decoder.bias"].clone()}
+
+    def merge_baseline_state_dicts(self, shard_sds) -> dict:
+        """The inverse of shard_baseline_state_dict: the state_dicts of ranks 0 .. G-1, in rank order, -> one
+        BaselineSparseAutoencoder state_dict (encoder rows and decoder columns concatenated, rank 0's decoder.bias).
+        Raises ValueError if the shards do not fit this plan or the replicated decoder.bias differs between them."""
+        if len(shard_sds) != self.world_size:
+            raise ValueError(f"expected {self.world_size} shard state_dicts, got {len(shard_sds)}")
+        hs = self.shard_latents
+        for r, sd in enumerate(shard_sds):
+            if sd["encoder.0.weight"].shape[0] != hs or sd["encoder.0.bias"].shape[0] != hs or sd["decoder.weight"].shape[1] != hs:
+                raise ValueError(f"shard {r} does not hold {hs} latents")
+        bias = shard_sds[0]["decoder.bias"]
+        for r, sd in enumerate(shard_sds[1:], 1):
+            if not torch.equal(sd["decoder.bias"], bias):
+                raise ValueError(f"decoder.bias of rank {r} differs from rank 0's: the replicas diverged")
+        return {"encoder.0.weight": torch.cat([sd["encoder.0.weight"] for sd in shard_sds], 0),
+                "encoder.0.bias": torch.cat([sd["encoder.0.bias"] for sd in shard_sds], 0),
+                "decoder.weight": torch.cat([sd["decoder.weight"] for sd in shard_sds], 1),
+                "decoder.bias": bias.clone()}
 
     def shard_baseline_state_dict(self, full: dict) -> dict:
         """Slice a full BaselineSparseAutoencoder state_dict (sae/baseline.py layout) down to this rank's shard. The
@@ -182,6 +212,12 @@ class CudaBaselineShardOps(_CudaEncoderOps):
     def decode_partial(self, vals, idx, plan: ShardPlan, with_bias: bool, out: torch.Tensor | None = None) -> torch.Tensor:
         return _lib.decode_rows_f32_range(vals, idx, self._dec_rows(), plan.latent_begin, 1.0,
                                           self.m.decoder.bias.detach() if with_bias else None, out=out)
+
+    def backward_local(self, x, vals, idx, g, g_vals, plan: ShardPlan):
+        """This shard's gradients from the global winners (vals, idx) [B, k], the gathered g = d loss / d recon [B, D]
+        and the summed g_vals = d loss / d vals [B, k] -> (grad W_enc [H/G, D], grad b_enc [H/G], grad W_dec [D, H/G],
+        grad b_dec [D] over the whole batch)."""
+        return _lib.baseline_backward_range(x, vals, idx, g, g_vals, self._dec_rows(), plan.latent_begin)
 
 
 class PeerExchange:
@@ -485,6 +521,41 @@ class DictionaryShardedBinarySAE(_DictionaryShardedForward):
         return latents, rows, self.polarize_loss(x)
 
 
+class _ShardedBaselineFn(torch.autograd.Function):
+    """(x, W_enc, b_enc, W_dec, b_dec) of one rank -> (values [B, k], indices [B, k], this rank's recon rows): the
+    sharded forward behind one autograd node. The backward runs the same collectives on every rank, in a fixed order
+    (see the module docstring), so every rank must run it."""
+
+    @staticmethod
+    def forward(ctx, x, w_enc, b_enc, w_dec, b_dec, module):
+        ctx.set_materialize_grads(False)
+        x = x.contiguous().float()
+        lat, rows = module._sharded_forward(x)
+        ctx.module = module
+        ctx.save_for_backward(x, lat.values, lat.indices)
+        ctx.mark_non_differentiable(lat.indices)
+        return lat.values, lat.indices, rows
+
+    @staticmethod
+    def backward(ctx, g_vals, _g_idx, g_rows):
+        m = ctx.module
+        plan = m.plan
+        x, vals, idx = ctx.saved_tensors
+        B, D = x.shape
+        a, b = plan.row_range(B)
+        g_rows = (torch.zeros((b - a, D), dtype=torch.float32, device=x.device) if g_rows is None
+                  else g_rows.detach().contiguous().float())
+        g = m._gather_rows(g_rows, B).contiguous()                            # collective 1: g [B, D]
+        gv = torch.zeros_like(vals) if g_vals is None else g_vals.detach().contiguous().float()
+        if plan.world_size > 1:
+            parts = m._all_gather(gv)                                         # collective 2: [G, B, k]
+            gv = parts[0].clone()
+            for r in range(1, plan.world_size):                               # rank order: the same bits on every run
+                gv += parts[r]
+        gwe, gbe, gwd, gbd = m.ops.backward_local(x, vals, idx, g, gv, plan)
+        return None, gwe, gbe, gwd, gbd, None
+
+
 class DictionaryShardedBaselineSAE(_DictionaryShardedForward):
     """Rank-local shard of BaselineSparseAutoencoder(input_dim, hidden_dim) (sae/baseline.py): the top-k baseline at
     2^20 latents, split over G ranks by latents.
@@ -496,7 +567,19 @@ class DictionaryShardedBaselineSAE(_DictionaryShardedForward):
     forward(x) -> (SparseLatents over all H latents with global indices, recon rows): this rank's [B/G, D] rows after
     the reduce-scatter, or the gathered [B, D] with `gather_output`. There is no dense [B, H] latent (the single-GPU
     module's `return_dense`): at H = 2^20 and B = 4096 it would take 17 GB. `SparseLatents.to_dense()` builds it on
-    request. Inference and analysis only: there is no backward."""
+    request.
+
+    Training: with `autograd = True` (not part of the state_dict) and grad mode on, the forward is the same forward
+    behind one autograd node (_ShardedBaselineFn), and `lat.values` is differentiable. The objective is the SUM of the
+    ranks' losses: each rank takes its loss on its own rows (rows of x in plan.row_range(B)), e.g.
+    0.5 * ((rows - x[a:b]) ** 2).sum() / (B * D), plus any term on lat.values. After loss.backward() the .grad of
+    encoder.0.weight, encoder.0.bias and decoder.weight is bit-equal to the single-GPU module's gradient of that
+    objective sliced to this shard, and decoder.bias.grad is the full gradient, the same bits on every rank (replicated
+    biases stay identical under any optimizer). EVERY rank must call backward() on a loss that depends on its rows: the
+    backward's two all-gathers are unconditional and issued in a fixed order, and a rank that skips them hangs the
+    others. Refused in training: gather_output (every rank would take its loss over the whole batch, counted G times)
+    and an x that requires grad (its gradient would need an all-reduce). ShardPlan.merge_baseline_state_dicts joins
+    the ranks' state_dicts into the single-GPU checkpoint layout."""
 
     def __init__(self, input_dim, hidden_dim, *, rank=None, world_size=None, process_group=None, ops=None):
         super().__init__(hidden_dim, rank, world_size, process_group)
@@ -506,6 +589,8 @@ class DictionaryShardedBaselineSAE(_DictionaryShardedForward):
         self.encoder = nn.Sequential(nn.Linear(input_dim, hs))
         self.decoder = nn.Linear(hs, input_dim)
         self.topk = 32
+        # True: forward builds one autograd node (_ShardedBaselineFn) whenever grad mode is on
+        self.autograd = False
         # ops=False defers the choice (tests install their own backend after construction)
         self.ops = CudaBaselineShardOps(self) if ops is None else (ops or None)
 
@@ -513,7 +598,17 @@ class DictionaryShardedBaselineSAE(_DictionaryShardedForward):
         return int(self.topk)                         # a count over the FULL dictionary, as sae/baseline.py:35
 
     def forward(self, x: torch.Tensor):
-        return self._sharded_forward(x)
+        if not (self.autograd and torch.is_grad_enabled()):
+            return self._sharded_forward(x)
+        if self.gather_output:
+            raise RuntimeError("DictionaryShardedBaselineSAE: gather_output is not supported in training (every rank would "
+                               "hold the whole batch, and a loss over it would be counted once per rank)")
+        if x.requires_grad:
+            raise RuntimeError("DictionaryShardedBaselineSAE: x.requires_grad is not supported in training (x is "
+                               "replicated: its gradient would need an all-reduce across the ranks)")
+        lin, dec = self.encoder[0], self.decoder
+        vals, idx, rows = _ShardedBaselineFn.apply(x, lin.weight, lin.bias, dec.weight, dec.bias, self)
+        return SparseLatents(vals, idx, (x.shape[0], self.hidden_dim)), rows
 
     def normalize_decoder_weights(self):
         """Unit-norm decoder columns (sae/baseline.py:42-50). A column is one latent, so every norm is local to the

@@ -49,6 +49,8 @@ baseline_sae  `baseline_forward(model, x)` (what `BaselineSparseAutoencoder.forw
             from one latent-major pass over the entries grouped by latent (one writer per element, no atomics);
             grad b_dec = column sums of g (two fixed-order levels); grad x = gv W_enc (the sparse row decoder).
         Every gradient is bit-deterministic.
+        Dictionary-sharded (sharded.py, `_ShardedBaselineFn`): the same backward over each rank's latent range
+        (qsae_baseline_backward_range), after all-gathers of d loss / d rows and d loss / d values.
 No CPU fallback: CUDA tensors only.
 """
 from __future__ import annotations
